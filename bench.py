@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's own CPU implementation, host cores
+    python bench.py --dump-outputs DIR ...    # also the last timed step's disparity maps as DIR/*.npy, to compare two builds
 
 A step = one pass of the hot path over one batch of synthetic stereo pairs (both directions per
 pair, like the reference's disparitySSDPair, main.cpp:21-48).  Workload at every N: per GPU a batch
@@ -267,6 +268,40 @@ def oracle_band_check(L, Rt, R, nd, cost, got_l, got_r, r0, n):
     return rep
 
 
+DUMP_BYTES = 64_000_000      # --dump-outputs: all files of all ranks together
+
+
+def dump_maps(out_dir, maps, budget, suffix=""):
+    """--dump-outputs: every tensor of `maps` ({name: disparity maps [..., rows, cols]}, one image shape) as float32
+    `out_dir/<name><suffix>.npy`.  Maps larger than `budget` bytes together keep one fixed, seeded sample of pixel positions
+    (the same for every map, increasing); its flat indices (row * cols + col) go to `sample_index<suffix>.npy` as float64.
+    Returns a description for the JSON line."""
+    import torch
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    rows, cols = next(iter(maps.values())).shape[-2:]
+    pix = rows * cols
+    n_maps = sum(t.numel() // pix for t in maps.values())
+    idx = None
+    files = []
+    if n_maps * pix * 4 > budget:
+        k = (budget - 1024) // (n_maps * 4 + 8)          # 1024: the .npy headers; 8: the float64 index of a sampled pixel
+        idx = np.sort(np.random.default_rng(0).choice(pix, k, replace=False))
+        np.save(out_dir / f"sample_index{suffix}.npy", idx.astype(np.float64))
+        files.append(f"sample_index{suffix}.npy")
+    for name, t in maps.items():
+        if idx is None:
+            a = t.to(torch.float32).cpu().numpy()
+        else:
+            a = t.reshape(-1, pix)[:, torch.from_numpy(idx).to(t.device)].to(torch.float32).cpu().numpy().reshape(*t.shape[:-2], -1)
+        np.save(out_dir / f"{name}{suffix}.npy", a)
+        files.append(f"{name}{suffix}.npy")
+    rep = {"dir": str(out_dir), "files": files, "pixels_per_map": pix if idx is None else int(idx.size), "of_pixels": pix}
+    if idx is not None:
+        rep["sample_index"] = "flat pixel index row * cols + col, stored as float64 (exact below 2^53)"
+    return rep
+
+
 # ---------------------------------------------------------------------------------------------------
 # our arm
 # ---------------------------------------------------------------------------------------------------
@@ -421,6 +456,12 @@ def run_ours(args, wl):
     sampler.start()
     dev_ms, launches = timed_pairs(G, args.steps)
     clocks = sampler.stop()
+    dump = None
+    if args.dump_outputs:     # before any later step reuses d_out
+        last = nwarm + args.steps - 1
+        dump = dump_maps(args.dump_outputs, {"disparity_left": d_out[last & 1, 0], "disparity_right": d_out[last & 1, 1]},
+                         DUMP_BYTES // world, f"_rank{rank}" if world > 1 else "")
+        dump.update(step=last, input_set=last % S, input_roll_rows=17 * (last % S))
     hot_ms, hot_n = 0.0, 0
     # hot-kernel time of the last step (events recorded by the library on the same stream)
     ms, nmeas = ctx.last_hot_kernel_ms()
@@ -666,6 +707,8 @@ def run_ours(args, wl):
             "gpu_launches": launches, "e2e_gpu_launches": e2e_launches, "clocks": clocks,
             "parity_check": parity,
         }
+        if dump is not None:
+            line["dump_outputs"] = dump
         if gather_sub:
             line["gather_variants"] = gather_sub
         if bands_sub is not None:
@@ -839,7 +882,7 @@ def suite_ps2_lines(torch, lib, ctx, dev, stream, steps, peak_lane_ops):
                       f"{steps}; the reference's published figure is its kernel alone (GpuTimer, DisparitySSD.cu:192-203)"}
 
 
-def bands_line(args, wl, lib, ctx, cost, dev, rank, world, local, steps, gather_kind, use_graph=True):
+def bands_line(args, wl, lib, ctx, cost, dev, rank, world, local, steps, gather_kind, use_graph=True, dump_dir=None):
     """BASELINE config 4: ONE synthetic pair, output rows sharded over the ranks (R+1 halo rows from the rank's own slab, no
     neighbour exchange), both maps of the band from one launch sequence, the bands gathered inside the timed step: pushed by
     the copy engines into rank 0's buffer (root), into every rank's (all), or all_gather'ed (nccl).  Strong scaling: a step is
@@ -929,6 +972,11 @@ def bands_line(args, wl, lib, ctx, cost, dev, rank, world, local, steps, gather_
         evs.append((e0, e1))
     barrier()
     clocks = sampler.stop()
+    dump = None
+    if dump_dir:              # this rank's band of both maps, as the last timed step left it
+        dump = dump_maps(dump_dir, {"disparity_left": mine[0, :r1 - r0], "disparity_right": mine[1, :r1 - r0]},
+                         DUMP_BYTES // world, f"_rank{rank}" if world > 1 else "")
+        dump.update(rows=[r0, r1])
     t = torch.tensor([sum(a.elapsed_time(b) for a, b in evs)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -967,6 +1015,8 @@ def bands_line(args, wl, lib, ctx, cost, dev, rank, world, local, steps, gather_
                                                      "nvlink_rx_busiest_rank": (world - 1) * band_bytes if world > 1 else 0},
                            "launch": graph_note, "l2": "flushed between steps"},
                 "gpu_launches": launches_per_step * steps, "clocks": clocks, "parity_check": parity}
+        if dump is not None:
+            line["dump_outputs"] = dump
     if pg is not None:
         # cross-rank check: every slot the consumer holds equals what that rank computed
         dist.barrier()
@@ -985,7 +1035,8 @@ def bands_line(args, wl, lib, ctx, cost, dev, rank, world, local, steps, gather_
 
 def run_bands(args, wl, lib, ctx, cost, dev, rank, world, local):
     import torch.distributed as dist
-    line = bands_line(args, wl, lib, ctx, cost, dev, rank, world, local, args.steps, args.gather, use_graph=not args.no_graph)
+    line = bands_line(args, wl, lib, ctx, cost, dev, rank, world, local, args.steps, args.gather, use_graph=not args.no_graph,
+                      dump_dir=args.dump_outputs)
     if rank == 0:
         print(json.dumps(line), flush=True)
     ctx.close()
@@ -1014,7 +1065,14 @@ def main():
     ap.add_argument("--mode", default="pairs", choices=["pairs", "bands"],
                     help="pairs: batch sharded by pair, weak scaling (default, the driver's line); "
                          "bands: ONE image sharded by row band with halo, strong scaling (BASELINE config 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write both disparity maps of the last timed step as float32 DIR/<name>.npy "
+                         f"(at most {DUMP_BYTES // 10**6} MB in all: a fixed, seeded sample of pixels when the maps are larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the maps of --impl ours")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference_arm(args, wl)

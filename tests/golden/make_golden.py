@@ -112,5 +112,54 @@ def main() -> None:
     print("wrote", OUT / "ps2_golden.npz", (OUT / "ps2_golden.npz").stat().st_size, "bytes")
 
 
+def record_reference_cases(from_restatement: bool) -> None:
+    """tests/golden/ref_cases.npz: the reference's own compiled SSD / NCC loop (int8 maps, as it stores them) on the inputs
+    of tests/test_oracle.py's compiled-reference tests, and that it throws on the NCC case without candidates - so those
+    tests compare the restatement with the reference where oracle/_ref cannot be built.
+
+        python tests/golden/make_golden.py --ref-cases                      # needs oracle/_ref (the reference sources)
+        python tests/golden/make_golden.py --ref-cases --from-restatement
+
+    The committed file was written with --from-restatement: the C restatement's outputs, on exactly these inputs, were
+    the reference's outputs.  At commit fb8d8c2, with oracle/_ref built from the reference sources, every one of these
+    live comparisons passed.  oracle/, introtocomputervision_b200/synth.py and the test inputs are unchanged since.
+    Wherever oracle/_ref is built, the tests check each recorded map against the live reference."""
+    sys.path.insert(0, str(ROOT / "tests"))
+    import test_oracle as t  # noqa: E402
+    if not from_restatement:
+        oracle.build()
+        assert oracle.have_ref() and oracle.have_ref_ncc(), "oracle/_ref not built (reference sources absent)"
+        ssd_lit = ssd_fast = oracle.ref_ssd
+        ncc_lit = ncc_fast = oracle.ref_ncorr
+    else:
+        def i8(f):                 # the functions each test compares the reference with, stored like the reference stores
+            return lambda *a: oracle.narrow_i8(f(*a))
+        ssd_lit, ssd_fast, ncc_lit, ncc_fast = i8(oracle.ssd), i8(oracle.ssd_fast), i8(oracle.ncorr), i8(oracle.ncorr_fast)
+    blob = {}
+    for seed in range(6):
+        blob[f"ssd_random/{seed}"] = ssd_lit(*t.ssd_random_case(seed))
+    for seed in range(8):
+        blob[f"ncc_random/{seed}"] = ncc_lit(*t.ncc_random_case(seed))
+    for cases, base, fn, kind in ((t.SSD_PAIR_RANGES, 400, ssd_fast, "ssd"), (t.NCC_PAIR_RANGES, 500, ncc_fast, "ncc")):
+        for rows, cols, R, rng in cases:
+            L, Rt = t.pair_range_images(rows, cols, rng, base)
+            blob[f"{kind}_pair/{rows}x{cols}_R{R}_{rng}/LR"] = fn(L, Rt, R, -rng, 0)
+            blob[f"{kind}_pair/{rows}x{cols}_R{R}_{rng}/RL"] = fn(Rt, L, R, 0, rng)
+    shape, R, a, b = t.NCC_EMPTY_CASE
+    img = np.ones(shape, np.float32)
+    try:
+        ncc_lit(img, img, R, a, b)
+        throws = 0
+    except oracle.OracleError:
+        throws = 1
+    blob["ncc_empty/throws"] = np.array([throws], np.int8)
+    assert all(v.dtype == np.int8 for v in blob.values())
+    np.savez_compressed(OUT / "ref_cases.npz", **blob)
+    print("wrote", OUT / "ref_cases.npz", (OUT / "ref_cases.npz").stat().st_size, "bytes,", len(blob), "arrays")
+
+
 if __name__ == "__main__":
-    main()
+    if "--ref-cases" in sys.argv:
+        record_reference_cases("--from-restatement" in sys.argv)
+    else:
+        main()
