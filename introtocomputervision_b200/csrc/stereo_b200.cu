@@ -12,6 +12,8 @@
 #include <cstdarg>
 #include <thread>
 #include <new>
+#include <initializer_list>
+#include <utility>
 #include <vector>
 
 namespace sb {
@@ -85,6 +87,28 @@ static int validate(const Problem& p, size_t ref_min_step, size_t tgt_min_step) 
     return STEREO_OK;
 }
 
+// ---- problems -----------------------------------------------------------------------------------
+
+// One direction: output rows [row_begin, row_end) of a rows x cols image pair whose buffers - addressed from the image's
+// row 0 - hold rows [avail_begin, avail_end).
+static Problem direction(int cost, PixType type, const void* ref, size_t ref_step, const void* tgt, size_t tgt_step, int rows,
+                         int cols, int row_begin, int row_end, int avail_begin, int avail_end, int R, int dmin, int dmax,
+                         void* disp, size_t disp_step, int elem, void* best, size_t best_step) {
+    return Problem{cost, ImageView{ref, ref_step, type}, ImageView{tgt, tgt_step, type}, rows, cols, row_begin, row_end,
+                   avail_begin, avail_end, R, dmin, dmax, OutView{disp, disp_step, elem}, OutView{best, best_step, 4}};
+}
+
+// Pair k of np: L->R over [-range, 0] at ps[k], then R->L with the images swapped over [0, +range] at ps[np + k]
+// (main.cpp:21-48).  Left-referenced problems first is the order a fused launch takes pairs in (fused_layout).
+static void pair_problems(Problem* ps, int np, int k, int cost, PixType type, const void* left, size_t left_step,
+                          const void* right, size_t right_step, int rows, int cols, int row_begin, int row_end, int avail_begin,
+                          int avail_end, int R, int range, void* disp_left, void* disp_right, size_t disp_step, int elem) {
+    ps[k] = direction(cost, type, left, left_step, right, right_step, rows, cols, row_begin, row_end, avail_begin, avail_end, R,
+                      -range, 0, disp_left, disp_step, elem, nullptr, 0);
+    ps[np + k] = direction(cost, type, right, right_step, left, left_step, rows, cols, row_begin, row_end, avail_begin, avail_end,
+                           R, 0, range, disp_right, disp_step, elem, nullptr, 0);
+}
+
 // ---- exact path ---------------------------------------------------------------------------------
 
 static size_t exact_scratch_bytes(const Problem& p) {
@@ -135,8 +159,6 @@ static int run_exact(stereo_ctx* ctx, const Problem& p, cudaStream_t st) {
 
 // ---- path selection -------------------------------------------------------------------------------
 
-static bool fused_layout(const stereo_ctx* ctx, const Problem* ps, int n);
-
 // Float images: which kernel family applies (decided from the device-side classification, see classify_convert_kernel).
 enum { CLS_U8 = 0, CLS_F32_FAST = 1, CLS_EXACT = 2 };
 
@@ -185,95 +207,26 @@ static int classify_images(stereo_ctx* ctx, const Problem& p, cudaStream_t st, u
     return STEREO_OK;
 }
 
-// Enqueues one direction.
-static int run_problem(stereo_ctx* ctx, Problem p, cudaStream_t st, bool reset_arena = true) {
-    const bool is_f32 = p.ref.type == PixType::F32;
-    const size_t min_step = size_t(p.cols) * (is_f32 ? 4 : 1);
-    int rc = validate(p, min_step, min_step);
-    if (rc != STEREO_OK) return rc;
-    if (p.ref.type != p.tgt.type) { set_error("mixed pixel types (internal)"); return STEREO_ERR_INVALID_ARG; }
+// Grows the scratch arena to `need` bytes; nothing enqueued by earlier calls may still use it then.
+static int reserve_arena(stereo_ctx* ctx, cudaStream_t st, size_t need) {
+    if (need <= ctx->arena.cap) return STEREO_OK;
+    const int rc = quiesce(ctx, st);
+    return rc != STEREO_OK ? rc : ctx->arena.reserve(need);
+}
 
-    const bool fast_ok = fast_supported(p) && ctx->force_path != STEREO_PATH_EXACT_F32;
-    size_t need = exact_scratch_bytes(p);
-    if (fast_ok) need = is_f32 ? f32_scratch_bytes(ctx, p, 1) : (need > fast_scratch_bytes(ctx, p) ? need : fast_scratch_bytes(ctx, p));
-    if (need > ctx->arena.cap) {
-        rc = quiesce(ctx, st);
-        if (rc != STEREO_OK) return rc;
-        rc = ctx->arena.reserve(need);
-        if (rc != STEREO_OK) return rc;
-    }
-    if (reset_arena) ctx->arena.reset();
-
-    int cls = is_f32 ? CLS_EXACT : CLS_U8;
-    if (fast_ok && is_f32) {
-        const size_t pitch = align256(p.cols);
-        uint8_t* a8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
-        uint8_t* b8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
-        if (!a8 || !b8) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
-        rc = classify_images(ctx, p, st, a8, b8, pitch, &cls);
-        if (rc != STEREO_OK) return rc;
-        if (cls == CLS_U8) { p.ref = ImageView{a8, pitch, PixType::U8}; p.tgt = ImageView{b8, pitch, PixType::U8}; }
-    }
-    if (fast_ok && cls != CLS_EXACT) {
-        ctx->last_path = cls == CLS_U8 ? STEREO_PATH_FAST_U8 : STEREO_PATH_FAST_F32;
-        return run_fast(ctx, p, st);
-    }
+// Enqueues one direction on the exact kernels.
+static int run_exact_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st) {
     if (ctx->force_path == STEREO_PATH_FAST_U8 || ctx->force_path == STEREO_PATH_FAST_F32) {
         set_error("fast path forced but not applicable (pixel values or window/range outside what the running-sum kernels cover)");
         return STEREO_ERR_UNSUPPORTED;
     }
+    const int rc = reserve_arena(ctx, st, exact_scratch_bytes(p));
+    if (rc != STEREO_OK) return rc;
+    ctx->arena.reset();
     ctx->last_path = STEREO_PATH_EXACT_F32;
     return run_exact(ctx, p, st);
 }
 
-// Both directions of ONE pair of float images (ps[0] left-referenced, ps[1] right-referenced, the same two device images):
-// classified once, then both maps from one launch sequence - one cost volume where the pair is fusable.
-static int run_pair_f32(stereo_ctx* ctx, Problem* ps, cudaStream_t st) {
-    const Problem& p = ps[0];
-    const size_t min_step = size_t(p.cols) * 4;
-    int rc = STEREO_OK;
-    for (int d = 0; d < 2 && rc == STEREO_OK; ++d) rc = validate(ps[d], min_step, min_step);
-    if (rc != STEREO_OK) return rc;
-    const size_t need = f32_scratch_bytes(ctx, p, 2);
-    if (need > ctx->arena.cap) {
-        rc = quiesce(ctx, st);
-        if (rc != STEREO_OK) return rc;
-        rc = ctx->arena.reserve(need);
-        if (rc != STEREO_OK) return rc;
-    }
-    ctx->arena.reset();
-    const size_t pitch = align256(p.cols);
-    uint8_t* a8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
-    uint8_t* b8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
-    if (!a8 || !b8) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
-    int cls = CLS_EXACT;
-    rc = classify_images(ctx, p, st, a8, b8, pitch, &cls);
-    if (rc != STEREO_OK) return rc;
-    if (cls == CLS_EXACT) {
-        if (ctx->force_path == STEREO_PATH_FAST_U8 || ctx->force_path == STEREO_PATH_FAST_F32) {
-            set_error("fast path forced but not applicable (pixel values outside what the running-sum kernels cover)");
-            return STEREO_ERR_UNSUPPORTED;
-        }
-        ctx->last_path = STEREO_PATH_EXACT_F32;
-        for (int d = 0; d < 2; ++d) {
-            ctx->arena.reset();
-            rc = run_exact(ctx, ps[d], st);
-            if (rc != STEREO_OK) return rc;
-        }
-        return STEREO_OK;
-    }
-    if (cls == CLS_U8) {
-        // ps[0]: ref = left, tgt = right; ps[1] the other way round
-        ps[0].ref = ImageView{a8, pitch, PixType::U8}; ps[0].tgt = ImageView{b8, pitch, PixType::U8};
-        ps[1].ref = ImageView{b8, pitch, PixType::U8}; ps[1].tgt = ImageView{a8, pitch, PixType::U8};
-    }
-    ctx->last_path = cls == CLS_U8 ? STEREO_PATH_FAST_U8 : STEREO_PATH_FAST_F32;
-    return run_fast_batch(ctx, ps, 2, st, fused_layout(ctx, ps, 2) ? 1 : 0);
-}
-
-// Enqueues `n` u8 problems that all take the packed path, several directions per launch sequence where they
-// are batchable (same shape, band, window, cost and candidate count).  `batch_budget` bounds the scratch one
-// launch sequence may hold.
 // True when ps = n/2 left-referenced problems followed by their right-referenced partners, each pair fusable.
 static bool fused_layout(const stereo_ctx* ctx, const Problem* ps, int n) {
     if (!ctx->fuse_pairs || n < 2 || (n & 1) || n > FMAXJOBS) return false;
@@ -283,42 +236,80 @@ static bool fused_layout(const stereo_ctx* ctx, const Problem* ps, int n) {
     return true;
 }
 
+// The float images of ONE image pair - ps[0], and its mirror ps[1] when n == 2 - classified once, then every direction
+// from one launch sequence (one cost volume where the pair is fusable) on u8 copies or the float operands, or from the
+// exact kernels.
+static int run_f32_pair(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
+    const Problem& p = ps[0];
+    int rc = reserve_arena(ctx, st, f32_scratch_bytes(ctx, p, n));
+    if (rc != STEREO_OK) return rc;
+    ctx->arena.reset();
+    const size_t pitch = align256(p.cols);
+    uint8_t* a8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
+    uint8_t* b8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
+    if (!a8 || !b8) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
+    int cls = CLS_EXACT;
+    rc = classify_images(ctx, p, st, a8, b8, pitch, &cls);
+    if (rc != STEREO_OK) return rc;
+    if (cls == CLS_EXACT) {
+        for (int d = 0; d < n && rc == STEREO_OK; ++d) rc = run_exact_direction(ctx, ps[d], st);
+        return rc;
+    }
+    if (cls == CLS_U8) {
+        // ps[0]: ref = left, tgt = right; ps[1] the other way round
+        ps[0].ref = ImageView{a8, pitch, PixType::U8}; ps[0].tgt = ImageView{b8, pitch, PixType::U8};
+        if (n == 2) { ps[1].ref = ps[0].tgt; ps[1].tgt = ps[0].ref; }
+    }
+    ctx->last_path = cls == CLS_U8 ? STEREO_PATH_FAST_U8 : STEREO_PATH_FAST_F32;
+    return run_fast_batch(ctx, ps, n, st, fused_layout(ctx, ps, n) ? n / 2 : 0);
+}
+
 // One launch sequence over batchable problems, fused when they are whole pairs.
 static int run_fast_auto(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t st) {
     return run_fast_batch(ctx, ps, n, st, fused_layout(ctx, ps, n) ? n / 2 : 0);
 }
 
+// Enqueues `n` u8 problems that all take the packed path, several directions per launch sequence where they are
+// batchable (same shape, band, window, cost and candidate count), one fused launch sequence when they are whole pairs.
+// `budget` bounds the scratch one unfused launch sequence may hold.
 static int run_fast_jobs(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t st) {
     const size_t budget = size_t(3) << 30;
-    if (fused_layout(ctx, ps, n)) {          // (n <= FMAXJOBS: one launch sequence)
-        const size_t need = size_t(n) * fast_scratch_bytes(ctx, ps[0]);
-        if (need > ctx->arena.cap) {
-            int rc = quiesce(ctx, st);
-            if (rc != STEREO_OK) return rc;
-            rc = ctx->arena.reserve(need);
-            if (rc != STEREO_OK) return rc;
-        }
-        ctx->arena.reset();
-        ctx->last_path = STEREO_PATH_FAST_U8;
-        return run_fast_batch(ctx, ps, n, st, n / 2);
-    }
-    int i = 0;
-    while (i < n) {
+    const bool fused = fused_layout(ctx, ps, n);         // (n <= FMAXJOBS: one launch sequence)
+    for (int i = 0, m = 0; i < n; i += m) {
         const size_t per_job = fast_scratch_bytes(ctx, ps[i]);
-        int m = 1;
+        m = fused ? n : 1;
         while (i + m < n && m < FMAXJOBS && fast_batchable(ps[i], ps[i + m]) && size_t(m + 1) * per_job <= budget) ++m;
-        const size_t need = size_t(m) * per_job;
-        if (need > ctx->arena.cap) {
-            int rc = quiesce(ctx, st);
-            if (rc != STEREO_OK) return rc;
-            rc = ctx->arena.reserve(need);
-            if (rc != STEREO_OK) return rc;
-        }
+        int rc = reserve_arena(ctx, st, size_t(m) * per_job);
+        if (rc != STEREO_OK) return rc;
         ctx->arena.reset();
         ctx->last_path = STEREO_PATH_FAST_U8;
-        int rc = run_fast_batch(ctx, ps + i, m, st);
+        rc = run_fast_batch(ctx, ps + i, m, st, fused ? n / 2 : 0);
         if (rc != STEREO_OK) return rc;
-        i += m;
+    }
+    return STEREO_OK;
+}
+
+// Enqueues every direction of a call: one problem, or n/2 left-referenced problems followed by their right-referenced
+// partners (pair k = ps[k], ps[n/2 + k]).  The one place that picks the kernel family.
+static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
+    bool fast = ctx->force_path != STEREO_PATH_EXACT_F32, u8 = true;
+    for (int i = 0; i < n; ++i) {
+        const Problem& p = ps[i];
+        const size_t row = size_t(p.cols) * (p.ref.type == PixType::F32 ? 4 : 1);
+        const int rc = validate(p, row, row);
+        if (rc != STEREO_OK) return rc;
+        if (p.ref.type != p.tgt.type) { set_error("mixed pixel types (internal)"); return STEREO_ERR_INVALID_ARG; }
+        fast = fast && fast_supported(p);
+        u8 = u8 && p.ref.type == PixType::U8;
+    }
+    if (fast && u8) return run_fast_jobs(ctx, ps, n, st);
+    if (fast && n <= 2) return run_f32_pair(ctx, ps, n, st);      // (float images come one pair per call)
+    const int np = n / 2;
+    if (np == 0) return run_exact_direction(ctx, ps[0], st);
+    for (int k = 0; k < np; ++k) {
+        int rc = run_exact_direction(ctx, ps[k], st);
+        if (rc == STEREO_OK) rc = run_exact_direction(ctx, ps[np + k], st);
+        if (rc != STEREO_OK) return rc;
     }
     return STEREO_OK;
 }
@@ -533,11 +524,8 @@ static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, in
     const bool any_f32 = type == PixType::F32 && !pack, any_pack = pack;
     const size_t f_pitch = align256(size_t(cols) * 4), u8_pitch = align256(cols), d_pitch = align256(size_t(cols) * elem);
     // validate each direction on a full-image problem (pointers only need to be non-null here)
-    Problem full{};
-    full.cost = cost; full.rows = rows; full.cols = cols; full.row_begin = 0; full.row_end = rows;
-    full.avail_begin = 0; full.avail_end = rows; full.R = R;
-    full.ref = ImageView{in, u8_pitch, PixType::U8}; full.tgt = full.ref;
-    full.disp = OutView{ctx, d_pitch, elem}; full.best = OutView{nullptr, 0, 4};
+    Problem full = direction(cost, PixType::U8, in, u8_pitch, in, u8_pitch, rows, cols, 0, rows, 0, rows, R, 0, 0, ctx, d_pitch,
+                             elem, nullptr, 0);
     const int nb_uniform = pipe_bands(ctx, n_pairs, rows);
     const int cp = pipe_chunk_pairs(n_pairs, nb_uniform, rows, cols);
     const int n_items = (n_pairs + cp - 1) / cp;
@@ -796,20 +784,92 @@ static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, in
     return STEREO_OK;
 }
 
-// Host-buffer single direction: upload (2D async copies), compute, download, synchronize — the
-// shape of cuda::disparitySSD (DisparitySSD.cu:171-206) without per-call allocation.
+// What every host entry point checks before it touches a buffer: the context, non-null pointers, an image of at most
+// 32768 pixels a side (validate() reports larger ones to device callers as UNSUPPORTED), a disparity element of 1, 2 or
+// 4 bytes and every {step, row bytes} step at least its row.  A pair's negative `range` is rejected with `range_rc`.
+static int check_host_args(stereo_ctx* ctx, std::initializer_list<const void*> ptrs, int rows, int cols, int elem,
+                           std::initializer_list<std::pair<size_t, size_t>> steps, int range = 0,
+                           int range_rc = STEREO_ERR_INVALID_RANGE) {
+    const int rc = check_ctx(ctx);
+    if (rc != STEREO_OK) return rc;
+    for (const void* p : ptrs)
+        if (!p) { set_error("null pointer"); return STEREO_ERR_INVALID_ARG; }
+    if (rows <= 0 || cols <= 0 || rows > 32768 || cols > 32768) { set_error("bad image size %d x %d", rows, cols); return STEREO_ERR_INVALID_ARG; }
+    if (elem != 1 && elem != 2 && elem != 4) { set_error("disp_elem_bytes must be 1, 2 or 4"); return STEREO_ERR_INVALID_ARG; }
+    for (const auto& s : steps)
+        if (s.first < s.second) { set_error("a step is smaller than its row"); return STEREO_ERR_INVALID_ARG; }
+    if (range < 0) { set_error("disparity_range must be >= 0"); return range_rc; }
+    return STEREO_OK;
+}
+
+// Sequential host call: upload (2D async copies), compute, download, synchronize - the shape of cuda::disparitySSD
+// (DisparitySSD.cu:171-206) without per-call allocation.
+struct HostRows { const void* ptr; size_t step, row_bytes; };     // host input rows
+struct HostMap { void* ptr; size_t step, row_bytes; };            // host output rows; ptr == nullptr: not wanted
+struct DevRows { char* ptr; size_t pitch; };
+
+// Uploads in_rows rows of both inputs, runs compute(device inputs, device outputs) on ctx->stream and downloads out_rows
+// rows of every wanted output.  `compute` brackets its kernels with begin_call / end_call, so the copies stay out of
+// last_kernel_ms.  The stream is synchronized on every return, errors included: nothing may still touch the caller's buffers.
+template <class Compute>
+static int staged_host_call(stereo_ctx* ctx, const HostRows (&in)[2], int in_rows, const HostMap (&out)[2], int out_rows,
+                            Compute compute) {
+    cudaStream_t st = ctx->stream;
+    DevRows din[2], dout[2] = {};
+    size_t need = 1024;
+    for (const HostRows& h : in) need += align256(h.row_bytes) * in_rows;
+    for (const HostMap& h : out) need += h.ptr ? align256(h.row_bytes) * out_rows : 0;
+    if (need > ctx->io.cap) {
+        SB_CUDA(cudaStreamSynchronize(st));
+        const int rc = ctx->io.reserve(need);
+        if (rc != STEREO_OK) return rc;
+    }
+    ctx->io.reset();
+    bool ok = true;
+    for (int i = 0; i < 2; ++i) {
+        din[i].pitch = align256(in[i].row_bytes);
+        din[i].ptr = static_cast<char*>(ctx->io.take(din[i].pitch * in_rows));
+        ok = ok && din[i].ptr;
+        if (!out[i].ptr) continue;
+        dout[i].pitch = align256(out[i].row_bytes);
+        dout[i].ptr = static_cast<char*>(ctx->io.take(dout[i].pitch * out_rows));
+        ok = ok && dout[i].ptr;
+    }
+    if (!ok) { set_error("io arena too small (internal)"); return STEREO_ERR_ALLOC; }
+    cudaError_t e = cudaSuccess;
+    for (int i = 0; i < 2 && e == cudaSuccess; ++i)
+        e = cudaMemcpy2DAsync(din[i].ptr, din[i].pitch, in[i].ptr, in[i].step, in[i].row_bytes, in_rows, cudaMemcpyHostToDevice, st);
+    int rc = e == cudaSuccess ? compute(din, dout) : STEREO_ERR_CUDA;
+    for (int i = 0; i < 2 && rc == STEREO_OK && e == cudaSuccess; ++i)
+        if (out[i].ptr)
+            e = cudaMemcpy2DAsync(out[i].ptr, out[i].step, dout[i].ptr, dout[i].pitch, out[i].row_bytes, out_rows, cudaMemcpyDeviceToHost, st);
+    if (e != cudaSuccess) { set_error("host copy failed: %s", cudaGetErrorString(e)); rc = STEREO_ERR_CUDA; }
+    e = cudaStreamSynchronize(st);
+    if (rc == STEREO_OK && e != cudaSuccess) { set_error("host call failed: %s", cudaGetErrorString(e)); rc = STEREO_ERR_CUDA; }
+    return rc;
+}
+
+// One call of a device entry point: every direction on `stream` (nullptr: the context's stream).
+static int device_call(stereo_ctx* ctx, Problem* ps, int n, void* stream) {
+    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    begin_call(ctx, st);
+    const int rc = run_directions(ctx, ps, n, st);
+    end_call(ctx, st);
+    return rc;
+}
+
+static int device_single(stereo_ctx* ctx, Problem p, void* stream) {
+    const int rc = check_ctx(ctx);
+    return rc != STEREO_OK ? rc : device_call(ctx, &p, 1, stream);
+}
+
 static int host_single(stereo_ctx* ctx, int cost, PixType type, const void* ref, size_t ref_step, const void* tgt,
                        size_t tgt_step, int rows, int cols, int R, int dmin, int dmax, void* disp_out,
                        size_t disp_step, int elem, void* best_out, size_t best_step) {
-    int rc = check_ctx(ctx);
+    const size_t row = size_t(cols) * (type == PixType::F32 ? 4 : 1), disp_row = size_t(cols) * elem, best_row = size_t(cols) * 4;
+    int rc = check_host_args(ctx, {ref, tgt, disp_out}, rows, cols, elem,
+                             {{ref_step, row}, {tgt_step, row}, {disp_step, disp_row}, {best_step, best_out ? best_row : 0}});
     if (rc != STEREO_OK) return rc;
-    if (!ref || !tgt || !disp_out) { set_error("null pointer"); return STEREO_ERR_INVALID_ARG; }
-    if (rows <= 0 || cols <= 0 || rows > 32768 || cols > 32768) { set_error("bad image size %d x %d", rows, cols); return STEREO_ERR_INVALID_ARG; }
-    if (elem != 1 && elem != 2 && elem != 4) { set_error("disp_elem_bytes must be 1, 2 or 4"); return STEREO_ERR_INVALID_ARG; }
-    const size_t px = type == PixType::F32 ? 4 : 1;
-    if (ref_step < cols * px || tgt_step < cols * px || disp_step < size_t(cols) * elem || (best_out && best_step < size_t(cols) * 4)) {
-        set_error("a step is smaller than its row"); return STEREO_ERR_INVALID_ARG;
-    }
     if (!best_out) {      // pipelined band-by-band; falls through to the sequential path when the packed kernels do not apply
         const HostPairIn in{ref, ref_step, tgt, tgt_step};
         void* outs[1] = {disp_out};
@@ -817,59 +877,13 @@ static int host_single(stereo_ctx* ctx, int cost, PixType type, const void* ref,
         rc = pairs_host_pipelined(ctx, cost, type, 1, &in, &dir, 1, rows, cols, R, disp_step, elem);
         if (rc <= STEREO_OK) return rc;
     }
-    cudaStream_t st = ctx->stream;
-    const size_t in_pitch = align256(cols * px), d_pitch = align256(size_t(cols) * elem), b_pitch = align256(size_t(cols) * 4);
-    const size_t need = 2 * in_pitch * rows + d_pitch * rows + (best_out ? b_pitch * rows : 0) + 1024;
-    if (need > ctx->io.cap) {
-        SB_CUDA(cudaStreamSynchronize(st));
-        rc = ctx->io.reserve(need);
-        if (rc != STEREO_OK) return rc;
-    }
-    ctx->io.reset();
-    char* d_ref = static_cast<char*>(ctx->io.take(in_pitch * rows));
-    char* d_tgt = static_cast<char*>(ctx->io.take(in_pitch * rows));
-    char* d_disp = static_cast<char*>(ctx->io.take(d_pitch * rows));
-    char* d_best = best_out ? static_cast<char*>(ctx->io.take(b_pitch * rows)) : nullptr;
-    SB_CUDA(cudaMemcpy2DAsync(d_ref, in_pitch, ref, ref_step, cols * px, rows, cudaMemcpyHostToDevice, st));
-    SB_CUDA(cudaMemcpy2DAsync(d_tgt, in_pitch, tgt, tgt_step, cols * px, rows, cudaMemcpyHostToDevice, st));
-    Problem p{};
-    p.cost = cost;
-    p.ref = ImageView{d_ref, in_pitch, type};
-    p.tgt = ImageView{d_tgt, in_pitch, type};
-    p.rows = rows; p.cols = cols; p.row_begin = 0; p.row_end = rows; p.avail_begin = 0; p.avail_end = rows;
-    p.R = R; p.dmin = dmin; p.dmax = dmax;
-    p.disp = OutView{d_disp, d_pitch, elem};
-    p.best = OutView{d_best, b_pitch, 4};
-    begin_call(ctx, st);
-    rc = run_problem(ctx, p, st);
-    end_call(ctx, st);
-    if (rc != STEREO_OK) return rc;
-    SB_CUDA(cudaMemcpy2DAsync(disp_out, disp_step, d_disp, d_pitch, size_t(cols) * elem, rows, cudaMemcpyDeviceToHost, st));
-    if (best_out) SB_CUDA(cudaMemcpy2DAsync(best_out, best_step, d_best, b_pitch, size_t(cols) * 4, rows, cudaMemcpyDeviceToHost, st));
-    SB_CUDA(cudaStreamSynchronize(st));
-    return STEREO_OK;
-}
-
-static int device_single(stereo_ctx* ctx, int cost, PixType type, const void* ref, size_t ref_step, const void* tgt,
-                         size_t tgt_step, int rows, int cols, int row_begin, int row_end, int R, int dmin, int dmax,
-                         void* disp_out, size_t disp_step, int elem, void* best_out, size_t best_step, void* stream,
-                         int avail_begin = 0, int avail_end = -1) {
-    int rc = check_ctx(ctx);
-    if (rc != STEREO_OK) return rc;
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    Problem p{};
-    p.cost = cost;
-    p.ref = ImageView{ref, ref_step, type};
-    p.tgt = ImageView{tgt, tgt_step, type};
-    p.rows = rows; p.cols = cols; p.row_begin = row_begin; p.row_end = row_end;
-    p.avail_begin = avail_begin; p.avail_end = avail_end < 0 ? rows : avail_end;
-    p.R = R; p.dmin = dmin; p.dmax = dmax;
-    p.disp = OutView{disp_out, disp_step, elem};
-    p.best = OutView{best_out, best_step, 4};
-    begin_call(ctx, st);
-    rc = run_problem(ctx, p, st);
-    end_call(ctx, st);
-    return rc;
+    const HostRows in[2] = {{ref, ref_step, row}, {tgt, tgt_step, row}};
+    const HostMap out[2] = {{disp_out, disp_step, disp_row}, {best_out, best_step, best_row}};
+    return staged_host_call(ctx, in, rows, out, rows, [&](const DevRows* d, const DevRows* o) {
+        Problem p = direction(cost, type, d[0].ptr, d[0].pitch, d[1].ptr, d[1].pitch, rows, cols, 0, rows, 0, rows, R, dmin, dmax,
+                              o[0].ptr, o[0].pitch, elem, o[1].ptr, o[1].pitch);
+        return device_call(ctx, &p, 1, ctx->stream);
+    });
 }
 
 } // namespace sb
@@ -1079,18 +1093,9 @@ int stereo_launch_plan(int cost, int float_operands, int n_pairs, int rows, int 
     tmp.sm_count = sm_count;
     Problem ps[FMAXJOBS];
     static const char dummy_l = 0, dummy_r = 0;
-    for (int k = 0; k < n_pairs; ++k) {
-        Problem two[2];
-        const PixType t = float_operands ? PixType::F32 : PixType::U8;
-        two[0] = Problem{};
-        two[0].cost = cost; two[0].rows = rows; two[0].cols = cols; two[0].row_begin = 0; two[0].row_end = rows;
-        two[0].avail_begin = 0; two[0].avail_end = rows; two[0].R = window_rad;
-        two[1] = two[0];
-        two[0].ref = ImageView{&dummy_l + k, size_t(cols), t}; two[0].tgt = ImageView{&dummy_r + k, size_t(cols), t};
-        two[0].dmin = -disparity_range; two[0].dmax = 0;
-        two[1].ref = two[0].tgt; two[1].tgt = two[0].ref; two[1].dmin = 0; two[1].dmax = disparity_range;
-        ps[k] = two[0]; ps[n_pairs + k] = two[1];
-    }
+    for (int k = 0; k < n_pairs; ++k)
+        pair_problems(ps, n_pairs, k, cost, float_operands ? PixType::F32 : PixType::U8, &dummy_l + k, size_t(cols), &dummy_r + k,
+                      size_t(cols), rows, cols, 0, rows, 0, rows, window_rad, disparity_range, nullptr, nullptr, 0, 1);
     if (!fast_supported(ps[0])) { set_error("outside what the running-sum kernels cover"); return STEREO_ERR_UNSUPPORTED; }
     tmp.fuse_pairs = fuse ? 1 : 0;
     const bool fused = fused_layout(&tmp, ps, 2 * n_pairs);
@@ -1362,60 +1367,41 @@ int stereo_disparity_refgpu_f32_device(stereo_ctx* ctx, int cost, const float* r
 int stereo_disparity_refgpu_f32_host(stereo_ctx* ctx, int cost, const float* ref, size_t ref_step, const float* tgt, size_t tgt_step,
                                      int rows, int cols, int window_rad, int min_disp, int max_disp, int8_t* disp_out,
                                      size_t disp_step, float* best_out, size_t best_step) {
-    int rc = check_ctx(ctx);
+    const size_t row = size_t(cols) * 4;
+    const int rc = check_host_args(ctx, {ref, tgt, disp_out}, rows, cols, 1, {{ref_step, row}, {tgt_step, row}});
     if (rc != STEREO_OK) return rc;
-    if (!ref || !tgt || !disp_out || rows <= 0 || cols <= 0 || rows > 32768 || cols > 32768) { set_error("bad arguments"); return STEREO_ERR_INVALID_ARG; }
-    if (ref_step < size_t(cols) * 4 || tgt_step < size_t(cols) * 4) { set_error("a step is smaller than its row"); return STEREO_ERR_INVALID_ARG; }
-    cudaStream_t st = ctx->stream;
-    const size_t in_pitch = align256(size_t(cols) * 4), d_pitch = align256(cols);
-    const size_t need = 3 * in_pitch * rows + d_pitch * rows + 1024;
-    if (need > ctx->io.cap) {
-        SB_CUDA(cudaStreamSynchronize(st));
-        rc = ctx->io.reserve(need);
-        if (rc != STEREO_OK) return rc;
-    }
-    ctx->io.reset();
-    char* d_ref = static_cast<char*>(ctx->io.take(in_pitch * rows));
-    char* d_tgt = static_cast<char*>(ctx->io.take(in_pitch * rows));
-    char* d_best = static_cast<char*>(ctx->io.take(in_pitch * rows));
-    char* d_disp = static_cast<char*>(ctx->io.take(d_pitch * rows));
-    SB_CUDA(cudaMemcpy2DAsync(d_ref, in_pitch, ref, ref_step, size_t(cols) * 4, rows, cudaMemcpyHostToDevice, st));
-    SB_CUDA(cudaMemcpy2DAsync(d_tgt, in_pitch, tgt, tgt_step, size_t(cols) * 4, rows, cudaMemcpyHostToDevice, st));
-    rc = stereo_disparity_refgpu_f32_device(ctx, cost, reinterpret_cast<const float*>(d_ref), in_pitch, reinterpret_cast<const float*>(d_tgt), in_pitch,
-                                            rows, cols, window_rad, min_disp, max_disp, reinterpret_cast<int8_t*>(d_disp), d_pitch,
-                                            best_out ? reinterpret_cast<float*>(d_best) : nullptr, in_pitch, st);
-    if (rc == STEREO_OK) {
-        cudaError_t e = cudaMemcpy2DAsync(disp_out, disp_step, d_disp, d_pitch, cols, rows, cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess && best_out) e = cudaMemcpy2DAsync(best_out, best_step, d_best, in_pitch, size_t(cols) * 4, rows, cudaMemcpyDeviceToHost, st);
-        if (e != cudaSuccess) { set_error("download failed: %s", cudaGetErrorString(e)); rc = STEREO_ERR_CUDA; }
-    }
-    cudaError_t e = cudaStreamSynchronize(st);
-    if (rc == STEREO_OK && e != cudaSuccess) { set_error("compat call failed: %s", cudaGetErrorString(e)); rc = STEREO_ERR_CUDA; }
-    return rc;
+    const HostRows in[2] = {{ref, ref_step, row}, {tgt, tgt_step, row}};
+    const HostMap out[2] = {{disp_out, disp_step, size_t(cols)}, {best_out, best_step, row}};
+    return staged_host_call(ctx, in, rows, out, rows, [&](const DevRows* d, const DevRows* o) {
+        return stereo_disparity_refgpu_f32_device(ctx, cost, reinterpret_cast<const float*>(d[0].ptr), d[0].pitch,
+                                                  reinterpret_cast<const float*>(d[1].ptr), d[1].pitch, rows, cols, window_rad, min_disp,
+                                                  max_disp, reinterpret_cast<int8_t*>(o[0].ptr), o[0].pitch,
+                                                  reinterpret_cast<float*>(o[1].ptr), o[1].pitch, ctx->stream);
+    });
 }
 
 int stereo_disparity_f32_device(stereo_ctx* ctx, int cost, const float* ref, size_t ref_step, const float* tgt,
                                 size_t tgt_step, int rows, int cols, int window_rad, int min_disp, int max_disp,
                                 void* disp_out, size_t disp_step, int disp_elem_bytes, void* best_out,
                                 size_t best_step, void* cuda_stream) {
-    return device_single(ctx, cost, PixType::F32, ref, ref_step, tgt, tgt_step, rows, cols, 0, rows, window_rad,
-                         min_disp, max_disp, disp_out, disp_step, disp_elem_bytes, best_out, best_step, cuda_stream);
+    return device_single(ctx, direction(cost, PixType::F32, ref, ref_step, tgt, tgt_step, rows, cols, 0, rows, 0, rows, window_rad,
+                                        min_disp, max_disp, disp_out, disp_step, disp_elem_bytes, best_out, best_step), cuda_stream);
 }
 
 int stereo_disparity_u8_device(stereo_ctx* ctx, int cost, const uint8_t* ref, size_t ref_step, const uint8_t* tgt,
                                size_t tgt_step, int rows, int cols, int window_rad, int min_disp, int max_disp,
                                void* disp_out, size_t disp_step, int disp_elem_bytes, void* best_out,
                                size_t best_step, void* cuda_stream) {
-    return device_single(ctx, cost, PixType::U8, ref, ref_step, tgt, tgt_step, rows, cols, 0, rows, window_rad,
-                         min_disp, max_disp, disp_out, disp_step, disp_elem_bytes, best_out, best_step, cuda_stream);
+    return device_single(ctx, direction(cost, PixType::U8, ref, ref_step, tgt, tgt_step, rows, cols, 0, rows, 0, rows, window_rad,
+                                        min_disp, max_disp, disp_out, disp_step, disp_elem_bytes, best_out, best_step), cuda_stream);
 }
 
 int stereo_disparity_band_u8_device(stereo_ctx* ctx, int cost, const uint8_t* ref, size_t ref_step,
                                     const uint8_t* tgt, size_t tgt_step, int rows, int cols, int row_begin,
                                     int row_end, int window_rad, int min_disp, int max_disp, void* disp_out,
                                     size_t disp_step, int disp_elem_bytes, void* cuda_stream) {
-    return device_single(ctx, cost, PixType::U8, ref, ref_step, tgt, tgt_step, rows, cols, row_begin, row_end,
-                         window_rad, min_disp, max_disp, disp_out, disp_step, disp_elem_bytes, nullptr, 0, cuda_stream);
+    return device_single(ctx, direction(cost, PixType::U8, ref, ref_step, tgt, tgt_step, rows, cols, row_begin, row_end, 0, rows,
+                                        window_rad, min_disp, max_disp, disp_out, disp_step, disp_elem_bytes, nullptr, 0), cuda_stream);
 }
 
 int stereo_disparity_band_halo_u8_device(stereo_ctx* ctx, int cost, const uint8_t* ref_halo, size_t ref_step,
@@ -1429,9 +1415,9 @@ int stereo_disparity_band_halo_u8_device(stereo_ctx* ctx, int cost, const uint8_
     // into the available range, which changes nothing when the halo covers what the band needs.
     const uint8_t* ref0 = ref_halo - size_t(halo_begin) * ref_step;
     const uint8_t* tgt0 = tgt_halo - size_t(halo_begin) * tgt_step;
-    return device_single(ctx, cost, PixType::U8, ref0, ref_step, tgt0, tgt_step, rows, cols, row_begin, row_end,
-                         window_rad, min_disp, max_disp, disp_out, disp_step, disp_elem_bytes, nullptr, 0, cuda_stream,
-                         halo_begin, halo_end);
+    return device_single(ctx, direction(cost, PixType::U8, ref0, ref_step, tgt0, tgt_step, rows, cols, row_begin, row_end, halo_begin,
+                                        halo_end, window_rad, min_disp, max_disp, disp_out, disp_step, disp_elem_bytes, nullptr, 0),
+                         cuda_stream);
 }
 
 int stereo_band_halo_rows(int rows, int row_begin, int row_end, int window_rad, int* halo_begin, int* halo_end) {
@@ -1448,59 +1434,24 @@ int stereo_band_halo_rows(int rows, int row_begin, int row_end, int window_rad, 
 
 // ---- pairs: L->R over [-range, 0], then R->L with images swapped over [0, +range] (main.cpp:21-48) ----
 
-static void pair_problems(Problem* p, int cost, PixType type, const void* left, size_t left_step, const void* right,
-                          size_t right_step, int rows, int cols, int R, int range, void* disp_left, void* disp_right,
-                          size_t disp_step, int elem) {
-    p[0] = Problem{};
-    p[0].cost = cost;
-    p[0].rows = rows; p[0].cols = cols; p[0].row_begin = 0; p[0].row_end = rows; p[0].avail_begin = 0; p[0].avail_end = rows; p[0].R = R;
-    p[0].best = OutView{nullptr, 0, 4};
-    p[1] = p[0];
-    p[0].ref = ImageView{left, left_step, type}; p[0].tgt = ImageView{right, right_step, type};
-    p[0].dmin = -range; p[0].dmax = 0; p[0].disp = OutView{disp_left, disp_step, elem};
-    p[1].ref = ImageView{right, right_step, type}; p[1].tgt = ImageView{left, left_step, type};
-    p[1].dmin = 0; p[1].dmax = range; p[1].disp = OutView{disp_right, disp_step, elem};
-}
-
-// true when every problem can go straight to the packed kernels (u8 images, supported window / range)
-static bool all_fast(const stereo_ctx* ctx, const Problem* ps, int n) {
-    if (ctx->force_path == STEREO_PATH_EXACT_F32) return false;
-    for (int i = 0; i < n; ++i)
-        if (ps[i].ref.type != PixType::U8 || ps[i].tgt.type != PixType::U8 || !fast_supported(ps[i])) return false;
-    return true;
-}
-
+// Both maps of a pair of device images, or of a row band of them (avail_begin / avail_end as in direction()).
 static int pair_device(stereo_ctx* ctx, int cost, PixType type, const void* left, size_t left_step, const void* right,
-                       size_t right_step, int rows, int cols, int R, int range, void* disp_left, void* disp_right,
-                       size_t disp_step, int elem, cudaStream_t st) {
+                       size_t right_step, int rows, int cols, int row_begin, int row_end, int avail_begin, int avail_end, int R,
+                       int range, void* disp_left, void* disp_right, size_t disp_step, int elem, void* stream) {
     if (range < 0) { set_error("disparity_range must be >= 0"); return STEREO_ERR_INVALID_RANGE; }
     Problem p[2];
-    pair_problems(p, cost, type, left, left_step, right, right_step, rows, cols, R, range, disp_left, disp_right, disp_step, elem);
-    if (all_fast(ctx, p, 2)) {       // both directions in one launch sequence
-        for (int d = 0; d < 2; ++d) {
-            int rc = validate(p[d], size_t(cols), size_t(cols));
-            if (rc != STEREO_OK) return rc;
-        }
-        return run_fast_jobs(ctx, p, 2, st);
-    }
-    if (type == PixType::F32 && fast_supported(p[0]) && fast_supported(p[1]) && ctx->force_path != STEREO_PATH_EXACT_F32)
-        return run_pair_f32(ctx, p, st);
-    int rc = run_problem(ctx, p[0], st);
-    if (rc != STEREO_OK) return rc;
-    return run_problem(ctx, p[1], st);
+    pair_problems(p, 1, 0, cost, type, left, left_step, right, right_step, rows, cols, row_begin, row_end, avail_begin, avail_end, R,
+                  range, disp_left, disp_right, disp_step, elem);
+    return device_call(ctx, p, 2, stream);
 }
 
 static int pair_host(stereo_ctx* ctx, int cost, PixType type, const void* left, size_t left_step, const void* right,
                      size_t right_step, int rows, int cols, int R, int range, void* disp_left, void* disp_right,
                      size_t disp_step, int elem) {
-    int rc = check_ctx(ctx);
+    const size_t row = size_t(cols) * (type == PixType::F32 ? 4 : 1), disp_row = size_t(cols) * elem;
+    int rc = check_host_args(ctx, {left, right, disp_left, disp_right}, rows, cols, elem,
+                             {{left_step, row}, {right_step, row}, {disp_step, disp_row}}, range);
     if (rc != STEREO_OK) return rc;
-    if (!left || !right || !disp_left || !disp_right) { set_error("null pointer"); return STEREO_ERR_INVALID_ARG; }
-    if (rows <= 0 || cols <= 0 || rows > 32768 || cols > 32768) { set_error("bad image size %d x %d", rows, cols); return STEREO_ERR_INVALID_ARG; }
-    if (elem != 1 && elem != 2 && elem != 4) { set_error("disp_elem_bytes must be 1, 2 or 4"); return STEREO_ERR_INVALID_ARG; }
-    const size_t px = type == PixType::F32 ? 4 : 1;
-    if (left_step < cols * px || right_step < cols * px || disp_step < size_t(cols) * elem) { set_error("a step is smaller than its row"); return STEREO_ERR_INVALID_ARG; }
-    if (range < 0) { set_error("disparity_range must be >= 0"); return STEREO_ERR_INVALID_RANGE; }
     {
         const HostPairIn in{left, left_step, right, right_step};
         void* outs_l[1] = {disp_left};
@@ -1509,29 +1460,12 @@ static int pair_host(stereo_ctx* ctx, int cost, PixType type, const void* left, 
         rc = pairs_host_pipelined(ctx, cost, type, 1, &in, dirs, 2, rows, cols, R, disp_step, elem);
         if (rc <= STEREO_OK) return rc;
     }
-    cudaStream_t st = ctx->stream;
-    const size_t in_pitch = align256(cols * px), d_pitch = align256(size_t(cols) * elem);
-    const size_t need = 2 * in_pitch * rows + 2 * d_pitch * rows + 1024;
-    if (need > ctx->io.cap) {
-        SB_CUDA(cudaStreamSynchronize(st));
-        rc = ctx->io.reserve(need);
-        if (rc != STEREO_OK) return rc;
-    }
-    ctx->io.reset();
-    char* d_l = static_cast<char*>(ctx->io.take(in_pitch * rows));
-    char* d_r = static_cast<char*>(ctx->io.take(in_pitch * rows));
-    char* d_dl = static_cast<char*>(ctx->io.take(d_pitch * rows));
-    char* d_dr = static_cast<char*>(ctx->io.take(d_pitch * rows));
-    SB_CUDA(cudaMemcpy2DAsync(d_l, in_pitch, left, left_step, cols * px, rows, cudaMemcpyHostToDevice, st));
-    SB_CUDA(cudaMemcpy2DAsync(d_r, in_pitch, right, right_step, cols * px, rows, cudaMemcpyHostToDevice, st));
-    begin_call(ctx, st);
-    rc = pair_device(ctx, cost, type, d_l, in_pitch, d_r, in_pitch, rows, cols, R, range, d_dl, d_dr, d_pitch, elem, st);
-    end_call(ctx, st);
-    if (rc != STEREO_OK) return rc;
-    SB_CUDA(cudaMemcpy2DAsync(disp_left, disp_step, d_dl, d_pitch, size_t(cols) * elem, rows, cudaMemcpyDeviceToHost, st));
-    SB_CUDA(cudaMemcpy2DAsync(disp_right, disp_step, d_dr, d_pitch, size_t(cols) * elem, rows, cudaMemcpyDeviceToHost, st));
-    SB_CUDA(cudaStreamSynchronize(st));
-    return STEREO_OK;
+    const HostRows in[2] = {{left, left_step, row}, {right, right_step, row}};
+    const HostMap out[2] = {{disp_left, disp_step, disp_row}, {disp_right, disp_step, disp_row}};
+    return staged_host_call(ctx, in, rows, out, rows, [&](const DevRows* d, const DevRows* o) {
+        return pair_device(ctx, cost, type, d[0].ptr, d[0].pitch, d[1].ptr, d[1].pitch, rows, cols, 0, rows, 0, rows, R, range,
+                           o[0].ptr, o[1].ptr, o[0].pitch, elem, ctx->stream);
+    });
 }
 
 int stereo_disparity_pair_f32_host(stereo_ctx* ctx, int cost, const float* left, size_t left_step, const float* right,
@@ -1553,28 +1487,20 @@ int stereo_disparity_pair_u8_device(stereo_ctx* ctx, int cost, const uint8_t* le
                                     const uint8_t* right, size_t right_step, int rows, int cols, int window_rad,
                                     int disparity_range, void* disp_left, void* disp_right, size_t disp_step,
                                     int disp_elem_bytes, void* cuda_stream) {
-    int rc = check_ctx(ctx);
+    const int rc = check_ctx(ctx);
     if (rc != STEREO_OK) return rc;
-    cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream;
-    begin_call(ctx, st);
-    rc = pair_device(ctx, cost, PixType::U8, left, left_step, right, right_step, rows, cols, window_rad,
-                     disparity_range, disp_left, disp_right, disp_step, disp_elem_bytes, st);
-    end_call(ctx, st);
-    return rc;
+    return pair_device(ctx, cost, PixType::U8, left, left_step, right, right_step, rows, cols, 0, rows, 0, rows, window_rad,
+                       disparity_range, disp_left, disp_right, disp_step, disp_elem_bytes, cuda_stream);
 }
 
 int stereo_disparity_pair_f32_device(stereo_ctx* ctx, int cost, const float* left, size_t left_step, const float* right,
                                      size_t right_step, int rows, int cols, int window_rad, int disparity_range,
                                      void* disp_left, void* disp_right, size_t disp_step, int disp_elem_bytes,
                                      void* cuda_stream) {
-    int rc = check_ctx(ctx);
+    const int rc = check_ctx(ctx);
     if (rc != STEREO_OK) return rc;
-    cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream;
-    begin_call(ctx, st);
-    rc = pair_device(ctx, cost, PixType::F32, left, left_step, right, right_step, rows, cols, window_rad,
-                     disparity_range, disp_left, disp_right, disp_step, disp_elem_bytes, st);
-    end_call(ctx, st);
-    return rc;
+    return pair_device(ctx, cost, PixType::F32, left, left_step, right, right_step, rows, cols, 0, rows, 0, rows, window_rad,
+                       disparity_range, disp_left, disp_right, disp_step, disp_elem_bytes, cuda_stream);
 }
 
 // Both maps of a row band from one launch sequence (one rank's share of a row-band sharded PAIR, BASELINE config 4).
@@ -1583,28 +1509,14 @@ int stereo_disparity_pair_band_halo_u8_device(stereo_ctx* ctx, int cost, const u
                                               int row_begin, int row_end, int halo_begin, int halo_end, int window_rad,
                                               int disparity_range, void* disp_left, void* disp_right, size_t disp_step,
                                               int disp_elem_bytes, void* cuda_stream) {
-    int rc = check_ctx(ctx);
+    const int rc = check_ctx(ctx);
     if (rc != STEREO_OK) return rc;
     if (!left_halo || !right_halo || !disp_left || !disp_right) { set_error("null pointer"); return STEREO_ERR_INVALID_ARG; }
     if (halo_begin < 0 || halo_end > rows || halo_begin >= halo_end) { set_error("bad halo rows [%d, %d)", halo_begin, halo_end); return STEREO_ERR_INVALID_ARG; }
-    if (disparity_range < 0) { set_error("disparity_range must be >= 0"); return STEREO_ERR_INVALID_RANGE; }
-    cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream;
     const uint8_t* l0 = left_halo - size_t(halo_begin) * left_step;       // full-image origins, see above
     const uint8_t* r0 = right_halo - size_t(halo_begin) * right_step;
-    Problem p[2];
-    pair_problems(p, cost, PixType::U8, l0, left_step, r0, right_step, rows, cols, window_rad, disparity_range, disp_left, disp_right,
-                  disp_step, disp_elem_bytes);
-    for (int d = 0; d < 2; ++d) { p[d].row_begin = row_begin; p[d].row_end = row_end; p[d].avail_begin = halo_begin; p[d].avail_end = halo_end; }
-    begin_call(ctx, st);
-    if (all_fast(ctx, p, 2)) {
-        for (int d = 0; d < 2 && rc == STEREO_OK; ++d) rc = validate(p[d], size_t(cols), size_t(cols));
-        if (rc == STEREO_OK) rc = run_fast_jobs(ctx, p, 2, st);
-    } else {
-        rc = run_problem(ctx, p[0], st);
-        if (rc == STEREO_OK) rc = run_problem(ctx, p[1], st);
-    }
-    end_call(ctx, st);
-    return rc;
+    return pair_device(ctx, cost, PixType::U8, l0, left_step, r0, right_step, rows, cols, row_begin, row_end, halo_begin, halo_end,
+                       window_rad, disparity_range, disp_left, disp_right, disp_step, disp_elem_bytes, cuda_stream);
 }
 
 // ---- one row band of a pair from HOST images (a device's share of a row-band sharded pair) ------------------------------
@@ -1615,38 +1527,19 @@ int stereo_disparity_pair_band_halo_u8_device(stereo_ctx* ctx, int cost, const u
 static int pair_band_host(stereo_ctx* ctx, int cost, PixType type, const void* left, size_t left_step, const void* right,
                           size_t right_step, int rows, int cols, int row_begin, int row_end, int R, int range,
                           void* disp_left, void* disp_right, size_t disp_step, int elem) {
-    int rc = check_ctx(ctx);
+    const size_t row = size_t(cols) * (type == PixType::F32 ? 4 : 1), disp_row = size_t(cols) * elem;
+    int rc = check_host_args(ctx, {left, right, disp_left, disp_right}, rows, cols, elem,
+                             {{left_step, row}, {right_step, row}, {disp_step, disp_row}}, range, STEREO_ERR_INVALID_ARG);
     if (rc != STEREO_OK) return rc;
-    if (!left || !right || !disp_left || !disp_right) { set_error("null pointer"); return STEREO_ERR_INVALID_ARG; }
-    if (rows <= 0 || cols <= 0 || rows > 32768 || cols > 32768) { set_error("bad image size %d x %d", rows, cols); return STEREO_ERR_INVALID_ARG; }
-    if (row_begin < 0 || row_end > rows || row_begin >= row_end) { set_error("bad row band [%d, %d)", row_begin, row_end); return STEREO_ERR_INVALID_ARG; }
-    if (elem != 1 && elem != 2 && elem != 4) { set_error("disp_elem_bytes must be 1, 2 or 4"); return STEREO_ERR_INVALID_ARG; }
-    const size_t px = type == PixType::F32 ? 4 : 1;
-    if (left_step < cols * px || right_step < cols * px || disp_step < size_t(cols) * elem) { set_error("a step is smaller than its row"); return STEREO_ERR_INVALID_ARG; }
-    if (R < 0 || range < 0) { set_error("window_rad and disparity_range must be >= 0"); return STEREO_ERR_INVALID_ARG; }
     int h0 = 0, h1 = 0;
-    rc = stereo_band_halo_rows(rows, row_begin, row_end, R, &h0, &h1);
+    rc = stereo_band_halo_rows(rows, row_begin, row_end, R, &h0, &h1);      // (rejects a bad band or window radius)
     if (rc != STEREO_OK) return rc;
-    const int nh = h1 - h0, nb = row_end - row_begin;
-    cudaStream_t st = ctx->stream;
-    const size_t u8_pitch = align256(cols), d_pitch = align256(size_t(cols) * elem);
-    const size_t need = 2 * u8_pitch * nh + 2 * d_pitch * nb + 1024;
-    if (need > ctx->io.cap) {
-        SB_CUDA(cudaStreamSynchronize(st));
-        rc = ctx->io.reserve(need);
-        if (rc != STEREO_OK) return rc;
-    }
-    ctx->io.reset();
-    uint8_t* d_l = static_cast<uint8_t*>(ctx->io.take(u8_pitch * nh));
-    uint8_t* d_r = static_cast<uint8_t*>(ctx->io.take(u8_pitch * nh));
-    char* d_dl = static_cast<char*>(ctx->io.take(d_pitch * nb));
-    char* d_dr = static_cast<char*>(ctx->io.take(d_pitch * nb));
-    if (!d_l || !d_r || !d_dl || !d_dr) { set_error("io arena too small (internal)"); return STEREO_ERR_ALLOC; }
-    const char* hl = static_cast<const char*>(left) + size_t(h0) * left_step;
-    const char* hr = static_cast<const char*>(right) + size_t(h0) * right_step;
+    const int nh = h1 - h0;
+    HostRows in[2] = {{static_cast<const char*>(left) + size_t(h0) * left_step, left_step, size_t(cols)},
+                      {static_cast<const char*>(right) + size_t(h0) * right_step, right_step, size_t(cols)}};
     if (type == PixType::F32) {
         const size_t stg_pitch = (size_t(cols) + 63) & ~size_t(63);
-        SB_CUDA(cudaStreamSynchronize(st));                     // (the staging may still feed an earlier upload)
+        SB_CUDA(cudaStreamSynchronize(ctx->stream));            // (the staging may still feed an earlier upload)
         rc = ensure_pinned(ctx, 2 * stg_pitch * nh);
         if (rc != STEREO_OK) return rc;
         if (ctx->host_threads == 0) ctx->host_threads = default_host_threads();
@@ -1655,25 +1548,18 @@ static int pair_band_host(stereo_ctx* ctx, int cost, PixType type, const void* l
         if (!ctx->pool) { set_error("out of host memory"); return STEREO_ERR_ALLOC; }
         uint8_t* sl = static_cast<uint8_t*>(ctx->pinned);
         uint8_t* sr = sl + stg_pitch * nh;
-        const bool ok = pack_f32_u8(*ctx->pool, reinterpret_cast<const float*>(hl), left_step, sl, stg_pitch, nh, cols) &&
-                        pack_f32_u8(*ctx->pool, reinterpret_cast<const float*>(hr), right_step, sr, stg_pitch, nh, cols);
+        const bool ok = pack_f32_u8(*ctx->pool, static_cast<const float*>(in[0].ptr), left_step, sl, stg_pitch, nh, cols) &&
+                        pack_f32_u8(*ctx->pool, static_cast<const float*>(in[1].ptr), right_step, sr, stg_pitch, nh, cols);
         if (!ok) { set_error("row-band entry points take 8-bit-valued images only"); return STEREO_ERR_UNSUPPORTED; }
-        SB_CUDA(cudaMemcpy2DAsync(d_l, u8_pitch, sl, stg_pitch, cols, nh, cudaMemcpyHostToDevice, st));
-        SB_CUDA(cudaMemcpy2DAsync(d_r, u8_pitch, sr, stg_pitch, cols, nh, cudaMemcpyHostToDevice, st));
-    } else {
-        SB_CUDA(cudaMemcpy2DAsync(d_l, u8_pitch, hl, left_step, cols, nh, cudaMemcpyHostToDevice, st));
-        SB_CUDA(cudaMemcpy2DAsync(d_r, u8_pitch, hr, right_step, cols, nh, cudaMemcpyHostToDevice, st));
+        in[0] = HostRows{sl, stg_pitch, size_t(cols)};
+        in[1] = HostRows{sr, stg_pitch, size_t(cols)};
     }
-    rc = stereo_disparity_pair_band_halo_u8_device(ctx, cost, d_l, u8_pitch, d_r, u8_pitch, rows, cols, row_begin, row_end, h0, h1, R, range,
-                                                   d_dl, d_dr, d_pitch, elem, st);
-    if (rc == STEREO_OK) {
-        cudaError_t e = cudaMemcpy2DAsync(disp_left, disp_step, d_dl, d_pitch, size_t(cols) * elem, nb, cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess) e = cudaMemcpy2DAsync(disp_right, disp_step, d_dr, d_pitch, size_t(cols) * elem, nb, cudaMemcpyDeviceToHost, st);
-        if (e != cudaSuccess) { set_error("download failed: %s", cudaGetErrorString(e)); rc = STEREO_ERR_CUDA; }
-    }
-    cudaError_t e = cudaStreamSynchronize(st);                  // also on errors: nothing may still touch the caller's buffers
-    if (rc == STEREO_OK && e != cudaSuccess) { set_error("band call failed: %s", cudaGetErrorString(e)); rc = STEREO_ERR_CUDA; }
-    return rc;
+    const HostMap out[2] = {{disp_left, disp_step, disp_row}, {disp_right, disp_step, disp_row}};
+    return staged_host_call(ctx, in, nh, out, row_end - row_begin, [&](const DevRows* d, const DevRows* o) {
+        return stereo_disparity_pair_band_halo_u8_device(ctx, cost, reinterpret_cast<const uint8_t*>(d[0].ptr), d[0].pitch,
+                                                         reinterpret_cast<const uint8_t*>(d[1].ptr), d[1].pitch, rows, cols, row_begin,
+                                                         row_end, h0, h1, R, range, o[0].ptr, o[1].ptr, o[0].pitch, elem, ctx->stream);
+    });
 }
 
 int stereo_disparity_pair_band_u8_host(stereo_ctx* ctx, int cost, const uint8_t* left, size_t left_step, const uint8_t* right,
@@ -1707,24 +1593,14 @@ int stereo_disparity_pair_batch_u8_device(stereo_ctx* ctx, int cost, int n_pairs
     Problem ps[FMAXJOBS];
     for (int i0 = 0; i0 < n_pairs && rc == STEREO_OK; i0 += CHUNK) {
         const int np = (n_pairs - i0 < CHUNK) ? n_pairs - i0 : CHUNK;
-        // left-referenced maps first, then right-referenced ones: jobs with the same range sign are neighbours
         for (int k = 0; k < np; ++k) {
-            Problem two[2];
             const int i = i0 + k;
-            pair_problems(two, cost, PixType::U8, left + size_t(i) * pair_stride, img_step, right + size_t(i) * pair_stride, img_step,
-                          rows, cols, window_rad, disparity_range, static_cast<char*>(disp_left) + size_t(i) * disp_pair_stride,
+            pair_problems(ps, np, k, cost, PixType::U8, left + size_t(i) * pair_stride, img_step, right + size_t(i) * pair_stride,
+                          img_step, rows, cols, 0, rows, 0, rows, window_rad, disparity_range,
+                          static_cast<char*>(disp_left) + size_t(i) * disp_pair_stride,
                           static_cast<char*>(disp_right) + size_t(i) * disp_pair_stride, disp_step, disp_elem_bytes);
-            ps[k] = two[0]; ps[np + k] = two[1];
         }
-        if (all_fast(ctx, ps, 2 * np)) {
-            for (int k = 0; k < 2 * np && rc == STEREO_OK; ++k) rc = validate(ps[k], size_t(cols), size_t(cols));
-            if (rc == STEREO_OK) rc = run_fast_jobs(ctx, ps, 2 * np, st);
-        } else {
-            for (int k = 0; k < np && rc == STEREO_OK; ++k) {
-                rc = run_problem(ctx, ps[k], st);
-                if (rc == STEREO_OK) rc = run_problem(ctx, ps[np + k], st);
-            }
-        }
+        rc = run_directions(ctx, ps, 2 * np, st);
     }
     end_call(ctx, st);
     return rc;
@@ -1734,16 +1610,13 @@ int stereo_disparity_pair_batch_u8_device(stereo_ctx* ctx, int cost, int n_pairs
 static int pair_batch_host(stereo_ctx* ctx, int cost, PixType type, int n_pairs, const void* left_v, const void* right_v,
                            size_t img_step, size_t pair_stride, int rows, int cols, int window_rad, int disparity_range,
                            void* disp_left, void* disp_right, size_t disp_step, size_t disp_pair_stride, int disp_elem_bytes) {
-    int rc = check_ctx(ctx);
-    if (rc != STEREO_OK) return rc;
     const char* left = static_cast<const char*>(left_v);
     const char* right = static_cast<const char*>(right_v);
     const size_t px = type == PixType::F32 ? 4 : 1;
     if (n_pairs <= 0) { set_error("n_pairs must be positive"); return STEREO_ERR_INVALID_ARG; }
-    if (!left || !right || !disp_left || !disp_right) { set_error("null pointer"); return STEREO_ERR_INVALID_ARG; }
-    if (rows <= 0 || cols <= 0 || rows > 32768 || cols > 32768 || img_step < size_t(cols) * px || disp_step < size_t(cols) * disp_elem_bytes) { set_error("bad size/step"); return STEREO_ERR_INVALID_ARG; }
-    if (disp_elem_bytes != 1 && disp_elem_bytes != 2 && disp_elem_bytes != 4) { set_error("disp_elem_bytes must be 1, 2 or 4"); return STEREO_ERR_INVALID_ARG; }
-    if (disparity_range < 0) { set_error("disparity_range must be >= 0"); return STEREO_ERR_INVALID_RANGE; }
+    int rc = check_host_args(ctx, {left, right, disp_left, disp_right}, rows, cols, disp_elem_bytes,
+                             {{img_step, size_t(cols) * px}, {disp_step, size_t(cols) * disp_elem_bytes}}, disparity_range);
+    if (rc != STEREO_OK) return rc;
     {   // pipelined: item i+1 uploads while item i computes and item i-1 downloads (3 device slots)
         std::vector<HostPairIn> in(n_pairs);
         std::vector<void*> outs_l(n_pairs), outs_r(n_pairs);
