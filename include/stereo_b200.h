@@ -178,6 +178,30 @@ int stereo_ctx_set_fuse_pairs(stereo_ctx* ctx, int on);
 /* Image pairs of the last call whose two maps came out of one cost volume. */
 int stereo_ctx_last_fused_pairs(const stereo_ctx* ctx);
 
+/* Left-right consistency check of pair calls (OpenCV's disp12MaxDiff occlusion / mismatch filter), on the device right
+ * after both maps are computed.  max_diff < 0 (the default) switches it off: results are then exactly those without it.
+ * max_diff >= 0 switches it on for every pair entry point of this context - pair host and device, f32 and u8, the batches,
+ * the host row band and the device band halo; single-direction and stereo_disparity_refgpu_* calls ignore it.  For every
+ * output row y of every pair of a call, with both maps read as they were before any pixel was invalidated:
+ *   left pixel x, value dL, is consistent when xr = x + dL lies in [0, cols) and |dL + dR(y, xr)| <= max_diff;
+ *   right pixel x, value dR, is consistent when xl = x + dR lies in [0, cols) and |dR + dL(y, xl)| <= max_diff.
+ * An inconsistent pixel gets -(disparity_range + 1) in either map (below every valid disparity of both, OpenCV's
+ * minDisparity - 1); every other pixel keeps its value.  SSD candidates centred in the replicate padding have their
+ * partner outside the image and so are inconsistent.  The sentinel must fit the map: disp_elem_bytes 1 needs
+ * disparity_range <= 127, 2 needs <= 32767; a pair call with the check on that breaks this returns STEREO_ERR_UNSUPPORTED
+ * before it enqueues or uploads anything and leaves the outputs untouched.  The check needs no scratch: device calls with
+ * it stay capturable in CUDA graphs. */
+int stereo_ctx_set_lr_check(stereo_ctx* ctx, int max_diff);
+/* The context's current max_diff (-1: off). */
+int stereo_ctx_lr_check(const stereo_ctx* ctx);
+/* The same check in place on two device maps the caller holds: rows x cols elements of disp_elem_bytes each, row stride
+ * disp_step bytes, disp_left over [-disparity_range, 0] and disp_right over [0, +disparity_range] (values outside those
+ * ranges are checked by the same rule).  Asynchronous on `cuda_stream` (NULL = the context's stream), like every device
+ * entry point.  max_diff must be >= 0; arguments are checked like those of the pair device entry points, and a sentinel
+ * that does not fit the element type returns STEREO_ERR_UNSUPPORTED. */
+int stereo_lr_check_device(stereo_ctx* ctx, void* disp_left, void* disp_right, size_t disp_step, int disp_elem_bytes,
+                           int rows, int cols, int disparity_range, int max_diff, void* cuda_stream);
+
 /* ---- single direction, HOST buffers (the drop-in form) ------------------------------------ */
 /*
  * One disparity map for reference image `ref` searched in `tgt` over [min_disp, max_disp].
@@ -400,6 +424,9 @@ void stereo_mgpu_destroy(stereo_mgpu* mg);
 int stereo_mgpu_device_count(const stereo_mgpu* mg);
 /* The context of the index-th listed device (for stereo_ctx_set_* knobs); owned by the stereo_mgpu. */
 stereo_ctx* stereo_mgpu_ctx(stereo_mgpu* mg, int index);
+/* stereo_ctx_set_lr_check on every device's context.  The check works row by row, so row bands and pair shards give the
+ * single-GPU result. */
+int stereo_mgpu_set_lr_check(stereo_mgpu* mg, int max_diff);
 /* Batches (BASELINE config 5): same arguments as stereo_disparity_pair_batch_{u8,f32}_host. */
 int stereo_mgpu_disparity_pair_batch_u8_host(stereo_mgpu* mg, int cost, int n_pairs,
                                              const uint8_t* left, const uint8_t* right, size_t img_step, size_t pair_stride,

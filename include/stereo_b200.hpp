@@ -174,6 +174,12 @@ inline void disparityNCorrWide(const MatT& l, const MatT& r, size_t rad, int dmi
     detail::run(STEREO_COST_NCORR, l, r, rad, dmin, dmax, d, S16C1, ctx);
 }
 
+// Left-right consistency check of the pair calls on `ctx` (default: the default context): maxDiff >= 0 switches it on,
+// < 0 off (stereo_ctx_set_lr_check).
+inline void setLrCheck(int maxDiff, stereo_ctx* ctx = nullptr) {
+    check(stereo_ctx_set_lr_check(ctx ? ctx : default_ctx(), maxDiff), "stereo_ctx_set_lr_check");
+}
+
 // Kernel time of the last call on the default context, the quantity the reference logs as
 // "disparitySSDKernel execution took {} ms" (DisparitySSD.cu:203).
 inline float lastKernelMs() { return stereo_ctx_last_kernel_ms(default_ctx()); }
@@ -218,6 +224,7 @@ public:
     MultiGpu& operator=(const MultiGpu&) = delete;
     int deviceCount() const { return stereo_mgpu_device_count(mg_); }
     stereo_mgpu* handle() { return mg_; }
+    void setLrCheck(int maxDiff) { check(stereo_mgpu_set_lr_check(mg_, maxDiff), "stereo_mgpu_set_lr_check"); }
 
     // disparitySSDPair / disparityNCorrPair (main.cpp:21-78) with the output rows sharded over the devices
     void disparityPairBands(int cost, const MatT& left, const MatT& right, size_t windowRad, int disparityRange, MatT& disparityLeft,

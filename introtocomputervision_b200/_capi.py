@@ -47,6 +47,10 @@ SIGNATURES = {
     "stereo_launch_plan": (_i, [_i, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "stereo_host_pack_f32_u8": (_i, [_vp, _sz, _vp, _sz, _i, _i, _i, C.POINTER(_i)]),
     "stereo_ctx_last_fused_pairs": (_i, [_vp]),
+    "stereo_ctx_set_lr_check": (_i, [_vp, _i]),
+    "stereo_ctx_lr_check": (_i, [_vp]),
+    "stereo_lr_check_device": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _i, _i, _vp]),
+    "stereo_mgpu_set_lr_check": (_i, [_vp, _i]),
     "stereo_ctx_synchronize": (_i, [_vp, _vp]),
     "stereo_disparity_f32_host": (_i, _SINGLE_HOST),
     "stereo_disparity_u8_host": (_i, _SINGLE_HOST),

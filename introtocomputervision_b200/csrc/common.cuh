@@ -104,6 +104,7 @@ struct stereo_ctx {
     int force_path = 0;
     int pipe_bands = 0;       // 0 = automatic
     int fuse_pairs = 1;       // both maps of a pair from one cost volume where the problem allows it
+    int lr_max_diff = -1;     // pair calls: left-right consistency check with this disp12MaxDiff (< 0: off)
     // device time of the hot kernels only (fast_*_kernel), per direction, for the roofline report
     static constexpr int HOT_EVENTS = 16;
     cudaEvent_t hot0[HOT_EVENTS] = {}, hot1[HOT_EVENTS] = {};

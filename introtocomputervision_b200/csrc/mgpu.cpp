@@ -141,6 +141,15 @@ stereo_ctx* stereo_mgpu_ctx(stereo_mgpu* mg, int index) {
     return mg->ctx[index];
 }
 
+int stereo_mgpu_set_lr_check(stereo_mgpu* mg, int max_diff) {
+    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
+    for (stereo_ctx* c : mg->ctx) {
+        const int rc = stereo_ctx_set_lr_check(c, max_diff);
+        if (rc != STEREO_OK) return rc;
+    }
+    return STEREO_OK;
+}
+
 int stereo_mgpu_disparity_pair_batch_u8_host(stereo_mgpu* mg, int cost, int n_pairs, const uint8_t* left, const uint8_t* right,
                                              size_t img_step, size_t pair_stride, int rows, int cols, int window_rad,
                                              int disparity_range, void* disp_left, void* disp_right, size_t disp_step,

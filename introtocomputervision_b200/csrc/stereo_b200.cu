@@ -5,6 +5,7 @@
 #include "fast.cuh"
 #include "compat.cuh"
 #include "imgproc.cuh"
+#include "lrcheck.cuh"
 #include "host_pack.hpp"
 
 #include <atomic>
@@ -107,6 +108,33 @@ static void pair_problems(Problem* ps, int np, int k, int cost, PixType type, co
                       -range, 0, disp_left, disp_step, elem, nullptr, 0);
     ps[np + k] = direction(cost, type, right, right_step, left, left_step, rows, cols, row_begin, row_end, avail_begin, avail_end,
                            R, 0, range, disp_right, disp_step, elem, nullptr, 0);
+}
+
+// ---- left-right consistency check (lrcheck.cuh) -----------------------------------------------------
+
+// The check marks a pair's inconsistent pixels with -(range + 1), which must fit the maps' element type.  (An int8 map of
+// more than 127 disparities already holds wrapped values.)
+static bool lr_sentinel_fits(int elem, int range) { return range <= (elem == 1 ? 127 : elem == 2 ? 32767 : 32768); }
+
+static int check_lr_sentinel(int elem, int range) {
+    if (lr_sentinel_fits(elem, range)) return STEREO_OK;
+    set_error("left-right check: the sentinel -(%d + 1) does not fit a %d-byte disparity element", range, elem);
+    return STEREO_ERR_UNSUPPORTED;
+}
+
+// The check over output rows [row_begin, row_end) of the maps of n/2 pairs laid out as pair_problems builds them: ps[k]
+// left-referenced, ps[n/2 + k] its partner.  Every pair of one call has the same shape, band, range and element type.
+static int lr_check_pairs(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t st) {
+    static_assert(FMAXJOBS / 2 <= LR_MAXPAIRS, "one check launch covers the pairs of one launch sequence");
+    const int np = n / 2;
+    LrParams P{};
+    for (int k = 0; k < np; ++k)
+        P.pair[k] = LrMaps{ps[k].disp.ptr, ps[np + k].disp.ptr, ps[k].disp.step, ps[np + k].disp.step};
+    P.cols = ps[0].cols;
+    P.max_diff = ctx->lr_max_diff;
+    P.sentinel = -(ps[np].dmax + 1);
+    ctx->last_launches += 1;
+    return lr_check_launch(P, ps[0].row_end - ps[0].row_begin, np, ps[0].disp.elem, st);
 }
 
 // ---- exact path ---------------------------------------------------------------------------------
@@ -291,6 +319,20 @@ static int run_fast_jobs(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t
 
 // Enqueues every direction of a call: one problem, or n/2 left-referenced problems followed by their right-referenced
 // partners (pair k = ps[k], ps[n/2 + k]).  The one place that picks the kernel family.
+static int run_families(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bool fast, bool u8) {
+    if (fast && u8) return run_fast_jobs(ctx, ps, n, st);
+    if (fast && n <= 2) return run_f32_pair(ctx, ps, n, st);      // (float images come one pair per call)
+    const int np = n / 2;
+    if (np == 0) return run_exact_direction(ctx, ps[0], st);
+    for (int k = 0; k < np; ++k) {
+        int rc = run_exact_direction(ctx, ps[k], st);
+        if (rc == STEREO_OK) rc = run_exact_direction(ctx, ps[np + k], st);
+        if (rc != STEREO_OK) return rc;
+    }
+    return STEREO_OK;
+}
+
+// Validates every direction, runs them, then - pairs with the context's left-right check on - checks the pairs' maps.
 static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
     bool fast = ctx->force_path != STEREO_PATH_EXACT_F32, u8 = true;
     for (int i = 0; i < n; ++i) {
@@ -302,16 +344,13 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
         fast = fast && fast_supported(p);
         u8 = u8 && p.ref.type == PixType::U8;
     }
-    if (fast && u8) return run_fast_jobs(ctx, ps, n, st);
-    if (fast && n <= 2) return run_f32_pair(ctx, ps, n, st);      // (float images come one pair per call)
-    const int np = n / 2;
-    if (np == 0) return run_exact_direction(ctx, ps[0], st);
-    for (int k = 0; k < np; ++k) {
-        int rc = run_exact_direction(ctx, ps[k], st);
-        if (rc == STEREO_OK) rc = run_exact_direction(ctx, ps[np + k], st);
+    const bool lr = n >= 2 && ctx->lr_max_diff >= 0;
+    for (int k = 0; lr && k < n / 2; ++k) {
+        const int rc = check_lr_sentinel(ps[k].disp.elem, ps[n / 2 + k].dmax);
         if (rc != STEREO_OK) return rc;
     }
-    return STEREO_OK;
+    const int rc = run_families(ctx, ps, n, st, fast, u8);
+    return rc == STEREO_OK && lr ? lr_check_pairs(ctx, ps, n, st) : rc;
 }
 
 // Every call of a context shares one scratch arena (and the classification flag), so calls are ordered: a call
@@ -749,6 +788,8 @@ static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, in
                 } else {
                     for (int k = 0; k < nj && rc == STEREO_OK; ++k) { ctx->arena.reset(); rc = run_fast(ctx, pd[k], s_cmp); }
                 }
+                // two directions: pd holds the np left-referenced problems, then their partners
+                if (rc == STEREO_OK && n_dirs == 2 && ctx->lr_max_diff >= 0) rc = lr_check_pairs(ctx, pd, nj, s_cmp);
                 if (rc != STEREO_OK) return rc;
             }
             SB_CUDA(cudaEventRecord(ev(w, b, 1), s_cmp));
@@ -786,7 +827,8 @@ static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, in
 
 // What every host entry point checks before it touches a buffer: the context, non-null pointers, an image of at most
 // 32768 pixels a side (validate() reports larger ones to device callers as UNSUPPORTED), a disparity element of 1, 2 or
-// 4 bytes and every {step, row bytes} step at least its row.  A pair's negative `range` is rejected with `range_rc`.
+// 4 bytes and every {step, row bytes} step at least its row.  A pair's negative `range` is rejected with `range_rc`, and
+// with the left-right check on, a `range` whose sentinel does not fit `elem` (single directions pass range 0).
 static int check_host_args(stereo_ctx* ctx, std::initializer_list<const void*> ptrs, int rows, int cols, int elem,
                            std::initializer_list<std::pair<size_t, size_t>> steps, int range = 0,
                            int range_rc = STEREO_ERR_INVALID_RANGE) {
@@ -799,7 +841,7 @@ static int check_host_args(stereo_ctx* ctx, std::initializer_list<const void*> p
     for (const auto& s : steps)
         if (s.first < s.second) { set_error("a step is smaller than its row"); return STEREO_ERR_INVALID_ARG; }
     if (range < 0) { set_error("disparity_range must be >= 0"); return range_rc; }
-    return STEREO_OK;
+    return ctx->lr_max_diff >= 0 ? check_lr_sentinel(elem, range) : STEREO_OK;
 }
 
 // Sequential host call: upload (2D async copies), compute, download, synchronize - the shape of cuda::disparitySSD
@@ -960,6 +1002,7 @@ int stereo_ctx_create(int device, stereo_ctx** ctx_out) {
         return STEREO_ERR_CUDA;
     }
     int rc = fast_ctx_init(c);
+    if (rc == STEREO_OK) rc = lr_check_init();
     if (rc != STEREO_OK) { stereo_ctx_destroy(c); return rc; }
     *ctx_out = c;
     return STEREO_OK;
@@ -1160,6 +1203,40 @@ int stereo_ctx_set_fuse_pairs(stereo_ctx* ctx, int on) {
     if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
     ctx->fuse_pairs = on ? 1 : 0;
     return STEREO_OK;
+}
+
+int stereo_ctx_set_lr_check(stereo_ctx* ctx, int max_diff) {
+    if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
+    ctx->lr_max_diff = max_diff < 0 ? -1 : max_diff;
+    return STEREO_OK;
+}
+
+int stereo_ctx_lr_check(const stereo_ctx* ctx) { return ctx ? ctx->lr_max_diff : -1; }
+
+int stereo_lr_check_device(stereo_ctx* ctx, void* disp_left, void* disp_right, size_t disp_step, int disp_elem_bytes, int rows,
+                           int cols, int disparity_range, int max_diff, void* cuda_stream) {
+    int rc = check_ctx(ctx);
+    if (rc != STEREO_OK) return rc;
+    if (!disp_left || !disp_right) { set_error("null map pointer"); return STEREO_ERR_INVALID_ARG; }
+    if (rows <= 0 || cols <= 0) { set_error("rows/cols must be positive (got %d x %d)", rows, cols); return STEREO_ERR_INVALID_ARG; }
+    if (rows > 32768 || cols > LR_MAXCOLS) { set_error("map larger than 32768 in a dimension"); return STEREO_ERR_UNSUPPORTED; }
+    if (disp_elem_bytes != 1 && disp_elem_bytes != 2 && disp_elem_bytes != 4) { set_error("disp_elem_bytes must be 1, 2 or 4"); return STEREO_ERR_INVALID_ARG; }
+    if (disp_step < size_t(cols) * disp_elem_bytes) { set_error("disp_step smaller than a row"); return STEREO_ERR_INVALID_ARG; }
+    if (disparity_range < 0 || disparity_range > 32768) { set_error("disparity_range must be in [0, 32768]"); return STEREO_ERR_INVALID_RANGE; }
+    if (max_diff < 0) { set_error("max_diff must be >= 0"); return STEREO_ERR_INVALID_ARG; }
+    rc = check_lr_sentinel(disp_elem_bytes, disparity_range);
+    if (rc != STEREO_OK) return rc;
+    cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream;
+    begin_call(ctx, st);
+    LrParams P{};
+    P.pair[0] = LrMaps{disp_left, disp_right, disp_step, disp_step};
+    P.cols = cols;
+    P.max_diff = max_diff;
+    P.sentinel = -(disparity_range + 1);
+    ctx->last_launches = 1;
+    rc = lr_check_launch(P, rows, 1, disp_elem_bytes, st);
+    end_call(ctx, st);
+    return rc;
 }
 
 // ---- peer gather: results pushed into other ranks' buffers by the copy engines ---------------------

@@ -117,6 +117,19 @@ class Context:
         """Pair calls: both maps from one cost volume where possible (default on; results identical either way)."""
         _check(_capi.lib().stereo_ctx_set_fuse_pairs(self._h, int(bool(on))), "stereo_ctx_set_fuse_pairs")
 
+    def set_lr_check(self, max_diff: Optional[int]) -> None:
+        """Pair calls: left-right consistency check (``disp12MaxDiff``).  Pixels whose partner in the other map is outside
+        the image or differs by more than ``max_diff`` get ``-(disparity_range + 1)`` in both maps.  ``None`` or a negative
+        value switches it off (the default)."""
+        v = -1 if max_diff is None or max_diff < 0 else int(max_diff)
+        _check(_capi.lib().stereo_ctx_set_lr_check(self._h, v), "stereo_ctx_set_lr_check")
+
+    @property
+    def lr_check(self) -> Optional[int]:
+        """The left-right check's ``max_diff``, or None when the check is off."""
+        v = int(_capi.lib().stereo_ctx_lr_check(self._h))
+        return None if v < 0 else v
+
     def set_host_threads(self, threads: int) -> None:
         """Host threads that convert CV_32FC1 host images to u8 before the upload (0 = automatic, -1 = off)."""
         _check(_capi.lib().stereo_ctx_set_host_threads(self._h, int(threads)), "stereo_ctx_set_host_threads")
@@ -252,6 +265,11 @@ class MultiGpu:
 
     def __exit__(self, *exc):
         self.close()
+
+    def set_lr_check(self, max_diff: Optional[int]) -> None:
+        """:meth:`Context.set_lr_check` on every device's context."""
+        v = -1 if max_diff is None or max_diff < 0 else int(max_diff)
+        _check(_capi.lib().stereo_mgpu_set_lr_check(self._h, v), "stereo_mgpu_set_lr_check")
 
     def disparity_pair_bands(self, cost: int, left: np.ndarray, right: np.ndarray, window_rad: int, disparity_range: int,
                              dtype=np.int8) -> Tuple[np.ndarray, np.ndarray]:
