@@ -202,6 +202,32 @@ int stereo_ctx_lr_check(const stereo_ctx* ctx);
 int stereo_lr_check_device(stereo_ctx* ctx, void* disp_left, void* disp_right, size_t disp_step, int disp_elem_bytes,
                            int rows, int cols, int disparity_range, int max_diff, void* cuda_stream);
 
+/* Speckle filter of pair calls (OpenCV's cv::filterSpeckles, StereoSGBM's speckleWindowSize / speckleRange), on the device
+ * after both maps are computed and, with it on too, after the left-right check.  max_size <= 0 (the default) switches it
+ * off: results are then exactly those without it.  max_size > 0 switches it on for the pair entry points of this context
+ * that compute whole maps - pair host and device, f32 and u8, the batches - and needs max_diff >= 0
+ * (STEREO_ERR_INVALID_ARG otherwise).  In each map, two 4-neighbours are connected when neither holds the sentinel and
+ * their values differ by at most max_diff (disparity units); every pixel of a connected component of at most max_size
+ * pixels gets the sentinel -(disparity_range + 1), every other pixel keeps its value.  Pixels the left-right check
+ * invalidated therefore split regions.  The sentinel rule is the left-right check's (disp_elem_bytes 1 needs
+ * disparity_range <= 127, 2 needs <= 32767; otherwise STEREO_ERR_UNSUPPORTED before anything is enqueued or uploaded).
+ * A speckle region can cross a band seam, so the row-band entry points (stereo_disparity_pair_band_halo_u8_device,
+ * stereo_disparity_pair_band_{u8,f32}_host) accept only the whole image as their band, and stereo_mgpu_disparity_pair_bands_*
+ * refuse: those calls return STEREO_ERR_UNSUPPORTED and enqueue, upload and write nothing.  Callers of band-sharded pairs
+ * filter the gathered maps with stereo_filter_speckles_device.  Single-direction and stereo_disparity_refgpu_* calls
+ * ignore the setting.  The filter takes about 8 bytes of scratch per pixel and map from the context's arena; after one
+ * call of a shape, device calls of that shape allocate nothing and stay capturable in CUDA graphs. */
+int stereo_ctx_set_speckle_filter(stereo_ctx* ctx, int max_size, int max_diff);
+/* The context's current setting (max_size 0: off). */
+int stereo_ctx_speckle_filter(const stereo_ctx* ctx, int* max_size, int* max_diff);
+/* cv::filterSpeckles(map, new_val, max_size, max_diff) in place on one device map the caller holds: rows x cols elements
+ * of disp_elem_bytes each (signed), row stride disp_step bytes; the bytes past a row's cols elements are never touched.
+ * Asynchronous on `cuda_stream` (NULL = the context's stream), like every device entry point.  A null map, a non-positive
+ * size, an element size other than 1, 2 or 4, a short step, a negative max_size or max_diff or a new_val the element type
+ * cannot hold return STEREO_ERR_INVALID_ARG; rows or cols over 32768 STEREO_ERR_UNSUPPORTED; max_size 0 is a valid no-op. */
+int stereo_filter_speckles_device(stereo_ctx* ctx, void* disp, size_t disp_step, int disp_elem_bytes, int rows, int cols,
+                                  int new_val, int max_size, int max_diff, void* cuda_stream);
+
 /* ---- single direction, HOST buffers (the drop-in form) ------------------------------------ */
 /*
  * One disparity map for reference image `ref` searched in `tgt` over [min_disp, max_disp].
@@ -427,6 +453,9 @@ stereo_ctx* stereo_mgpu_ctx(stereo_mgpu* mg, int index);
 /* stereo_ctx_set_lr_check on every device's context.  The check works row by row, so row bands and pair shards give the
  * single-GPU result. */
 int stereo_mgpu_set_lr_check(stereo_mgpu* mg, int max_diff);
+/* stereo_ctx_set_speckle_filter on every device's context.  Pair batches shard whole pairs and so give the single-GPU
+ * result; row-band sharded pairs return STEREO_ERR_UNSUPPORTED while the filter is on. */
+int stereo_mgpu_set_speckle_filter(stereo_mgpu* mg, int max_size, int max_diff);
 /* Batches (BASELINE config 5): same arguments as stereo_disparity_pair_batch_{u8,f32}_host. */
 int stereo_mgpu_disparity_pair_batch_u8_host(stereo_mgpu* mg, int cost, int n_pairs,
                                              const uint8_t* left, const uint8_t* right, size_t img_step, size_t pair_stride,

@@ -180,6 +180,12 @@ inline void setLrCheck(int maxDiff, stereo_ctx* ctx = nullptr) {
     check(stereo_ctx_set_lr_check(ctx ? ctx : default_ctx(), maxDiff), "stereo_ctx_set_lr_check");
 }
 
+// Speckle filter of the pair calls on `ctx` (default: the default context): maxSize > 0 switches it on, <= 0 off
+// (stereo_ctx_set_speckle_filter).
+inline void setSpeckleFilter(int maxSize, int maxDiff, stereo_ctx* ctx = nullptr) {
+    check(stereo_ctx_set_speckle_filter(ctx ? ctx : default_ctx(), maxSize, maxDiff), "stereo_ctx_set_speckle_filter");
+}
+
 // Kernel time of the last call on the default context, the quantity the reference logs as
 // "disparitySSDKernel execution took {} ms" (DisparitySSD.cu:203).
 inline float lastKernelMs() { return stereo_ctx_last_kernel_ms(default_ctx()); }
@@ -225,6 +231,9 @@ public:
     int deviceCount() const { return stereo_mgpu_device_count(mg_); }
     stereo_mgpu* handle() { return mg_; }
     void setLrCheck(int maxDiff) { check(stereo_mgpu_set_lr_check(mg_, maxDiff), "stereo_mgpu_set_lr_check"); }
+    void setSpeckleFilter(int maxSize, int maxDiff) {
+        check(stereo_mgpu_set_speckle_filter(mg_, maxSize, maxDiff), "stereo_mgpu_set_speckle_filter");
+    }
 
     // disparitySSDPair / disparityNCorrPair (main.cpp:21-78) with the output rows sharded over the devices
     void disparityPairBands(int cost, const MatT& left, const MatT& right, size_t windowRad, int disparityRange, MatT& disparityLeft,

@@ -51,6 +51,10 @@ SIGNATURES = {
     "stereo_ctx_lr_check": (_i, [_vp]),
     "stereo_lr_check_device": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _i, _i, _vp]),
     "stereo_mgpu_set_lr_check": (_i, [_vp, _i]),
+    "stereo_ctx_set_speckle_filter": (_i, [_vp, _i, _i]),
+    "stereo_ctx_speckle_filter": (_i, [_vp, C.POINTER(_i), C.POINTER(_i)]),
+    "stereo_filter_speckles_device": (_i, [_vp, _vp, _sz, _i, _i, _i, _i, _i, _i, _vp]),
+    "stereo_mgpu_set_speckle_filter": (_i, [_vp, _i, _i]),
     "stereo_ctx_synchronize": (_i, [_vp, _vp]),
     "stereo_disparity_f32_host": (_i, _SINGLE_HOST),
     "stereo_disparity_u8_host": (_i, _SINGLE_HOST),

@@ -105,6 +105,8 @@ struct stereo_ctx {
     int pipe_bands = 0;       // 0 = automatic
     int fuse_pairs = 1;       // both maps of a pair from one cost volume where the problem allows it
     int lr_max_diff = -1;     // pair calls: left-right consistency check with this disp12MaxDiff (< 0: off)
+    int spk_max_size = 0;     // pair calls: speckle filter of components up to this many pixels (0: off) ...
+    int spk_max_diff = 0;     // ... whose neighbours differ by at most this much
     // device time of the hot kernels only (fast_*_kernel), per direction, for the roofline report
     static constexpr int HOT_EVENTS = 16;
     cudaEvent_t hot0[HOT_EVENTS] = {}, hot1[HOT_EVENTS] = {};

@@ -75,6 +75,15 @@ int pair_bands(stereo_mgpu* mg, int cost, const T* left, size_t left_step, const
                int window_rad, int disparity_range, void* disp_left, void* disp_right, size_t disp_step, int elem, bool f32) {
     if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
     if (rows <= 0) { sb::set_error("rows must be positive"); return STEREO_ERR_INVALID_ARG; }
+    // a speckle region can cross a band seam: no band is filtered on its own (and no whole-pair call stands in for the bands)
+    for (stereo_ctx* c : mg->ctx) {
+        int max_size = 0, max_diff = 0;
+        stereo_ctx_speckle_filter(c, &max_size, &max_diff);
+        if (max_size > 0) {
+            sb::set_error("speckle filter on: row-band sharded pairs are not filtered (filter the gathered map with stereo_filter_speckles_device)");
+            return STEREO_ERR_UNSUPPORTED;
+        }
+    }
     int parts = int(mg->ctx.size());
     const int band = (rows + parts - 1) / parts;            // equal bands of ceil(rows / parts) rows, the last one(s) shorter or empty
     int rc = for_each_device(mg, [&](int k) -> int {
@@ -145,6 +154,15 @@ int stereo_mgpu_set_lr_check(stereo_mgpu* mg, int max_diff) {
     if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
     for (stereo_ctx* c : mg->ctx) {
         const int rc = stereo_ctx_set_lr_check(c, max_diff);
+        if (rc != STEREO_OK) return rc;
+    }
+    return STEREO_OK;
+}
+
+int stereo_mgpu_set_speckle_filter(stereo_mgpu* mg, int max_size, int max_diff) {
+    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
+    for (stereo_ctx* c : mg->ctx) {
+        const int rc = stereo_ctx_set_speckle_filter(c, max_size, max_diff);
         if (rc != STEREO_OK) return rc;
     }
     return STEREO_OK;

@@ -6,6 +6,7 @@
 #include "compat.cuh"
 #include "imgproc.cuh"
 #include "lrcheck.cuh"
+#include "speckle.cuh"
 #include "host_pack.hpp"
 
 #include <atomic>
@@ -118,7 +119,7 @@ static bool lr_sentinel_fits(int elem, int range) { return range <= (elem == 1 ?
 
 static int check_lr_sentinel(int elem, int range) {
     if (lr_sentinel_fits(elem, range)) return STEREO_OK;
-    set_error("left-right check: the sentinel -(%d + 1) does not fit a %d-byte disparity element", range, elem);
+    set_error("left-right check / speckle filter: the sentinel -(%d + 1) does not fit a %d-byte disparity element", range, elem);
     return STEREO_ERR_UNSUPPORTED;
 }
 
@@ -135,6 +136,40 @@ static int lr_check_pairs(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_
     P.sentinel = -(ps[np].dmax + 1);
     ctx->last_launches += 1;
     return lr_check_launch(P, ps[0].row_end - ps[0].row_begin, np, ps[0].disp.elem, st);
+}
+
+// ---- speckle filter (speckle.cuh) ---------------------------------------------------------------------------------
+
+// The filter over n whole rows x cols maps of one element type, in place.  Its scratch comes from the arena, which the
+// caller sized for speckle_scratch_bytes(n, rows, cols) before it enqueued anything: the filter itself never grows it.
+static int speckle_maps(stereo_ctx* ctx, const OutView* maps, int n, int rows, int cols, int new_val, int max_size, int max_diff,
+                        cudaStream_t st) {
+    SpeckleParams P{};
+    for (int k = 0; k < n; ++k) P.map[k] = SpeckleMap{maps[k].ptr, maps[k].step, nullptr, nullptr};
+    P.rows = rows; P.cols = cols; P.new_val = new_val; P.max_size = max_size; P.max_diff = max_diff;
+    ctx->arena.reset();
+    void* s = ctx->arena.take(speckle_scratch_bytes(n, rows, cols));
+    if (!s) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
+    speckle_bind_scratch(P, n, s);
+    ctx->last_launches += SPK_LAUNCHES;
+    return speckle_launch(P, n, maps[0].elem, st);
+}
+
+// A speckle region can cross a band seam, so with the filter on a pair call takes the whole map only.
+static int check_speckle_band(const stereo_ctx* ctx, int row_begin, int row_end, int rows) {
+    if (ctx->spk_max_size <= 0 || (row_begin == 0 && row_end == rows)) return STEREO_OK;
+    set_error("speckle filter: rows [%d, %d) are not the whole map (filter the gathered map with stereo_filter_speckles_device)",
+              row_begin, row_end);
+    return STEREO_ERR_UNSUPPORTED;
+}
+
+// The context's filter over both maps of the n/2 whole-image pairs of ps (laid out as pair_problems builds them), with the
+// left-right check's sentinel as the value of removed pixels.
+static int speckle_pairs(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t st) {
+    static_assert(FMAXJOBS <= SPK_MAXMAPS, "one filter launch covers the maps of one launch sequence");
+    OutView maps[FMAXJOBS];
+    for (int k = 0; k < n; ++k) maps[k] = ps[k].disp;
+    return speckle_maps(ctx, maps, n, ps[0].rows, ps[0].cols, -(ps[n / 2].dmax + 1), ctx->spk_max_size, ctx->spk_max_diff, st);
 }
 
 // ---- exact path ---------------------------------------------------------------------------------
@@ -332,7 +367,8 @@ static int run_families(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bo
     return STEREO_OK;
 }
 
-// Validates every direction, runs them, then - pairs with the context's left-right check on - checks the pairs' maps.
+// Validates every direction, runs them, then - pairs with the context's left-right check or speckle filter on - checks
+// and filters the pairs' maps, in that order (StereoSGBM's).
 static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
     bool fast = ctx->force_path != STEREO_PATH_EXACT_F32, u8 = true;
     for (int i = 0; i < n; ++i) {
@@ -344,13 +380,20 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
         fast = fast && fast_supported(p);
         u8 = u8 && p.ref.type == PixType::U8;
     }
-    const bool lr = n >= 2 && ctx->lr_max_diff >= 0;
-    for (int k = 0; lr && k < n / 2; ++k) {
+    const bool lr = n >= 2 && ctx->lr_max_diff >= 0, spk = n >= 2 && ctx->spk_max_size > 0;
+    for (int k = 0; (lr || spk) && k < n / 2; ++k) {
         const int rc = check_lr_sentinel(ps[k].disp.elem, ps[n / 2 + k].dmax);
         if (rc != STEREO_OK) return rc;
     }
-    const int rc = run_families(ctx, ps, n, st, fast, u8);
-    return rc == STEREO_OK && lr ? lr_check_pairs(ctx, ps, n, st) : rc;
+    if (spk) {
+        int rc = check_speckle_band(ctx, ps[0].row_begin, ps[0].row_end, ps[0].rows);
+        if (rc == STEREO_OK) rc = reserve_arena(ctx, st, speckle_scratch_bytes(n, ps[0].rows, ps[0].cols));
+        if (rc != STEREO_OK) return rc;
+    }
+    int rc = run_families(ctx, ps, n, st, fast, u8);
+    if (rc == STEREO_OK && lr) rc = lr_check_pairs(ctx, ps, n, st);
+    if (rc == STEREO_OK && spk) rc = speckle_pairs(ctx, ps, n, st);
+    return rc;
 }
 
 // Every call of a context shares one scratch arena (and the classification flag), so calls are ordered: a call
@@ -599,6 +642,9 @@ static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, in
             }
         }
     }
+    // pairs with the speckle filter: an item's maps are filtered whole after its last band, then downloaded
+    const bool spk = n_dirs == 2 && ctx->spk_max_size > 0;
+    if (spk && speckle_scratch_bytes(2 * cp, rows, cols) > scratch) scratch = speckle_scratch_bytes(2 * cp, rows, cols);
     constexpr int NSTG = 4;                               // pinned staging ring of the host-packed uploads
     int rc = ensure_pipe(ctx, 3 * n_units + 4 + NSTG);
     if (rc != STEREO_OK) return rc;
@@ -790,15 +836,21 @@ static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, in
                 }
                 // two directions: pd holds the np left-referenced problems, then their partners
                 if (rc == STEREO_OK && n_dirs == 2 && ctx->lr_max_diff >= 0) rc = lr_check_pairs(ctx, pd, nj, s_cmp);
+                if (rc == STEREO_OK && spk && b == nbw(w) - 1) {
+                    OutView maps[2 * PIPE_CPMAX];
+                    for (int k = 0; k < nj; ++k) maps[k] = OutView{sl[k % np].out[k / np], d_pitch, elem};
+                    rc = speckle_maps(ctx, maps, nj, rows, cols, -(dirs[1].dmax + 1), ctx->spk_max_size, ctx->spk_max_diff, s_cmp);
+                }
                 if (rc != STEREO_OK) return rc;
             }
             SB_CUDA(cudaEventRecord(ev(w, b, 1), s_cmp));
-            // ---- download
+            // ---- download: this band's rows, or with the speckle filter every row of the item after its last band
             SB_CUDA(cudaStreamWaitEvent(s_out, ev(w, b, 1), 0));
-            for (int c = 0; c < np; ++c)
+            const int d0 = !spk ? rb : (b == nbw(w) - 1 ? 0 : re);
+            for (int c = 0; c < np && re > d0; ++c)
                 for (int d = 0; d < n_dirs; ++d)
-                    SB_CUDA(cudaMemcpy2DAsync(static_cast<char*>(dirs[d].out[i0 + c]) + size_t(rb) * disp_step, disp_step, sl[c].out[d] + size_t(rb) * d_pitch, d_pitch,
-                                              size_t(cols) * elem, re - rb, cudaMemcpyDeviceToHost, s_out));
+                    SB_CUDA(cudaMemcpy2DAsync(static_cast<char*>(dirs[d].out[i0 + c]) + size_t(d0) * disp_step, disp_step, sl[c].out[d] + size_t(d0) * d_pitch, d_pitch,
+                                              size_t(cols) * elem, re - d0, cudaMemcpyDeviceToHost, s_out));
             SB_CUDA(cudaEventRecord(ev(w, b, 2), s_out));
         }
     }
@@ -828,7 +880,8 @@ static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, in
 // What every host entry point checks before it touches a buffer: the context, non-null pointers, an image of at most
 // 32768 pixels a side (validate() reports larger ones to device callers as UNSUPPORTED), a disparity element of 1, 2 or
 // 4 bytes and every {step, row bytes} step at least its row.  A pair's negative `range` is rejected with `range_rc`, and
-// with the left-right check on, a `range` whose sentinel does not fit `elem` (single directions pass range 0).
+// with the left-right check or the speckle filter on, a `range` whose sentinel does not fit `elem` (single directions pass
+// range 0).
 static int check_host_args(stereo_ctx* ctx, std::initializer_list<const void*> ptrs, int rows, int cols, int elem,
                            std::initializer_list<std::pair<size_t, size_t>> steps, int range = 0,
                            int range_rc = STEREO_ERR_INVALID_RANGE) {
@@ -841,7 +894,7 @@ static int check_host_args(stereo_ctx* ctx, std::initializer_list<const void*> p
     for (const auto& s : steps)
         if (s.first < s.second) { set_error("a step is smaller than its row"); return STEREO_ERR_INVALID_ARG; }
     if (range < 0) { set_error("disparity_range must be >= 0"); return range_rc; }
-    return ctx->lr_max_diff >= 0 ? check_lr_sentinel(elem, range) : STEREO_OK;
+    return ctx->lr_max_diff >= 0 || ctx->spk_max_size > 0 ? check_lr_sentinel(elem, range) : STEREO_OK;
 }
 
 // Sequential host call: upload (2D async copies), compute, download, synchronize - the shape of cuda::disparitySSD
@@ -1239,6 +1292,43 @@ int stereo_lr_check_device(stereo_ctx* ctx, void* disp_left, void* disp_right, s
     return rc;
 }
 
+int stereo_ctx_set_speckle_filter(stereo_ctx* ctx, int max_size, int max_diff) {
+    if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
+    if (max_size > 0 && max_diff < 0) { set_error("max_diff must be >= 0"); return STEREO_ERR_INVALID_ARG; }
+    ctx->spk_max_size = max_size > 0 ? max_size : 0;
+    ctx->spk_max_diff = max_size > 0 ? max_diff : 0;
+    return STEREO_OK;
+}
+
+int stereo_ctx_speckle_filter(const stereo_ctx* ctx, int* max_size, int* max_diff) {
+    if (!ctx || !max_size || !max_diff) { set_error("null argument"); return STEREO_ERR_INVALID_ARG; }
+    *max_size = ctx->spk_max_size;
+    *max_diff = ctx->spk_max_diff;
+    return STEREO_OK;
+}
+
+int stereo_filter_speckles_device(stereo_ctx* ctx, void* disp, size_t disp_step, int disp_elem_bytes, int rows, int cols, int new_val,
+                                  int max_size, int max_diff, void* cuda_stream) {
+    int rc = check_ctx(ctx);
+    if (rc != STEREO_OK) return rc;
+    if (!disp) { set_error("null map pointer"); return STEREO_ERR_INVALID_ARG; }
+    if (rows <= 0 || cols <= 0) { set_error("rows/cols must be positive (got %d x %d)", rows, cols); return STEREO_ERR_INVALID_ARG; }
+    if (rows > SPK_MAXDIM || cols > SPK_MAXDIM) { set_error("map larger than 32768 in a dimension"); return STEREO_ERR_UNSUPPORTED; }
+    if (disp_elem_bytes != 1 && disp_elem_bytes != 2 && disp_elem_bytes != 4) { set_error("disp_elem_bytes must be 1, 2 or 4"); return STEREO_ERR_INVALID_ARG; }
+    if (disp_step < size_t(cols) * disp_elem_bytes) { set_error("disp_step smaller than a row"); return STEREO_ERR_INVALID_ARG; }
+    if (max_size < 0 || max_diff < 0) { set_error("max_size and max_diff must be >= 0"); return STEREO_ERR_INVALID_ARG; }
+    const int lim = disp_elem_bytes == 1 ? 127 : disp_elem_bytes == 2 ? 32767 : INT32_MAX;
+    if (new_val > lim || new_val < -lim - 1) { set_error("new_val %d does not fit a %d-byte element", new_val, disp_elem_bytes); return STEREO_ERR_INVALID_ARG; }
+    cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream;
+    if (max_size > 0) rc = reserve_arena(ctx, st, speckle_scratch_bytes(1, rows, cols));
+    if (rc != STEREO_OK) return rc;
+    begin_call(ctx, st);
+    const OutView map{disp, disp_step, disp_elem_bytes};
+    if (max_size > 0) rc = speckle_maps(ctx, &map, 1, rows, cols, new_val, max_size, max_diff, st);
+    end_call(ctx, st);
+    return rc;
+}
+
 // ---- peer gather: results pushed into other ranks' buffers by the copy engines ---------------------
 static int ensure_peer(stereo_ctx* ctx) {
     if (ctx->peer_ready) return STEREO_OK;
@@ -1610,6 +1700,8 @@ static int pair_band_host(stereo_ctx* ctx, int cost, PixType type, const void* l
     if (rc != STEREO_OK) return rc;
     int h0 = 0, h1 = 0;
     rc = stereo_band_halo_rows(rows, row_begin, row_end, R, &h0, &h1);      // (rejects a bad band or window radius)
+    if (rc != STEREO_OK) return rc;
+    rc = check_speckle_band(ctx, row_begin, row_end, rows);      // (as run_directions would, but before staging)
     if (rc != STEREO_OK) return rc;
     const int nh = h1 - h0;
     HostRows in[2] = {{static_cast<const char*>(left) + size_t(h0) * left_step, left_step, size_t(cols)},

@@ -130,6 +130,20 @@ class Context:
         v = int(_capi.lib().stereo_ctx_lr_check(self._h))
         return None if v < 0 else v
 
+    def set_speckle_filter(self, max_size: Optional[int], max_diff: int = 1) -> None:
+        """Pair calls: speckle filter (``cv::filterSpeckles``), after the left-right check when both are on.  In each map,
+        connected regions of at most ``max_size`` pixels whose 4-neighbours differ by at most ``max_diff`` get
+        ``-(disparity_range + 1)``.  ``None`` or a value <= 0 switches it off (the default)."""
+        v = 0 if max_size is None or max_size <= 0 else int(max_size)
+        _check(_capi.lib().stereo_ctx_set_speckle_filter(self._h, v, int(max_diff)), "stereo_ctx_set_speckle_filter")
+
+    @property
+    def speckle_filter(self) -> Optional[Tuple[int, int]]:
+        """``(max_size, max_diff)`` of the speckle filter, or None when it is off."""
+        size, diff = C.c_int(), C.c_int()
+        _check(_capi.lib().stereo_ctx_speckle_filter(self._h, C.byref(size), C.byref(diff)), "stereo_ctx_speckle_filter")
+        return None if size.value <= 0 else (size.value, diff.value)
+
     def set_host_threads(self, threads: int) -> None:
         """Host threads that convert CV_32FC1 host images to u8 before the upload (0 = automatic, -1 = off)."""
         _check(_capi.lib().stereo_ctx_set_host_threads(self._h, int(threads)), "stereo_ctx_set_host_threads")
@@ -270,6 +284,11 @@ class MultiGpu:
         """:meth:`Context.set_lr_check` on every device's context."""
         v = -1 if max_diff is None or max_diff < 0 else int(max_diff)
         _check(_capi.lib().stereo_mgpu_set_lr_check(self._h, v), "stereo_mgpu_set_lr_check")
+
+    def set_speckle_filter(self, max_size: Optional[int], max_diff: int = 1) -> None:
+        """:meth:`Context.set_speckle_filter` on every device's context (row-band sharded pairs refuse while it is on)."""
+        v = 0 if max_size is None or max_size <= 0 else int(max_size)
+        _check(_capi.lib().stereo_mgpu_set_speckle_filter(self._h, v, int(max_diff)), "stereo_mgpu_set_speckle_filter")
 
     def disparity_pair_bands(self, cost: int, left: np.ndarray, right: np.ndarray, window_rad: int, disparity_range: int,
                              dtype=np.int8) -> Tuple[np.ndarray, np.ndarray]:

@@ -1,0 +1,549 @@
+"""Speckle filter on the B200 (stereo_ctx_set_speckle_filter, stereo_filter_speckles_device): the kernel alone against the
+filter's restatement (speckle_oracle.filter_speckles) on adversarial maps and shapes, with padded rows; every pair entry
+point with the filter on against the restatement applied to the same call's maps with it off, alone and after the
+left-right check, for both costs, fused and unfused, on each kernel family; a 16-pair 720p batch and a 4K pair; the
+rejections (partial bands, the sentinel rule, bad settings and arguments) and the default and off states; and a CUDA
+graph around a device pair call."""
+import ctypes as C
+
+import numpy as np
+import pytest
+
+import introtocomputervision_b200 as sb
+from introtocomputervision_b200 import _capi, synth
+from lr_oracle import lr_check
+from speckle_oracle import filter_speckles
+from test_entry_points import EXPECTED, PITCH, ROWS, _args
+from test_lr_check import FAMILIES, RANGE_T, _images, _run, _set_fuse
+
+pytestmark = pytest.mark.gpu
+
+ARG, UNSUP = _capi.ERR_INVALID_ARG, _capi.ERR_UNSUPPORTED
+DT = {1: np.int8, 2: np.int16, 4: np.int32}
+MAX_SIZE, MAX_DIFF = 30, 0
+
+
+def _torch():
+    import torch
+    return torch
+
+
+def _ok(rc, where=""):
+    assert rc == _capi.STEREO_OK, f"{where}: {rc} ({_capi.last_error()})"
+
+
+@pytest.fixture(scope="module")
+def sctx():
+    c = sb.Context(0)
+    yield c
+    c.close()
+
+
+@pytest.fixture(scope="module")
+def mg():
+    m = sb.MultiGpu([0, 0])
+    yield m
+    m.close()
+
+
+# ---- 1. the kernel alone ---------------------------------------------------------------------------------------------
+
+def _blobs(g, rows, cols):
+    """Random walks along the rows and down the columns: long, thin regions of every size, plus 5 % sentinel pixels."""
+    d = np.cumsum(g.integers(-1, 2, (rows, cols)), axis=1) + np.cumsum(g.integers(-1, 2, (rows, 1)), axis=0)
+    return d % 50
+
+
+def _serpentine(rows, cols):
+    """One 1-pixel-wide path through the whole map: even rows are path (0), odd rows wall (9) with one opening, at the
+    right end and the left end in turn.  The deepest union-find trees a map of this size can give."""
+    d = np.zeros((rows, cols), np.int64)
+    d[1::2] = 9
+    for k, y in enumerate(range(1, rows, 2)):
+        d[y, cols - 1 if k % 2 == 0 else 0] = 0
+    return d
+
+
+def _comb(rows, cols):
+    """Teeth (0) on even columns that join only in the last row; odd columns (5) stay separate columns."""
+    d = np.zeros((rows, cols), np.int64)
+    d[:-1, 1::2] = 5
+    return d
+
+
+def _checker(rows, cols, max_diff):
+    y, x = np.mgrid[:rows, :cols]
+    return ((x + y) % 2) * (max_diff + 1)
+
+
+def _padded(a, pad):
+    rows, cols = a.shape
+    buf = np.full((rows, cols * a.itemsize + pad), 0x5A, np.uint8)
+    buf[:, :cols * a.itemsize] = a.view(np.uint8).reshape(rows, -1)
+    return buf
+
+
+def _device_filter(ctx, d, new_val, max_size, max_diff, pad=96):
+    """d filtered by stereo_filter_speckles_device in a row-padded device buffer; checks the padding is untouched."""
+    torch = _torch()
+    rows, cols = d.shape
+    buf = _padded(d, pad)
+    t = torch.from_numpy(buf).cuda()
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+    _ok(_capi.lib().stereo_filter_speckles_device(ctx.handle, t.data_ptr(), buf.shape[1], d.itemsize, rows, cols, new_val, max_size,
+                                                  max_diff, C.c_void_p(side.cuda_stream)), "stereo_filter_speckles_device")
+    assert ctx.last_launches == (4 if max_size > 0 else 0)
+    torch.cuda.synchronize()
+    out = t.cpu().numpy()
+    n = cols * d.itemsize
+    assert (out[:, n:] == 0x5A).all(), "row padding written"
+    return out[:, :n].copy().view(d.dtype)
+
+
+def _check_kernel(ctx, d, new_val, settings, min_changed=0.0):
+    for max_size, max_diff in settings:
+        got = _device_filter(ctx, d, new_val, max_size, max_diff)
+        want = filter_speckles(d, new_val, max_size, max_diff)
+        bad = np.argwhere(got != want)
+        assert bad.size == 0, f"{d.shape} {d.dtype} {max_size}/{max_diff}: differs at {bad[:5].tolist()} (of {len(bad)})"
+        if max_size == settings[0][0]:
+            assert np.mean(want != d) >= min_changed
+
+
+@pytest.mark.parametrize("elem", [1, 2, 4])
+@pytest.mark.parametrize("kind", ["serpentine", "comb", "checker", "whole", "blobs"])
+def test_kernel_alone_adversarial_maps(sctx, elem, kind):
+    rows, cols, nv = 150, 333, -100
+    g = np.random.default_rng(elem * 10 + len(kind))
+    d = {"serpentine": _serpentine(rows, cols), "comb": _comb(rows, cols), "checker": _checker(rows, cols, 2),
+         "whole": np.full((rows, cols), 3), "blobs": _blobs(g, rows, cols)}[kind].astype(DT[elem])
+    if kind == "blobs":
+        d[g.random((rows, cols)) < 0.05] = nv
+    big = rows * cols
+    settings = {"serpentine": [(big, 0), (big // 2, 0), (cols, 0)],      # the path (~big/2 px) goes, then stays; walls go
+                "comb": [(big // 2, 1), (big, 4), (rows, 1)],
+                "checker": [(1, 2), (1, 3), (2, 3)],                      # max_diff 2: all singletons; 3: one component
+                "whole": [(big, 0), (big - 1, 0)],
+                "blobs": [(20, 0), (100, 1), (400, 2), (0, 1)]}[kind]
+    _check_kernel(sctx, d, nv, settings)
+
+
+def test_kernel_alone_int32_near_the_limits(sctx):
+    lo, hi = np.iinfo(np.int32).min, np.iinfo(np.int32).max
+    g = np.random.default_rng(5)
+    rows, cols = 70, 90
+    d = np.where(g.random((rows, cols)) < 0.5, lo + g.integers(0, 3, (rows, cols)), hi - g.integers(0, 3, (rows, cols)))
+    d = d.astype(np.int32)
+    d[g.random((rows, cols)) < 0.1] = 0
+    # lo and hi differ by 2^32 - 1, more than any max_diff: a 32-bit difference would wrap to 1 and link them
+    _check_kernel(sctx, d, 0, [(30, 1), (30, 2), (rows * cols, 2 ** 31 - 1), (5, 2 ** 31 - 1)])
+
+
+SHAPES = [(1, 1), (1, 640), (640, 1), (7, 640), (2160, 3840), (2, 32768), (32768, 2)]
+
+
+@pytest.mark.parametrize("elem", [1, 2, 4])
+@pytest.mark.parametrize("shape", SHAPES)
+def test_kernel_alone_shapes(sctx, elem, shape):
+    rows, cols = shape
+    nv = -100
+    g = np.random.default_rng(rows * 7 + cols + elem)
+    d = _blobs(g, rows, cols).astype(DT[elem])
+    d[g.random((rows, cols)) < 0.05] = nv
+    settings = [(20, 1), (1, 0)] if rows * cols < 10 ** 6 else [(100, 1)]
+    _check_kernel(sctx, d, nv, settings, min_changed=0.001 if rows * cols > 100 else 0.0)
+
+
+def test_kernel_alone_4k_serpentine(sctx):
+    d = _serpentine(2160, 3840).astype(np.int16)
+    _check_kernel(sctx, d, -300, [(2160 * 3840 // 2 + 600, 0)], min_changed=0.4)
+
+
+def test_kernel_alone_argument_checks(sctx):
+    torch = _torch()
+    buf = torch.zeros((4, 256), dtype=torch.uint8, device="cuda")
+    a = buf.data_ptr()
+    lib = _capi.lib()
+
+    def call(p=a, step=256, elem=2, rows=4, cols=64, nv=-11, max_size=5, max_diff=1, ctx=sctx.handle):
+        return lib.stereo_filter_speckles_device(ctx, p, step, elem, rows, cols, nv, max_size, max_diff, None)
+
+    assert call() == _capi.STEREO_OK and call(max_size=0) == _capi.STEREO_OK
+    assert sctx.last_launches == 0
+    assert call(p=None) == ARG and call(ctx=None) == ARG
+    assert call(rows=0) == ARG and call(cols=0) == ARG and call(rows=-1) == ARG
+    assert call(rows=32769) == UNSUP and call(cols=32769, step=32769 * 2) == UNSUP
+    assert call(elem=3) == ARG and call(step=127) == ARG
+    assert call(max_size=-1) == ARG and call(max_diff=-1) == ARG
+    assert call(elem=1, nv=-129) == ARG and call(elem=1, nv=128) == ARG and call(elem=2, nv=32768) == ARG
+    assert call(elem=1, nv=-128) == _capi.STEREO_OK and call(elem=2, nv=-32768) == _capi.STEREO_OK
+    assert call(elem=4, nv=-2 ** 31) == _capi.STEREO_OK
+    sctx.synchronize()
+
+
+# ---- 2. every pair entry point ---------------------------------------------------------------------------------------
+
+ENTRIES = ["pair_host", "pair_device", "batch_device", "batch_host", "band_host", "band_halo_device", "mgpu_batch"]
+
+
+def _run_whole(h, entry, cost, Ls, Rs, win, rng, dt):
+    """_run, with the band entry points called once for the whole image."""
+    if entry not in ("band_host", "band_halo_device"):
+        return _run(h, entry, cost, Ls, Rs, win, rng, dt)
+    lib = _capi.lib()
+    n, rows, cols = Ls.shape
+    dt = np.dtype(dt)
+    elem = dt.itemsize
+    out_l, out_r = np.empty((n, rows, cols), dt), np.empty((n, rows, cols), dt)
+    for i in range(n):
+        L, R = np.ascontiguousarray(Ls[i]), np.ascontiguousarray(Rs[i])
+        if entry == "band_host":
+            fn = lib.stereo_disparity_pair_band_f32_host if L.dtype == np.float32 else lib.stereo_disparity_pair_band_u8_host
+            _ok(fn(h.handle, cost, L.ctypes.data, L.strides[0], R.ctypes.data, R.strides[0], rows, cols, 0, rows, win, rng,
+                   out_l[i].ctypes.data, out_r[i].ctypes.data, cols * elem, elem), entry)
+        else:
+            torch = _torch()
+            tl, tr = torch.from_numpy(L).cuda(), torch.from_numpy(R).cuda()
+            ol = torch.empty((rows, cols), dtype={1: torch.int8, 2: torch.int16, 4: torch.int32}[elem], device="cuda")
+            orr = torch.empty_like(ol)
+            _ok(lib.stereo_disparity_pair_band_halo_u8_device(h.handle, cost, tl.data_ptr(), cols, tr.data_ptr(), cols, rows, cols, 0, rows,
+                                                              0, rows, win, rng, ol.data_ptr(), orr.data_ptr(), cols * elem, elem,
+                                                              C.c_void_p(torch.cuda.current_stream().cuda_stream)), entry)
+            torch.cuda.synchronize()
+            out_l[i], out_r[i] = ol.cpu().numpy(), orr.cpu().numpy()
+    return out_l, out_r
+
+
+def _filtered_equals_oracle_of_off(h, entry, cost, Ls, Rs, win, rng, dt, lr, max_size=MAX_SIZE, max_diff=MAX_DIFF, min_share=0.001):
+    try:
+        h.set_lr_check(None)
+        h.set_speckle_filter(None)
+        off = _run_whole(h, entry, cost, Ls, Rs, win, rng, dt)
+        h.set_lr_check(1 if lr else None)
+        h.set_speckle_filter(max_size, max_diff)
+        on = _run_whole(h, entry, cost, Ls, Rs, win, rng, dt)
+    finally:
+        h.set_lr_check(None)
+        h.set_speckle_filter(None)
+    nv = -(rng + 1)
+    changed = 0
+    for i in range(len(Ls)):
+        base = lr_check(off[0][i], off[1][i], rng, 1) if lr else (off[0][i], off[1][i])
+        for side in (0, 1):
+            want = filter_speckles(base[side], nv, max_size, max_diff)
+            bad = np.argwhere(on[side][i] != want)
+            assert bad.size == 0, f"{entry} pair {i} map {side}: differs at {bad[:5].tolist()} (of {len(bad)})"
+            changed += int(np.sum(want != base[side]))
+    share = changed / (2 * Ls.size)
+    assert changed > 0 and min_share <= share < 0.9, f"the filter changed {changed} pixels, {share:.4f} of them"
+    return off, on
+
+
+@pytest.mark.parametrize("lr", [False, True])
+@pytest.mark.parametrize("family", list(FAMILIES))
+@pytest.mark.parametrize("fuse", [True, False])
+@pytest.mark.parametrize("cost", [sb.COST_SSD, sb.COST_NCORR])
+@pytest.mark.parametrize("entry", ENTRIES)
+def test_every_pair_entry_point_equals_the_oracle_filter(sctx, mg, entry, cost, fuse, family, lr):
+    kind, win, dt = FAMILIES[family]
+    if kind != "u8" and entry in ("batch_device", "band_halo_device"):
+        pytest.skip("8-bit device entry point")
+    if kind == "noisy" and entry == "band_host":
+        pytest.skip("the host row-band entry points take 8-bit-valued images only")
+    h = mg if entry.startswith("mgpu_") else sctx
+    n = 5 if "batch" in entry else 1
+    Ls, Rs = _images(kind, n, 500 + 7 * ENTRIES.index(entry))
+    _set_fuse(h, fuse)
+    try:
+        # (the 17 x 17 window of the exact family leaves smooth maps: after the left-right check a few pixels at most)
+        _filtered_equals_oracle_of_off(h, entry, cost, Ls, Rs, win, RANGE_T, dt, lr, min_share=0.0 if family == "exact" else 0.001)
+    finally:
+        _set_fuse(h, True)
+
+
+@pytest.mark.parametrize("bands", [0, 3])
+@pytest.mark.parametrize("kind", ["u8", "f32"])
+def test_host_pipeline_items_and_bands(sctx, bands, kind):
+    Ls, Rs = _images(kind, 7, 901)
+    sctx.set_pipe_bands(bands)
+    try:
+        for cost in (sb.COST_SSD, sb.COST_NCORR):
+            for lr in (False, True):
+                _filtered_equals_oracle_of_off(sctx, "batch_host", cost, Ls, Rs, 3, RANGE_T, np.int16, lr, 30, 0)
+    finally:
+        sctx.set_pipe_bands(0)
+
+
+def test_launches_of_a_filtered_pair_call(sctx):
+    Ls, Rs = _images("u8", 1, 41)
+    sctx.set_speckle_filter(None)
+    _run(sctx, "pair_device", sb.COST_SSD, Ls, Rs, 3, RANGE_T, np.int16)
+    off = sctx.last_launches
+    sctx.set_speckle_filter(MAX_SIZE, MAX_DIFF)
+    try:
+        _run(sctx, "pair_device", sb.COST_SSD, Ls, Rs, 3, RANGE_T, np.int16)
+        assert sctx.last_launches == off + 4
+    finally:
+        sctx.set_speckle_filter(None)
+
+
+# ---- 3. / 4. full-size batches ---------------------------------------------------------------------------------------
+
+def _device_batch(ctx, Ls, Rs, win, rng, elem):
+    torch = _torch()
+    n, rows, cols = Ls.shape
+    tl, tr = torch.from_numpy(Ls).cuda(), torch.from_numpy(Rs).cuda()
+    out = torch.empty((2, n, rows, cols), dtype={1: torch.int8, 2: torch.int16}[elem], device="cuda")
+    _ok(_capi.lib().stereo_disparity_pair_batch_u8_device(ctx.handle, sb.COST_SSD, n, tl.data_ptr(), tr.data_ptr(), cols, rows * cols,
+                                                          rows, cols, win, rng, out[0].data_ptr(), out[1].data_ptr(), cols * elem,
+                                                          rows * cols * elem, elem, C.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    torch.cuda.synchronize()
+    return out.cpu().numpy()
+
+
+@pytest.mark.parametrize("shape,nd,win,n,elem", [((720, 1280), 64, 4, 16, 1), ((2160, 3840), 256, 5, 1, 2)])
+def test_full_size_batch_equals_the_oracle(sctx, shape, nd, win, n, elem):
+    rows, cols = shape
+    rng = nd - 1
+    pairs = [synth.make_pair(rows, cols, nd, 60 + i)[:2] for i in range(min(n, 4))]
+    Ls = np.stack([pairs[i % len(pairs)][0] for i in range(n)])
+    Rs = np.stack([pairs[i % len(pairs)][1] for i in range(n)])
+    sctx.set_speckle_filter(None)
+    off = _device_batch(sctx, Ls, Rs, win, rng, elem)
+    sctx.set_speckle_filter(100, 1)
+    try:
+        on = _device_batch(sctx, Ls, Rs, win, rng, elem)
+        launches = sctx.last_launches
+    finally:
+        sctx.set_speckle_filter(None)
+    cache = {}
+    for side in (0, 1):
+        for i in range(n):
+            key = (side, i % len(pairs))
+            if key not in cache:
+                cache[key] = filter_speckles(off[side, i], -(rng + 1), 100, 1)
+            assert np.array_equal(on[side, i], cache[key]), (side, i)
+    assert np.mean(on != off) > 0.002
+    if n == 16:
+        _device_batch(sctx, Ls, Rs, win, rng, elem)
+        assert launches == sctx.last_launches + 4    # every map of the 16 pairs in one set of filter launches
+
+
+# ---- 5. rejections, default and off ----------------------------------------------------------------------------------
+
+def _fill(dev, shape, value):
+    torch = _torch()
+    a = np.full(shape, value, np.uint8)
+    return torch.from_numpy(a).cuda() if dev else a
+
+
+def test_partial_bands_are_rejected_and_write_nothing(sctx, mg):
+    torch = _torch()
+    lib = _capi.lib()
+    rows, cols, win, rng = 48, 96, 3, 16
+    L, Rt, _ = synth.make_pair(rows, cols, rng + 4, 88)
+    Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
+    sctx.set_speckle_filter(MAX_SIZE, MAX_DIFF)
+    mg.set_speckle_filter(MAX_SIZE, MAX_DIFF)
+    try:
+        for r0, r1 in ((0, 24), (24, 48), (10, 20)):
+            for fn, a, b in ((lib.stereo_disparity_pair_band_u8_host, L, Rt), (lib.stereo_disparity_pair_band_f32_host, Lf, Rf)):
+                ol, orr = _fill(False, (rows, cols * 2), 0x3C), _fill(False, (rows, cols * 2), 0x3C)
+                rc = fn(sctx.handle, sb.COST_SSD, a.ctypes.data, a.strides[0], b.ctypes.data, b.strides[0], rows, cols, r0, r1, win, rng,
+                        ol[r0:].ctypes.data, orr[r0:].ctypes.data, cols * 2, 2)
+                assert rc == UNSUP, (fn.__name__, r0, r1, rc)
+                assert (ol == 0x3C).all() and (orr == 0x3C).all()
+            h0, h1 = C.c_int(), C.c_int()
+            _ok(lib.stereo_band_halo_rows(rows, r0, r1, win, C.byref(h0), C.byref(h1)))
+            tl, tr = torch.from_numpy(L).cuda(), torch.from_numpy(Rt).cuda()
+            ol, orr = _fill(True, (rows, cols * 2), 0x3C), _fill(True, (rows, cols * 2), 0x3C)
+            rc = lib.stereo_disparity_pair_band_halo_u8_device(sctx.handle, sb.COST_SSD, tl[h0.value].data_ptr(), cols, tr[h0.value].data_ptr(),
+                                                               cols, rows, cols, r0, r1, h0.value, h1.value, win, rng, ol[r0].data_ptr(),
+                                                               orr[r0].data_ptr(), cols * 2, 2, None)
+            torch.cuda.synchronize()
+            assert rc == UNSUP, ("band_halo", r0, r1, rc)
+            assert (ol == 0x3C).all().item() and (orr == 0x3C).all().item()
+        for fn, a, b in ((lib.stereo_mgpu_disparity_pair_bands_u8_host, L, Rt), (lib.stereo_mgpu_disparity_pair_bands_f32_host, Lf, Rf),
+                         # float images that are not 8-bit: no whole-pair call stands in for the refused bands either
+                         (lib.stereo_mgpu_disparity_pair_bands_f32_host, synth.noisy_variant(L, 1), synth.noisy_variant(Rt, 2))):
+            ol, orr = _fill(False, (rows, cols * 2), 0x3C), _fill(False, (rows, cols * 2), 0x3C)
+            rc = fn(mg._h, sb.COST_SSD, a.ctypes.data, a.strides[0], b.ctypes.data, b.strides[0], rows, cols, win, rng,
+                    ol.ctypes.data, orr.ctypes.data, cols * 2, 2)
+            assert rc == UNSUP, (fn.__name__, rc)
+            assert (ol == 0x3C).all() and (orr == 0x3C).all()
+    finally:
+        sctx.set_speckle_filter(None)
+        mg.set_speckle_filter(None)
+    # off again: the same partial band is computed
+    ol = np.zeros((rows, cols), np.int16)
+    orr = np.zeros((rows, cols), np.int16)
+    _ok(lib.stereo_disparity_pair_band_u8_host(sctx.handle, sb.COST_SSD, L.ctypes.data, cols, Rt.ctypes.data, cols, rows, cols, 10, 20,
+                                               win, rng, ol[10:].ctypes.data, orr[10:].ctypes.data, cols * 2, 2))
+    dl, dr = mg.disparity_pair_bands(sb.COST_SSD, L, Rt, win, rng, dtype=np.int16)
+    assert dl.shape == (rows, cols)
+
+
+PAIR_ENTRY_POINTS = [n for n in EXPECTED if n.startswith("stereo_disparity_pair_")]
+MGPU_ENTRY_POINTS = {"stereo_mgpu_disparity_pair_batch_u8_host": "stereo_disparity_pair_batch_u8_host",
+                     "stereo_mgpu_disparity_pair_batch_f32_host": "stereo_disparity_pair_batch_f32_host"}
+
+
+@pytest.mark.parametrize("elem,rng", [(1, 128), (2, 32768)])
+@pytest.mark.parametrize("name", PAIR_ENTRY_POINTS + list(MGPU_ENTRY_POINTS))
+def test_sentinel_that_does_not_fit_is_rejected_with_the_filter_alone(sctx, mg, name, elem, rng):
+    torch = _torch()
+    h = mg if name.startswith("stereo_mgpu_") else sctx
+    as_name = MGPU_ENTRY_POINTS.get(name, name)
+    dev = as_name.endswith("_device")
+    imgs = [_fill(dev, (2, ROWS, PITCH), 0) for _ in range(2)]
+    outs = [_fill(dev, (2, ROWS, PITCH), 0x3C) for _ in range(2)]
+    ptrs = [t.data_ptr() for t in imgs + outs] if dev else [a.ctypes.data for a in imgs + outs]
+    handle = h._h if isinstance(h, sb.MultiGpu) else h.handle
+    fn = getattr(_capi.lib(), name)
+    # (the band entry points are called with a band of the whole image here: the sentinel alone rejects them)
+    args = _args(as_name, handle, ptrs, rng=rng, elem=elem)
+    if "band" in as_name:
+        args = _whole_band_args(as_name, args)
+    h.set_speckle_filter(MAX_SIZE, MAX_DIFF)
+    try:
+        rc = fn(*args)
+        torch.cuda.synchronize()
+        assert rc == UNSUP, f"{name}: {rc} ({_capi.last_error()})"
+        assert "sentinel" in _capi.last_error()
+        for o in outs:
+            a = o.cpu().numpy() if dev else o
+            assert (a == 0x3C).all(), f"{name} wrote its outputs"
+    finally:
+        h.set_speckle_filter(None)
+    _ok(fn(*args), name)
+    torch.cuda.synchronize()
+
+
+def _whole_band_args(name, args):
+    """test_entry_points._args of a band entry point, with the band [4, 12) widened to the whole image [0, ROWS)."""
+    a = list(args)
+    i = a.index(4)
+    assert a[i + 1] == 12
+    a[i], a[i + 1] = 0, ROWS
+    if name == "stereo_disparity_pair_band_halo_u8_device":
+        a[i + 2], a[i + 3] = 0, ROWS
+    return a
+
+
+def test_setter_checks_and_default_state(sctx, mg):
+    lib = _capi.lib()
+    fresh = sb.Context(0)
+    try:
+        assert fresh.speckle_filter is None
+        assert lib.stereo_ctx_set_speckle_filter(None, 5, 1) == ARG
+        assert lib.stereo_mgpu_set_speckle_filter(None, 5, 1) == ARG
+        assert lib.stereo_ctx_set_speckle_filter(fresh.handle, 5, -1) == ARG
+        assert fresh.speckle_filter is None
+        _ok(lib.stereo_ctx_set_speckle_filter(fresh.handle, 0, -1))          # off: max_diff does not matter
+        _ok(lib.stereo_ctx_set_speckle_filter(fresh.handle, -3, 7))
+        assert fresh.speckle_filter is None
+        fresh.set_speckle_filter(40, 2)
+        assert fresh.speckle_filter == (40, 2)
+        fresh.set_speckle_filter(7)
+        assert fresh.speckle_filter == (7, 1)
+        fresh.set_speckle_filter(None)
+        assert fresh.speckle_filter is None
+        with pytest.raises(sb.StereoError):
+            fresh.set_speckle_filter(10, -1)
+        with pytest.raises(sb.StereoError):
+            mg.set_speckle_filter(10, -1)
+        size, diff = C.c_int(), C.c_int()
+        assert lib.stereo_ctx_speckle_filter(None, C.byref(size), C.byref(diff)) == ARG
+        mg.set_speckle_filter(9, 0)
+        for i in range(mg.device_count):
+            _ok(lib.stereo_ctx_speckle_filter(lib.stereo_mgpu_ctx(mg._h, i), C.byref(size), C.byref(diff)))
+            assert (size.value, diff.value) == (9, 0)
+        mg.set_speckle_filter(None)
+    finally:
+        fresh.close()
+        mg.set_speckle_filter(None)
+
+
+def test_off_again_is_byte_identical_to_a_fresh_context(sctx):
+    Ls, Rs = _images("u8", 3, 78)
+    fresh = sb.Context(0)
+    try:
+        for entry in ("pair_host", "pair_device", "batch_device", "batch_host"):
+            for cost in (sb.COST_SSD, sb.COST_NCORR):
+                want = _run(fresh, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
+                sctx.set_speckle_filter(MAX_SIZE, MAX_DIFF)
+                on = _run(sctx, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
+                sctx.set_speckle_filter(0)
+                assert sctx.speckle_filter is None
+                got = _run(sctx, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
+                assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1]), (entry, cost)
+                assert (on[0] != want[0]).any()
+    finally:
+        fresh.close()
+        sctx.set_speckle_filter(None)
+
+
+def test_single_direction_and_refgpu_calls_ignore_the_filter(sctx):
+    L, Rt, _ = synth.make_pair(48, 160, 24, 516)
+    Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
+
+    def singles(c):
+        return [c.disparity(sb.COST_SSD, Lf, Rf, 3, -20, 0, dtype=np.int16), c.disparity(sb.COST_NCORR, L, Rt, 3, 0, 20),
+                c.disparity_refgpu(sb.COST_SSD, Lf, Rf, 3, -20, 0)]
+
+    fresh = sb.Context(0)
+    try:
+        want = singles(fresh)
+        sctx.set_speckle_filter(1000, 3)
+        got = singles(sctx)
+    finally:
+        fresh.close()
+        sctx.set_speckle_filter(None)
+    for a, b in zip(got, want):
+        assert np.array_equal(a, b)
+
+
+# ---- 6. graph capture -------------------------------------------------------------------------------------------------
+
+def test_device_pair_call_with_the_filter_replays_in_a_cuda_graph(sctx):
+    torch = _torch()
+    rows, cols, win, rng = 120, 256, 3, 30
+    inputs = [synth.make_pair(rows, cols, rng + 4, 3030 + k)[:2] for k in range(3)]
+    s = torch.cuda.Stream()
+    tl = torch.from_numpy(inputs[0][0]).cuda()
+    tr = torch.from_numpy(inputs[0][1]).cuda()
+    out = torch.full((2, rows, cols), 99, dtype=torch.int16, device="cuda")
+    s.wait_stream(torch.cuda.current_stream())
+
+    def call(c):
+        _ok(_capi.lib().stereo_disparity_pair_u8_device(c.handle, sb.COST_SSD, tl.data_ptr(), cols, tr.data_ptr(), cols, rows, cols, win,
+                                                        rng, out[0].data_ptr(), out[1].data_ptr(), cols * 2, 2, C.c_void_p(s.cuda_stream)))
+
+    offc = sb.Context(0)
+    try:
+        sctx.set_speckle_filter(MAX_SIZE, MAX_DIFF)
+        with torch.cuda.stream(s):
+            call(sctx)                                  # warm-up: sizes the scratch arena
+        s.synchronize()
+        g = torch.cuda.CUDAGraph()
+        out.fill_(99)
+        torch.cuda.synchronize()
+        with torch.cuda.graph(g, stream=s, capture_error_mode="thread_local"):
+            call(sctx)
+        assert (out == 99).all().item()                 # captured, not run
+        for L, Rt in inputs[1:]:
+            tl.copy_(torch.from_numpy(L))
+            tr.copy_(torch.from_numpy(Rt))
+            torch.cuda.synchronize()
+            g.replay()
+            torch.cuda.synchronize()
+            got = out.cpu().numpy()
+            off_l, off_r = offc.disparity_pair(sb.COST_SSD, L, Rt, win, rng, dtype=np.int16)
+            want_l = filter_speckles(off_l, -(rng + 1), MAX_SIZE, MAX_DIFF)
+            want_r = filter_speckles(off_r, -(rng + 1), MAX_SIZE, MAX_DIFF)
+            assert np.array_equal(got[0], want_l) and np.array_equal(got[1], want_r)
+            assert (want_l != off_l).any()
+    finally:
+        offc.close()
+        sctx.set_speckle_filter(None)
