@@ -74,7 +74,10 @@ typedef enum stereo_path {
     STEREO_PATH_FAST_U8 = 2,    /* integer-valued 0..255 inputs: packed dot-product running sums */
     STEREO_PATH_REFGPU = 4,     /* stereo_disparity_refgpu_*: the function the reference's GPU kernels compute (SURVEY.md A.3) */
     STEREO_PATH_FAST_F32 = 3    /* general float inputs of bounded range (noise / contrast variants, main.cpp:140-153,191-193):
-                                   per-element round((l-r)^2) as exact int32 running sums (SSD), float32 running sums (NCC) */
+                                   per-element round((l-r)^2) as exact int32 running sums (SSD), float32 running sums (NCC).
+                                   Bounds: SSD keys 128*SSD + position < 2^32 and (l-r)^2 < 2^23; NCC |v| < 1e6 and, when
+                                   every value has one sign, (hi-lo)^2 / (lo^2 + hi^2) >= 2^-4 - a larger DC offset crowds
+                                   every score towards 1 below the keys' ~2^-16 resolution (DESIGN.md §4.5) */
 } stereo_path;
 
 typedef struct stereo_ctx stereo_ctx;

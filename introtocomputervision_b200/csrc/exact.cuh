@@ -160,8 +160,10 @@ __global__ void classify_convert_kernel(const float* __restrict__ img0, size_t s
     }
     if (__syncthreads_or(bad)) {
         __shared__ unsigned smax[2][8];
-        const float vv = nonfinite ? 0.f : v;
-        const unsigned hi = __reduce_max_sync(0xffffffffu, f32_ordered(vv)), lo = __reduce_max_sync(0xffffffffu, f32_ordered(-vv));
+        // threads outside the image and non-finite pixels track nothing: the range is that of the block's finite pixels
+        const bool track = x < cols && y < rows && !nonfinite;
+        const unsigned hi = __reduce_max_sync(0xffffffffu, track ? f32_ordered(v) : 0u);
+        const unsigned lo = __reduce_max_sync(0xffffffffu, track ? f32_ordered(-v) : 0u);
         const int tid = threadIdx.y * blockDim.x + threadIdx.x, warp = tid >> 5;
         if ((tid & 31) == 0) { smax[0][warp] = lo; smax[1][warp] = hi; }
         const int anynf = __syncthreads_or(nonfinite);
