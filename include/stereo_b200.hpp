@@ -186,6 +186,12 @@ inline void setSpeckleFilter(int maxSize, int maxDiff, stereo_ctx* ctx = nullptr
     check(stereo_ctx_set_speckle_filter(ctx ? ctx : default_ctx(), maxSize, maxDiff), "stereo_ctx_set_speckle_filter");
 }
 
+// Semi-global matching of the SSD pair calls on `ctx` (default: the default context): paths 4 or 8 switch it on, 0 off
+// (stereo_ctx_set_sgm).
+inline void setSgm(int paths, int p1 = 0, int p2 = 0, stereo_ctx* ctx = nullptr) {
+    check(stereo_ctx_set_sgm(ctx ? ctx : default_ctx(), paths, p1, p2), "stereo_ctx_set_sgm");
+}
+
 // Kernel time of the last call on the default context, the quantity the reference logs as
 // "disparitySSDKernel execution took {} ms" (DisparitySSD.cu:203).
 inline float lastKernelMs() { return stereo_ctx_last_kernel_ms(default_ctx()); }
@@ -234,6 +240,7 @@ public:
     void setSpeckleFilter(int maxSize, int maxDiff) {
         check(stereo_mgpu_set_speckle_filter(mg_, maxSize, maxDiff), "stereo_mgpu_set_speckle_filter");
     }
+    void setSgm(int paths, int p1 = 0, int p2 = 0) { check(stereo_mgpu_set_sgm(mg_, paths, p1, p2), "stereo_mgpu_set_sgm"); }
 
     // disparitySSDPair / disparityNCorrPair (main.cpp:21-78) with the output rows sharded over the devices
     void disparityPairBands(int cost, const MatT& left, const MatT& right, size_t windowRad, int disparityRange, MatT& disparityLeft,

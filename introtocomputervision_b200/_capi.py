@@ -16,7 +16,7 @@ LIB_PATH = Path(os.environ.get("STEREO_B200_LIB") or
 STEREO_OK = 0
 ERR_INVALID_ARG, ERR_INVALID_RANGE, ERR_NO_DEVICE, ERR_CUDA, ERR_ALLOC, ERR_UNSUPPORTED = -1, -2, -3, -4, -5, -6
 COST_SSD, COST_NCORR = 0, 1
-PATH_NONE, PATH_EXACT_F32, PATH_FAST_U8, PATH_FAST_F32, PATH_REFGPU = 0, 1, 2, 3, 4
+PATH_NONE, PATH_EXACT_F32, PATH_FAST_U8, PATH_FAST_F32, PATH_REFGPU, PATH_SGM = 0, 1, 2, 3, 4, 5
 
 _vp, _sz, _i = C.c_void_p, C.c_size_t, C.c_int
 
@@ -55,6 +55,9 @@ SIGNATURES = {
     "stereo_ctx_speckle_filter": (_i, [_vp, C.POINTER(_i), C.POINTER(_i)]),
     "stereo_filter_speckles_device": (_i, [_vp, _vp, _sz, _i, _i, _i, _i, _i, _i, _vp]),
     "stereo_mgpu_set_speckle_filter": (_i, [_vp, _i, _i]),
+    "stereo_ctx_set_sgm": (_i, [_vp, _i, _i, _i]),
+    "stereo_ctx_sgm": (_i, [_vp, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i)]),
+    "stereo_mgpu_set_sgm": (_i, [_vp, _i, _i, _i]),
     "stereo_ctx_synchronize": (_i, [_vp, _vp]),
     "stereo_disparity_f32_host": (_i, _SINGLE_HOST),
     "stereo_disparity_u8_host": (_i, _SINGLE_HOST),

@@ -84,6 +84,12 @@ int pair_bands(stereo_mgpu* mg, int cost, const T* left, size_t left_step, const
             return STEREO_ERR_UNSUPPORTED;
         }
     }
+    // SGM paths cross band seams: no band is aggregated on its own
+    for (stereo_ctx* c : mg->ctx) {
+        int paths = 0, p1 = 0, p2 = 0;
+        stereo_ctx_sgm(c, &paths, &p1, &p2);
+        if (paths > 0) { sb::set_error("SGM on: row-band sharded pairs are not aggregated (shard whole pairs)"); return STEREO_ERR_UNSUPPORTED; }
+    }
     int parts = int(mg->ctx.size());
     const int band = (rows + parts - 1) / parts;            // equal bands of ceil(rows / parts) rows, the last one(s) shorter or empty
     int rc = for_each_device(mg, [&](int k) -> int {
@@ -163,6 +169,15 @@ int stereo_mgpu_set_speckle_filter(stereo_mgpu* mg, int max_size, int max_diff) 
     if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
     for (stereo_ctx* c : mg->ctx) {
         const int rc = stereo_ctx_set_speckle_filter(c, max_size, max_diff);
+        if (rc != STEREO_OK) return rc;
+    }
+    return STEREO_OK;
+}
+
+int stereo_mgpu_set_sgm(stereo_mgpu* mg, int paths, int p1, int p2) {
+    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
+    for (stereo_ctx* c : mg->ctx) {
+        const int rc = stereo_ctx_set_sgm(c, paths, p1, p2);
         if (rc != STEREO_OK) return rc;
     }
     return STEREO_OK;

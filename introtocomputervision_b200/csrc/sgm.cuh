@@ -1,0 +1,178 @@
+// Semi-global matching (path aggregation of the SSD cost along scanlines) for one direction of a pair.
+//   C(y, x, d)  the reference's SSD window sum of candidate d (exact.cuh's ssd_elem per element, the flat-index row-wrap
+//               reads included), for the present candidates: those with s = x + R + d in [0, Wp - 1].
+//   L_r(p, d) = C(p, d) + min(L_r(q, d), L_r(q, d -+ 1) + P1, m(q) + P2) - m(q),  q = p - r,  m(q) = min_e L_r(q, e);
+//               L_r(p, d) = C(p, d) where q lies outside the image.  Terms of candidates absent at q are left out.
+//   S(p, d)   = sum over the 4 or 8 paths r of L_r(p, d);  disparity = the first minimum of S over the present candidates.
+// Launches per direction: two replicate pads (exact.cuh), sgm_cost_kernel, then one sgm_path_kernel per path in stream
+// order; the first path writes S, the later ones read-add-write it, the last one also writes the winner-take-all map.
+// Layout: candidate index j = d - dlo innermost, padded to Dp = 32 K (K candidates per lane of the path kernels).  Absent
+// and padding candidates hold SGM_ABSENT in C and L; S of an absent candidate is 0xFFFFFFFF, above every present sum as
+// an unsigned value.  With paths * (C_max + P2) <= 2^31 - 1 (checked by the caller), every present L is below 2^29, m(q)
+// + P2 below 2^30 = SGM_ABSENT, and SGM_ABSENT + P1 below 2^31: absent terms never win a minimum and nothing overflows.
+#pragma once
+#include "common.cuh"
+#include "exact.cuh"
+
+namespace sb {
+
+constexpr int SGM_ABSENT = 1 << 30;
+constexpr int SGM_MAXK = 16;               // candidates per lane (one instantiation each): at most 512 per pixel
+constexpr int SGM_XT = 256;                // output columns of one cost block
+constexpr int SGM_COST_THREADS = 256;      // 8 warps, SGM_XT / 8 consecutive columns each
+constexpr int SGM_PATH_WARPS = 4;          // scanlines (one warp each) per path block
+
+// C for output rows [y0, y0 + rows_per_block) x columns [x0, x0 + SGM_XT) x candidates [j0, j0 + 32) of one block.
+// Vertical window sums V(c, d) of the element image E(r, c, d) = ssd_elem(Lp[r][c], Rp_flat[r Wp + c + d]) are kept in
+// shared memory for the block's columns and slide down one row at a time (E is recomputed for the row that leaves);
+// each warp then slides the horizontal window along its 32 columns with the candidate in the lane, so every row of C is
+// written as 128-byte lines.  Reads outside [-R, Hp Wp + R) - only ever of absent or padding candidates - count as 0.
+__global__ void __launch_bounds__(SGM_COST_THREADS)
+sgm_cost_kernel(const float* __restrict__ Lp, const float* __restrict__ Rp, int rows, int cols, int R, int dlo, int D, int Dp,
+                int rows_per_block, int32_t* __restrict__ C) {
+    extern __shared__ int32_t V[];                       // [(SGM_XT + 2R) columns][32 candidates]
+    const int Wp = cols + 2 * R, w = 2 * R + 1, nc = SGM_XT + 2 * R;
+    const long long flat_lo = -R, flat_hi = (long long)(rows + 2 * R) * Wp + R;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int x0 = blockIdx.x * SGM_XT, y0 = blockIdx.y * rows_per_block, j = blockIdx.z * 32 + lane;
+    const int d = dlo + j;
+    const int y1 = min(rows, y0 + rows_per_block);
+    auto E = [&](int r, int c) -> int {                  // r, c: padded coordinates
+        const long long f = (long long)r * Wp + c + d;
+        if (c >= Wp || f < flat_lo || f >= flat_hi) return 0;
+        return ssd_elem(__ldg(Lp + (long long)r * Wp + c), __ldg(Rp + f));
+    };
+    for (int ci = warp; ci < nc; ci += SGM_COST_THREADS / 32) {
+        int v = 0;
+        for (int r = y0; r < y0 + w; ++r) v += E(r, x0 + ci);
+        V[ci * 32 + lane] = v;
+    }
+    constexpr int SEG = SGM_XT / (SGM_COST_THREADS / 32);
+    const int xs = x0 + warp * SEG;
+    for (int y = y0;;) {
+        __syncthreads();
+        if (xs < cols) {
+            int h = 0;
+            for (int k = 0; k < w; ++k) h += V[(warp * SEG + k) * 32 + lane];
+            int32_t* out = C + ((size_t)y * cols + xs) * Dp + j;
+            const int xe = min(cols, xs + SEG);
+            for (int x = xs; x < xe; ++x, out += Dp) {
+                const int s = x + R + d;
+                *out = (j < D && s >= 0 && s < Wp) ? h : SGM_ABSENT;
+                const int ci = x - x0;
+                if (x + 1 < xe) h += V[(ci + w) * 32 + lane] - V[ci * 32 + lane];
+            }
+        }
+        if (++y >= y1) break;
+        __syncthreads();
+        for (int ci = warp; ci < nc; ci += SGM_COST_THREADS / 32)
+            V[ci * 32 + lane] += E(y - 1 + w, x0 + ci) - E(y - 1, x0 + ci);
+    }
+}
+
+// Scanlines of direction (dy, dx): every pixel whose predecessor p - r lies outside the image starts one.
+__host__ __device__ inline int sgm_lines(int rows, int cols, int dy, int dx) {
+    return (dy ? cols : 0) + (dx ? (dy ? rows - 1 : rows) : 0);
+}
+
+struct SgmOut { void* ptr; size_t step; int elem; int dlo; };    // the map the last path writes (ptr == nullptr: none)
+
+// One path direction, one warp per scanline, lane l holding candidates [l K, l K + K) (Dp = 32 K).  The previous pixel's L_r stays in
+// registers; d -+ 1 across lanes come through shuffles and m(q) is one warp minimum.  first: S = L; otherwise S += L.
+// With out.ptr, the winner-take-all of the final S (first minimum, unsigned) is stored in out's element type.
+template <int K>
+__global__ void __launch_bounds__(SGM_PATH_WARPS * 32)
+sgm_path_kernel(const int32_t* __restrict__ C, int32_t* __restrict__ S, int rows, int cols, int dy, int dx, int P1, int P2,
+                int first, SgmOut out) {
+    constexpr int Dp = 32 * K;
+    const int lane = threadIdx.x & 31;
+    const int line = blockIdx.x * SGM_PATH_WARPS + (threadIdx.x >> 5);
+    if (line >= sgm_lines(rows, cols, dy, dx)) return;
+    int y, x;
+    if (dy && line < cols) { y = dy > 0 ? 0 : rows - 1; x = line; }
+    else {
+        const int t = dy ? line - cols : line;
+        x = dx > 0 ? 0 : cols - 1;
+        y = (dy > 0) ? t + 1 : t;
+    }
+    const int steps = min(dy > 0 ? rows - y : dy < 0 ? y + 1 : 0x7FFFFFFF, dx > 0 ? cols - x : dx < 0 ? x + 1 : 0x7FFFFFFF);
+    const long long stride = ((long long)dy * cols + dx) * Dp;
+    long long base = ((long long)y * cols + x) * Dp + lane * K;
+    // C and S of the next PF pixels are in flight while this one is computed (S of a pixel is only ever touched by the one
+    // warp whose scanline crosses it, and by earlier launches)
+    constexpr int PF = K <= 3 ? 4 : K <= 8 ? 2 : 1;
+    int Lq[K], cq[PF][K], sq[PF][K];
+#pragma unroll
+    for (int u = 0; u < PF; ++u)
+#pragma unroll
+        for (int i = 0; i < K; ++i) {
+            cq[u][i] = u < steps ? __ldg(C + base + u * stride + i) : SGM_ABSENT;
+            sq[u][i] = u < steps && !first ? S[base + u * stride + i] : 0;
+        }
+#pragma unroll
+    for (int i = 0; i < K; ++i) Lq[i] = SGM_ABSENT;
+    int mq = 0;
+    for (int s0 = 0; s0 < steps; s0 += PF) {
+#pragma unroll
+    for (int u = 0; u < PF; ++u) {
+        const int st = s0 + u;
+        if (st >= steps) break;
+        int c[K], so[K];
+#pragma unroll
+        for (int i = 0; i < K; ++i) { c[i] = cq[u][i]; so[i] = sq[u][i]; }
+        if (st + PF < steps) {
+#pragma unroll
+            for (int i = 0; i < K; ++i) {
+                cq[u][i] = __ldg(C + base + PF * stride + i);
+                sq[u][i] = first ? 0 : S[base + PF * stride + i];
+            }
+        }
+        // neighbours across lanes: the last candidate of lane - 1 and the first of lane + 1
+        int lm = __shfl_up_sync(0xffffffffu, Lq[K - 1], 1);
+        int rp = __shfl_down_sync(0xffffffffu, Lq[0], 1);
+        if (lane == 0) lm = SGM_ABSENT;
+        if (lane == 31) rp = SGM_ABSENT;
+        int L[K];
+        int lmin = SGM_ABSENT;
+#pragma unroll
+        for (int i = 0; i < K; ++i) {
+            if (st == 0 || c[i] == SGM_ABSENT) L[i] = c[i];
+            else {
+                const int a = i == 0 ? lm : Lq[i > 0 ? i - 1 : 0];           // (indices stay constant and in range)
+                const int b = i + 1 < K ? Lq[i + 1 < K ? i + 1 : i] : rp;
+                L[i] = c[i] + min(min(Lq[i], min(a, b) + P1), mq + P2) - mq;
+            }
+            lmin = min(lmin, L[i]);
+        }
+        mq = __reduce_min_sync(0xffffffffu, lmin);
+        unsigned sn[K];
+#pragma unroll
+        for (int i = 0; i < K; ++i) {
+            Lq[i] = L[i];
+            sn[i] = c[i] == SGM_ABSENT ? 0xFFFFFFFFu : unsigned(first ? L[i] : so[i] + L[i]);
+            S[base + i] = int(sn[i]);
+        }
+        if (out.ptr) {
+            unsigned best = 0xFFFFFFFFu; int bi = 0;
+#pragma unroll
+            for (int i = K - 1; i >= 0; --i) if (sn[i] <= best) { best = sn[i]; bi = i; }
+            const unsigned wmin = __reduce_min_sync(0xffffffffu, best);
+            const unsigned ball = __ballot_sync(0xffffffffu, best == wmin);
+            const int src = __ffs(ball) - 1;
+            const int jw = __shfl_sync(0xffffffffu, lane * K + bi, src);
+            if (lane == 0) {
+                const long long pix = base / Dp;
+                const int py = int(pix / cols), px = int(pix - (long long)py * cols);
+                char* row = static_cast<char*>(out.ptr) + size_t(py) * out.step;
+                const int dv = out.dlo + jw;
+                if (out.elem == 1) reinterpret_cast<int8_t*>(row)[px] = int8_t(uint8_t(uint32_t(dv) & 0xFFu));
+                else if (out.elem == 2) reinterpret_cast<int16_t*>(row)[px] = int16_t(dv);
+                else reinterpret_cast<int32_t*>(row)[px] = dv;
+            }
+        }
+        base += stride;
+    }
+    }
+}
+
+} // namespace sb

@@ -7,6 +7,7 @@
 #include "imgproc.cuh"
 #include "lrcheck.cuh"
 #include "speckle.cuh"
+#include "sgm.cuh"
 #include "host_pack.hpp"
 
 #include <atomic>
@@ -237,9 +238,9 @@ static size_t f32_scratch_bytes(stereo_ctx* ctx, const Problem& p, int dirs) {
     return need + 2 * align256(size_t(p.rows) * align256(p.cols)) + 4096;
 }
 
-// Converts both float images to u8 copies while classifying them, reads the verdict back (one 16-byte copy and a stream
-// synchronize: the kernel family is a host decision) and says which family serves this image pair.
-static int classify_images(stereo_ctx* ctx, const Problem& p, cudaStream_t st, uint8_t* a8, uint8_t* b8, size_t pitch, int* cls) {
+// Converts both float images to u8 copies while classifying them and reads the verdict back into ctx->h_flag (one 16-byte
+// copy and a stream synchronize: the kernel family is a host decision).
+static int classify_flags(stereo_ctx* ctx, const Problem& p, cudaStream_t st, uint8_t* a8, uint8_t* b8, size_t pitch) {
     SB_CUDA(cudaMemsetAsync(ctx->d_flag, 0, 4 * sizeof(int), st));
     dim3 cb(32, 8), cg(div_round_up(p.cols, 32), div_round_up(p.rows, 8), 2);
     classify_convert_kernel<<<cg, cb, 0, st>>>(static_cast<const float*>(p.ref.ptr), p.ref.step, a8, static_cast<const float*>(p.tgt.ptr), p.tgt.step, b8,
@@ -250,15 +251,30 @@ static int classify_images(stereo_ctx* ctx, const Problem& p, cudaStream_t st, u
     SB_CUDA(cudaStreamSynchronize(st));
     SB_CUDA(cudaEventRecord(ctx->ev_gap1, st));          // (the kernels chosen below follow this mark)
     ctx->gap_recorded = true;
+    return STEREO_OK;
+}
+
+// The tracked extremes [tlo, thi] of the blocks that hold a non-8-bit pixel, and the value range [lo, hi] of both images:
+// [0, 255] for the blocks without a non-8-bit pixel, the tracked extremes for the others.
+static void classified_range(const stereo_ctx* ctx, double* tlo, double* thi, double* lo, double* hi) {
+    const unsigned* hf = reinterpret_cast<const unsigned*>(ctx->h_flag);
+    *tlo = hf[1] ? -double(f32_from_ordered(hf[1])) : 0.0;
+    *thi = hf[2] ? double(f32_from_ordered(hf[2])) : 0.0;
+    *lo = *tlo < 0.0 ? *tlo : 0.0;
+    *hi = *thi > 255.0 ? *thi : 255.0;
+}
+
+// Classifies the float images of one pair and says which kernel family serves it.
+static int classify_images(stereo_ctx* ctx, const Problem& p, cudaStream_t st, uint8_t* a8, uint8_t* b8, size_t pitch, int* cls) {
+    const int rc = classify_flags(ctx, p, st, a8, b8, pitch);
+    if (rc != STEREO_OK) return rc;
     const unsigned* hf = reinterpret_cast<const unsigned*>(ctx->h_flag);
     if (hf[0] == 0 && ctx->force_path != STEREO_PATH_FAST_F32) { *cls = CLS_U8; return STEREO_OK; }
     *cls = CLS_EXACT;
     if (hf[0] & 2u) return STEREO_OK;                                  // a pixel that is not finite
     if (ctx->force_path == STEREO_PATH_FAST_U8) return STEREO_OK;      // (reported as "not applicable" by the caller)
-    // the tracked extremes of the blocks that hold a non-8-bit pixel
-    const double tlo = hf[1] ? -double(f32_from_ordered(hf[1])) : 0.0, thi = hf[2] ? double(f32_from_ordered(hf[2])) : 0.0;
-    // value range: [0, 255] for the blocks without a non-8-bit pixel, the tracked extremes for the others
-    const double lo = tlo < 0.0 ? tlo : 0.0, hi = thi > 255.0 ? thi : 255.0;
+    double tlo, thi, lo, hi;
+    classified_range(ctx, &tlo, &thi, &lo, &hi);
     const double range = (hi - lo) * (1.0 + 1e-6), wnd = double(2 * p.R + 1) * (2 * p.R + 1);
     bool ok;
     if (p.cost == STEREO_COST_SSD) {
@@ -376,8 +392,146 @@ static int run_families(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bo
     return STEREO_OK;
 }
 
-// Validates every direction, runs them, then - pairs with the context's left-right check or speckle filter on - checks
-// and filters the pairs' maps, in that order (StereoSGBM's).
+// ---- semi-global matching (sgm.cuh) ----------------------------------------------------------------------------------
+
+// Candidates of one direction: [dmin, dmax] clipped to the ones some pixel has present (|d| <= cols - 1 + R), padded to
+// 32 K for the path kernels.
+struct SgmShape { int dlo, D, K; size_t Dp; };
+static SgmShape sgm_shape(const Problem& p) {
+    const int lim = p.cols - 1 + p.R;
+    const int dlo = p.dmin > -lim ? p.dmin : -lim, dhi = p.dmax < lim ? p.dmax : lim;
+    const int D = dhi - dlo + 1, K = (D + 31) / 32;
+    return SgmShape{dlo, D, K, size_t(32) * K};
+}
+
+static size_t sgm_padded_elems(const Problem& p) {
+    return size_t(p.rows + 2 * p.R) * (p.cols + 2 * p.R) + 2 * (size_t(p.R) + 64);
+}
+
+// One direction's scratch: both padded images, the cost volume and the aggregate (plus, for float images, the u8 copies
+// the classification writes).  Directions of a call run one after the other on the same scratch.
+static size_t sgm_scratch_bytes(const Problem& p) {
+    const size_t cells = size_t(p.rows) * p.cols * sgm_shape(p).Dp;
+    size_t need = 2 * align256(sgm_padded_elems(p) * sizeof(float)) + 2 * align256(cells * 4) + 4096;
+    if (p.ref.type == PixType::F32) need += 2 * align256(size_t(p.rows) * align256(p.cols));
+    return need;
+}
+
+// Every L_r is at most C_max + P2 with C_max = (2R + 1)^2 M, M the largest per-element term: S stays in int32 when
+// paths (C_max + P2) <= 2^31 - 1.
+static int check_sgm_bound(const stereo_ctx* ctx, int R, double M) {
+    const double w = double(2 * R + 1) * (2 * R + 1);
+    if (double(ctx->sgm_paths) * (w * M + ctx->sgm_p2) <= 2147483647.0) return STEREO_OK;
+    set_error("SGM: %d paths x ((2 * %d + 1)^2 x %.0f + P2 %d) exceeds 2^31 - 1", ctx->sgm_paths, R, M, ctx->sgm_p2);
+    return STEREO_ERR_UNSUPPORTED;
+}
+
+// What an SGM pair call must satisfy before anything is staged or enqueued: the SSD cost and whole maps (paths cross
+// band seams).  run_sgm checks the candidate count and the int32 bound.
+static int check_sgm_call(const stereo_ctx* ctx, int cost, int row_begin, int row_end, int rows) {
+    if (ctx->sgm_paths <= 0) return STEREO_OK;
+    if (cost != STEREO_COST_SSD) { set_error("SGM aggregates the SSD cost only (switch it off for NCC calls)"); return STEREO_ERR_UNSUPPORTED; }
+    if (row_begin != 0 || row_end != rows) {
+        set_error("SGM: rows [%d, %d) are not the whole map (vertical and diagonal paths cross band seams)", row_begin, row_end);
+        return STEREO_ERR_UNSUPPORTED;
+    }
+    return STEREO_OK;
+}
+
+// One direction by SGM into p.disp, on scratch the caller reserved.  ref / tgt: the caller's images (u8 or float).
+static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st) {
+    static constexpr int DIRS[8][2] = {{0, 1}, {0, -1}, {1, 0}, {-1, 0}, {1, 1}, {1, -1}, {-1, 1}, {-1, -1}};
+    const SgmShape g = sgm_shape(p);
+    const int Hp = p.rows + 2 * p.R, Wp = p.cols + 2 * p.R;
+    const size_t guard = size_t(p.R) + 64, cells = size_t(p.rows) * p.cols * g.Dp;
+    float* lbuf = static_cast<float*>(ctx->arena.take(sgm_padded_elems(p) * sizeof(float)));
+    float* rbuf = static_cast<float*>(ctx->arena.take(sgm_padded_elems(p) * sizeof(float)));
+    int32_t* C = static_cast<int32_t*>(ctx->arena.take(cells * 4));
+    int32_t* S = static_cast<int32_t*>(ctx->arena.take(cells * 4));
+    if (!lbuf || !rbuf || !C || !S) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
+    SB_CUDA(cudaMemsetAsync(rbuf, 0, guard * sizeof(float), st));
+    SB_CUDA(cudaMemsetAsync(rbuf + guard + size_t(Hp) * Wp, 0, guard * sizeof(float), st));
+    float* Lp = lbuf + guard;
+    float* Rp = rbuf + guard;
+    dim3 pb(32, 8), pg(div_round_up(Wp, 32), div_round_up(Hp, 8));
+    if (p.ref.type == PixType::F32) {
+        pad_replicate_kernel<float><<<pg, pb, 0, st>>>(static_cast<const float*>(p.ref.ptr), p.ref.step, p.rows, p.cols, p.R, Lp, Hp, Wp, 0, p.rows);
+        pad_replicate_kernel<float><<<pg, pb, 0, st>>>(static_cast<const float*>(p.tgt.ptr), p.tgt.step, p.rows, p.cols, p.R, Rp, Hp, Wp, 0, p.rows);
+    } else {
+        pad_replicate_kernel<uint8_t><<<pg, pb, 0, st>>>(static_cast<const uint8_t*>(p.ref.ptr), p.ref.step, p.rows, p.cols, p.R, Lp, Hp, Wp, 0, p.rows);
+        pad_replicate_kernel<uint8_t><<<pg, pb, 0, st>>>(static_cast<const uint8_t*>(p.tgt.ptr), p.tgt.step, p.rows, p.cols, p.R, Rp, Hp, Wp, 0, p.rows);
+    }
+    // rows per cost block: as many as still leave about four blocks per SM (each block recomputes 2R + 1 rows first)
+    const long long tiles = (long long)div_round_up(p.cols, SGM_XT) * (g.Dp / 32);
+    int rpb = 64;
+    while (rpb > 8 && tiles * div_round_up(p.rows, rpb) < 4LL * ctx->sm_count) rpb /= 2;
+    const dim3 cg(div_round_up(p.cols, SGM_XT), div_round_up(p.rows, rpb), unsigned(g.Dp / 32));
+    const size_t smem = size_t(SGM_XT + 2 * p.R) * 32 * sizeof(int32_t);
+    sgm_cost_kernel<<<cg, SGM_COST_THREADS, smem, st>>>(Lp, Rp, p.rows, p.cols, p.R, g.dlo, g.D, int(g.Dp), rpb, C);
+    ctx->last_launches += 3;
+    for (int k = 0; k < ctx->sgm_paths; ++k) {
+        const int dy = DIRS[k][0], dx = DIRS[k][1];
+        const bool last = k == ctx->sgm_paths - 1;
+        const SgmOut out{last ? p.disp.ptr : nullptr, p.disp.step, p.disp.elem, g.dlo};
+        const unsigned blocks = div_round_up(sgm_lines(p.rows, p.cols, dy, dx), SGM_PATH_WARPS);
+#define SB_SGM_PATH(K) case K: sgm_path_kernel<K><<<blocks, SGM_PATH_WARPS * 32, 0, st>>>(C, S, p.rows, p.cols, dy, dx, ctx->sgm_p1, ctx->sgm_p2, k == 0, out); break
+        switch (g.K) {
+            SB_SGM_PATH(1); SB_SGM_PATH(2); SB_SGM_PATH(3); SB_SGM_PATH(4); SB_SGM_PATH(5); SB_SGM_PATH(6); SB_SGM_PATH(7); SB_SGM_PATH(8);
+            SB_SGM_PATH(9); SB_SGM_PATH(10); SB_SGM_PATH(11); SB_SGM_PATH(12); SB_SGM_PATH(13); SB_SGM_PATH(14); SB_SGM_PATH(15); SB_SGM_PATH(16);
+            default: set_error("SGM: no path kernel for %d candidates per lane (internal)", g.K); return STEREO_ERR_UNSUPPORTED;
+        }
+#undef SB_SGM_PATH
+        ctx->last_launches += 1;
+    }
+    SB_CUDA(cudaGetLastError());
+    return STEREO_OK;
+}
+
+// Every direction of a pair call by SGM: n/2 left-referenced problems and their partners, one at a time on one scratch.
+// 8-bit images are checked against the int32 bound with M = 255^2 before anything is enqueued; float images (one pair
+// per call) are classified first, refused when a pixel is not finite, and checked with M = ceil((hi - lo)^2) of their
+// value range (widened by 1e-6 for the float rounding of l - r and its square).
+static int run_sgm(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bool u8) {
+    size_t need = 0;
+    for (int i = 0; i < n; ++i) {
+        if (sgm_shape(ps[i]).K > SGM_MAXK) {
+            set_error("SGM: %d candidates per pixel, at most %d are supported", sgm_shape(ps[i]).D, 32 * SGM_MAXK);
+            return STEREO_ERR_UNSUPPORTED;
+        }
+        const size_t b = sgm_scratch_bytes(ps[i]);
+        if (b > need) need = b;
+    }
+    int rc = u8 ? check_sgm_bound(ctx, ps[0].R, 255.0 * 255.0) : STEREO_OK;
+    if (rc == STEREO_OK) rc = reserve_arena(ctx, st, need);
+    if (rc != STEREO_OK) return rc;
+    if (!u8) {
+        const Problem& p = ps[0];
+        ctx->arena.reset();
+        const size_t pitch = align256(p.cols);
+        uint8_t* a8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
+        uint8_t* b8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
+        if (!a8 || !b8) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
+        rc = classify_flags(ctx, p, st, a8, b8, pitch);
+        if (rc != STEREO_OK) return rc;
+        const unsigned flags = *reinterpret_cast<const unsigned*>(ctx->h_flag);
+        if (flags & 2u) { set_error("SGM: an image holds a pixel that is not finite"); return STEREO_ERR_UNSUPPORTED; }
+        double tlo, thi, lo, hi;
+        classified_range(ctx, &tlo, &thi, &lo, &hi);
+        const double range = (hi - lo) * (1.0 + 1e-6);
+        rc = check_sgm_bound(ctx, p.R, flags == 0 ? 255.0 * 255.0 : ceil(range * range));
+        if (rc != STEREO_OK) return rc;
+    }
+    ctx->last_path = STEREO_PATH_SGM;
+    for (int i = 0; i < n && rc == STEREO_OK; ++i) {
+        ctx->arena.reset();
+        rc = run_sgm_direction(ctx, ps[i], st);
+    }
+    return rc;
+}
+
+// Validates every direction, runs them - pairs with the context's SGM on by SGM, everything else on the kernel family
+// run_families picks - then, pairs with the context's left-right check or speckle filter on, checks and filters the
+// pairs' maps, in that order (StereoSGBM's).
 static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
     bool fast = ctx->force_path != STEREO_PATH_EXACT_F32, u8 = true;
     for (int i = 0; i < n; ++i) {
@@ -389,7 +543,11 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
         fast = fast && fast_supported(p);
         u8 = u8 && p.ref.type == PixType::U8;
     }
-    const bool lr = n >= 2 && ctx->lr_max_diff >= 0, spk = n >= 2 && ctx->spk_max_size > 0;
+    const bool lr = n >= 2 && ctx->lr_max_diff >= 0, spk = n >= 2 && ctx->spk_max_size > 0, sgm = n >= 2 && ctx->sgm_paths > 0;
+    if (sgm) {
+        const int rc = check_sgm_call(ctx, ps[0].cost, ps[0].row_begin, ps[0].row_end, ps[0].rows);
+        if (rc != STEREO_OK) return rc;
+    }
     for (int k = 0; (lr || spk) && k < n / 2; ++k) {
         const int rc = check_lr_sentinel(ps[k].disp.elem, ps[n / 2 + k].dmax);
         if (rc != STEREO_OK) return rc;
@@ -399,7 +557,7 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
         if (rc == STEREO_OK) rc = reserve_arena(ctx, st, speckle_scratch_bytes(n, ps[0].rows, ps[0].cols));
         if (rc != STEREO_OK) return rc;
     }
-    int rc = run_families(ctx, ps, n, st, fast, u8);
+    int rc = sgm ? run_sgm(ctx, ps, n, st, u8) : run_families(ctx, ps, n, st, fast, u8);
     if (rc == STEREO_OK && lr) rc = lr_check_pairs(ctx, ps, n, st);
     if (rc == STEREO_OK && spk) rc = speckle_pairs(ctx, ps, n, st);
     return rc;
@@ -599,6 +757,7 @@ static bool host_sample_is_8bit(const void* img, size_t step, int rows, int cols
 static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, int n_pairs, const HostPairIn* in,
                                      const HostDir* dirs, int n_dirs, int rows, int cols, int R, size_t disp_step, int elem) {
     if (ctx->force_path == STEREO_PATH_EXACT_F32 || ctx->force_path == STEREO_PATH_FAST_F32) return PIPE_NOT_APPLICABLE;
+    if (n_dirs == 2 && ctx->sgm_paths > 0) return PIPE_NOT_APPLICABLE;      // (SGM maps are computed whole, run_directions)
     const auto t_call = std::chrono::steady_clock::now();       // (trace only)
     double t_pack = 0.0, t_ring = 0.0;
     auto since = [](std::chrono::steady_clock::time_point t0) { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(); };
@@ -1316,6 +1475,24 @@ int stereo_ctx_speckle_filter(const stereo_ctx* ctx, int* max_size, int* max_dif
     return STEREO_OK;
 }
 
+int stereo_ctx_set_sgm(stereo_ctx* ctx, int paths, int p1, int p2) {
+    if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
+    if (paths != 0 && paths != 4 && paths != 8) { set_error("SGM paths must be 0, 4 or 8 (got %d)", paths); return STEREO_ERR_INVALID_ARG; }
+    if (p1 < 0 || p1 > p2) { set_error("SGM penalties need 0 <= P1 <= P2 (got %d, %d)", p1, p2); return STEREO_ERR_INVALID_ARG; }
+    ctx->sgm_paths = paths;
+    ctx->sgm_p1 = paths ? p1 : 0;
+    ctx->sgm_p2 = paths ? p2 : 0;
+    return STEREO_OK;
+}
+
+int stereo_ctx_sgm(const stereo_ctx* ctx, int* paths, int* p1, int* p2) {
+    if (!ctx || !paths || !p1 || !p2) { set_error("null argument"); return STEREO_ERR_INVALID_ARG; }
+    *paths = ctx->sgm_paths;
+    *p1 = ctx->sgm_p1;
+    *p2 = ctx->sgm_p2;
+    return STEREO_OK;
+}
+
 int stereo_filter_speckles_device(stereo_ctx* ctx, void* disp, size_t disp_step, int disp_elem_bytes, int rows, int cols, int new_val,
                                   int max_size, int max_diff, void* cuda_stream) {
     int rc = check_ctx(ctx);
@@ -1627,6 +1804,7 @@ static int pair_host(stereo_ctx* ctx, int cost, PixType type, const void* left, 
     const size_t row = size_t(cols) * (type == PixType::F32 ? 4 : 1), disp_row = size_t(cols) * elem;
     int rc = check_host_args(ctx, {left, right, disp_left, disp_right}, rows, cols, elem,
                              {{left_step, row}, {right_step, row}, {disp_step, disp_row}}, range);
+    if (rc == STEREO_OK) rc = check_sgm_call(ctx, cost, 0, rows, rows);      // (as run_directions would, but before staging)
     if (rc != STEREO_OK) return rc;
     {
         const HostPairIn in{left, left_step, right, right_step};
@@ -1711,6 +1889,7 @@ static int pair_band_host(stereo_ctx* ctx, int cost, PixType type, const void* l
     rc = stereo_band_halo_rows(rows, row_begin, row_end, R, &h0, &h1);      // (rejects a bad band or window radius)
     if (rc != STEREO_OK) return rc;
     rc = check_speckle_band(ctx, row_begin, row_end, rows);      // (as run_directions would, but before staging)
+    if (rc == STEREO_OK) rc = check_sgm_call(ctx, cost, row_begin, row_end, rows);
     if (rc != STEREO_OK) return rc;
     const int nh = h1 - h0;
     HostRows in[2] = {{static_cast<const char*>(left) + size_t(h0) * left_step, left_step, size_t(cols)},
@@ -1794,6 +1973,7 @@ static int pair_batch_host(stereo_ctx* ctx, int cost, PixType type, int n_pairs,
     if (n_pairs <= 0) { set_error("n_pairs must be positive"); return STEREO_ERR_INVALID_ARG; }
     int rc = check_host_args(ctx, {left, right, disp_left, disp_right}, rows, cols, disp_elem_bytes,
                              {{img_step, size_t(cols) * px}, {disp_step, size_t(cols) * disp_elem_bytes}}, disparity_range);
+    if (rc == STEREO_OK) rc = check_sgm_call(ctx, cost, 0, rows, rows);
     if (rc != STEREO_OK) return rc;
     {   // pipelined: item i+1 uploads while item i computes and item i-1 downloads (3 device slots)
         std::vector<HostPairIn> in(n_pairs);

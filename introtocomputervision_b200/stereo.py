@@ -144,6 +144,20 @@ class Context:
         _check(_capi.lib().stereo_ctx_speckle_filter(self._h, C.byref(size), C.byref(diff)), "stereo_ctx_speckle_filter")
         return None if size.value <= 0 else (size.value, diff.value)
 
+    def set_sgm(self, paths: Optional[int], p1: int = 0, p2: int = 0) -> None:
+        """SSD pair calls: semi-global matching over ``paths`` (4 or 8) scanline directions with penalties
+        ``0 <= p1 <= p2``, before the left-right check and the speckle filter.  ``None`` or 0 switches it off (the
+        default)."""
+        v = 0 if paths is None else int(paths)
+        _check(_capi.lib().stereo_ctx_set_sgm(self._h, v, int(p1), int(p2)), "stereo_ctx_set_sgm")
+
+    @property
+    def sgm(self) -> Optional[Tuple[int, int, int]]:
+        """``(paths, p1, p2)`` of semi-global matching, or None when it is off."""
+        paths, p1, p2 = C.c_int(), C.c_int(), C.c_int()
+        _check(_capi.lib().stereo_ctx_sgm(self._h, C.byref(paths), C.byref(p1), C.byref(p2)), "stereo_ctx_sgm")
+        return None if paths.value <= 0 else (paths.value, p1.value, p2.value)
+
     def set_host_threads(self, threads: int) -> None:
         """Host threads that convert CV_32FC1 host images to u8 before the upload (0 = automatic, -1 = off)."""
         _check(_capi.lib().stereo_ctx_set_host_threads(self._h, int(threads)), "stereo_ctx_set_host_threads")
@@ -289,6 +303,11 @@ class MultiGpu:
         """:meth:`Context.set_speckle_filter` on every device's context (row-band sharded pairs refuse while it is on)."""
         v = 0 if max_size is None or max_size <= 0 else int(max_size)
         _check(_capi.lib().stereo_mgpu_set_speckle_filter(self._h, v, int(max_diff)), "stereo_mgpu_set_speckle_filter")
+
+    def set_sgm(self, paths: Optional[int], p1: int = 0, p2: int = 0) -> None:
+        """:meth:`Context.set_sgm` on every device's context (row-band sharded pairs refuse while it is on)."""
+        v = 0 if paths is None else int(paths)
+        _check(_capi.lib().stereo_mgpu_set_sgm(self._h, v, int(p1), int(p2)), "stereo_mgpu_set_sgm")
 
     def disparity_pair_bands(self, cost: int, left: np.ndarray, right: np.ndarray, window_rad: int, disparity_range: int,
                              dtype=np.int8) -> Tuple[np.ndarray, np.ndarray]:
