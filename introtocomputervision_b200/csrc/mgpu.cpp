@@ -75,19 +75,16 @@ int pair_bands(stereo_mgpu* mg, int cost, const T* left, size_t left_step, const
                int window_rad, int disparity_range, void* disp_left, void* disp_right, size_t disp_step, int elem, bool f32) {
     if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
     if (rows <= 0) { sb::set_error("rows must be positive"); return STEREO_ERR_INVALID_ARG; }
-    // a speckle region can cross a band seam: no band is filtered on its own (and no whole-pair call stands in for the bands)
+    // speckle regions and SGM paths cross band seams: no band is filtered or aggregated on its own (and no whole-pair call
+    // stands in for the bands)
     for (stereo_ctx* c : mg->ctx) {
-        int max_size = 0, max_diff = 0;
+        int max_size = 0, max_diff = 0, paths = 0, p1 = 0, p2 = 0;
         stereo_ctx_speckle_filter(c, &max_size, &max_diff);
+        stereo_ctx_sgm(c, &paths, &p1, &p2);
         if (max_size > 0) {
             sb::set_error("speckle filter on: row-band sharded pairs are not filtered (filter the gathered map with stereo_filter_speckles_device)");
             return STEREO_ERR_UNSUPPORTED;
         }
-    }
-    // SGM paths cross band seams: no band is aggregated on its own
-    for (stereo_ctx* c : mg->ctx) {
-        int paths = 0, p1 = 0, p2 = 0;
-        stereo_ctx_sgm(c, &paths, &p1, &p2);
         if (paths > 0) { sb::set_error("SGM on: row-band sharded pairs are not aggregated (shard whole pairs)"); return STEREO_ERR_UNSUPPORTED; }
     }
     int parts = int(mg->ctx.size());

@@ -112,34 +112,50 @@ static void pair_problems(Problem* ps, int np, int k, int cost, PixType type, co
                            R, 0, range, disp_right, disp_step, elem, nullptr, 0);
 }
 
-// ---- left-right consistency check (lrcheck.cuh) -----------------------------------------------------
+// ---- pair options: left-right check (lrcheck.cuh), speckle filter (speckle.cuh), SGM (sgm.cuh) ----------------------
 
-// The check marks a pair's inconsistent pixels with -(range + 1), which must fit the maps' element type.  (An int8 map of
+// The check and the filter mark removed pixels with -(range + 1), which must fit the maps' element type.  (An int8 map of
 // more than 127 disparities already holds wrapped values.)
-static bool lr_sentinel_fits(int elem, int range) { return range <= (elem == 1 ? 127 : elem == 2 ? 32767 : 32768); }
-
 static int check_lr_sentinel(int elem, int range) {
-    if (lr_sentinel_fits(elem, range)) return STEREO_OK;
+    if (range <= (elem == 1 ? 127 : elem == 2 ? 32767 : 32768)) return STEREO_OK;
     set_error("left-right check / speckle filter: the sentinel -(%d + 1) does not fit a %d-byte disparity element", range, elem);
     return STEREO_ERR_UNSUPPORTED;
 }
 
-// The check over output rows [row_begin, row_end) of the maps of n/2 pairs laid out as pair_problems builds them: ps[k]
-// left-referenced, ps[n/2 + k] its partner.  Every pair of one call has the same shape, band, range and element type.
-static int lr_check_pairs(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t st) {
-    static_assert(FMAXJOBS / 2 <= LR_MAXPAIRS, "one check launch covers the pairs of one launch sequence");
-    const int np = n / 2;
-    LrParams P{};
-    for (int k = 0; k < np; ++k)
-        P.pair[k] = LrMaps{ps[k].disp.ptr, ps[np + k].disp.ptr, ps[k].disp.step, ps[np + k].disp.step};
-    P.cols = ps[0].cols;
-    P.max_diff = ctx->lr_max_diff;
-    P.sentinel = -(ps[np].dmax + 1);
-    ctx->last_launches += 1;
-    return lr_check_launch(P, ps[0].row_end - ps[0].row_begin, np, ps[0].disp.elem, st);
+// What a pair call must satisfy for the context's options, checked once per call before anything is staged or enqueued:
+// the sentinel fits (left-right check or speckle filter on), SGM aggregates the SSD cost, and SGM paths and speckle
+// regions, which cross band seams, get whole maps.  run_sgm checks the candidate count and the int32 bound.
+static int check_pair_options(const stereo_ctx* ctx, int cost, int elem, int range, int row_begin, int row_end, int rows) {
+    const bool sgm = ctx->sgm_paths > 0, spk = ctx->spk_max_size > 0, whole = row_begin == 0 && row_end == rows;
+    if (ctx->lr_max_diff >= 0 || spk) {
+        const int rc = check_lr_sentinel(elem, range);
+        if (rc != STEREO_OK) return rc;
+    }
+    if (sgm && cost != STEREO_COST_SSD) { set_error("SGM aggregates the SSD cost only (switch it off for NCC calls)"); return STEREO_ERR_UNSUPPORTED; }
+    if (sgm && !whole) {
+        set_error("SGM: rows [%d, %d) are not the whole map (vertical and diagonal paths cross band seams)", row_begin, row_end);
+        return STEREO_ERR_UNSUPPORTED;
+    }
+    if (spk && !whole) {
+        set_error("speckle filter: rows [%d, %d) are not the whole map (filter the gathered map with stereo_filter_speckles_device)",
+                  row_begin, row_end);
+        return STEREO_ERR_UNSUPPORTED;
+    }
+    return STEREO_OK;
 }
 
-// ---- speckle filter (speckle.cuh) ---------------------------------------------------------------------------------
+// The check over `rows` rows of np pairs of maps, in place: maps[k] the left map of pair k, maps[np + k] its right map,
+// each at its first row, all of one element type.
+static int lr_check_pairs(stereo_ctx* ctx, const OutView* maps, int np, int rows, int cols, int max_diff, int sentinel,
+                          cudaStream_t st) {
+    LrParams P{};
+    for (int k = 0; k < np; ++k) P.pair[k] = LrMaps{maps[k].ptr, maps[np + k].ptr, maps[k].step, maps[np + k].step};
+    P.cols = cols;
+    P.max_diff = max_diff;
+    P.sentinel = sentinel;
+    ctx->last_launches += 1;
+    return lr_check_launch(P, rows, np, maps[0].elem, st);
+}
 
 // The filter over n whole rows x cols maps of one element type, in place.  Its scratch comes from the arena, which the
 // caller sized for speckle_scratch_bytes(n, rows, cols) before it enqueued anything: the filter itself never grows it.
@@ -156,57 +172,74 @@ static int speckle_maps(stereo_ctx* ctx, const OutView* maps, int n, int rows, i
     return speckle_launch(P, n, maps[0].elem, st);
 }
 
-// A speckle region can cross a band seam, so with the filter on a pair call takes the whole map only.
-static int check_speckle_band(const stereo_ctx* ctx, int row_begin, int row_end, int rows) {
-    if (ctx->spk_max_size <= 0 || (row_begin == 0 && row_end == rows)) return STEREO_OK;
-    set_error("speckle filter: rows [%d, %d) are not the whole map (filter the gathered map with stereo_filter_speckles_device)",
-              row_begin, row_end);
-    return STEREO_ERR_UNSUPPORTED;
+// The arena scratch finish_pairs needs for the n maps of a pair call.
+static size_t finish_scratch_bytes(const stereo_ctx* ctx, int n, int rows, int cols) {
+    return ctx->spk_max_size > 0 ? speckle_scratch_bytes(n, rows, cols) : 0;
 }
 
-// The context's filter over both maps of the n/2 whole-image pairs of ps (laid out as pair_problems builds them), with the
-// left-right check's sentinel as the value of removed pixels.
-static int speckle_pairs(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t st) {
+// The context's left-right check and speckle filter on the maps of the n/2 pairs of ps (laid out as pair_problems builds
+// them), in that order (StereoSGBM's): the check on the rows of ps, then, once `maps_complete` says every row of the maps
+// is computed, the filter on the whole maps.
+static int finish_pairs(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t st, bool maps_complete) {
+    static_assert(FMAXJOBS / 2 <= LR_MAXPAIRS, "one check launch covers the pairs of one launch sequence");
     static_assert(FMAXJOBS <= SPK_MAXMAPS, "one filter launch covers the maps of one launch sequence");
+    const Problem& p = ps[0];
+    const int sentinel = -(ps[n / 2].dmax + 1);
     OutView maps[FMAXJOBS];
     for (int k = 0; k < n; ++k) maps[k] = ps[k].disp;
-    return speckle_maps(ctx, maps, n, ps[0].rows, ps[0].cols, -(ps[n / 2].dmax + 1), ctx->spk_max_size, ctx->spk_max_diff, st);
+    int rc = STEREO_OK;
+    if (ctx->lr_max_diff >= 0) rc = lr_check_pairs(ctx, maps, n / 2, p.row_end - p.row_begin, p.cols, ctx->lr_max_diff, sentinel, st);
+    if (rc != STEREO_OK || !maps_complete || ctx->spk_max_size <= 0) return rc;
+    for (int k = 0; k < n; ++k) maps[k].ptr = static_cast<char*>(maps[k].ptr) - size_t(ps[k].row_begin) * maps[k].step;
+    return speckle_maps(ctx, maps, n, p.rows, p.cols, sentinel, ctx->spk_max_size, ctx->spk_max_diff, st);
 }
 
 // ---- exact path ---------------------------------------------------------------------------------
 
+// Floats of one replicate-padded image of p with its guards (pad_images).
+static size_t padded_elems(const Problem& p) {
+    return size_t(p.rows + 2 * p.R) * (p.cols + 2 * p.R) + 2 * (size_t(p.R) + 64);
+}
+
 static size_t exact_scratch_bytes(const Problem& p) {
-    const size_t Hp = p.rows + 2 * p.R, Wp = p.cols + 2 * p.R, guard = size_t(p.R) + 64;
-    const size_t img = align256((Hp * Wp + 2 * guard) * sizeof(float));
     const size_t band = size_t(p.row_end - p.row_begin) * p.cols;
-    return 2 * img + 2 * align256(band * 4) + 4096;
+    return 2 * align256(padded_elems(p) * sizeof(float)) + 2 * align256(band * 4) + 4096;
+}
+
+// Both images of p, padded by R with replicated borders, into two float images taken from the arena, each with R + 64
+// guard floats on both sides; *Lp and *Rp point at their first pixels.  The target's guards are zeroed: they stand in for
+// the reference's out-of-allocation reads.
+static int pad_images(stereo_ctx* ctx, const Problem& p, cudaStream_t st, float** Lp, float** Rp) {
+    const int Hp = p.rows + 2 * p.R, Wp = p.cols + 2 * p.R;
+    const size_t guard = size_t(p.R) + 64;
+    float* lbuf = static_cast<float*>(ctx->arena.take(padded_elems(p) * sizeof(float)));
+    float* rbuf = static_cast<float*>(ctx->arena.take(padded_elems(p) * sizeof(float)));
+    if (!lbuf || !rbuf) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
+    SB_CUDA(cudaMemsetAsync(rbuf, 0, guard * sizeof(float), st));
+    SB_CUDA(cudaMemsetAsync(rbuf + guard + size_t(Hp) * Wp, 0, guard * sizeof(float), st));
+    *Lp = lbuf + guard;
+    *Rp = rbuf + guard;
+    dim3 pb(32, 8), pg(div_round_up(Wp, 32), div_round_up(Hp, 8));
+    if (p.ref.type == PixType::F32)
+        pad_replicate_kernel<float><<<pg, pb, 0, st>>>(static_cast<const float*>(p.ref.ptr), p.ref.step, p.rows, p.cols, p.R, *Lp, Hp, Wp, p.avail_begin, p.avail_end);
+    else
+        pad_replicate_kernel<uint8_t><<<pg, pb, 0, st>>>(static_cast<const uint8_t*>(p.ref.ptr), p.ref.step, p.rows, p.cols, p.R, *Lp, Hp, Wp, p.avail_begin, p.avail_end);
+    if (p.tgt.type == PixType::F32)
+        pad_replicate_kernel<float><<<pg, pb, 0, st>>>(static_cast<const float*>(p.tgt.ptr), p.tgt.step, p.rows, p.cols, p.R, *Rp, Hp, Wp, p.avail_begin, p.avail_end);
+    else
+        pad_replicate_kernel<uint8_t><<<pg, pb, 0, st>>>(static_cast<const uint8_t*>(p.tgt.ptr), p.tgt.step, p.rows, p.cols, p.R, *Rp, Hp, Wp, p.avail_begin, p.avail_end);
+    ctx->last_launches += 2;
+    return STEREO_OK;
 }
 
 static int run_exact(stereo_ctx* ctx, const Problem& p, cudaStream_t st) {
-    const int Hp = p.rows + 2 * p.R, Wp = p.cols + 2 * p.R;
-    const size_t guard = size_t(p.R) + 64;
-    const size_t img_elems = size_t(Hp) * Wp + 2 * guard;
-    float* lbuf = static_cast<float*>(ctx->arena.take(img_elems * sizeof(float)));
-    float* rbuf = static_cast<float*>(ctx->arena.take(img_elems * sizeof(float)));
+    float *Lp, *Rp;
+    const int rc = pad_images(ctx, p, st, &Lp, &Rp);
+    if (rc != STEREO_OK) return rc;
     const int band_rows = p.row_end - p.row_begin;
     int32_t* d_disp = static_cast<int32_t*>(ctx->arena.take(size_t(band_rows) * p.cols * 4));
     uint32_t* d_best = static_cast<uint32_t*>(ctx->arena.take(size_t(band_rows) * p.cols * 4));
-    if (!lbuf || !rbuf || !d_disp || !d_best) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
-    // zero guards (the tgt guard stands in for the reference's out-of-allocation reads)
-    SB_CUDA(cudaMemsetAsync(rbuf, 0, guard * sizeof(float), st));
-    SB_CUDA(cudaMemsetAsync(rbuf + guard + size_t(Hp) * Wp, 0, guard * sizeof(float), st));
-    float* Lp = lbuf + guard;
-    float* Rp = rbuf + guard;
-    dim3 pb(32, 8), pg(div_round_up(Wp, 32), div_round_up(Hp, 8));
-    if (p.ref.type == PixType::F32)
-        pad_replicate_kernel<float><<<pg, pb, 0, st>>>(static_cast<const float*>(p.ref.ptr), p.ref.step, p.rows, p.cols, p.R, Lp, Hp, Wp, p.avail_begin, p.avail_end);
-    else
-        pad_replicate_kernel<uint8_t><<<pg, pb, 0, st>>>(static_cast<const uint8_t*>(p.ref.ptr), p.ref.step, p.rows, p.cols, p.R, Lp, Hp, Wp, p.avail_begin, p.avail_end);
-    if (p.tgt.type == PixType::F32)
-        pad_replicate_kernel<float><<<pg, pb, 0, st>>>(static_cast<const float*>(p.tgt.ptr), p.tgt.step, p.rows, p.cols, p.R, Rp, Hp, Wp, p.avail_begin, p.avail_end);
-    else
-        pad_replicate_kernel<uint8_t><<<pg, pb, 0, st>>>(static_cast<const uint8_t*>(p.tgt.ptr), p.tgt.step, p.rows, p.cols, p.R, Rp, Hp, Wp, p.avail_begin, p.avail_end);
-    ctx->last_launches += 2;
+    if (!d_disp || !d_best) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
     dim3 kb(128), kg(div_round_up(p.cols, 128), band_rows);
     if (p.cost == STEREO_COST_SSD)
         ssd_exact_kernel<<<kg, kb, 0, st>>>(Lp, Rp, p.rows, p.cols, p.R, p.dmin, p.dmax, p.row_begin, d_disp,
@@ -228,6 +261,9 @@ enum { CLS_U8 = 0, CLS_F32_FAST = 1, CLS_EXACT = 2 };
 
 static Problem as_u8(Problem p) { p.ref.type = PixType::U8; p.tgt.type = PixType::U8; return p; }
 
+// The two u8 copies classify_flags takes from the arena.
+static size_t u8_copies_bytes(const Problem& p) { return 2 * align256(size_t(p.rows) * align256(p.cols)); }
+
 // Scratch for a float problem whose kernel family is only known after the classification: the larger of the three
 // families' needs plus the u8 copies of both images.  `dirs` = directions that share one launch sequence.
 static size_t f32_scratch_bytes(stereo_ctx* ctx, const Problem& p, int dirs) {
@@ -235,12 +271,20 @@ static size_t f32_scratch_bytes(stereo_ctx* ctx, const Problem& p, int dirs) {
     const size_t f = size_t(dirs) * fast_scratch_bytes(ctx, p), u = size_t(dirs) * fast_scratch_bytes(ctx, as_u8(p));
     if (f > need) need = f;
     if (u > need) need = u;
-    return need + 2 * align256(size_t(p.rows) * align256(p.cols)) + 4096;
+    return need + u8_copies_bytes(p) + 4096;
 }
 
-// Converts both float images to u8 copies while classifying them and reads the verdict back into ctx->h_flag (one 16-byte
-// copy and a stream synchronize: the kernel family is a host decision).
-static int classify_flags(stereo_ctx* ctx, const Problem& p, cudaStream_t st, uint8_t* a8, uint8_t* b8, size_t pitch) {
+// Resets the arena and converts both float images of p into u8 copies at its start (u8[0] of ref, u8[1] of tgt) while
+// classifying them, then reads the verdict back into ctx->h_flag (one 16-byte copy and a stream synchronize: the kernel
+// family is a host decision).
+static int classify_flags(stereo_ctx* ctx, const Problem& p, cudaStream_t st, ImageView u8[2]) {
+    ctx->arena.reset();
+    const size_t pitch = align256(p.cols);
+    uint8_t* a8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
+    uint8_t* b8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
+    if (!a8 || !b8) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
+    u8[0] = ImageView{a8, pitch, PixType::U8};
+    u8[1] = ImageView{b8, pitch, PixType::U8};
     SB_CUDA(cudaMemsetAsync(ctx->d_flag, 0, 4 * sizeof(int), st));
     dim3 cb(32, 8), cg(div_round_up(p.cols, 32), div_round_up(p.rows, 8), 2);
     classify_convert_kernel<<<cg, cb, 0, st>>>(static_cast<const float*>(p.ref.ptr), p.ref.step, a8, static_cast<const float*>(p.tgt.ptr), p.tgt.step, b8,
@@ -264,9 +308,9 @@ static void classified_range(const stereo_ctx* ctx, double* tlo, double* thi, do
     *hi = *thi > 255.0 ? *thi : 255.0;
 }
 
-// Classifies the float images of one pair and says which kernel family serves it.
-static int classify_images(stereo_ctx* ctx, const Problem& p, cudaStream_t st, uint8_t* a8, uint8_t* b8, size_t pitch, int* cls) {
-    const int rc = classify_flags(ctx, p, st, a8, b8, pitch);
+// Classifies the float images of one pair (classify_flags) and says which kernel family serves it.
+static int classify_images(stereo_ctx* ctx, const Problem& p, cudaStream_t st, ImageView u8[2], int* cls) {
+    const int rc = classify_flags(ctx, p, st, u8);
     if (rc != STEREO_OK) return rc;
     const unsigned* hf = reinterpret_cast<const unsigned*>(ctx->h_flag);
     if (hf[0] == 0 && ctx->force_path != STEREO_PATH_FAST_F32) { *cls = CLS_U8; return STEREO_OK; }
@@ -331,13 +375,9 @@ static int run_f32_pair(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
     const Problem& p = ps[0];
     int rc = reserve_arena(ctx, st, f32_scratch_bytes(ctx, p, n));
     if (rc != STEREO_OK) return rc;
-    ctx->arena.reset();
-    const size_t pitch = align256(p.cols);
-    uint8_t* a8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
-    uint8_t* b8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
-    if (!a8 || !b8) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
+    ImageView u8[2];
     int cls = CLS_EXACT;
-    rc = classify_images(ctx, p, st, a8, b8, pitch, &cls);
+    rc = classify_images(ctx, p, st, u8, &cls);
     if (rc != STEREO_OK) return rc;
     if (cls == CLS_EXACT) {
         for (int d = 0; d < n && rc == STEREO_OK; ++d) rc = run_exact_direction(ctx, ps[d], st);
@@ -345,7 +385,7 @@ static int run_f32_pair(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
     }
     if (cls == CLS_U8) {
         // ps[0]: ref = left, tgt = right; ps[1] the other way round
-        ps[0].ref = ImageView{a8, pitch, PixType::U8}; ps[0].tgt = ImageView{b8, pitch, PixType::U8};
+        ps[0].ref = u8[0]; ps[0].tgt = u8[1];
         if (n == 2) { ps[1].ref = ps[0].tgt; ps[1].tgt = ps[0].ref; }
     }
     ctx->last_path = cls == CLS_U8 ? STEREO_PATH_FAST_U8 : STEREO_PATH_FAST_F32;
@@ -404,17 +444,12 @@ static SgmShape sgm_shape(const Problem& p) {
     return SgmShape{dlo, D, K, size_t(32) * K};
 }
 
-static size_t sgm_padded_elems(const Problem& p) {
-    return size_t(p.rows + 2 * p.R) * (p.cols + 2 * p.R) + 2 * (size_t(p.R) + 64);
-}
-
 // One direction's scratch: both padded images, the cost volume and the aggregate (plus, for float images, the u8 copies
 // the classification writes).  Directions of a call run one after the other on the same scratch.
 static size_t sgm_scratch_bytes(const Problem& p) {
     const size_t cells = size_t(p.rows) * p.cols * sgm_shape(p).Dp;
-    size_t need = 2 * align256(sgm_padded_elems(p) * sizeof(float)) + 2 * align256(cells * 4) + 4096;
-    if (p.ref.type == PixType::F32) need += 2 * align256(size_t(p.rows) * align256(p.cols));
-    return need;
+    const size_t need = 2 * align256(padded_elems(p) * sizeof(float)) + 2 * align256(cells * 4) + 4096;
+    return p.ref.type == PixType::F32 ? need + u8_copies_bytes(p) : need;
 }
 
 // Every L_r is at most C_max + P2 with C_max = (2R + 1)^2 M, M the largest per-element term: S stays in int32 when
@@ -426,41 +461,17 @@ static int check_sgm_bound(const stereo_ctx* ctx, int R, double M) {
     return STEREO_ERR_UNSUPPORTED;
 }
 
-// What an SGM pair call must satisfy before anything is staged or enqueued: the SSD cost and whole maps (paths cross
-// band seams).  run_sgm checks the candidate count and the int32 bound.
-static int check_sgm_call(const stereo_ctx* ctx, int cost, int row_begin, int row_end, int rows) {
-    if (ctx->sgm_paths <= 0) return STEREO_OK;
-    if (cost != STEREO_COST_SSD) { set_error("SGM aggregates the SSD cost only (switch it off for NCC calls)"); return STEREO_ERR_UNSUPPORTED; }
-    if (row_begin != 0 || row_end != rows) {
-        set_error("SGM: rows [%d, %d) are not the whole map (vertical and diagonal paths cross band seams)", row_begin, row_end);
-        return STEREO_ERR_UNSUPPORTED;
-    }
-    return STEREO_OK;
-}
-
 // One direction by SGM into p.disp, on scratch the caller reserved.  ref / tgt: the caller's images (u8 or float).
 static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st) {
     static constexpr int DIRS[8][2] = {{0, 1}, {0, -1}, {1, 0}, {-1, 0}, {1, 1}, {1, -1}, {-1, 1}, {-1, -1}};
     const SgmShape g = sgm_shape(p);
-    const int Hp = p.rows + 2 * p.R, Wp = p.cols + 2 * p.R;
-    const size_t guard = size_t(p.R) + 64, cells = size_t(p.rows) * p.cols * g.Dp;
-    float* lbuf = static_cast<float*>(ctx->arena.take(sgm_padded_elems(p) * sizeof(float)));
-    float* rbuf = static_cast<float*>(ctx->arena.take(sgm_padded_elems(p) * sizeof(float)));
+    const size_t cells = size_t(p.rows) * p.cols * g.Dp;
+    float *Lp, *Rp;
+    const int rc = pad_images(ctx, p, st, &Lp, &Rp);
+    if (rc != STEREO_OK) return rc;
     int32_t* C = static_cast<int32_t*>(ctx->arena.take(cells * 4));
     int32_t* S = static_cast<int32_t*>(ctx->arena.take(cells * 4));
-    if (!lbuf || !rbuf || !C || !S) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
-    SB_CUDA(cudaMemsetAsync(rbuf, 0, guard * sizeof(float), st));
-    SB_CUDA(cudaMemsetAsync(rbuf + guard + size_t(Hp) * Wp, 0, guard * sizeof(float), st));
-    float* Lp = lbuf + guard;
-    float* Rp = rbuf + guard;
-    dim3 pb(32, 8), pg(div_round_up(Wp, 32), div_round_up(Hp, 8));
-    if (p.ref.type == PixType::F32) {
-        pad_replicate_kernel<float><<<pg, pb, 0, st>>>(static_cast<const float*>(p.ref.ptr), p.ref.step, p.rows, p.cols, p.R, Lp, Hp, Wp, 0, p.rows);
-        pad_replicate_kernel<float><<<pg, pb, 0, st>>>(static_cast<const float*>(p.tgt.ptr), p.tgt.step, p.rows, p.cols, p.R, Rp, Hp, Wp, 0, p.rows);
-    } else {
-        pad_replicate_kernel<uint8_t><<<pg, pb, 0, st>>>(static_cast<const uint8_t*>(p.ref.ptr), p.ref.step, p.rows, p.cols, p.R, Lp, Hp, Wp, 0, p.rows);
-        pad_replicate_kernel<uint8_t><<<pg, pb, 0, st>>>(static_cast<const uint8_t*>(p.tgt.ptr), p.tgt.step, p.rows, p.cols, p.R, Rp, Hp, Wp, 0, p.rows);
-    }
+    if (!C || !S) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
     // rows per cost block: as many as still leave about four blocks per SM (each block recomputes 2R + 1 rows first)
     const long long tiles = (long long)div_round_up(p.cols, SGM_XT) * (g.Dp / 32);
     int rpb = 64;
@@ -468,7 +479,7 @@ static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st)
     const dim3 cg(div_round_up(p.cols, SGM_XT), div_round_up(p.rows, rpb), unsigned(g.Dp / 32));
     const size_t smem = size_t(SGM_XT + 2 * p.R) * 32 * sizeof(int32_t);
     sgm_cost_kernel<<<cg, SGM_COST_THREADS, smem, st>>>(Lp, Rp, p.rows, p.cols, p.R, g.dlo, g.D, int(g.Dp), rpb, C);
-    ctx->last_launches += 3;
+    ctx->last_launches += 1;
     for (int k = 0; k < ctx->sgm_paths; ++k) {
         const int dy = DIRS[k][0], dx = DIRS[k][1];
         const bool last = k == ctx->sgm_paths - 1;
@@ -506,12 +517,8 @@ static int run_sgm(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bool u8
     if (rc != STEREO_OK) return rc;
     if (!u8) {
         const Problem& p = ps[0];
-        ctx->arena.reset();
-        const size_t pitch = align256(p.cols);
-        uint8_t* a8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
-        uint8_t* b8 = static_cast<uint8_t*>(ctx->arena.take(size_t(p.rows) * pitch));
-        if (!a8 || !b8) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
-        rc = classify_flags(ctx, p, st, a8, b8, pitch);
+        ImageView copies[2];
+        rc = classify_flags(ctx, p, st, copies);
         if (rc != STEREO_OK) return rc;
         const unsigned flags = *reinterpret_cast<const unsigned*>(ctx->h_flag);
         if (flags & 2u) { set_error("SGM: an image holds a pixel that is not finite"); return STEREO_ERR_UNSUPPORTED; }
@@ -530,8 +537,7 @@ static int run_sgm(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bool u8
 }
 
 // Validates every direction, runs them - pairs with the context's SGM on by SGM, everything else on the kernel family
-// run_families picks - then, pairs with the context's left-right check or speckle filter on, checks and filters the
-// pairs' maps, in that order (StereoSGBM's).
+// run_families picks - then finishes pairs with the context's left-right check and speckle filter (finish_pairs).
 static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
     bool fast = ctx->force_path != STEREO_PATH_EXACT_F32, u8 = true;
     for (int i = 0; i < n; ++i) {
@@ -543,24 +549,15 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
         fast = fast && fast_supported(p);
         u8 = u8 && p.ref.type == PixType::U8;
     }
-    const bool lr = n >= 2 && ctx->lr_max_diff >= 0, spk = n >= 2 && ctx->spk_max_size > 0, sgm = n >= 2 && ctx->sgm_paths > 0;
-    if (sgm) {
-        const int rc = check_sgm_call(ctx, ps[0].cost, ps[0].row_begin, ps[0].row_end, ps[0].rows);
+    const bool pair = n >= 2;      // (every pair of a call has the same shape, band, range and element type)
+    if (pair) {
+        const Problem& p = ps[0];
+        int rc = check_pair_options(ctx, p.cost, p.disp.elem, ps[n / 2].dmax, p.row_begin, p.row_end, p.rows);
+        if (rc == STEREO_OK) rc = reserve_arena(ctx, st, finish_scratch_bytes(ctx, n, p.rows, p.cols));
         if (rc != STEREO_OK) return rc;
     }
-    for (int k = 0; (lr || spk) && k < n / 2; ++k) {
-        const int rc = check_lr_sentinel(ps[k].disp.elem, ps[n / 2 + k].dmax);
-        if (rc != STEREO_OK) return rc;
-    }
-    if (spk) {
-        int rc = check_speckle_band(ctx, ps[0].row_begin, ps[0].row_end, ps[0].rows);
-        if (rc == STEREO_OK) rc = reserve_arena(ctx, st, speckle_scratch_bytes(n, ps[0].rows, ps[0].cols));
-        if (rc != STEREO_OK) return rc;
-    }
-    int rc = sgm ? run_sgm(ctx, ps, n, st, u8) : run_families(ctx, ps, n, st, fast, u8);
-    if (rc == STEREO_OK && lr) rc = lr_check_pairs(ctx, ps, n, st);
-    if (rc == STEREO_OK && spk) rc = speckle_pairs(ctx, ps, n, st);
-    return rc;
+    const int rc = pair && ctx->sgm_paths > 0 ? run_sgm(ctx, ps, n, st, u8) : run_families(ctx, ps, n, st, fast, u8);
+    return rc == STEREO_OK && pair ? finish_pairs(ctx, ps, n, st, true) : rc;
 }
 
 // Every call of a context shares one scratch arena (and the classification flag), so calls are ordered: a call
@@ -812,7 +809,8 @@ static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, in
     }
     // pairs with the speckle filter: an item's maps are filtered whole after its last band, then downloaded
     const bool spk = n_dirs == 2 && ctx->spk_max_size > 0;
-    if (spk && speckle_scratch_bytes(2 * cp, rows, cols) > scratch) scratch = speckle_scratch_bytes(2 * cp, rows, cols);
+    const size_t finish = n_dirs == 2 ? finish_scratch_bytes(ctx, 2 * cp, rows, cols) : 0;
+    if (finish > scratch) scratch = finish;
     constexpr int NSTG = 4;                               // pinned staging ring of the host-packed uploads
     int rc = ensure_pipe(ctx, 3 * n_units + 4 + NSTG);
     if (rc != STEREO_OK) return rc;
@@ -1003,12 +1001,7 @@ static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, in
                     for (int k = 0; k < nj && rc == STEREO_OK; ++k) { ctx->arena.reset(); rc = run_fast(ctx, pd[k], s_cmp); }
                 }
                 // two directions: pd holds the np left-referenced problems, then their partners
-                if (rc == STEREO_OK && n_dirs == 2 && ctx->lr_max_diff >= 0) rc = lr_check_pairs(ctx, pd, nj, s_cmp);
-                if (rc == STEREO_OK && spk && b == nbw(w) - 1) {
-                    OutView maps[2 * PIPE_CPMAX];
-                    for (int k = 0; k < nj; ++k) maps[k] = OutView{sl[k % np].out[k / np], d_pitch, elem};
-                    rc = speckle_maps(ctx, maps, nj, rows, cols, -(dirs[1].dmax + 1), ctx->spk_max_size, ctx->spk_max_diff, s_cmp);
-                }
+                if (rc == STEREO_OK && n_dirs == 2) rc = finish_pairs(ctx, pd, nj, s_cmp, b == nbw(w) - 1);
                 if (rc != STEREO_OK) return rc;
             }
             SB_CUDA(cudaEventRecord(ev(w, b, 1), s_cmp));
@@ -1047,9 +1040,8 @@ static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, in
 
 // What every host entry point checks before it touches a buffer: the context, non-null pointers, an image of at most
 // 32768 pixels a side (validate() reports larger ones to device callers as UNSUPPORTED), a disparity element of 1, 2 or
-// 4 bytes and every {step, row bytes} step at least its row.  A pair's negative `range` is rejected with `range_rc`, and
-// with the left-right check or the speckle filter on, a `range` whose sentinel does not fit `elem` (single directions pass
-// range 0).
+// 4 bytes and every {step, row bytes} step at least its row.  A pair's negative `range` is rejected with `range_rc` (single
+// directions pass range 0).
 static int check_host_args(stereo_ctx* ctx, std::initializer_list<const void*> ptrs, int rows, int cols, int elem,
                            std::initializer_list<std::pair<size_t, size_t>> steps, int range = 0,
                            int range_rc = STEREO_ERR_INVALID_RANGE) {
@@ -1062,7 +1054,7 @@ static int check_host_args(stereo_ctx* ctx, std::initializer_list<const void*> p
     for (const auto& s : steps)
         if (s.first < s.second) { set_error("a step is smaller than its row"); return STEREO_ERR_INVALID_ARG; }
     if (range < 0) { set_error("disparity_range must be >= 0"); return range_rc; }
-    return ctx->lr_max_diff >= 0 || ctx->spk_max_size > 0 ? check_lr_sentinel(elem, range) : STEREO_OK;
+    return STEREO_OK;
 }
 
 // Sequential host call: upload (2D async copies), compute, download, synchronize - the shape of cuda::disparitySSD
@@ -1449,13 +1441,8 @@ int stereo_lr_check_device(stereo_ctx* ctx, void* disp_left, void* disp_right, s
     if (rc != STEREO_OK) return rc;
     cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream;
     begin_call(ctx, st);
-    LrParams P{};
-    P.pair[0] = LrMaps{disp_left, disp_right, disp_step, disp_step};
-    P.cols = cols;
-    P.max_diff = max_diff;
-    P.sentinel = -(disparity_range + 1);
-    ctx->last_launches = 1;
-    rc = lr_check_launch(P, rows, 1, disp_elem_bytes, st);
+    const OutView maps[2] = {{disp_left, disp_step, disp_elem_bytes}, {disp_right, disp_step, disp_elem_bytes}};
+    rc = lr_check_pairs(ctx, maps, 1, rows, cols, max_diff, -(disparity_range + 1), st);
     end_call(ctx, st);
     return rc;
 }
@@ -1804,7 +1791,7 @@ static int pair_host(stereo_ctx* ctx, int cost, PixType type, const void* left, 
     const size_t row = size_t(cols) * (type == PixType::F32 ? 4 : 1), disp_row = size_t(cols) * elem;
     int rc = check_host_args(ctx, {left, right, disp_left, disp_right}, rows, cols, elem,
                              {{left_step, row}, {right_step, row}, {disp_step, disp_row}}, range);
-    if (rc == STEREO_OK) rc = check_sgm_call(ctx, cost, 0, rows, rows);      // (as run_directions would, but before staging)
+    if (rc == STEREO_OK) rc = check_pair_options(ctx, cost, elem, range, 0, rows, rows);      // (as run_directions would, but before staging)
     if (rc != STEREO_OK) return rc;
     {
         const HostPairIn in{left, left_step, right, right_step};
@@ -1888,8 +1875,7 @@ static int pair_band_host(stereo_ctx* ctx, int cost, PixType type, const void* l
     int h0 = 0, h1 = 0;
     rc = stereo_band_halo_rows(rows, row_begin, row_end, R, &h0, &h1);      // (rejects a bad band or window radius)
     if (rc != STEREO_OK) return rc;
-    rc = check_speckle_band(ctx, row_begin, row_end, rows);      // (as run_directions would, but before staging)
-    if (rc == STEREO_OK) rc = check_sgm_call(ctx, cost, row_begin, row_end, rows);
+    rc = check_pair_options(ctx, cost, elem, range, row_begin, row_end, rows);      // (as run_directions would, but before staging)
     if (rc != STEREO_OK) return rc;
     const int nh = h1 - h0;
     HostRows in[2] = {{static_cast<const char*>(left) + size_t(h0) * left_step, left_step, size_t(cols)},
@@ -1973,7 +1959,7 @@ static int pair_batch_host(stereo_ctx* ctx, int cost, PixType type, int n_pairs,
     if (n_pairs <= 0) { set_error("n_pairs must be positive"); return STEREO_ERR_INVALID_ARG; }
     int rc = check_host_args(ctx, {left, right, disp_left, disp_right}, rows, cols, disp_elem_bytes,
                              {{img_step, size_t(cols) * px}, {disp_step, size_t(cols) * disp_elem_bytes}}, disparity_range);
-    if (rc == STEREO_OK) rc = check_sgm_call(ctx, cost, 0, rows, rows);
+    if (rc == STEREO_OK) rc = check_pair_options(ctx, cost, disp_elem_bytes, disparity_range, 0, rows, rows);
     if (rc != STEREO_OK) return rc;
     {   // pipelined: item i+1 uploads while item i computes and item i-1 downloads (3 device slots)
         std::vector<HostPairIn> in(n_pairs);

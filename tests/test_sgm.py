@@ -12,12 +12,12 @@ from introtocomputervision_b200 import _capi, synth
 from lr_oracle import lr_check
 from sgm_oracle import sgm_pair
 from speckle_oracle import filter_speckles
-from test_lr_check import FAMILIES, RANGE_T, _images, _run
-from test_speckle_filter import ENTRIES, _device_batch, _run_whole
+from pair_calls import FAMILIES, RANGE_T, _device_batch, _images, _run
 
 pytestmark = pytest.mark.gpu
 
 ARG, UNSUP = _capi.ERR_INVALID_ARG, _capi.ERR_UNSUPPORTED
+ENTRIES = ["pair_host", "pair_device", "batch_device", "batch_host", "band_host", "band_halo_device", "mgpu_batch"]
 
 
 def _torch():
@@ -96,7 +96,7 @@ def test_every_pair_entry_point_equals_the_restatement(gctx, mg, entry, kind):
     for paths, p1, p2, R, rng, dt, lr, spk in CONFIGS:
         _set(h, paths, p1, p2, lr, spk)
         try:
-            on = _run_whole(h, entry, sb.COST_SSD, Ls, Rs, R, rng, dt)
+            on = _run(h, entry, sb.COST_SSD, Ls, Rs, R, rng, dt, bands=[(0, Ls.shape[1])])
         finally:
             _reset(h)
         want = _expected(Ls, Rs, R, rng, dt, paths, p1, p2, lr, spk)

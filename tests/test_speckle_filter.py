@@ -13,8 +13,8 @@ import introtocomputervision_b200 as sb
 from introtocomputervision_b200 import _capi, synth
 from lr_oracle import lr_check
 from speckle_oracle import filter_speckles
+from pair_calls import FAMILIES, RANGE_T, _device_batch, _images, _run, _set_fuse
 from test_entry_points import EXPECTED, PITCH, ROWS, _args
-from test_lr_check import FAMILIES, RANGE_T, _images, _run, _set_fuse
 
 pytestmark = pytest.mark.gpu
 
@@ -187,42 +187,15 @@ def test_kernel_alone_argument_checks(sctx):
 ENTRIES = ["pair_host", "pair_device", "batch_device", "batch_host", "band_host", "band_halo_device", "mgpu_batch"]
 
 
-def _run_whole(h, entry, cost, Ls, Rs, win, rng, dt):
-    """_run, with the band entry points called once for the whole image."""
-    if entry not in ("band_host", "band_halo_device"):
-        return _run(h, entry, cost, Ls, Rs, win, rng, dt)
-    lib = _capi.lib()
-    n, rows, cols = Ls.shape
-    dt = np.dtype(dt)
-    elem = dt.itemsize
-    out_l, out_r = np.empty((n, rows, cols), dt), np.empty((n, rows, cols), dt)
-    for i in range(n):
-        L, R = np.ascontiguousarray(Ls[i]), np.ascontiguousarray(Rs[i])
-        if entry == "band_host":
-            fn = lib.stereo_disparity_pair_band_f32_host if L.dtype == np.float32 else lib.stereo_disparity_pair_band_u8_host
-            _ok(fn(h.handle, cost, L.ctypes.data, L.strides[0], R.ctypes.data, R.strides[0], rows, cols, 0, rows, win, rng,
-                   out_l[i].ctypes.data, out_r[i].ctypes.data, cols * elem, elem), entry)
-        else:
-            torch = _torch()
-            tl, tr = torch.from_numpy(L).cuda(), torch.from_numpy(R).cuda()
-            ol = torch.empty((rows, cols), dtype={1: torch.int8, 2: torch.int16, 4: torch.int32}[elem], device="cuda")
-            orr = torch.empty_like(ol)
-            _ok(lib.stereo_disparity_pair_band_halo_u8_device(h.handle, cost, tl.data_ptr(), cols, tr.data_ptr(), cols, rows, cols, 0, rows,
-                                                              0, rows, win, rng, ol.data_ptr(), orr.data_ptr(), cols * elem, elem,
-                                                              C.c_void_p(torch.cuda.current_stream().cuda_stream)), entry)
-            torch.cuda.synchronize()
-            out_l[i], out_r[i] = ol.cpu().numpy(), orr.cpu().numpy()
-    return out_l, out_r
-
-
 def _filtered_equals_oracle_of_off(h, entry, cost, Ls, Rs, win, rng, dt, lr, max_size=MAX_SIZE, max_diff=MAX_DIFF, min_share=0.001):
+    whole = [(0, Ls.shape[1])]          # (the band entry points take only a whole-image band with the filter on)
     try:
         h.set_lr_check(None)
         h.set_speckle_filter(None)
-        off = _run_whole(h, entry, cost, Ls, Rs, win, rng, dt)
+        off = _run(h, entry, cost, Ls, Rs, win, rng, dt, bands=whole)
         h.set_lr_check(1 if lr else None)
         h.set_speckle_filter(max_size, max_diff)
-        on = _run_whole(h, entry, cost, Ls, Rs, win, rng, dt)
+        on = _run(h, entry, cost, Ls, Rs, win, rng, dt, bands=whole)
     finally:
         h.set_lr_check(None)
         h.set_speckle_filter(None)
@@ -289,18 +262,6 @@ def test_launches_of_a_filtered_pair_call(sctx):
 
 
 # ---- 3. / 4. full-size batches ---------------------------------------------------------------------------------------
-
-def _device_batch(ctx, Ls, Rs, win, rng, elem):
-    torch = _torch()
-    n, rows, cols = Ls.shape
-    tl, tr = torch.from_numpy(Ls).cuda(), torch.from_numpy(Rs).cuda()
-    out = torch.empty((2, n, rows, cols), dtype={1: torch.int8, 2: torch.int16}[elem], device="cuda")
-    _ok(_capi.lib().stereo_disparity_pair_batch_u8_device(ctx.handle, sb.COST_SSD, n, tl.data_ptr(), tr.data_ptr(), cols, rows * cols,
-                                                          rows, cols, win, rng, out[0].data_ptr(), out[1].data_ptr(), cols * elem,
-                                                          rows * cols * elem, elem, C.c_void_p(torch.cuda.current_stream().cuda_stream)))
-    torch.cuda.synchronize()
-    return out.cpu().numpy()
-
 
 @pytest.mark.parametrize("shape,nd,win,n,elem", [((720, 1280), 64, 4, 16, 1), ((2160, 3840), 256, 5, 1, 2)])
 def test_full_size_batch_equals_the_oracle(sctx, shape, nd, win, n, elem):
