@@ -2,8 +2,9 @@
 to it: R > 7, more than 4096 candidates, the FAST_F32 value-range bound for SSD at its edge, the classification of single
 edge values, and the float NCC family across DC offsets.
 
-SSD: bit-exact disparities and costs against oracle.ssd / oracle.ssd_fast.  NCC: the BASELINE contract (>= 99.9 % equal
-disparities, scores within 1e-5) against the literal oracle.ncorr.  Every value stays where the reference is defined: per
+SSD: bit-exact disparities and costs against oracle.ssd / oracle.ssd_fast.  NCC: against the literal oracle.ncorr, the exact
+family identical (tests/ncc_check.py, tau = 0), the fast families within their key resolution at every pixel, plus the BASELINE
+contract (>= 99.9 % equal disparities, scores within 1e-5).  Every value stays where the reference is defined: per
 element (l - r)^2 < 2^31 and window sums within int32."""
 import ctypes as C
 
@@ -12,6 +13,7 @@ import pytest
 
 import oracle
 import exact_cases as ec
+import ncc_check as nc
 from lr_oracle import lr_check
 from speckle_oracle import filter_speckles
 import introtocomputervision_b200 as sb
@@ -20,7 +22,6 @@ from introtocomputervision_b200 import _capi, synth
 pytestmark = pytest.mark.gpu
 
 NCC_SCORE_RTOL = 1e-5
-NCC_DISP_AGREE = 0.999
 UNSUP, RANGE = _capi.ERR_UNSUPPORTED, _capi.ERR_INVALID_RANGE
 
 
@@ -38,10 +39,10 @@ def _tdt(dt):
     return {1: t.int8, 2: t.int16, 4: t.int32}[np.dtype(dt).itemsize]
 
 
-def assert_ncc_close(d, s, d_ref, s_ref):
-    agree = float(np.mean(d == d_ref))
-    assert agree >= NCC_DISP_AGREE, f"disparity agreement {agree:.5f}"
+def assert_ncc_close(d, s, d_ref, s_ref, ref, tgt, R, dmin, dmax, family):
+    nc.check_ncc_map(d, ref, tgt, R, dmin, dmax, family, oracle_disp=d_ref)
     np.testing.assert_allclose(s, s_ref, rtol=NCC_SCORE_RTOL, atol=1e-7)
+    nc.check_best(s, d, ref, tgt, R, dmin, dmax, mask=d != d_ref)
 
 
 def _mgpu_devices():
@@ -106,7 +107,7 @@ def test_exact_shapes_ncc_vs_oracle(ctx, rows, cols, R, dmin, dmax, dt):
             continue
         d, s = ctx.disparity(sb.COST_NCORR, a, b, R, dmin, dmax, dtype=np.int32, return_best=True)
         assert ctx.last_path == sb.PATH_EXACT_F32, name
-        assert_ncc_close(d, s, d_ref, s_ref)
+        assert_ncc_close(d, s, d_ref, s_ref, af, bf, R, dmin, dmax, "exact")
         if np.dtype(dt) != np.int32:
             _check_map(ctx.disparity(sb.COST_NCORR, a, b, R, dmin, dmax, dtype=dt), d, dt)
 
@@ -165,13 +166,20 @@ def _ep_refs(cost, kind):
     return _EP_CACHE[key]
 
 
-def _same(cost, got, want):
+def _same(cost, got, want, ncc=None):
+    """SSD: identical maps.  NCC: ncc = (ref, tgt, R, dmin, dmax, family) of the map, checked pixel by pixel (ncc_check)."""
     if cost == sb.COST_SSD:
         bad = np.argwhere(got != want.astype(got.dtype))
         assert bad.size == 0, f"differs at {bad[:5].tolist()} (of {len(bad)})"
     else:
-        agree = float(np.mean(got == want.astype(got.dtype)))
-        assert agree >= NCC_DISP_AGREE, agree
+        ref, tgt, R, dmin, dmax, family = ncc
+        nc.check_ncc_map(got, ref, tgt, R, dmin, dmax, family, oracle_disp=want)
+
+
+def _ep(a, b, side):
+    """The NCC check arguments of the EP shape's L->R (side 0) or R->L (side 1) map of images a, b (EXACT_F32: R > 7)."""
+    a, b = a.astype(np.float32), b.astype(np.float32)
+    return (a, b, EP_R, -EP_RNG, 0, "exact") if side == 0 else (b, a, EP_R, 0, EP_RNG, "exact")
 
 
 def _single_device(ctx, cost, a, b, dmin, dmax, f32):
@@ -248,18 +256,18 @@ def test_every_pair_entry_point_reaches_the_exact_family(ctx, cost, entry, kind)
     Ls, Rs, refs = _ep_refs(cost, kind)
     dl, dr = _pair_entry(ctx, entry, cost, Ls[0], Rs[0])
     assert ctx.last_path == sb.PATH_EXACT_F32
-    _same(cost, dl, refs[0][0])
-    _same(cost, dr, refs[0][1])
+    _same(cost, dl, refs[0][0], _ep(Ls[0], Rs[0], 0))
+    _same(cost, dr, refs[0][1], _ep(Ls[0], Rs[0], 1))
 
 
 @pytest.mark.parametrize("cost", [sb.COST_SSD, sb.COST_NCORR])
 @pytest.mark.parametrize("kind", ["u8", "f32"])
 def test_single_host_and_device_reach_the_exact_family(ctx, cost, kind):
     Ls, Rs, refs = _ep_refs(cost, kind)
-    for a, b, dmin, dmax, want in ((Ls[0], Rs[0], -EP_RNG, 0, refs[0][0]), (Rs[0], Ls[0], 0, EP_RNG, refs[0][1])):
-        _same(cost, ctx.disparity(cost, a, b, EP_R, dmin, dmax, dtype=EP_DT), want)
+    for side, (a, b, dmin, dmax, want) in enumerate(((Ls[0], Rs[0], -EP_RNG, 0, refs[0][0]), (Rs[0], Ls[0], 0, EP_RNG, refs[0][1]))):
+        _same(cost, ctx.disparity(cost, a, b, EP_R, dmin, dmax, dtype=EP_DT), want, _ep(Ls[0], Rs[0], side))
         assert ctx.last_path == sb.PATH_EXACT_F32
-        _same(cost, _single_device(ctx, cost, a, b, dmin, dmax, kind == "f32"), want)
+        _same(cost, _single_device(ctx, cost, a, b, dmin, dmax, kind == "f32"), want, _ep(Ls[0], Rs[0], side))
         assert ctx.last_path == sb.PATH_EXACT_F32
 
 
@@ -292,8 +300,8 @@ def test_batch_and_multi_gpu_entry_points_reach_the_exact_family(ctx, cost, entr
                 pairs = [mg.disparity_pair_bands(cost, Ls[i], Rs[i], EP_R, EP_RNG, dtype=EP_DT) for i in range(n)]
                 bl, br = np.stack([p[0] for p in pairs]), np.stack([p[1] for p in pairs])
     for i in range(n):
-        _same(cost, bl[i], refs[i][0])
-        _same(cost, br[i], refs[i][1])
+        _same(cost, bl[i], refs[i][0], _ep(Ls[i], Rs[i], 0))
+        _same(cost, br[i], refs[i][1], _ep(Ls[i], Rs[i], 1))
 
 
 def test_pair_band_f32_host_refuses_images_that_are_not_8bit(ctx):
@@ -465,7 +473,7 @@ def test_single_edge_value_classifies_and_matches_the_oracle(ctx, rows, cols, va
         n_ref, s_ref = oracle.ncorr(Lf, Rf, CLS_R, CLS_DMIN, 0, return_score=True)
         n, s = ctx.disparity(sb.COST_NCORR, Lf, Rf, CLS_R, CLS_DMIN, 0, dtype=np.int32, return_best=True)
         assert ctx.last_path == path, (y, x)
-        assert_ncc_close(n, s, n_ref, s_ref)
+        assert_ncc_close(n, s, n_ref, s_ref, Lf, Rf, CLS_R, CLS_DMIN, 0, nc.family_of(ctx))
 
 
 @pytest.mark.parametrize("rows,cols", CLS_SHAPES)
@@ -504,7 +512,9 @@ def test_non_finite_pixel_routes_to_the_exact_family(ctx, rows, cols, value):
         n_ref, s_ref = oracle.ncorr(Lf, Rf, CLS_R, CLS_DMIN, 0, return_score=True)
         n, s = ctx.disparity(sb.COST_NCORR, Lf, Rf, CLS_R, CLS_DMIN, 0, dtype=np.int32, return_best=True)
         assert ctx.last_path == sb.PATH_EXACT_F32, (y, x)
-        assert_ncc_close(n[clean], s[clean], n_ref[clean], s_ref[clean])
+        # (the exact kernels ARE the literal oracle: identical wherever the reference is defined)
+        assert np.array_equal(n[clean], n_ref[clean]), (y, x)
+        assert np.array_equal(s[clean].view(np.uint32), s_ref[clean].view(np.uint32)), (y, x)
 
 
 @pytest.mark.parametrize("cost", [sb.COST_SSD, sb.COST_NCORR])
@@ -518,8 +528,10 @@ def test_host_f32_batch_with_one_exact_pair(ctx, cost):
     fn = oracle.ssd_fast if cost == sb.COST_SSD else oracle.ncorr
     for i in range(n):
         want_l, want_r = fn(Ls[i], Rs[i], R, -rng, 0), fn(Rs[i], Ls[i], R, 0, rng)
-        _same(cost, bl[i], want_l)
-        _same(cost, br[i], want_r)
+        # NCC: pair 2 (x5, not 8-bit) takes the float kernels, the others the packed ones, fused or not ("u8" covers both)
+        family = "f32" if i == 2 else "u8"
+        _same(cost, bl[i], want_l, (Ls[i], Rs[i], R, -rng, 0, family))
+        _same(cost, br[i], want_r, (Rs[i], Ls[i], R, 0, rng, family))
     dl, _ = ctx.disparity_pair(cost, Ls[2], Rs[2], R, rng, dtype=np.int16)
     assert ctx.last_path == (sb.PATH_EXACT_F32 if cost == sb.COST_SSD else sb.PATH_FAST_F32)
     assert np.array_equal(dl, bl[2])
@@ -543,13 +555,15 @@ def _ncc_agreement(ctx, Lf, Rf):
     d_ref, s_ref = oracle.ncorr(Lf, Rf, R, -D, 0, return_score=True)
     r_ref = oracle.ncorr(Rf, Lf, R, 0, D)
     d, s = ctx.disparity(sb.COST_NCORR, Lf, Rf, R, -D, 0, dtype=np.int32, return_best=True)
-    path = ctx.last_path
+    path, family = ctx.last_path, nc.family_of(ctx)
     dl, dr = ctx.disparity_pair(sb.COST_NCORR, Lf, Rf, R, D, dtype=np.int16)
     assert ctx.last_path == path
+    pair_family = nc.family_of(ctx)
     agree = (float(np.mean(d == d_ref)), float(np.mean(dl == d_ref)), float(np.mean(dr == r_ref)))
     print(f"NCC agreement path={path} single={agree[0]:.5f} pair L->R={agree[1]:.5f} R->L={agree[2]:.5f}")
-    assert_ncc_close(d, s, d_ref, s_ref)
-    assert min(agree) >= NCC_DISP_AGREE, agree
+    assert_ncc_close(d, s, d_ref, s_ref, Lf, Rf, R, -D, 0, family)
+    nc.check_ncc_map(dl, Lf, Rf, R, -D, 0, pair_family, oracle_disp=d_ref, what="pair L->R")
+    nc.check_ncc_map(dr, Rf, Lf, R, 0, D, pair_family, oracle_disp=r_ref, what="pair R->L")
     return path
 
 

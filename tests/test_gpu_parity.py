@@ -1,12 +1,14 @@
 """GPU parity tests: the CUDA path, called through the C ABI, against the oracle on the same inputs.
 
 SSD: bit-exact disparities (and costs).  NCC: winning score within 1e-5 relative and disparity equal
-on >= 99.9 % of pixels (BASELINE.json north_star); the exact path is expected to be identical.
+on >= 99.9 % of pixels (BASELINE.json north_star); every pixel that differs names a candidate whose oracle score is within
+the key resolution of the oracle's winner (tests/ncc_check.py), and the exact path is identical.
 """
 import numpy as np
 import pytest
 
 import oracle
+import ncc_check as nc
 import introtocomputervision_b200 as sb
 from introtocomputervision_b200 import synth
 
@@ -21,10 +23,12 @@ def _cases(cost):
     return Golden().names(cost)
 
 
-def assert_ncc_close(d, s, d_ref, s_ref):
-    agree = float(np.mean(d == d_ref))
-    assert agree >= NCC_DISP_AGREE, f"disparity agreement {agree:.5f}"
+def assert_ncc_close(d, s, d_ref, s_ref, ref, tgt, R, dmin, dmax, family, min_agree=NCC_DISP_AGREE):
+    """Per-pixel check of the map against the oracle's (ncc_check), the north-star fraction, the scores within 1e-5, and where
+    the disparity differs the returned score is the oracle's score of the returned candidate, bit for bit."""
+    nc.check_ncc_map(d, ref, tgt, R, dmin, dmax, family, oracle_disp=d_ref, min_agree=min_agree)
     np.testing.assert_allclose(s, s_ref, rtol=NCC_SCORE_RTOL, atol=1e-7)
+    nc.check_best(s, d, ref, tgt, R, dmin, dmax, mask=d != d_ref)
 
 
 # ---- golden vectors (reference-generated) ----------------------------------------------------------
@@ -44,12 +48,12 @@ def test_ssd_golden(ctx, golden, name, R, dmin, dmax):
 def test_ncc_golden(ctx, golden, name, R, dmin, dmax):
     g = golden.get("ncc", name)
     L, Rt = g["left"], g["right"]
-    d, s = ctx.disparity(sb.COST_NCORR, L.astype(np.float32), Rt.astype(np.float32), R, dmin, dmax,
-                         dtype=np.int16, return_best=True)
-    assert_ncc_close(d, s, g["disp"], g["score"])
+    Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
+    d, s = ctx.disparity(sb.COST_NCORR, Lf, Rf, R, dmin, dmax, dtype=np.int16, return_best=True)
+    assert_ncc_close(d, s, g["disp"], g["score"], Lf, Rf, R, dmin, dmax, nc.family_of(ctx))
     if L.dtype == np.uint8:
         d8, s8 = ctx.disparity(sb.COST_NCORR, L, Rt, R, dmin, dmax, dtype=np.int16, return_best=True)
-        assert_ncc_close(d8, s8, g["disp"], g["score"])
+        assert_ncc_close(d8, s8, g["disp"], g["score"], Lf, Rf, R, dmin, dmax, nc.family_of(ctx))
 
 
 # ---- seeded random inputs against the oracle ----------------------------------------------------------
@@ -90,7 +94,7 @@ def test_ncc_random_vs_oracle(ctx, seed):
         Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
     d_ref, s_ref = oracle.ncorr(Lf, Rf, R, dmin, dmax, return_score=True)
     d, s = ctx.disparity(sb.COST_NCORR, Lf, Rf, R, dmin, dmax, dtype=np.int32, return_best=True)
-    assert_ncc_close(d, s, d_ref, s_ref)
+    assert_ncc_close(d, s, d_ref, s_ref, Lf, Rf, R, dmin, dmax, nc.family_of(ctx))
 
 
 # ---- BASELINE config shapes ------------------------------------------------------------------------------
@@ -123,7 +127,7 @@ def test_ncc_pair1_band_variants_vs_oracle(ctx):
         for (a, b, dmin, dmax) in ((Lf, Rf, -95, 0), (Rf, Lf, 0, 95)):
             d_ref, s_ref = oracle.ncorr(a, b, 7, dmin, dmax, return_score=True)
             d, s = ctx.disparity(sb.COST_NCORR, a, b, 7, dmin, dmax, dtype=np.int16, return_best=True)
-            assert_ncc_close(d, s, d_ref, s_ref)
+            assert_ncc_close(d, s, d_ref, s_ref, a, b, 7, dmin, dmax, nc.family_of(ctx))
 
 
 # ---- API behaviour ------------------------------------------------------------------------------------------
@@ -167,6 +171,7 @@ def test_device_batch_launch_chunks_vs_oracle(ctx, n, rng, R):
         assert rc == 0, _capi.last_error()
         ctx.synchronize()
         assert ctx.last_path == sb.PATH_FAST_U8
+        family = nc.family_of(ctx)
         bl, br = ol.cpu().numpy(), orr.cpu().numpy()
         for i in range(n):
             Lf, Rf = Ls[i].astype(np.float32), Rs[i].astype(np.float32)
@@ -174,8 +179,8 @@ def test_device_batch_launch_chunks_vs_oracle(ctx, n, rng, R):
                 assert np.array_equal(bl[i], oracle.ssd_fast(Lf, Rf, R, -rng, 0)), f"pair {i} L->R"
                 assert np.array_equal(br[i], oracle.ssd_fast(Rf, Lf, R, 0, rng)), f"pair {i} R->L"
             else:
-                assert float(np.mean(bl[i] == oracle.ncorr_fast(Lf, Rf, R, -rng, 0))) >= 0.999
-                assert float(np.mean(br[i] == oracle.ncorr_fast(Rf, Lf, R, 0, rng))) >= 0.999
+                nc.check_ncc_map(bl[i], Lf, Rf, R, -rng, 0, family, what=f"pair {i} L->R")
+                nc.check_ncc_map(br[i], Rf, Lf, R, 0, rng, family, what=f"pair {i} R->L")
 
 
 def test_config5_shape_batch_pairs_vs_oracle(ctx):
@@ -192,8 +197,10 @@ def test_config5_shape_batch_pairs_vs_oracle(ctx):
         assert np.array_equal(bl[i], oracle.narrow_i8(oracle.ssd_fast(Lf, Rf, 4, -63, 0)))
         assert np.array_equal(br[i], oracle.narrow_i8(oracle.ssd_fast(Rf, Lf, 4, 0, 63)))
     nl, nr = ctx.disparity_pair_batch(sb.COST_NCORR, Ls[:1], Rs[:1], 4, 63)
-    assert float(np.mean(nl[0] == oracle.narrow_i8(oracle.ncorr_fast(Ls[0].astype(np.float32), Rs[0].astype(np.float32), 4, -63, 0)))) >= 0.999
-    assert float(np.mean(nr[0] == oracle.narrow_i8(oracle.ncorr_fast(Rs[0].astype(np.float32), Ls[0].astype(np.float32), 4, 0, 63)))) >= 0.999
+    family = nc.family_of(ctx)
+    Lf, Rf = Ls[0].astype(np.float32), Rs[0].astype(np.float32)
+    nc.check_ncc_map(nl[0], Lf, Rf, 4, -63, 0, family, what="L->R")
+    nc.check_ncc_map(nr[0], Rf, Lf, 4, 0, 63, family, what="R->L")
 
 
 def test_wide_disparity_needs_wide_output(ctx):
@@ -244,7 +251,7 @@ def test_device_pointer_and_band_entry_points(ctx):
             if cost == sb.COST_SSD:
                 assert np.array_equal(full.cpu().numpy(), ref.astype(np.int16))
             else:
-                assert float(np.mean(full.cpu().numpy() == ref)) >= NCC_DISP_AGREE
+                nc.check_ncc_map(full.cpu().numpy(), a.cpu().numpy(), b.cpu().numpy(), 4, dmin, dmax, nc.family_of(ctx), oracle_disp=ref)
                 ref = full.cpu().numpy().astype(np.int32)        # bands must reproduce the full call exactly
             # row bands (with the R+1 halo the SSD wrap quirk needs) reproduce the same rows
             for (r0, r1) in ((0, 23), (23, 47), (47, 70)):
@@ -274,9 +281,10 @@ def test_pipelined_host_bands_vs_oracle(ctx, bands):
         assert np.array_equal(ctx.disparity(sb.COST_SSD, Rf, Lf, 5, 0, 39, dtype=np.int16), ref_r)
         # NCC: banded result == whole-image result, and close to the oracle
         dn = ctx.disparity(sb.COST_NCORR, Lf, Rf, 5, -39, 0, dtype=np.int16)
+        family = nc.family_of(ctx)
         ctx.set_pipe_bands(1)
         assert np.array_equal(dn, ctx.disparity(sb.COST_NCORR, Lf, Rf, 5, -39, 0, dtype=np.int16))
-        assert float(np.mean(dn == oracle.ncorr_fast(Lf, Rf, 5, -39, 0))) >= NCC_DISP_AGREE
+        nc.check_ncc_map(dn, Lf, Rf, 5, -39, 0, family)
     finally:
         ctx.set_pipe_bands(0)
 
@@ -314,14 +322,15 @@ def test_host_batch_chunked_items_vs_oracle(ctx, n, kind):
     for cost in (sb.COST_SSD, sb.COST_NCORR):
         bl, br = ctx.disparity_pair_batch(cost, Ls, Rs, R, rng, dtype=np.int16)
         assert ctx.last_path == sb.PATH_FAST_U8
+        family = nc.family_of(ctx)
         for i in range(n):
             Lf, Rf = Ls[i].astype(np.float32), Rs[i].astype(np.float32)
             if cost == sb.COST_SSD:
                 assert np.array_equal(bl[i], oracle.ssd_fast(Lf, Rf, R, -rng, 0)), f"pair {i} L->R"
                 assert np.array_equal(br[i], oracle.ssd_fast(Rf, Lf, R, 0, rng)), f"pair {i} R->L"
             else:
-                assert float(np.mean(bl[i] == oracle.ncorr_fast(Lf, Rf, R, -rng, 0))) >= NCC_DISP_AGREE
-                assert float(np.mean(br[i] == oracle.ncorr_fast(Rf, Lf, R, 0, rng))) >= NCC_DISP_AGREE
+                nc.check_ncc_map(bl[i], Lf, Rf, R, -rng, 0, family, what=f"pair {i} L->R")
+                nc.check_ncc_map(br[i], Rf, Lf, R, 0, rng, family, what=f"pair {i} R->L")
 
 
 @pytest.mark.parametrize("n,kind", [(3, np.float32), (3, np.uint8), (1, np.float32), (2, np.uint8)])
@@ -619,8 +628,8 @@ def test_ncc_fast_u8_vs_oracle(ctx, rows, cols, R, dmin, dmax):
     d_ref, s_ref = oracle.ncorr_fast(L.astype(np.float32), Rt.astype(np.float32), R, dmin, dmax, return_score=True)
     d, s = ctx.disparity(sb.COST_NCORR, L, Rt, R, dmin, dmax, dtype=np.int32, return_best=True)
     assert ctx.last_path == sb.PATH_FAST_U8
-    assert_ncc_close(d, s, d_ref, s_ref)
-    # where the disparity agrees the recomputed score is the oracle's, bit for bit
+    assert_ncc_close(d, s, d_ref, s_ref, L, Rt, R, dmin, dmax, nc.family_of(ctx))
+    # where the disparity agrees the recomputed score is the oracle's, bit for bit (elsewhere: assert_ncc_close)
     same = d == d_ref
     assert np.array_equal(s[same], s_ref[same])
     d2 = ctx.disparity(sb.COST_NCORR, L.astype(np.float32), Rt.astype(np.float32), R, dmin, dmax, dtype=np.int32)
@@ -645,7 +654,7 @@ def test_ncc_fast_flat_dark_and_saturated_images(ctx):
     for (a, b, dmin, dmax) in ((L, Rt, -30, 0), (Rt, L, 0, 30)):
         d_ref, s_ref = oracle.ncorr(a.astype(np.float32), b.astype(np.float32), 3, dmin, dmax, return_score=True)
         d, s = ctx.disparity(sb.COST_NCORR, a, b, 3, dmin, dmax, dtype=np.int32, return_best=True)
-        assert_ncc_close(d, s, d_ref, s_ref)
+        assert_ncc_close(d, s, d_ref, s_ref, a, b, 3, dmin, dmax, nc.family_of(ctx))
 
 
 def test_ncc_fast_smooth_low_texture(ctx):
@@ -656,9 +665,8 @@ def test_ncc_fast_smooth_low_texture(ctx):
     Rt = np.clip(60 + 0.3 * (xx + 7) + 0.2 * yy + rng.integers(-3, 4, xx.shape), 0, 255).astype(np.uint8)
     d_ref, s_ref = oracle.ncorr_fast(L.astype(np.float32), Rt.astype(np.float32), 4, -40, 0, return_score=True)
     d, s = ctx.disparity(sb.COST_NCORR, L, Rt, 4, -40, 0, dtype=np.int32, return_best=True)
-    np.testing.assert_allclose(s, s_ref, rtol=NCC_SCORE_RTOL, atol=1e-7)
-    agree = float(np.mean(d == d_ref))
-    assert agree >= 0.99, f"low-texture agreement {agree:.4f}"   # near-ties within ~2^-22 relative may resolve differently
+    # near-ties within ~2^-22 relative may resolve differently: a lower fraction, but every differing pixel within tau
+    assert_ncc_close(d, s, d_ref, s_ref, L, Rt, 4, -40, 0, nc.family_of(ctx), min_agree=0.99)
     # Why not 99.9 % here: this image is built so that dozens of candidates per pixel score within a few float32 ulps of each
     # other (scores ~ 0.99999).  The oracle ranks float32 scores (2^-24 relative near 1); a key holds 23 value bits of
     # C * rs in a power-of-two scale that can be up to twice the score's magnitude (2^-22 relative), so candidates the oracle
@@ -666,10 +674,8 @@ def test_ncc_fast_smooth_low_texture(ctx):
     # The pair call (fused NCC pairs, one scale per PIXEL instead of per strip row) behaves the same on it.
     fl, fr = ctx.disparity_pair(sb.COST_NCORR, L, Rt, 4, 40, dtype=np.int32)
     assert ctx.last_fused_pairs == 1
-    agree_pair = float(np.mean(fl == d_ref))
-    assert agree_pair >= 0.99, f"low-texture agreement of the pair call {agree_pair:.4f}"
-    d_ref_r = oracle.ncorr_fast(Rt.astype(np.float32), L.astype(np.float32), 4, 0, 40)
-    assert float(np.mean(fr == d_ref_r)) >= 0.99
+    nc.check_ncc_map(fl, L, Rt, 4, -40, 0, "u8_fused", oracle_disp=d_ref, min_agree=0.99, what="pair L->R")
+    nc.check_ncc_map(fr, Rt, L, 4, 0, 40, "u8_fused", min_agree=0.99, what="pair R->L")
 
 
 def test_ncc_fast_equals_exact_path(ctx):
@@ -682,7 +688,12 @@ def test_ncc_fast_equals_exact_path(ctx):
         ctx.force_path(0)
     d_fast, s_fast = ctx.disparity(sb.COST_NCORR, L, Rt, 5, -140, 0, dtype=np.int16, return_best=True)
     assert ctx.last_path == sb.PATH_FAST_U8
-    assert_ncc_close(d_fast, s_fast, d_exact, s_exact)
+    # the exact path IS the oracle (tau = 0) ...
+    Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
+    d_ref = oracle.ncorr_fast(Lf, Rf, 5, -140, 0)
+    nc.check_ncc_map(d_exact, Lf, Rf, 5, -140, 0, "exact", oracle_disp=d_ref)
+    # ... and the packed kernels are within their key resolution of it
+    assert_ncc_close(d_fast, s_fast, d_exact, s_exact, Lf, Rf, 5, -140, 0, nc.family_of(ctx))
 
 
 # ---- BASELINE config 3 at full size: 1920x1080, 128 disparities, 9x9, SSD and NCC ------------------------
@@ -696,7 +707,7 @@ def test_config3_full_size_ssd_and_ncc(ctx):
     d_ref, s_ref = oracle.ncorr_fast(Lf, Rf, 4, -127, 0, return_score=True)
     d, s = ctx.disparity(sb.COST_NCORR, L, Rt, 4, -127, 0, dtype=np.int16, return_best=True)
     assert ctx.last_path == sb.PATH_FAST_U8
-    assert_ncc_close(d, s, d_ref, s_ref)
+    assert_ncc_close(d, s, d_ref, s_ref, Lf, Rf, 4, -127, 0, nc.family_of(ctx))
 
 
 # ---- fused pair launches for any candidate count and every window radius (SURVEY.md §8 f2) ----------------------
@@ -781,7 +792,7 @@ def test_ps2_problem_shapes_full_size_clean(ctx):
             d_ref, s_ref = oracle.ncorr_fast(ref, tgt, R, lo, hi, return_score=True)
             d, s = ctx.disparity(sb.COST_NCORR, ref, tgt, R, lo, hi, dtype=np.int16, return_best=True)
             assert ctx.last_path == sb.PATH_FAST_U8
-            assert_ncc_close(d, s, d_ref, s_ref)
+            assert_ncc_close(d, s, d_ref, s_ref, ref, tgt, R, lo, hi, nc.family_of(ctx))
 
 
 def test_config4_full_size_fused_pair_and_ncc(ctx):
@@ -801,7 +812,7 @@ def test_config4_full_size_fused_pair_and_ncc(ctx):
     d_ref, s_ref = oracle.ncorr_fast(Lf, Rf, 5, -255, 0, return_score=True)
     d, s = ctx.disparity(sb.COST_NCORR, L, Rt, 5, -255, 0, dtype=np.int16, return_best=True)
     assert ctx.last_path == sb.PATH_FAST_U8
-    assert_ncc_close(d, s, d_ref, s_ref)
+    assert_ncc_close(d, s, d_ref, s_ref, Lf, Rf, 5, -255, 0, nc.family_of(ctx))
 
 
 # ---- the float running-sum kernels (general float32 images; VERDICT r1 row g1) ------------------------------------------
@@ -891,7 +902,10 @@ def test_float_kernels_on_8bit_images_equal_packed_kernels(ctx):
     finally:
         ctx.force_path(0)
     assert np.array_equal(dl8, dlf) and np.array_equal(dr8, drf)
-    assert_ncc_close(nf, sf, n8, s8)
+    # both families against the oracle, each within its own key resolution
+    n_ref, s_ref = oracle.ncorr_fast(Lf, Rf, 5, -100, 0, return_score=True)
+    assert_ncc_close(n8, s8, n_ref, s_ref, Lf, Rf, 5, -100, 0, "u8")
+    assert_ncc_close(nf, sf, n_ref, s_ref, Lf, Rf, 5, -100, 0, "f32")
 
 
 def test_float_kernels_hand_wide_value_ranges_to_the_exact_path(ctx):
@@ -914,7 +928,7 @@ def test_ncc_float_kernels_vs_oracle(ctx, rows, cols, R, dmin, dmax):
         d_ref, s_ref = oracle.ncorr_fast(Lf, Rf, R, dmin, dmax, return_score=True)
         d, s = ctx.disparity(sb.COST_NCORR, Lf, Rf, R, dmin, dmax, dtype=np.int32, return_best=True)
         assert ctx.last_path == sb.PATH_FAST_F32, name
-        assert_ncc_close(d, s, d_ref, s_ref)
+        assert_ncc_close(d, s, d_ref, s_ref, Lf, Rf, R, dmin, dmax, "f32")
 
 
 def test_ps2_problem_shapes_full_size_noisy_and_contrast(ctx):
@@ -931,7 +945,7 @@ def test_ps2_problem_shapes_full_size_noisy_and_contrast(ctx):
             d_ref, s_ref = oracle.ncorr_fast(ref, tgt, 7, lo, hi, return_score=True)
             d, s = ctx.disparity(sb.COST_NCORR, ref, tgt, 7, lo, hi, dtype=np.int16, return_best=True)
             assert ctx.last_path == sb.PATH_FAST_F32, name
-            assert_ncc_close(d, s, d_ref, s_ref)
+            assert_ncc_close(d, s, d_ref, s_ref, ref, tgt, 7, lo, hi, "f32")
 
 
 # ---- host-side packing of CV_32FC1 images (stereo_ctx_set_host_threads) ---------------------------------------------------
@@ -989,19 +1003,17 @@ def test_ncc_fused_pairs_vs_oracle(ctx, rows, cols, R, rng):
     (ref_l, _), (ref_r, _) = _ncc_pair_refs(Lf, Rf, R, rng)
     fl, fr = ctx.disparity_pair(sb.COST_NCORR, L, Rt, R, rng, dtype=np.int16)
     assert ctx.last_path == sb.PATH_FAST_U8 and ctx.last_fused_pairs == 1
-    al, ar = float(np.mean(fl == ref_l)), float(np.mean(fr == ref_r))
-    assert al >= NCC_DISP_AGREE and ar >= NCC_DISP_AGREE, (al, ar)
     ctx.set_fuse_pairs(False)
     try:
         ul, ur = ctx.disparity_pair(sb.COST_NCORR, L, Rt, R, rng, dtype=np.int16)
         assert ctx.last_fused_pairs == 0
     finally:
         ctx.set_fuse_pairs(True)
-    assert float(np.mean(ul == ref_l)) >= NCC_DISP_AGREE and float(np.mean(ur == ref_r)) >= NCC_DISP_AGREE
-    # wherever a map differs from the oracle's, the candidate it chose scores like the oracle's winner (a tie at float32 level)
-    for got, ref_d, (a, b, lo, hi) in ((fl, ref_l, (Lf, Rf, -rng, 0)), (fr, ref_r, (Rf, Lf, 0, rng))):
-        bad = np.argwhere(got != ref_d)
-        assert len(bad) <= max(1, int(0.001 * got.size)), len(bad)
+    # wherever a map differs from the oracle's, the candidate it chose scores like the oracle's winner (within the key
+    # resolution of the family), and the north-star fraction holds
+    for got, ref_d, family, (a, b, lo, hi) in ((fl, ref_l, "u8_fused", (Lf, Rf, -rng, 0)), (fr, ref_r, "u8_fused", (Rf, Lf, 0, rng)),
+                                               (ul, ref_l, "u8", (Lf, Rf, -rng, 0)), (ur, ref_r, "u8", (Rf, Lf, 0, rng))):
+        nc.check_ncc_map(got, a, b, R, lo, hi, family, oracle_disp=ref_d)
 
 
 def test_ncc_fused_pairs_low_texture_and_flat_images(ctx):
@@ -1021,8 +1033,8 @@ def test_ncc_fused_pairs_low_texture_and_flat_images(ctx):
         assert ctx.last_fused_pairs == 1
         # (the gradient image is full of near-ties at float32 level, see test_ncc_fast_smooth_low_texture; the flat images tie
         # exactly everywhere and must come out as the oracle's first maximum)
-        assert float(np.mean(fl == ref_l)) >= need, float(np.mean(fl == ref_l))
-        assert float(np.mean(fr == ref_r)) >= need, float(np.mean(fr == ref_r))
+        nc.check_ncc_map(fl, af, bf, R, -rng, 0, "u8_fused", oracle_disp=ref_l, min_agree=need, what="L->R")
+        nc.check_ncc_map(fr, bf, af, R, 0, rng, "u8_fused", oracle_disp=ref_r, min_agree=need, what="R->L")
 
 
 def test_ncc_fused_pairs_full_size_and_batches(ctx):
@@ -1033,8 +1045,8 @@ def test_ncc_fused_pairs_full_size_and_batches(ctx):
         (ref_l, _), (ref_r, _) = _ncc_pair_refs(Lf, Rf, R, rng)
         dl, dr = sb.disparityNCorrPair(Lf, Rf, sb.DisparityConfig(R, rng), ctx=ctx)
         assert ctx.last_path == sb.PATH_FAST_U8 and ctx.last_fused_pairs == 1
-        assert float(np.mean(dl == oracle.narrow_i8(ref_l))) >= NCC_DISP_AGREE
-        assert float(np.mean(dr == oracle.narrow_i8(ref_r))) >= NCC_DISP_AGREE
+        nc.check_ncc_map(dl, Lf, Rf, R, -rng, 0, "u8_fused", oracle_disp=ref_l, what="L->R")
+        nc.check_ncc_map(dr, Rf, Lf, R, 0, rng, "u8_fused", oracle_disp=ref_r, what="R->L")
     n = 6
     Ls, Rs = zip(*[synth.make_pair(33, 330, 64, 7100 + i)[:2] for i in range(n)])
     Ls, Rs = np.stack(Ls), np.stack(Rs)
@@ -1042,8 +1054,8 @@ def test_ncc_fused_pairs_full_size_and_batches(ctx):
     assert ctx.last_fused_pairs == n
     for i in range(n):
         a, b = Ls[i].astype(np.float32), Rs[i].astype(np.float32)
-        assert float(np.mean(bl[i] == oracle.narrow_i8(oracle.ncorr_fast(a, b, 4, -63, 0)))) >= NCC_DISP_AGREE, i
-        assert float(np.mean(br[i] == oracle.narrow_i8(oracle.ncorr_fast(b, a, 4, 0, 63)))) >= NCC_DISP_AGREE, i
+        nc.check_ncc_map(bl[i], a, b, 4, -63, 0, "u8_fused", what=f"pair {i} L->R")
+        nc.check_ncc_map(br[i], b, a, 4, 0, 63, "u8_fused", what=f"pair {i} R->L")
 
 
 def test_config4_full_size_ncc_pair_and_noisy_float_pair(ctx):
@@ -1054,8 +1066,8 @@ def test_config4_full_size_ncc_pair_and_noisy_float_pair(ctx):
     Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
     dl, dr = ctx.disparity_pair(sb.COST_NCORR, L, Rt, 5, 255, dtype=np.int16)
     assert ctx.last_path == sb.PATH_FAST_U8 and ctx.last_fused_pairs >= 1
-    assert float(np.mean(dl == oracle.ncorr_fast(Lf, Rf, 5, -255, 0))) >= NCC_DISP_AGREE
-    assert float(np.mean(dr == oracle.ncorr_fast(Rf, Lf, 5, 0, 255))) >= NCC_DISP_AGREE
+    nc.check_ncc_map(dl, Lf, Rf, 5, -255, 0, "u8_fused", what="4K L->R")
+    nc.check_ncc_map(dr, Rf, Lf, 5, 0, 255, "u8_fused", what="4K R->L")
     Ln, Rn = synth.noisy_variant(L, 21), synth.noisy_variant(Rt, 22)
     fl, fr = ctx.disparity_pair(sb.COST_SSD, Ln, Rn, 5, 255, dtype=np.int16)
     assert ctx.last_path == sb.PATH_FAST_F32 and ctx.last_fused_pairs >= 1

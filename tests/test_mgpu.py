@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 import oracle
+import ncc_check as nc
 import introtocomputervision_b200 as sb
 from introtocomputervision_b200 import _capi, synth
 
@@ -30,9 +31,10 @@ def test_mgpu_row_bands_equal_the_oracle(which):
                 bad = np.argwhere(dl != ref_l)
                 assert bad.size == 0, f"L->R differs at {bad[:5].tolist()} (of {len(bad)}), devices {devices}, R {R}"
                 assert np.array_equal(dr, ref_r), (devices, R, rng)
-        d_ref, _ = oracle.ncorr_fast(Lf, Rf, 4, -63, 0, return_score=True)
         dl, dr = mg.disparity_pair_bands(sb.COST_NCORR, L, Rt, 4, 63, dtype=np.int16)
-        assert float(np.mean(dl == d_ref)) >= 0.999
+        # packed kernels, fused or not per device context: "u8" (the per-strip tolerance) covers both
+        nc.check_ncc_map(dl, Lf, Rf, 4, -63, 0, "u8", what="L->R")
+        nc.check_ncc_map(dr, Rf, Lf, 4, 0, 63, "u8", what="R->L")
         # float images that are not 8-bit-valued: computed whole on the first device by the float kernels
         Ln, Rn = synth.noisy_variant(L, 1), synth.noisy_variant(Rt, 2)
         dl, dr = mg.disparity_pair_bands(sb.COST_SSD, Ln, Rn, 3, 40, dtype=np.int16)
