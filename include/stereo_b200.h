@@ -73,7 +73,7 @@ typedef enum stereo_path {
     STEREO_PATH_EXACT_F32 = 1,  /* any float input, window and range: per-element reference arithmetic, no running sums */
     STEREO_PATH_FAST_U8 = 2,    /* integer-valued 0..255 inputs: packed dot-product running sums */
     STEREO_PATH_REFGPU = 4,     /* stereo_disparity_refgpu_*: the function the reference's GPU kernels compute (SURVEY.md A.3) */
-    STEREO_PATH_SGM = 5,        /* SSD pair calls with stereo_ctx_set_sgm on: semi-global matching (sgm.cuh) */
+    STEREO_PATH_SGM = 5,        /* pair calls with stereo_ctx_set_sgm on: semi-global matching (sgm.cuh) */
     STEREO_PATH_FAST_F32 = 3    /* general float inputs of bounded range (noise / contrast variants, main.cpp:140-153,191-193):
                                    per-element round((l-r)^2) as exact int32 running sums (SSD), float32 running sums (NCC).
                                    Bounds: SSD keys 128*SSD + position < 2^32 and (l-r)^2 < 2^23; NCC |v| < 1e6 and, when
@@ -232,27 +232,29 @@ int stereo_ctx_speckle_filter(const stereo_ctx* ctx, int* max_size, int* max_dif
 int stereo_filter_speckles_device(stereo_ctx* ctx, void* disp, size_t disp_step, int disp_elem_bytes, int rows, int cols,
                                   int new_val, int max_size, int max_diff, void* cuda_stream);
 
-/* Semi-global matching of SSD pair calls: path aggregation of the matching cost along scanlines, in place of the
+/* Semi-global matching of pair calls: path aggregation of the matching cost along scanlines, in place of the
  * winner-take-all of the block matcher.  paths 0 (the default) switches it off: results are then exactly those without
  * it.  paths 4 or 8 switch it on for the pair entry points of this context that compute whole maps - pair host and
  * device, f32 and u8, the batches; any other paths, p1 < 0 or p1 > p2 return STEREO_ERR_INVALID_ARG and keep the old
  * setting.  Each direction of a pair is aggregated on its own (L->R over [-range, 0] referenced on the left image, R->L
- * over [0, +range] referenced on the right).  For reference image ref, radius R and padded column xp = x + R of a
+ * over [0, +range] referenced on the right).  SSD: for reference image ref, radius R and padded column xp = x + R of a
  * Wp = cols + 2R wide padded image, candidate d is present at (y, x) when xp + d lies in [0, Wp - 1] (the candidates the
  * SSD single-direction call evaluates; d = 0 always is).  C(p, d) is that call's window sum for the candidate (replicate
- * padding, the flat-index row-wrap reads, per element round(float((l - r)^2)), integer accumulation).  For each path
+ * padding, the flat-index row-wrap reads, per element round(float((l - r)^2)), integer accumulation).  NCC pair calls are
+ * served only while an NCC scale q is set (stereo_ctx_set_sgm_ncc_scale), with C defined there.  For each path
  * direction r - (0,+-1), (+-1,0), and with 8 paths also (+-1,+-1) - and q = p - r:
  *     L_r(p, d) = C(p, d)                                                               where q is outside the image,
  *     L_r(p, d) = C(p, d) + min(L_r(q, d), L_r(q, d-1) + p1, L_r(q, d+1) + p1, m(q) + p2) - m(q)   otherwise,
  * with m(q) the minimum of L_r(q, .) over the candidates present at q; terms of candidates absent at q are left out.
  * S(p, d) is the sum of L_r(p, d) over the paths, and the disparity the first minimum of S over the present candidates in
  * ascending d, stored in the map's element type as every other call does (1-byte maps narrow like the reference's char).
- * p1 = p2 = 0 gives L_r = C and so the SSD maps themselves (wherever every present window cost is below 99999999).
+ * For SSD, p1 = p2 = 0 gives L_r = C and so the SSD maps themselves (wherever every present window cost is below 99999999).
  * The left-right check, then the speckle filter, run on the SGM maps when they are on too (SGM -> check -> filter).
  * Refused with STEREO_ERR_UNSUPPORTED before anything is enqueued or written (float images: after their classification):
- * NCC pair calls; paths * ((2R + 1)^2 M + p2) > 2^31 - 1, with M = 255^2 for 8-bit-valued images and ceil((hi - lo)^2)
- * (widened by 1e-6 for float rounding) over the value range of other float images; float images with a pixel that is not
- * finite; more than 512 candidates after clipping [-range, range] to |d| <= cols - 1 + R.  Paths cross band seams, so
+ * NCC pair calls while the NCC scale is 0; SSD with paths * ((2R + 1)^2 M + p2) > 2^31 - 1, with M = 255^2 for 8-bit-valued
+ * images and ceil((hi - lo)^2) (widened by 1e-6 for float rounding) over the value range of other float images; float
+ * images with a pixel that is not finite; more than 512 candidates after clipping [-range, range] to |d| <= cols - 1 + R
+ * (SSD) or |d| <= cols - 1 (NCC).  Paths cross band seams, so
  * the row-band entry points (stereo_disparity_pair_band_halo_u8_device, stereo_disparity_pair_band_{u8,f32}_host) accept
  * only the whole image as their band and stereo_mgpu_disparity_pair_bands_* refuse.  Single-direction and
  * stereo_disparity_refgpu_* calls ignore the setting.  Calls served by SGM report STEREO_PATH_SGM, 0 fused pairs and no
@@ -262,6 +264,27 @@ int stereo_filter_speckles_device(stereo_ctx* ctx, void* disp, size_t disp_step,
 int stereo_ctx_set_sgm(stereo_ctx* ctx, int paths, int p1, int p2);
 /* The context's current setting (paths 0: off, with p1 = p2 = 0). */
 int stereo_ctx_sgm(const stereo_ctx* ctx, int* paths, int* p1, int* p2);
+
+/* Integer scale q of the NCC matching cost for SGM.  0 (the default): SGM refuses NCC pair calls, as before.
+ * 1 <= q <= 2^24: NCC pair calls are served by SGM while stereo_ctx_set_sgm is on.  Other values: STEREO_ERR_INVALID_ARG,
+ * old setting kept.  The scale and stereo_ctx_set_sgm are independent: switching SGM off keeps q, q alone changes nothing,
+ * and SSD calls ignore it.
+ * NCC cost.  Candidate d is present at (y, x) when 0 <= x + d <= cols - 1: the reference's own NCC candidates in both
+ * directions (L->R over [-range, 0] right-aligned, DisparityNCorr.cpp:67; R->L over [0, range] from startX = x), so
+ * [-range, range] is clipped to |d| <= cols - 1.  s(p, d) is the candidate's float32 TM_CCORR_NORMED score in the
+ * reference's arithmetic (the double numerator summed in (wy, k) order and rounded to float32, double window energies in
+ * the same order, the 10 FLT_EPSILON zero-energy rule and the 1.125 t rule; stereo_disparity_* with the exact kernels
+ * return it as best_out), and
+ *     C(p, d) = q - floor(fl32(q * s(p, d)))        in [0, 2q]
+ * (the product is exact for a power-of-two q and correctly rounded otherwise).  L_r, S and the first minimum of S are as
+ * above; the left-right check and the speckle filter follow.  Float images are classified once and refused when a pixel is
+ * not finite.  paths * (2q + p2) > 2^31 - 1 returns STEREO_ERR_UNSUPPORTED before anything is enqueued, whatever the
+ * image.  With p1 = p2 = 0 the map is the first d that maximises floor(fl32(q * s)): the block matcher's NCC map except
+ * where a candidate before the block matcher's winner falls in the same quantum of q * s (not an exact identity, as it is
+ * for SSD).  Scratch adds 16 bytes per pixel (the two images' window norms) to the SSD figure. */
+int stereo_ctx_set_sgm_ncc_scale(stereo_ctx* ctx, int q);
+/* The context's current q (0: off); STEREO_ERR_INVALID_ARG for a null context. */
+int stereo_ctx_sgm_ncc_scale(const stereo_ctx* ctx);
 
 /* ---- single direction, HOST buffers (the drop-in form) ------------------------------------ */
 /*
@@ -494,6 +517,8 @@ int stereo_mgpu_set_speckle_filter(stereo_mgpu* mg, int max_size, int max_diff);
 /* stereo_ctx_set_sgm on every device's context.  Pair batches shard whole pairs and so give the single-GPU result;
  * row-band sharded pairs return STEREO_ERR_UNSUPPORTED while SGM is on. */
 int stereo_mgpu_set_sgm(stereo_mgpu* mg, int paths, int p1, int p2);
+/* stereo_ctx_set_sgm_ncc_scale on every device's context. */
+int stereo_mgpu_set_sgm_ncc_scale(stereo_mgpu* mg, int q);
 /* Batches (BASELINE config 5): same arguments as stereo_disparity_pair_batch_{u8,f32}_host. */
 int stereo_mgpu_disparity_pair_batch_u8_host(stereo_mgpu* mg, int cost, int n_pairs,
                                              const uint8_t* left, const uint8_t* right, size_t img_step, size_t pair_stride,

@@ -186,10 +186,16 @@ inline void setSpeckleFilter(int maxSize, int maxDiff, stereo_ctx* ctx = nullptr
     check(stereo_ctx_set_speckle_filter(ctx ? ctx : default_ctx(), maxSize, maxDiff), "stereo_ctx_set_speckle_filter");
 }
 
-// Semi-global matching of the SSD pair calls on `ctx` (default: the default context): paths 4 or 8 switch it on, 0 off
+// Semi-global matching of the pair calls on `ctx` (default: the default context): paths 4 or 8 switch it on, 0 off
 // (stereo_ctx_set_sgm).
 inline void setSgm(int paths, int p1 = 0, int p2 = 0, stereo_ctx* ctx = nullptr) {
     check(stereo_ctx_set_sgm(ctx ? ctx : default_ctx(), paths, p1, p2), "stereo_ctx_set_sgm");
+}
+
+// Integer scale q (1 .. 2^24) of the NCC cost C = q - floor(fl32(q * score)) that lets SGM serve NCC pair calls; 0 (the
+// default) refuses them (stereo_ctx_set_sgm_ncc_scale).
+inline void setSgmNccScale(int q, stereo_ctx* ctx = nullptr) {
+    check(stereo_ctx_set_sgm_ncc_scale(ctx ? ctx : default_ctx(), q), "stereo_ctx_set_sgm_ncc_scale");
 }
 
 // Kernel time of the last call on the default context, the quantity the reference logs as
@@ -241,6 +247,7 @@ public:
         check(stereo_mgpu_set_speckle_filter(mg_, maxSize, maxDiff), "stereo_mgpu_set_speckle_filter");
     }
     void setSgm(int paths, int p1 = 0, int p2 = 0) { check(stereo_mgpu_set_sgm(mg_, paths, p1, p2), "stereo_mgpu_set_sgm"); }
+    void setSgmNccScale(int q) { check(stereo_mgpu_set_sgm_ncc_scale(mg_, q), "stereo_mgpu_set_sgm_ncc_scale"); }
 
     // disparitySSDPair / disparityNCorrPair (main.cpp:21-78) with the output rows sharded over the devices
     void disparityPairBands(int cost, const MatT& left, const MatT& right, size_t windowRad, int disparityRange, MatT& disparityLeft,

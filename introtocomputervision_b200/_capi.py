@@ -58,6 +58,9 @@ SIGNATURES = {
     "stereo_ctx_set_sgm": (_i, [_vp, _i, _i, _i]),
     "stereo_ctx_sgm": (_i, [_vp, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i)]),
     "stereo_mgpu_set_sgm": (_i, [_vp, _i, _i, _i]),
+    "stereo_ctx_set_sgm_ncc_scale": (_i, [_vp, _i]),
+    "stereo_ctx_sgm_ncc_scale": (_i, [_vp]),
+    "stereo_mgpu_set_sgm_ncc_scale": (_i, [_vp, _i]),
     "stereo_ctx_synchronize": (_i, [_vp, _vp]),
     "stereo_disparity_f32_host": (_i, _SINGLE_HOST),
     "stereo_disparity_u8_host": (_i, _SINGLE_HOST),

@@ -107,8 +107,9 @@ struct stereo_ctx {
     int lr_max_diff = -1;     // pair calls: left-right consistency check with this disp12MaxDiff (< 0: off)
     int spk_max_size = 0;     // pair calls: speckle filter of components up to this many pixels (0: off) ...
     int spk_max_diff = 0;     // ... whose neighbours differ by at most this much
-    int sgm_paths = 0;        // SSD pair calls: semi-global matching over 4 or 8 paths (0: off) ...
+    int sgm_paths = 0;        // pair calls: semi-global matching over 4 or 8 paths (0: off) ...
     int sgm_p1 = 0, sgm_p2 = 0;   // ... with these penalties
+    int sgm_ncc_scale = 0;    // ... and, for NCC pair calls, this integer scale of the NCC cost (0: NCC refused)
     // device time of the hot kernels only (fast_*_kernel), per direction, for the roofline report
     static constexpr int HOT_EVENTS = 16;
     cudaEvent_t hot0[HOT_EVENTS] = {}, hot1[HOT_EVENTS] = {};

@@ -59,6 +59,22 @@ ssd_exact_kernel(const float* __restrict__ Lp, const float* __restrict__ Rp, int
     cost[o] = bestCost;
 }
 
+// TM_CCORR_NORMED's normalisation of one candidate (opencv/modules/imgproc/src/templmatch.cpp common_matchTemplate), in
+// two halves: the target window's norm from its double energy wnd - 0 below the zero-energy threshold - and the float32
+// score of the double numerator acc against t = ncc_target_norm(wnd) * sqrt(reference energy).
+__device__ __forceinline__ double ncc_target_norm(double wnd) {
+    const double diff2 = wnd > 0 ? wnd : 0;
+    const double lim = fmin(0.5, 10 * double(FLT_EPSILON) * wnd);
+    return diff2 <= lim ? 0 : sqrt(diff2);
+}
+__device__ __forceinline__ float ncc_normalise(double acc, double t) {
+    double num = double(float(acc));
+    if (fabs(num) < t) num /= t;
+    else if (fabs(num) < t * 1.125) num = num > 0 ? 1 : -1;
+    else num = 0;
+    return float(num);
+}
+
 // NCC with TM_CCORR_NORMED's arithmetic (float32 numerator, double energies and normalisation,
 // float32 result; opencv/modules/imgproc/src/templmatch.cpp common_matchTemplate).
 __global__ void __launch_bounds__(128)
@@ -91,14 +107,7 @@ ncorr_exact_kernel(const float* __restrict__ Lp, const float* __restrict__ Rp, i
                 wnd += b * b;
             }
         }
-        double num = double(float(acc));
-        const double diff2 = wnd > 0 ? wnd : 0;
-        const double lim = fmin(0.5, 10 * double(FLT_EPSILON) * wnd);
-        const double t = (diff2 <= lim) ? 0 : sqrt(diff2) * templNorm;
-        if (fabs(num) < t) num /= t;
-        else if (fabs(num) < t * 1.125) num = num > 0 ? 1 : -1;
-        else num = 0;
-        const float sc = float(num);
+        const float sc = ncc_normalise(acc, ncc_target_norm(wnd) * templNorm);
         if (bestI < 0 || sc > bestScore) { bestScore = sc; bestI = i; }
     }
     const bool right_aligned = (dmin <= 0 && dmax <= 0);

@@ -180,6 +180,15 @@ int stereo_mgpu_set_sgm(stereo_mgpu* mg, int paths, int p1, int p2) {
     return STEREO_OK;
 }
 
+int stereo_mgpu_set_sgm_ncc_scale(stereo_mgpu* mg, int q) {
+    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
+    for (stereo_ctx* c : mg->ctx) {
+        const int rc = stereo_ctx_set_sgm_ncc_scale(c, q);
+        if (rc != STEREO_OK) return rc;
+    }
+    return STEREO_OK;
+}
+
 int stereo_mgpu_disparity_pair_batch_u8_host(stereo_mgpu* mg, int cost, int n_pairs, const uint8_t* left, const uint8_t* right,
                                              size_t img_step, size_t pair_stride, int rows, int cols, int window_rad,
                                              int disparity_range, void* disp_left, void* disp_right, size_t disp_step,

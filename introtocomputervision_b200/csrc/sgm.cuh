@@ -1,10 +1,13 @@
-// Semi-global matching (path aggregation of the SSD cost along scanlines) for one direction of a pair.
-//   C(y, x, d)  the reference's SSD window sum of candidate d (exact.cuh's ssd_elem per element, the flat-index row-wrap
-//               reads included), for the present candidates: those with s = x + R + d in [0, Wp - 1].
+// Semi-global matching (path aggregation of the matching cost along scanlines) for one direction of a pair.
+//   C(y, x, d)  SSD: the reference's SSD window sum of candidate d (exact.cuh's ssd_elem per element, the flat-index
+//               row-wrap reads included), for the present candidates: those with s = x + R + d in [0, Wp - 1].
+//               NCC: q - floor(fl32(q s)) of the candidate's float32 TM_CCORR_NORMED score s (exact.cuh's ncorr_exact_kernel
+//               arithmetic), for the present candidates: those with x + d in [0, cols - 1].
 //   L_r(p, d) = C(p, d) + min(L_r(q, d), L_r(q, d -+ 1) + P1, m(q) + P2) - m(q),  q = p - r,  m(q) = min_e L_r(q, e);
 //               L_r(p, d) = C(p, d) where q lies outside the image.  Terms of candidates absent at q are left out.
 //   S(p, d)   = sum over the 4 or 8 paths r of L_r(p, d);  disparity = the first minimum of S over the present candidates.
-// Launches per direction: two replicate pads (exact.cuh), sgm_cost_kernel, then one sgm_path_kernel per path in stream
+// Launches per direction: two replicate pads (exact.cuh), [NCC: sgm_ncc_norm_kernel,] the cost kernel - sgm_cost_kernel, or
+// sgm_ncc_cell_kernel for NCC on float images that are not 8-bit-valued - then one sgm_path_kernel per path in stream
 // order; the first path writes S, the later ones read-add-write it, the last one also writes the winner-take-all map.
 // Layout: candidate index j = d - dlo innermost, padded to Dp = 32 K (K candidates per lane of the path kernels).  Absent
 // and padding candidates hold SGM_ABSENT in C and L; S of an absent candidate is 0xFFFFFFFF, above every present sum as
@@ -22,14 +25,49 @@ constexpr int SGM_XT = 256;                // output columns of one cost block
 constexpr int SGM_COST_THREADS = 256;      // 8 warps, SGM_XT / 8 consecutive columns each
 constexpr int SGM_PATH_WARPS = 4;          // scanlines (one warp each) per path block
 
+// The NCC cost's per-pixel window norms (sgm_ncc_norm_kernel, rows x cols each) and its scale q.
+struct SgmNcc { const double* nref; const double* ntgt; int q; };
+
+// C of a present NCC candidate d at (y, x) from its double numerator acc: q - floor(fl32(q s)), in [0, 2q].
+__device__ __forceinline__ int32_t sgm_ncc_cost(double acc, const SgmNcc& n, int cols, int y, int x, int d) {
+    const size_t o = size_t(y) * cols + x;
+    const float s = ncc_normalise(acc, n.ntgt[o + d] * n.nref[o]);
+    return n.q - int(floorf(__fmul_rn(float(n.q), s)));
+}
+
+// Window norms of one direction's padded images at every (y, x): the double window energy E in the oracle's (wy, k)
+// order, then nref = sqrt(E) of the reference (blockIdx.z 0) and ntgt = ncc_target_norm(E) of the target (blockIdx.z 1),
+// so that ntgt(y, x + d) * nref(y, x) is ncorr_exact_kernel's t of candidate d bit for bit.
+__global__ void __launch_bounds__(128)
+sgm_ncc_norm_kernel(const float* __restrict__ Lp, const float* __restrict__ Rp, int cols, int R, double* __restrict__ nref,
+                    double* __restrict__ ntgt) {
+    const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
+    if (x >= cols) return;
+    const int Wp = cols + 2 * R, w = 2 * R + 1;
+    const float* img = blockIdx.z ? Rp : Lp;
+    double e = 0;
+    for (int wy = 0; wy < w; ++wy) {
+        const float* row = img + size_t(y + wy) * Wp + x;
+        for (int k = 0; k < w; ++k) { const double v = __ldg(row + k); e += v * v; }
+    }
+    const size_t o = size_t(y) * cols + x;
+    if (blockIdx.z) ntgt[o] = ncc_target_norm(e);
+    else nref[o] = sqrt(e);
+}
+
 // C for output rows [y0, y0 + rows_per_block) x columns [x0, x0 + SGM_XT) x candidates [j0, j0 + 32) of one block.
-// Vertical window sums V(c, d) of the element image E(r, c, d) = ssd_elem(Lp[r][c], Rp_flat[r Wp + c + d]) are kept in
-// shared memory for the block's columns and slide down one row at a time (E is recomputed for the row that leaves);
-// each warp then slides the horizontal window along its 32 columns with the candidate in the lane, so every row of C is
-// written as 128-byte lines.  Reads outside [-R, Hp Wp + R) - only ever of absent or padding candidates - count as 0.
+// Vertical window sums V(c, d) of the element image E(r, c, d) are kept in shared memory for the block's columns and
+// slide down one row at a time (E is recomputed for the row that leaves); each warp then slides the horizontal window
+// along its 32 columns with the candidate in the lane, so every row of C is written as 128-byte lines.
+//   SSD: E = ssd_elem(Lp[r][c], Rp_flat[r Wp + c + d]); reads outside [-R, Hp Wp + R) - only ever of absent or padding
+//        candidates - count as 0.
+//   NCC (8-bit-valued images only): E = Lp[r][c] Rp[r][c + d], 0 where c + d leaves the padded row (again only absent or
+//        padding candidates).  The products are integers, so the int32 window sum - below (2R + 1)^2 255^2 < 2^31 - is
+//        the oracle's double numerator exactly, whatever the order; the epilogue normalises it (sgm_ncc_cost).
+template <bool NCC>
 __global__ void __launch_bounds__(SGM_COST_THREADS)
 sgm_cost_kernel(const float* __restrict__ Lp, const float* __restrict__ Rp, int rows, int cols, int R, int dlo, int D, int Dp,
-                int rows_per_block, int32_t* __restrict__ C) {
+                int rows_per_block, SgmNcc ncc, int32_t* __restrict__ C) {
     extern __shared__ int32_t V[];                       // [(SGM_XT + 2R) columns][32 candidates]
     const int Wp = cols + 2 * R, w = 2 * R + 1, nc = SGM_XT + 2 * R;
     const long long flat_lo = -R, flat_hi = (long long)(rows + 2 * R) * Wp + R;
@@ -38,6 +76,10 @@ sgm_cost_kernel(const float* __restrict__ Lp, const float* __restrict__ Rp, int 
     const int d = dlo + j;
     const int y1 = min(rows, y0 + rows_per_block);
     auto E = [&](int r, int c) -> int {                  // r, c: padded coordinates
+        if (NCC) {
+            if (c >= Wp || c + d < 0 || c + d >= Wp) return 0;
+            return int(__ldg(Lp + (long long)r * Wp + c)) * int(__ldg(Rp + (long long)r * Wp + c + d));
+        }
         const long long f = (long long)r * Wp + c + d;
         if (c >= Wp || f < flat_lo || f >= flat_hi) return 0;
         return ssd_elem(__ldg(Lp + (long long)r * Wp + c), __ldg(Rp + f));
@@ -57,8 +99,8 @@ sgm_cost_kernel(const float* __restrict__ Lp, const float* __restrict__ Rp, int 
             int32_t* out = C + ((size_t)y * cols + xs) * Dp + j;
             const int xe = min(cols, xs + SEG);
             for (int x = xs; x < xe; ++x, out += Dp) {
-                const int s = x + R + d;
-                *out = (j < D && s >= 0 && s < Wp) ? h : SGM_ABSENT;
+                if (NCC) *out = (j < D && x + d >= 0 && x + d < cols) ? sgm_ncc_cost(double(h), ncc, cols, y, x, d) : SGM_ABSENT;
+                else *out = (j < D && x + R + d >= 0 && x + R + d < Wp) ? h : SGM_ABSENT;
                 const int ci = x - x0;
                 if (x + 1 < xe) h += V[(ci + w) * 32 + lane] - V[ci * 32 + lane];
             }
@@ -67,6 +109,48 @@ sgm_cost_kernel(const float* __restrict__ Lp, const float* __restrict__ Rp, int 
         __syncthreads();
         for (int ci = warp; ci < nc; ci += SGM_COST_THREADS / 32)
             V[ci * 32 + lane] += E(y - 1 + w, x0 + ci) - E(y - 1, x0 + ci);
+    }
+}
+
+// C of the NCC cost for float images that are not 8-bit-valued: their products round in double, so each cell's numerator
+// is summed on its own in the oracle's (wy, k) order.  One block: row y, columns [x0, x0 + SGM_CELL_XT), candidates
+// [j0, j0 + 32) with the candidate in the lane; each warp holds SGM_CELL_XT / 8 consecutive pixels' numerators.  Window
+// row by window row, the block stages the reference's and the targets' padded row segments in shared memory (0 outside
+// the row: only absent and padding candidates read there); the reference value is a broadcast, the target values are
+// consecutive across the lanes, and every row of C is written as 128-byte lines.
+constexpr int SGM_CELL_XT = 64;
+__global__ void __launch_bounds__(SGM_COST_THREADS)
+sgm_ncc_cell_kernel(const float* __restrict__ Lp, const float* __restrict__ Rp, int cols, int R, int dlo, int D, int Dp, SgmNcc ncc,
+                    int32_t* __restrict__ C) {
+    extern __shared__ float sh[];                        // reference [SGM_CELL_XT + 2R], target [SGM_CELL_XT + 31 + 2R]
+    constexpr int PX = SGM_CELL_XT / (SGM_COST_THREADS / 32);
+    const int Wp = cols + 2 * R, w = 2 * R + 1, nl = SGM_CELL_XT + 2 * R, nt = nl + 31;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int x0 = blockIdx.x * SGM_CELL_XT, y = blockIdx.y, j = blockIdx.z * 32 + lane, d = dlo + j;
+    const int t0 = x0 + dlo + blockIdx.z * 32;            // padded target column of the target segment's first value
+    float* Ls = sh;
+    float* Ts = sh + nl;
+    double acc[PX];
+#pragma unroll
+    for (int u = 0; u < PX; ++u) acc[u] = 0;
+    for (int wy = 0; wy < w; ++wy) {
+        const float* lrow = Lp + size_t(y + wy) * Wp;
+        const float* rrow = Rp + size_t(y + wy) * Wp;
+        for (int i = threadIdx.x; i < nl; i += SGM_COST_THREADS) Ls[i] = x0 + i < Wp ? __ldg(lrow + x0 + i) : 0.f;
+        for (int i = threadIdx.x; i < nt; i += SGM_COST_THREADS) Ts[i] = t0 + i >= 0 && t0 + i < Wp ? __ldg(rrow + t0 + i) : 0.f;
+        __syncthreads();
+#pragma unroll
+        for (int u = 0; u < PX; ++u) {
+            const int xi = warp * PX + u;
+            for (int k = 0; k < w; ++k) acc[u] += double(Ls[xi + k]) * double(Ts[xi + lane + k]);     // (exact products)
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int u = 0; u < PX; ++u) {
+        const int x = x0 + warp * PX + u;
+        if (x < cols)
+            C[(size_t(y) * cols + x) * Dp + j] = (j < D && x + d >= 0 && x + d < cols) ? sgm_ncc_cost(acc[u], ncc, cols, y, x, d) : SGM_ABSENT;
     }
 }
 

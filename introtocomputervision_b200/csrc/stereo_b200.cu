@@ -123,15 +123,19 @@ static int check_lr_sentinel(int elem, int range) {
 }
 
 // What a pair call must satisfy for the context's options, checked once per call before anything is staged or enqueued:
-// the sentinel fits (left-right check or speckle filter on), SGM aggregates the SSD cost, and SGM paths and speckle
-// regions, which cross band seams, get whole maps.  run_sgm checks the candidate count and the int32 bound.
+// the sentinel fits (left-right check or speckle filter on), SGM aggregates the SSD cost or, with an NCC scale set, the NCC
+// cost, and SGM paths and speckle regions, which cross band seams, get whole maps.  run_sgm checks the candidate count and
+// the int32 bound.
 static int check_pair_options(const stereo_ctx* ctx, int cost, int elem, int range, int row_begin, int row_end, int rows) {
     const bool sgm = ctx->sgm_paths > 0, spk = ctx->spk_max_size > 0, whole = row_begin == 0 && row_end == rows;
     if (ctx->lr_max_diff >= 0 || spk) {
         const int rc = check_lr_sentinel(elem, range);
         if (rc != STEREO_OK) return rc;
     }
-    if (sgm && cost != STEREO_COST_SSD) { set_error("SGM aggregates the SSD cost only (switch it off for NCC calls)"); return STEREO_ERR_UNSUPPORTED; }
+    if (sgm && cost != STEREO_COST_SSD && ctx->sgm_ncc_scale == 0) {
+        set_error("SGM aggregates the SSD cost only while no NCC scale is set (stereo_ctx_set_sgm_ncc_scale; or switch SGM off for NCC calls)");
+        return STEREO_ERR_UNSUPPORTED;
+    }
     if (sgm && !whole) {
         set_error("SGM: rows [%d, %d) are not the whole map (vertical and diagonal paths cross band seams)", row_begin, row_end);
         return STEREO_ERR_UNSUPPORTED;
@@ -434,35 +438,40 @@ static int run_families(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bo
 
 // ---- semi-global matching (sgm.cuh) ----------------------------------------------------------------------------------
 
-// Candidates of one direction: [dmin, dmax] clipped to the ones some pixel has present (|d| <= cols - 1 + R), padded to
-// 32 K for the path kernels.
+// Candidates of one direction: [dmin, dmax] clipped to the ones some pixel has present (|d| <= cols - 1 + R for SSD,
+// |d| <= cols - 1 for NCC), padded to 32 K for the path kernels.
 struct SgmShape { int dlo, D, K; size_t Dp; };
 static SgmShape sgm_shape(const Problem& p) {
-    const int lim = p.cols - 1 + p.R;
+    const int lim = p.cost == STEREO_COST_NCORR ? p.cols - 1 : p.cols - 1 + p.R;
     const int dlo = p.dmin > -lim ? p.dmin : -lim, dhi = p.dmax < lim ? p.dmax : lim;
     const int D = dhi - dlo + 1, K = (D + 31) / 32;
     return SgmShape{dlo, D, K, size_t(32) * K};
 }
 
-// One direction's scratch: both padded images, the cost volume and the aggregate (plus, for float images, the u8 copies
-// the classification writes).  Directions of a call run one after the other on the same scratch.
+// One direction's scratch: both padded images, the cost volume and the aggregate, for NCC the two window-norm maps (plus,
+// for float images, the u8 copies the classification writes).  Directions of a call run one after the other on the same
+// scratch.
 static size_t sgm_scratch_bytes(const Problem& p) {
     const size_t cells = size_t(p.rows) * p.cols * sgm_shape(p).Dp;
-    const size_t need = 2 * align256(padded_elems(p) * sizeof(float)) + 2 * align256(cells * 4) + 4096;
+    size_t need = 2 * align256(padded_elems(p) * sizeof(float)) + 2 * align256(cells * 4) + 4096;
+    if (p.cost == STEREO_COST_NCORR) need += 2 * align256(size_t(p.rows) * p.cols * sizeof(double));
     return p.ref.type == PixType::F32 ? need + u8_copies_bytes(p) : need;
 }
 
-// Every L_r is at most C_max + P2 with C_max = (2R + 1)^2 M, M the largest per-element term: S stays in int32 when
-// paths (C_max + P2) <= 2^31 - 1.
-static int check_sgm_bound(const stereo_ctx* ctx, int R, double M) {
-    const double w = double(2 * R + 1) * (2 * R + 1);
-    if (double(ctx->sgm_paths) * (w * M + ctx->sgm_p2) <= 2147483647.0) return STEREO_OK;
-    set_error("SGM: %d paths x ((2 * %d + 1)^2 x %.0f + P2 %d) exceeds 2^31 - 1", ctx->sgm_paths, R, M, ctx->sgm_p2);
+// Every L_r is at most C_max + P2: S stays in int32 when paths (C_max + P2) <= 2^31 - 1.  C_max is (2R + 1)^2 M for SSD,
+// M the largest per-element term, and 2q for NCC.
+static int check_sgm_bound(const stereo_ctx* ctx, double c_max, const char* what) {
+    if (double(ctx->sgm_paths) * (c_max + ctx->sgm_p2) <= 2147483647.0) return STEREO_OK;
+    set_error("SGM: %d paths x (C_max %.0f [%s] + P2 %d) exceeds 2^31 - 1", ctx->sgm_paths, c_max, what, ctx->sgm_p2);
     return STEREO_ERR_UNSUPPORTED;
+}
+static int check_ssd_sgm_bound(const stereo_ctx* ctx, int R, double M) {
+    return check_sgm_bound(ctx, double(2 * R + 1) * (2 * R + 1) * M, "(2R + 1)^2 x the largest element");
 }
 
 // One direction by SGM into p.disp, on scratch the caller reserved.  ref / tgt: the caller's images (u8 or float).
-static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st) {
+// `per_cell`: NCC on float images that are not 8-bit-valued, whose numerators are summed cell by cell (sgm_ncc_cell_kernel).
+static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st, bool per_cell) {
     static constexpr int DIRS[8][2] = {{0, 1}, {0, -1}, {1, 0}, {-1, 0}, {1, 1}, {1, -1}, {-1, 1}, {-1, -1}};
     const SgmShape g = sgm_shape(p);
     const size_t cells = size_t(p.rows) * p.cols * g.Dp;
@@ -472,13 +481,31 @@ static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st)
     int32_t* C = static_cast<int32_t*>(ctx->arena.take(cells * 4));
     int32_t* S = static_cast<int32_t*>(ctx->arena.take(cells * 4));
     if (!C || !S) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
-    // rows per cost block: as many as still leave about four blocks per SM (each block recomputes 2R + 1 rows first)
-    const long long tiles = (long long)div_round_up(p.cols, SGM_XT) * (g.Dp / 32);
-    int rpb = 64;
-    while (rpb > 8 && tiles * div_round_up(p.rows, rpb) < 4LL * ctx->sm_count) rpb /= 2;
-    const dim3 cg(div_round_up(p.cols, SGM_XT), div_round_up(p.rows, rpb), unsigned(g.Dp / 32));
-    const size_t smem = size_t(SGM_XT + 2 * p.R) * 32 * sizeof(int32_t);
-    sgm_cost_kernel<<<cg, SGM_COST_THREADS, smem, st>>>(Lp, Rp, p.rows, p.cols, p.R, g.dlo, g.D, int(g.Dp), rpb, C);
+    SgmNcc ncc{nullptr, nullptr, ctx->sgm_ncc_scale};
+    const bool is_ncc = p.cost == STEREO_COST_NCORR;
+    if (is_ncc) {
+        double* nref = static_cast<double*>(ctx->arena.take(size_t(p.rows) * p.cols * sizeof(double)));
+        double* ntgt = static_cast<double*>(ctx->arena.take(size_t(p.rows) * p.cols * sizeof(double)));
+        if (!nref || !ntgt) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
+        ncc.nref = nref;
+        ncc.ntgt = ntgt;
+        sgm_ncc_norm_kernel<<<dim3(div_round_up(p.cols, 128), p.rows, 2), 128, 0, st>>>(Lp, Rp, p.cols, p.R, nref, ntgt);
+        ctx->last_launches += 1;
+    }
+    if (per_cell) {
+        const dim3 cg(div_round_up(p.cols, SGM_CELL_XT), p.rows, unsigned(g.Dp / 32));
+        const size_t smem = size_t(2 * (SGM_CELL_XT + 2 * p.R) + 31) * sizeof(float);
+        sgm_ncc_cell_kernel<<<cg, SGM_COST_THREADS, smem, st>>>(Lp, Rp, p.cols, p.R, g.dlo, g.D, int(g.Dp), ncc, C);
+    } else {
+        // rows per cost block: as many as still leave about four blocks per SM (each block recomputes 2R + 1 rows first)
+        const long long tiles = (long long)div_round_up(p.cols, SGM_XT) * (g.Dp / 32);
+        int rpb = 64;
+        while (rpb > 8 && tiles * div_round_up(p.rows, rpb) < 4LL * ctx->sm_count) rpb /= 2;
+        const dim3 cg(div_round_up(p.cols, SGM_XT), div_round_up(p.rows, rpb), unsigned(g.Dp / 32));
+        const size_t smem = size_t(SGM_XT + 2 * p.R) * 32 * sizeof(int32_t);
+        if (is_ncc) sgm_cost_kernel<true><<<cg, SGM_COST_THREADS, smem, st>>>(Lp, Rp, p.rows, p.cols, p.R, g.dlo, g.D, int(g.Dp), rpb, ncc, C);
+        else sgm_cost_kernel<false><<<cg, SGM_COST_THREADS, smem, st>>>(Lp, Rp, p.rows, p.cols, p.R, g.dlo, g.D, int(g.Dp), rpb, ncc, C);
+    }
     ctx->last_launches += 1;
     for (int k = 0; k < ctx->sgm_paths; ++k) {
         const int dy = DIRS[k][0], dx = DIRS[k][1];
@@ -499,10 +526,13 @@ static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st)
 }
 
 // Every direction of a pair call by SGM: n/2 left-referenced problems and their partners, one at a time on one scratch.
-// 8-bit images are checked against the int32 bound with M = 255^2 before anything is enqueued; float images (one pair
-// per call) are classified first, refused when a pixel is not finite, and checked with M = ceil((hi - lo)^2) of their
-// value range (widened by 1e-6 for the float rounding of l - r and its square).
+// SSD: 8-bit images are checked against the int32 bound with M = 255^2 before anything is enqueued; float images (one
+// pair per call) are classified first, refused when a pixel is not finite, and checked with M = ceil((hi - lo)^2) of
+// their value range (widened by 1e-6 for the float rounding of l - r and its square).  NCC: the bound (C_max = 2q) is
+// checked before anything is enqueued; float images are classified, refused when a pixel is not finite, and take the
+// per-cell cost kernel unless they are 8-bit-valued.
 static int run_sgm(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bool u8) {
+    const bool ncc = ps[0].cost == STEREO_COST_NCORR;
     size_t need = 0;
     for (int i = 0; i < n; ++i) {
         if (sgm_shape(ps[i]).K > SGM_MAXK) {
@@ -512,9 +542,11 @@ static int run_sgm(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bool u8
         const size_t b = sgm_scratch_bytes(ps[i]);
         if (b > need) need = b;
     }
-    int rc = u8 ? check_sgm_bound(ctx, ps[0].R, 255.0 * 255.0) : STEREO_OK;
+    int rc = ncc ? check_sgm_bound(ctx, 2.0 * ctx->sgm_ncc_scale, "2q")
+           : u8 ? check_ssd_sgm_bound(ctx, ps[0].R, 255.0 * 255.0) : STEREO_OK;
     if (rc == STEREO_OK) rc = reserve_arena(ctx, st, need);
     if (rc != STEREO_OK) return rc;
+    bool per_cell = false;
     if (!u8) {
         const Problem& p = ps[0];
         ImageView copies[2];
@@ -522,16 +554,19 @@ static int run_sgm(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bool u8
         if (rc != STEREO_OK) return rc;
         const unsigned flags = *reinterpret_cast<const unsigned*>(ctx->h_flag);
         if (flags & 2u) { set_error("SGM: an image holds a pixel that is not finite"); return STEREO_ERR_UNSUPPORTED; }
-        double tlo, thi, lo, hi;
-        classified_range(ctx, &tlo, &thi, &lo, &hi);
-        const double range = (hi - lo) * (1.0 + 1e-6);
-        rc = check_sgm_bound(ctx, p.R, flags == 0 ? 255.0 * 255.0 : ceil(range * range));
-        if (rc != STEREO_OK) return rc;
+        per_cell = ncc && flags != 0;
+        if (!ncc) {
+            double tlo, thi, lo, hi;
+            classified_range(ctx, &tlo, &thi, &lo, &hi);
+            const double range = (hi - lo) * (1.0 + 1e-6);
+            rc = check_ssd_sgm_bound(ctx, p.R, flags == 0 ? 255.0 * 255.0 : ceil(range * range));
+            if (rc != STEREO_OK) return rc;
+        }
     }
     ctx->last_path = STEREO_PATH_SGM;
     for (int i = 0; i < n && rc == STEREO_OK; ++i) {
         ctx->arena.reset();
-        rc = run_sgm_direction(ctx, ps[i], st);
+        rc = run_sgm_direction(ctx, ps[i], st, per_cell);
     }
     return rc;
 }
@@ -1478,6 +1513,18 @@ int stereo_ctx_sgm(const stereo_ctx* ctx, int* paths, int* p1, int* p2) {
     *p1 = ctx->sgm_p1;
     *p2 = ctx->sgm_p2;
     return STEREO_OK;
+}
+
+int stereo_ctx_set_sgm_ncc_scale(stereo_ctx* ctx, int q) {
+    if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
+    if (q < 0 || q > (1 << 24)) { set_error("SGM NCC scale must be in [0, 2^24] (got %d)", q); return STEREO_ERR_INVALID_ARG; }
+    ctx->sgm_ncc_scale = q;
+    return STEREO_OK;
+}
+
+int stereo_ctx_sgm_ncc_scale(const stereo_ctx* ctx) {
+    if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
+    return ctx->sgm_ncc_scale;
 }
 
 int stereo_filter_speckles_device(stereo_ctx* ctx, void* disp, size_t disp_step, int disp_elem_bytes, int rows, int cols, int new_val,

@@ -145,9 +145,9 @@ class Context:
         return None if size.value <= 0 else (size.value, diff.value)
 
     def set_sgm(self, paths: Optional[int], p1: int = 0, p2: int = 0) -> None:
-        """SSD pair calls: semi-global matching over ``paths`` (4 or 8) scanline directions with penalties
+        """Pair calls: semi-global matching over ``paths`` (4 or 8) scanline directions with penalties
         ``0 <= p1 <= p2``, before the left-right check and the speckle filter.  ``None`` or 0 switches it off (the
-        default)."""
+        default).  NCC pair calls are served only while an NCC scale is set (:meth:`set_sgm_ncc_scale`)."""
         v = 0 if paths is None else int(paths)
         _check(_capi.lib().stereo_ctx_set_sgm(self._h, v, int(p1), int(p2)), "stereo_ctx_set_sgm")
 
@@ -157,6 +157,19 @@ class Context:
         paths, p1, p2 = C.c_int(), C.c_int(), C.c_int()
         _check(_capi.lib().stereo_ctx_sgm(self._h, C.byref(paths), C.byref(p1), C.byref(p2)), "stereo_ctx_sgm")
         return None if paths.value <= 0 else (paths.value, p1.value, p2.value)
+
+    def set_sgm_ncc_scale(self, q: int) -> None:
+        """Integer scale ``q`` (1 .. 2**24) of the NCC matching cost for SGM; 0 (the default) makes SGM refuse NCC pair
+        calls.  A candidate d is present at (y, x) when ``0 <= x + d <= cols - 1``; its cost is
+        ``C = q - floor(float32(q * s))`` in [0, 2q], with s the candidate's float32 TM_CCORR_NORMED score in the
+        reference's arithmetic.  Independent of :meth:`set_sgm`: switching SGM off keeps q, and q alone changes
+        nothing.  ``paths * (2q + p2)`` must not exceed 2**31 - 1."""
+        _check(_capi.lib().stereo_ctx_set_sgm_ncc_scale(self._h, int(q)), "stereo_ctx_set_sgm_ncc_scale")
+
+    @property
+    def sgm_ncc_scale(self) -> int:
+        """The NCC cost scale q of SGM (0: NCC pair calls refused while SGM is on)."""
+        return int(_capi.lib().stereo_ctx_sgm_ncc_scale(self._h))
 
     def set_host_threads(self, threads: int) -> None:
         """Host threads that convert CV_32FC1 host images to u8 before the upload (0 = automatic, -1 = off)."""
@@ -308,6 +321,11 @@ class MultiGpu:
         """:meth:`Context.set_sgm` on every device's context (row-band sharded pairs refuse while it is on)."""
         v = 0 if paths is None else int(paths)
         _check(_capi.lib().stereo_mgpu_set_sgm(self._h, v, int(p1), int(p2)), "stereo_mgpu_set_sgm")
+
+    def set_sgm_ncc_scale(self, q: int) -> None:
+        """:meth:`Context.set_sgm_ncc_scale` on every device's context: ``C = q - floor(float32(q * s))`` of the NCC
+        score s, 0 refuses NCC pair calls while SGM is on."""
+        _check(_capi.lib().stereo_mgpu_set_sgm_ncc_scale(self._h, int(q)), "stereo_mgpu_set_sgm_ncc_scale")
 
     def disparity_pair_bands(self, cost: int, left: np.ndarray, right: np.ndarray, window_rad: int, disparity_range: int,
                              dtype=np.int8) -> Tuple[np.ndarray, np.ndarray]:
