@@ -334,17 +334,20 @@ __device__ __forceinline__ void fast_row(int (&col)[FM][RowShape<R, K>::NC], con
     int rqv[S::NQ4];               // packed: u8x4 of the target image;                 OPF: the entering row
     int lov[OPF ? S::NC4 : 1];     // OPF: the leaving rows
     int rov[OPF ? S::NQ4 : 1];
+    // Packed operands are fetched four columns at a time, two quads ahead of their use (update below), not all at the start of
+    // the row: with every operand word of the row live next to the column sums, ptxas split the column sums' live ranges and
+    // copied them back into place every row (about 2 moves per pixel step of the fused 4K/256 kernel, 250 -> 233 registers).
+    auto fetch_lp = [&](int i) {
+        const int4 v = lds128(lp_row + 4 * i);
+        lpv[4 * i] = v.x; lpv[4 * i + 1] = v.y; lpv[4 * i + 2] = v.z; lpv[4 * i + 3] = v.w;
+    };
+    auto fetch_rq = [&](int i) {
+        const int4 v = lds128(rq_row + 4 * i);
+        rqv[4 * i] = v.x; rqv[4 * i + 1] = v.y; rqv[4 * i + 2] = v.z; rqv[4 * i + 3] = v.w;
+    };
     if (!OPF) {
 #pragma unroll
-        for (int i = 0; i < S::NC4 / 4; ++i) {
-            const int4 v = lds128(lp_row + 4 * i);
-            lpv[4 * i] = v.x; lpv[4 * i + 1] = v.y; lpv[4 * i + 2] = v.z; lpv[4 * i + 3] = v.w;
-        }
-#pragma unroll
-        for (int i = 0; i < S::NQ4 / 4; ++i) {
-            const int4 v = lds128(rq_row + 4 * i);
-            rqv[4 * i] = v.x; rqv[4 * i + 1] = v.y; rqv[4 * i + 2] = v.z; rqv[4 * i + 3] = v.w;
-        }
+        for (int i = 0; i < 2; ++i) { fetch_lp(i); fetch_rq(i); }
     }
     // OPF: operands are fetched four columns at a time right before their first use (twice the operand words of the
     // packed path would not fit next to the column sums)
@@ -389,6 +392,10 @@ __device__ __forceinline__ void fast_row(int (&col)[FM][RowShape<R, K>::NC], con
             }
             return;
         }
+        if ((c & 3) == 0) {           // column c uses lpv[c] and rqv[c .. c + 3]
+            if (c + 8 < S::NC4) fetch_lp(c / 4 + 2);
+            if (c + 8 < S::NQ4) fetch_rq(c / 4 + 2);
+        }
         const int a = (MODE == 0) ? (lpv[c] & 0xFFFF) : lpv[c];      // warm-up: entering row only
 #pragma unroll
         for (int m = 0; m < FM; ++m)
@@ -400,11 +407,16 @@ __device__ __forceinline__ void fast_row(int (&col)[FM][RowShape<R, K>::NC], con
         return;
     }
     int e2v[S::NE4];
-#pragma unroll
-    for (int i = 0; i < S::NE4 / 4; ++i) {
+    // likewise the energy / position words, one quad ahead (step k reads e2v[k .. k + 3]); MODE 3 and the fused NCC
+    // kernels derive per-position masks / scales from the whole row up front, and the float-operand kernels (which fetch
+    // their operands per quad anyway) spill more with it (R = 7 NCC: 144 -> 160 bytes)
+    constexpr bool E2LAZY = !OPF && MODE != 3 && !(FUSED && NCC);
+    auto fetch_e2 = [&](int i) {
         const int4 v = lds128(e2_row + 4 * i);
         e2v[4 * i] = v.x; e2v[4 * i + 1] = v.y; e2v[4 * i + 2] = v.z; e2v[4 * i + 3] = v.w;
-    }
+    };
+#pragma unroll
+    for (int i = 0; i < (E2LAZY ? 1 : S::NE4 / 4); ++i) fetch_e2(i);
     // MODE 3: the selects are turned into masks once per row - per position (K + 3 of them, each used by up to four
     // candidates) and per m - so that a candidate pays ONE three-input LOP3: key | inv[k + m] | mmask[m] (SSD: all-ones =
     // KEY_INVALID loses every min) or key & ok[k + m] & mmask[m] (NCC: 0 = NCC_KEY_NONE loses every max).
@@ -474,6 +486,7 @@ __device__ __forceinline__ void fast_row(int (&col)[FM][RowShape<R, K>::NC], con
 #pragma unroll
     for (int k = 0; k < K; ++k) {                 // [pixel-loop-begin] (tests/test_capi.py checks that nothing spills in here)
         update(k + 2 * R);
+        if (E2LAZY && (k & 3) == 0 && k + 4 < S::NE4) fetch_e2(k / 4 + 1);
         if (FUSED && (k & 3) == 0) {
             const int4 v = lds128(el_row + k);
             elv[0] = v.x; elv[1] = v.y; elv[2] = v.z; elv[3] = v.w;
