@@ -286,6 +286,35 @@ int stereo_ctx_set_sgm_ncc_scale(stereo_ctx* ctx, int q);
 /* The context's current q (0: off); STEREO_ERR_INVALID_ARG for a null context. */
 int stereo_ctx_sgm_ncc_scale(const stereo_ctx* ctx);
 
+/* Uniqueness ratio of pair calls (StereoSGBM's uniquenessRatio u), on the device before the left-right check and the
+ * speckle filter (StereoSGBM's order: uniqueness -> check -> filter; the check and the filter see the pixels it rejected).
+ * u = 0 (the default) switches it off: the rule below can then never fire and results are exactly those without it.
+ * 1 <= u <= 99 switches it on for the pair entry points of this context that compute whole maps - pair host and device,
+ * f32 and u8, the batches; any other u returns STEREO_ERR_INVALID_ARG and keeps the old setting.  For each map of each pair,
+ * over the candidates d present at the pixel (SSD: xp + d in [0, Wp - 1]; NCC: x + d in [0, cols - 1]; as defined for SGM
+ * above), V(d) is the value the map minimises - S(p, d) for SGM maps, the SSD window sum C(p, d) for block-matcher maps -
+ * and j* its first minimum in ascending d (the map's own winner), V* = V(j*).  The pixel gets the sentinel
+ * -(disparity_range + 1) when some present d with |d - j*| > 1 has
+ *     V(d) (100 - u) < V* 100        (in 64-bit; StereoSGBM's integer form),
+ * and, for block-matcher maps, when every present window cost is >= 99999999 (the map holds the reference's default 0
+ * there: no candidate was accepted).  Every other pixel keeps its value.  StereoBM's form (sad[d] <= minsad (1 + u / 100))
+ * is not offered: one rule serves both matchers.  OpenCV applies the ratio to its left map only; here it applies to both
+ * maps of a pair, each against its own V, because each direction is matched on its own.
+ * Refused with STEREO_ERR_UNSUPPORTED before anything is enqueued, uploaded or written (float images: after their
+ * classification): a sentinel that does not fit the map (the left-right check's rule); NCC pair calls with SGM off (the NCC
+ * block matcher ranks float32 scores, for which OpenCV has no ratio rule; NCC SGM maps are served); row bands other than the
+ * whole image and stereo_mgpu_disparity_pair_bands_*; and, with SGM off, more than 512 candidates after clipping (as SGM)
+ * or a window cost that can reach 2^30: (2R + 1)^2 M >= 2^30 with M as for SGM (255^2 for 8-bit images, ceil((hi - lo)^2)
+ * of other float images, none for a pixel that is not finite).  Single-direction and stereo_disparity_refgpu_* calls
+ * ignore the setting.
+ * Block-matcher maps come from the same kernels as without it (same last path, same fused pairs); a second pass then
+ * recomputes each direction's exact cost volume (SGM's cost kernel, 4 bytes per pixel and padded candidate, one direction
+ * at a time, plus the padded images) and reads it once.  SGM maps apply the ratio in their last path at no extra scratch.
+ * After one call of a shape, device calls of that shape allocate nothing and stay capturable in CUDA graphs. */
+int stereo_ctx_set_uniqueness(stereo_ctx* ctx, int uniqueness_ratio);
+/* The context's current u (0: off); STEREO_ERR_INVALID_ARG for a null context. */
+int stereo_ctx_uniqueness(const stereo_ctx* ctx);
+
 /* ---- single direction, HOST buffers (the drop-in form) ------------------------------------ */
 /*
  * One disparity map for reference image `ref` searched in `tgt` over [min_disp, max_disp].
@@ -519,6 +548,9 @@ int stereo_mgpu_set_speckle_filter(stereo_mgpu* mg, int max_size, int max_diff);
 int stereo_mgpu_set_sgm(stereo_mgpu* mg, int paths, int p1, int p2);
 /* stereo_ctx_set_sgm_ncc_scale on every device's context. */
 int stereo_mgpu_set_sgm_ncc_scale(stereo_mgpu* mg, int q);
+/* stereo_ctx_set_uniqueness on every device's context.  Pair batches shard whole pairs and so give the single-GPU result;
+ * row-band sharded pairs return STEREO_ERR_UNSUPPORTED while it is on. */
+int stereo_mgpu_set_uniqueness(stereo_mgpu* mg, int uniqueness_ratio);
 /* Batches (BASELINE config 5): same arguments as stereo_disparity_pair_batch_{u8,f32}_host. */
 int stereo_mgpu_disparity_pair_batch_u8_host(stereo_mgpu* mg, int cost, int n_pairs,
                                              const uint8_t* left, const uint8_t* right, size_t img_step, size_t pair_stride,

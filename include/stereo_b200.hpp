@@ -198,6 +198,12 @@ inline void setSgmNccScale(int q, stereo_ctx* ctx = nullptr) {
     check(stereo_ctx_set_sgm_ncc_scale(ctx ? ctx : default_ctx(), q), "stereo_ctx_set_sgm_ncc_scale");
 }
 
+// Uniqueness ratio (StereoSGBM's uniquenessRatio, 1 .. 99) of the pair calls on `ctx` (default: the default context); 0
+// switches it off (stereo_ctx_set_uniqueness).
+inline void setUniqueness(int uniquenessRatio, stereo_ctx* ctx = nullptr) {
+    check(stereo_ctx_set_uniqueness(ctx ? ctx : default_ctx(), uniquenessRatio), "stereo_ctx_set_uniqueness");
+}
+
 // Kernel time of the last call on the default context, the quantity the reference logs as
 // "disparitySSDKernel execution took {} ms" (DisparitySSD.cu:203).
 inline float lastKernelMs() { return stereo_ctx_last_kernel_ms(default_ctx()); }
@@ -248,6 +254,9 @@ public:
     }
     void setSgm(int paths, int p1 = 0, int p2 = 0) { check(stereo_mgpu_set_sgm(mg_, paths, p1, p2), "stereo_mgpu_set_sgm"); }
     void setSgmNccScale(int q) { check(stereo_mgpu_set_sgm_ncc_scale(mg_, q), "stereo_mgpu_set_sgm_ncc_scale"); }
+    void setUniqueness(int uniquenessRatio) {
+        check(stereo_mgpu_set_uniqueness(mg_, uniquenessRatio), "stereo_mgpu_set_uniqueness");
+    }
 
     // disparitySSDPair / disparityNCorrPair (main.cpp:21-78) with the output rows sharded over the devices
     void disparityPairBands(int cost, const MatT& left, const MatT& right, size_t windowRad, int disparityRange, MatT& disparityLeft,

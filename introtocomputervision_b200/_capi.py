@@ -61,6 +61,9 @@ SIGNATURES = {
     "stereo_ctx_set_sgm_ncc_scale": (_i, [_vp, _i]),
     "stereo_ctx_sgm_ncc_scale": (_i, [_vp]),
     "stereo_mgpu_set_sgm_ncc_scale": (_i, [_vp, _i]),
+    "stereo_ctx_set_uniqueness": (_i, [_vp, _i]),
+    "stereo_ctx_uniqueness": (_i, [_vp]),
+    "stereo_mgpu_set_uniqueness": (_i, [_vp, _i]),
     "stereo_ctx_synchronize": (_i, [_vp, _vp]),
     "stereo_disparity_f32_host": (_i, _SINGLE_HOST),
     "stereo_disparity_u8_host": (_i, _SINGLE_HOST),

@@ -110,6 +110,7 @@ struct stereo_ctx {
     int sgm_paths = 0;        // pair calls: semi-global matching over 4 or 8 paths (0: off) ...
     int sgm_p1 = 0, sgm_p2 = 0;   // ... with these penalties
     int sgm_ncc_scale = 0;    // ... and, for NCC pair calls, this integer scale of the NCC cost (0: NCC refused)
+    int uniq = 0;             // pair calls: StereoSGBM's uniquenessRatio, 1 .. 99 (0: off)
     // device time of the hot kernels only (fast_*_kernel), per direction, for the roofline report
     static constexpr int HOT_EVENTS = 16;
     cudaEvent_t hot0[HOT_EVENTS] = {}, hot1[HOT_EVENTS] = {};

@@ -9,6 +9,8 @@
 // Launches per direction: two replicate pads (exact.cuh), [NCC: sgm_ncc_norm_kernel,] the cost kernel - sgm_cost_kernel, or
 // sgm_ncc_cell_kernel for NCC on float images that are not 8-bit-valued - then one sgm_path_kernel per path in stream
 // order; the first path writes S, the later ones read-add-write it, the last one also writes the winner-take-all map.
+// The uniqueness pass over a block matcher's SSD map reuses the pads, sgm_cost_kernel<false> and one path kernel with
+// P1 = P2 = 0 (so L_r = C), S not stored and only the sentinel written (SgmOut::only_invalid).
 // Layout: candidate index j = d - dlo innermost, padded to Dp = 32 K (K candidates per lane of the path kernels).  Absent
 // and padding candidates hold SGM_ABSENT in C and L; S of an absent candidate is 0xFFFFFFFF, above every present sum as
 // an unsigned value.  With paths * (C_max + P2) <= 2^31 - 1 (checked by the caller), every present L is below 2^29, m(q)
@@ -159,11 +161,42 @@ __host__ __device__ inline int sgm_lines(int rows, int cols, int dy, int dx) {
     return (dy ? cols : 0) + (dx ? (dy ? rows - 1 : rows) : 0);
 }
 
-struct SgmOut { void* ptr; size_t step; int elem; int dlo; };    // the map the last path writes (ptr == nullptr: none)
+// The map the last path writes (ptr == nullptr: none).  uniq: the uniqueness ratio (0: off), whose rejected pixels get
+// `sentinel`.  only_invalid: the block matcher's map is already there; store only the sentinel, also at pixels whose every
+// present V is >= 99999999 (the reference's initial best cost, so its map holds the default 0 there).
+struct SgmOut { void* ptr; size_t step; int elem; int dlo; int uniq; int sentinel; int only_invalid; };
+
+constexpr unsigned SGM_BM_NO_WINNER = 99999999u;
+
+// Winner-take-all of one pixel's V across the warp, lane l holding candidates [l K, l K + K) (absent: 0xFFFFFFFF).
+// Returns j*, the first minimum, in every lane, and its V* in *vbest.  *unique is false when uniq > 0 and some present j with
+// |j - j*| > 1 has V(j) (100 - uniq) < V* 100 (StereoSGBM's uniquenessRatio rule, in 64-bit); true otherwise, also when every
+// other candidate is absent.
+template <int K>
+__device__ __forceinline__ int sgm_winner(const unsigned (&v)[K], int lane, int uniq, unsigned* vbest, bool* unique) {
+    unsigned best = 0xFFFFFFFFu; int bi = 0;
+#pragma unroll
+    for (int i = K - 1; i >= 0; --i) if (v[i] <= best) { best = v[i]; bi = i; }
+    const unsigned wmin = __reduce_min_sync(0xffffffffu, best);
+    const unsigned ball = __ballot_sync(0xffffffffu, best == wmin);
+    const int src = __ffs(ball) - 1;
+    const int jw = __shfl_sync(0xffffffffu, lane * K + bi, src);
+    *vbest = wmin;
+    *unique = true;
+    if (uniq) {
+        unsigned far = 0xFFFFFFFFu;
+#pragma unroll
+        for (int i = 0; i < K; ++i) if (abs(lane * K + i - jw) > 1) far = min(far, v[i]);
+        far = __reduce_min_sync(0xffffffffu, far);
+        *unique = far == 0xFFFFFFFFu || (unsigned long long)far * unsigned(100 - uniq) >= (unsigned long long)wmin * 100u;
+    }
+    return jw;
+}
 
 // One path direction, one warp per scanline, lane l holding candidates [l K, l K + K) (Dp = 32 K).  The previous pixel's L_r stays in
-// registers; d -+ 1 across lanes come through shuffles and m(q) is one warp minimum.  first: S = L; otherwise S += L.
-// With out.ptr, the winner-take-all of the final S (first minimum, unsigned) is stored in out's element type.
+// registers; d -+ 1 across lanes come through shuffles and m(q) is one warp minimum.  first: S = L; otherwise S += L; S ==
+// nullptr (only with first): S is not stored.  With out.ptr, the winner-take-all of the final S (first minimum, unsigned,
+// with out.uniq the uniqueness ratio: sgm_winner) is stored in out's element type.
 template <int K>
 __global__ void __launch_bounds__(SGM_PATH_WARPS * 32)
 sgm_path_kernel(const int32_t* __restrict__ C, int32_t* __restrict__ S, int rows, int cols, int dy, int dx, int P1, int P2,
@@ -234,21 +267,18 @@ sgm_path_kernel(const int32_t* __restrict__ C, int32_t* __restrict__ S, int rows
         for (int i = 0; i < K; ++i) {
             Lq[i] = L[i];
             sn[i] = c[i] == SGM_ABSENT ? 0xFFFFFFFFu : unsigned(first ? L[i] : so[i] + L[i]);
-            S[base + i] = int(sn[i]);
+            if (S) S[base + i] = int(sn[i]);
         }
         if (out.ptr) {
-            unsigned best = 0xFFFFFFFFu; int bi = 0;
-#pragma unroll
-            for (int i = K - 1; i >= 0; --i) if (sn[i] <= best) { best = sn[i]; bi = i; }
-            const unsigned wmin = __reduce_min_sync(0xffffffffu, best);
-            const unsigned ball = __ballot_sync(0xffffffffu, best == wmin);
-            const int src = __ffs(ball) - 1;
-            const int jw = __shfl_sync(0xffffffffu, lane * K + bi, src);
-            if (lane == 0) {
+            unsigned vbest;
+            bool unique;
+            const int jw = sgm_winner<K>(sn, lane, out.uniq, &vbest, &unique);
+            const bool invalid = !unique || (out.only_invalid && vbest >= SGM_BM_NO_WINNER);
+            if (lane == 0 && (invalid || !out.only_invalid)) {
                 const long long pix = base / Dp;
                 const int py = int(pix / cols), px = int(pix - (long long)py * cols);
                 char* row = static_cast<char*>(out.ptr) + size_t(py) * out.step;
-                const int dv = out.dlo + jw;
+                const int dv = invalid ? out.sentinel : out.dlo + jw;
                 if (out.elem == 1) reinterpret_cast<int8_t*>(row)[px] = int8_t(uint8_t(uint32_t(dv) & 0xFFu));
                 else if (out.elem == 2) reinterpret_cast<int16_t*>(row)[px] = int16_t(dv);
                 else reinterpret_cast<int32_t*>(row)[px] = dv;

@@ -112,25 +112,57 @@ static void pair_problems(Problem* ps, int np, int k, int cost, PixType type, co
                            R, 0, range, disp_right, disp_step, elem, nullptr, 0);
 }
 
-// ---- pair options: left-right check (lrcheck.cuh), speckle filter (speckle.cuh), SGM (sgm.cuh) ----------------------
+// ---- pair options: uniqueness ratio, left-right check (lrcheck.cuh), speckle filter (speckle.cuh), SGM (sgm.cuh) -------
 
-// The check and the filter mark removed pixels with -(range + 1), which must fit the maps' element type.  (An int8 map of
-// more than 127 disparities already holds wrapped values.)
+// The uniqueness ratio, the check and the filter mark removed pixels with -(range + 1), which must fit the maps' element
+// type.  (An int8 map of more than 127 disparities already holds wrapped values.)
 static int check_lr_sentinel(int elem, int range) {
     if (range <= (elem == 1 ? 127 : elem == 2 ? 32767 : 32768)) return STEREO_OK;
-    set_error("left-right check / speckle filter: the sentinel -(%d + 1) does not fit a %d-byte disparity element", range, elem);
+    set_error("uniqueness ratio / left-right check / speckle filter: the sentinel -(%d + 1) does not fit a %d-byte disparity element",
+              range, elem);
+    return STEREO_ERR_UNSUPPORTED;
+}
+
+// The uniqueness pass over the block matcher's SSD maps (run_uniqueness) holds C in int32 below SGM_ABSENT, the marker of
+// absent candidates, so that no present cost reads as absent and C + m(q) of its path kernel cannot overflow:
+// (2R + 1)^2 M < 2^30, M the largest per-element term as check_ssd_sgm_bound takes it.
+static int check_uniq_bound(int R, double M) {
+    if (double(2 * R + 1) * (2 * R + 1) * M < double(SGM_ABSENT)) return STEREO_OK;
+    set_error("uniqueness ratio: the block matcher's window cost (2R + 1)^2 x %.0f (R = %d) does not stay below 2^30", M, R);
     return STEREO_ERR_UNSUPPORTED;
 }
 
 // What a pair call must satisfy for the context's options, checked once per call before anything is staged or enqueued:
-// the sentinel fits (left-right check or speckle filter on), SGM aggregates the SSD cost or, with an NCC scale set, the NCC
-// cost, and SGM paths and speckle regions, which cross band seams, get whole maps.  run_sgm checks the candidate count and
-// the int32 bound.
-static int check_pair_options(const stereo_ctx* ctx, int cost, int elem, int range, int row_begin, int row_end, int rows) {
-    const bool sgm = ctx->sgm_paths > 0, spk = ctx->spk_max_size > 0, whole = row_begin == 0 && row_end == rows;
-    if (ctx->lr_max_diff >= 0 || spk) {
+// the sentinel fits (uniqueness ratio, left-right check or speckle filter on), SGM aggregates the SSD cost or, with an NCC
+// scale set, the NCC cost, and SGM paths, speckle regions and the uniqueness pass get whole maps.  The uniqueness ratio on
+// block-matcher maps needs the SSD cost, at most 512 candidates after clipping and, for 8-bit images, check_uniq_bound with
+// M = 255^2 (float images: after their classification, check_uniq_classified).  run_sgm checks SGM's candidate count and
+// int32 bound.
+static int check_pair_options(const stereo_ctx* ctx, int cost, PixType type, int elem, int range, int R, int cols, int row_begin,
+                              int row_end, int rows) {
+    const bool sgm = ctx->sgm_paths > 0, spk = ctx->spk_max_size > 0, uniq = ctx->uniq > 0, whole = row_begin == 0 && row_end == rows;
+    if (ctx->lr_max_diff >= 0 || spk || uniq) {
         const int rc = check_lr_sentinel(elem, range);
         if (rc != STEREO_OK) return rc;
+    }
+    if (uniq && !whole) {
+        set_error("uniqueness ratio: rows [%d, %d) are not the whole map (the uniqueness pass works on whole images)", row_begin, row_end);
+        return STEREO_ERR_UNSUPPORTED;
+    }
+    if (uniq && !sgm) {
+        if (cost != STEREO_COST_SSD) {
+            set_error("uniqueness ratio: NCC block-matcher maps rank float32 scores, for which it has no rule (switch SGM on with an NCC scale)");
+            return STEREO_ERR_UNSUPPORTED;
+        }
+        const int lim = cols - 1 + R, D = (range < lim ? range : lim) + 1;      // (sgm_shape's clipping of either direction)
+        if (D > 32 * SGM_MAXK) {
+            set_error("uniqueness ratio: %d candidates per pixel, at most %d are supported", D, 32 * SGM_MAXK);
+            return STEREO_ERR_UNSUPPORTED;
+        }
+        if (type == PixType::U8) {
+            const int rc = check_uniq_bound(R, 255.0 * 255.0);
+            if (rc != STEREO_OK) return rc;
+        }
     }
     if (sgm && cost != STEREO_COST_SSD && ctx->sgm_ncc_scale == 0) {
         set_error("SGM aggregates the SSD cost only while no NCC scale is set (stereo_ctx_set_sgm_ncc_scale; or switch SGM off for NCC calls)");
@@ -343,6 +375,25 @@ static int classify_images(stereo_ctx* ctx, const Problem& p, cudaStream_t st, I
     return STEREO_OK;
 }
 
+// M of check_ssd_sgm_bound for float images from their classification (classify_flags): 255^2 when 8-bit-valued, otherwise
+// ceil((hi - lo)^2) of their value range, widened by 1e-6 for the float rounding of l - r and its square.
+static double classified_ssd_max_elem(const stereo_ctx* ctx) {
+    if (*reinterpret_cast<const unsigned*>(ctx->h_flag) == 0) return 255.0 * 255.0;
+    double tlo, thi, lo, hi;
+    classified_range(ctx, &tlo, &thi, &lo, &hi);
+    const double range = (hi - lo) * (1.0 + 1e-6);
+    return ceil(range * range);
+}
+
+// check_uniq_bound for float images from the classification the call made; a pixel that is not finite has no bound.
+static int check_uniq_classified(const stereo_ctx* ctx, int R) {
+    if (*reinterpret_cast<const unsigned*>(ctx->h_flag) & 2u) {
+        set_error("uniqueness ratio: an image holds a pixel that is not finite");
+        return STEREO_ERR_UNSUPPORTED;
+    }
+    return check_uniq_bound(R, classified_ssd_max_elem(ctx));
+}
+
 // Grows the scratch arena to `need` bytes; nothing enqueued by earlier calls may still use it then.
 static int reserve_arena(stereo_ctx* ctx, cudaStream_t st, size_t need) {
     if (need <= ctx->arena.cap) return STEREO_OK;
@@ -382,6 +433,7 @@ static int run_f32_pair(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
     ImageView u8[2];
     int cls = CLS_EXACT;
     rc = classify_images(ctx, p, st, u8, &cls);
+    if (rc == STEREO_OK && n == 2 && ctx->uniq > 0) rc = check_uniq_classified(ctx, p.R);      // (before any map is written)
     if (rc != STEREO_OK) return rc;
     if (cls == CLS_EXACT) {
         for (int d = 0; d < n && rc == STEREO_OK; ++d) rc = run_exact_direction(ctx, ps[d], st);
@@ -469,9 +521,39 @@ static int check_ssd_sgm_bound(const stereo_ctx* ctx, int R, double M) {
     return check_sgm_bound(ctx, double(2 * R + 1) * (2 * R + 1) * M, "(2R + 1)^2 x the largest element");
 }
 
+// C of one direction (sgm_cost_kernel; SSD, or NCC of 8-bit-valued images) from its padded images.
+static void launch_sgm_cost(stereo_ctx* ctx, const Problem& p, const SgmShape& g, const float* Lp, const float* Rp, const SgmNcc& ncc,
+                            int32_t* C, cudaStream_t st) {
+    // rows per cost block: as many as still leave about four blocks per SM (each block recomputes 2R + 1 rows first)
+    const long long tiles = (long long)div_round_up(p.cols, SGM_XT) * (g.Dp / 32);
+    int rpb = 64;
+    while (rpb > 8 && tiles * div_round_up(p.rows, rpb) < 4LL * ctx->sm_count) rpb /= 2;
+    const dim3 cg(div_round_up(p.cols, SGM_XT), div_round_up(p.rows, rpb), unsigned(g.Dp / 32));
+    const size_t smem = size_t(SGM_XT + 2 * p.R) * 32 * sizeof(int32_t);
+    if (p.cost == STEREO_COST_NCORR) sgm_cost_kernel<true><<<cg, SGM_COST_THREADS, smem, st>>>(Lp, Rp, p.rows, p.cols, p.R, g.dlo, g.D, int(g.Dp), rpb, ncc, C);
+    else sgm_cost_kernel<false><<<cg, SGM_COST_THREADS, smem, st>>>(Lp, Rp, p.rows, p.cols, p.R, g.dlo, g.D, int(g.Dp), rpb, ncc, C);
+    ctx->last_launches += 1;
+}
+
+// One sgm_path_kernel launch of direction (dy, dx) over C of shape g.
+static int launch_sgm_path(stereo_ctx* ctx, const Problem& p, const SgmShape& g, const int32_t* C, int32_t* S, int dy, int dx, int P1,
+                           int P2, bool first, const SgmOut& out, cudaStream_t st) {
+    const unsigned blocks = div_round_up(sgm_lines(p.rows, p.cols, dy, dx), SGM_PATH_WARPS);
+#define SB_SGM_PATH(K) case K: sgm_path_kernel<K><<<blocks, SGM_PATH_WARPS * 32, 0, st>>>(C, S, p.rows, p.cols, dy, dx, P1, P2, first, out); break
+    switch (g.K) {
+        SB_SGM_PATH(1); SB_SGM_PATH(2); SB_SGM_PATH(3); SB_SGM_PATH(4); SB_SGM_PATH(5); SB_SGM_PATH(6); SB_SGM_PATH(7); SB_SGM_PATH(8);
+        SB_SGM_PATH(9); SB_SGM_PATH(10); SB_SGM_PATH(11); SB_SGM_PATH(12); SB_SGM_PATH(13); SB_SGM_PATH(14); SB_SGM_PATH(15); SB_SGM_PATH(16);
+        default: set_error("SGM: no path kernel for %d candidates per lane (internal)", g.K); return STEREO_ERR_UNSUPPORTED;
+    }
+#undef SB_SGM_PATH
+    ctx->last_launches += 1;
+    return STEREO_OK;
+}
+
 // One direction by SGM into p.disp, on scratch the caller reserved.  ref / tgt: the caller's images (u8 or float).
 // `per_cell`: NCC on float images that are not 8-bit-valued, whose numerators are summed cell by cell (sgm_ncc_cell_kernel).
-static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st, bool per_cell) {
+// `sentinel`: the value of pixels the uniqueness ratio rejects.
+static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st, bool per_cell, int sentinel) {
     static constexpr int DIRS[8][2] = {{0, 1}, {0, -1}, {1, 0}, {-1, 0}, {1, 1}, {1, -1}, {-1, 1}, {-1, -1}};
     const SgmShape g = sgm_shape(p);
     const size_t cells = size_t(p.rows) * p.cols * g.Dp;
@@ -496,30 +578,46 @@ static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st,
         const dim3 cg(div_round_up(p.cols, SGM_CELL_XT), p.rows, unsigned(g.Dp / 32));
         const size_t smem = size_t(2 * (SGM_CELL_XT + 2 * p.R) + 31) * sizeof(float);
         sgm_ncc_cell_kernel<<<cg, SGM_COST_THREADS, smem, st>>>(Lp, Rp, p.cols, p.R, g.dlo, g.D, int(g.Dp), ncc, C);
-    } else {
-        // rows per cost block: as many as still leave about four blocks per SM (each block recomputes 2R + 1 rows first)
-        const long long tiles = (long long)div_round_up(p.cols, SGM_XT) * (g.Dp / 32);
-        int rpb = 64;
-        while (rpb > 8 && tiles * div_round_up(p.rows, rpb) < 4LL * ctx->sm_count) rpb /= 2;
-        const dim3 cg(div_round_up(p.cols, SGM_XT), div_round_up(p.rows, rpb), unsigned(g.Dp / 32));
-        const size_t smem = size_t(SGM_XT + 2 * p.R) * 32 * sizeof(int32_t);
-        if (is_ncc) sgm_cost_kernel<true><<<cg, SGM_COST_THREADS, smem, st>>>(Lp, Rp, p.rows, p.cols, p.R, g.dlo, g.D, int(g.Dp), rpb, ncc, C);
-        else sgm_cost_kernel<false><<<cg, SGM_COST_THREADS, smem, st>>>(Lp, Rp, p.rows, p.cols, p.R, g.dlo, g.D, int(g.Dp), rpb, ncc, C);
-    }
-    ctx->last_launches += 1;
-    for (int k = 0; k < ctx->sgm_paths; ++k) {
-        const int dy = DIRS[k][0], dx = DIRS[k][1];
-        const bool last = k == ctx->sgm_paths - 1;
-        const SgmOut out{last ? p.disp.ptr : nullptr, p.disp.step, p.disp.elem, g.dlo};
-        const unsigned blocks = div_round_up(sgm_lines(p.rows, p.cols, dy, dx), SGM_PATH_WARPS);
-#define SB_SGM_PATH(K) case K: sgm_path_kernel<K><<<blocks, SGM_PATH_WARPS * 32, 0, st>>>(C, S, p.rows, p.cols, dy, dx, ctx->sgm_p1, ctx->sgm_p2, k == 0, out); break
-        switch (g.K) {
-            SB_SGM_PATH(1); SB_SGM_PATH(2); SB_SGM_PATH(3); SB_SGM_PATH(4); SB_SGM_PATH(5); SB_SGM_PATH(6); SB_SGM_PATH(7); SB_SGM_PATH(8);
-            SB_SGM_PATH(9); SB_SGM_PATH(10); SB_SGM_PATH(11); SB_SGM_PATH(12); SB_SGM_PATH(13); SB_SGM_PATH(14); SB_SGM_PATH(15); SB_SGM_PATH(16);
-            default: set_error("SGM: no path kernel for %d candidates per lane (internal)", g.K); return STEREO_ERR_UNSUPPORTED;
-        }
-#undef SB_SGM_PATH
         ctx->last_launches += 1;
+    } else {
+        launch_sgm_cost(ctx, p, g, Lp, Rp, ncc, C, st);
+    }
+    for (int k = 0; k < ctx->sgm_paths; ++k) {
+        const bool last = k == ctx->sgm_paths - 1;
+        const SgmOut out{last ? p.disp.ptr : nullptr, p.disp.step, p.disp.elem, g.dlo, ctx->uniq, sentinel, 0};
+        const int rc2 = launch_sgm_path(ctx, p, g, C, S, DIRS[k][0], DIRS[k][1], ctx->sgm_p1, ctx->sgm_p2, k == 0, out, st);
+        if (rc2 != STEREO_OK) return rc2;
+    }
+    SB_CUDA(cudaGetLastError());
+    return STEREO_OK;
+}
+
+// The uniqueness pass's scratch for one direction: both padded images and C (plus, for float images, the u8 copies a
+// classification writes).  Directions run one after the other on the same scratch.
+static size_t uniq_scratch_bytes(const Problem& p) {
+    const size_t need = 2 * align256(padded_elems(p) * sizeof(float)) + align256(size_t(p.rows) * p.cols * sgm_shape(p).Dp * 4) + 4096;
+    return p.ref.type == PixType::F32 ? need + u8_copies_bytes(p) : need;
+}
+
+// The uniqueness ratio on the block matcher's SSD maps of the n directions of ps (pair_problems' layout, the caller's
+// images), after the block matcher wrote them: per direction, on scratch the caller reserved, the padded images, C
+// (sgm_cost_kernel<false>, the block matcher's window costs exactly) and one vertical path kernel with P1 = P2 = 0, so
+// that L_r = C, which stores no S and writes only the sentinel (SgmOut::only_invalid).
+static int run_uniqueness(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t st) {
+    const int sentinel = -(ps[n / 2].dmax + 1);
+    for (int i = 0; i < n; ++i) {
+        const Problem& p = ps[i];
+        const SgmShape g = sgm_shape(p);
+        ctx->arena.reset();
+        float *Lp, *Rp;
+        int rc = pad_images(ctx, p, st, &Lp, &Rp);
+        if (rc != STEREO_OK) return rc;
+        int32_t* C = static_cast<int32_t*>(ctx->arena.take(size_t(p.rows) * p.cols * g.Dp * 4));
+        if (!C) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
+        launch_sgm_cost(ctx, p, g, Lp, Rp, SgmNcc{nullptr, nullptr, 0}, C, st);
+        const SgmOut out{p.disp.ptr, p.disp.step, p.disp.elem, g.dlo, ctx->uniq, sentinel, 1};
+        rc = launch_sgm_path(ctx, p, g, C, nullptr, 1, 0, 0, 0, true, out, st);
+        if (rc != STEREO_OK) return rc;
     }
     SB_CUDA(cudaGetLastError());
     return STEREO_OK;
@@ -556,23 +654,21 @@ static int run_sgm(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bool u8
         if (flags & 2u) { set_error("SGM: an image holds a pixel that is not finite"); return STEREO_ERR_UNSUPPORTED; }
         per_cell = ncc && flags != 0;
         if (!ncc) {
-            double tlo, thi, lo, hi;
-            classified_range(ctx, &tlo, &thi, &lo, &hi);
-            const double range = (hi - lo) * (1.0 + 1e-6);
-            rc = check_ssd_sgm_bound(ctx, p.R, flags == 0 ? 255.0 * 255.0 : ceil(range * range));
+            rc = check_ssd_sgm_bound(ctx, p.R, classified_ssd_max_elem(ctx));
             if (rc != STEREO_OK) return rc;
         }
     }
     ctx->last_path = STEREO_PATH_SGM;
     for (int i = 0; i < n && rc == STEREO_OK; ++i) {
         ctx->arena.reset();
-        rc = run_sgm_direction(ctx, ps[i], st, per_cell);
+        rc = run_sgm_direction(ctx, ps[i], st, per_cell, -(ps[n / 2].dmax + 1));
     }
     return rc;
 }
 
 // Validates every direction, runs them - pairs with the context's SGM on by SGM, everything else on the kernel family
-// run_families picks - then finishes pairs with the context's left-right check and speckle filter (finish_pairs).
+// run_families picks - then, for pairs of block-matcher maps, applies the context's uniqueness ratio (run_uniqueness;
+// SGM maps apply it in their last path) and finishes pairs with the left-right check and speckle filter (finish_pairs).
 static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
     bool fast = ctx->force_path != STEREO_PATH_EXACT_F32, u8 = true;
     for (int i = 0; i < n; ++i) {
@@ -585,13 +681,25 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
         u8 = u8 && p.ref.type == PixType::U8;
     }
     const bool pair = n >= 2;      // (every pair of a call has the same shape, band, range and element type)
+    const bool uniq_pass = pair && ctx->uniq > 0 && ctx->sgm_paths == 0;
     if (pair) {
         const Problem& p = ps[0];
-        int rc = check_pair_options(ctx, p.cost, p.disp.elem, ps[n / 2].dmax, p.row_begin, p.row_end, p.rows);
-        if (rc == STEREO_OK) rc = reserve_arena(ctx, st, finish_scratch_bytes(ctx, n, p.rows, p.cols));
+        int rc = check_pair_options(ctx, p.cost, p.ref.type, p.disp.elem, ps[n / 2].dmax, p.R, p.cols, p.row_begin, p.row_end, p.rows);
+        size_t need = finish_scratch_bytes(ctx, n, p.rows, p.cols);
+        if (uniq_pass && uniq_scratch_bytes(p) > need) need = uniq_scratch_bytes(p);      // (both directions have one shape)
+        if (rc == STEREO_OK) rc = reserve_arena(ctx, st, need);
+        if (rc == STEREO_OK && uniq_pass && !u8 && !(fast && n <= 2)) {
+            // float images the exact kernels take without a classification: classify them for the bound
+            ImageView copies[2];
+            rc = classify_flags(ctx, p, st, copies);
+            if (rc == STEREO_OK) rc = check_uniq_classified(ctx, p.R);
+        }
         if (rc != STEREO_OK) return rc;
     }
-    const int rc = pair && ctx->sgm_paths > 0 ? run_sgm(ctx, ps, n, st, u8) : run_families(ctx, ps, n, st, fast, u8);
+    Problem callers[FMAXJOBS];      // (run_f32_pair points ps at u8 copies in the arena, which the uniqueness pass reuses)
+    for (int i = 0; uniq_pass && i < n; ++i) callers[i] = ps[i];
+    int rc = pair && ctx->sgm_paths > 0 ? run_sgm(ctx, ps, n, st, u8) : run_families(ctx, ps, n, st, fast, u8);
+    if (rc == STEREO_OK && uniq_pass) rc = run_uniqueness(ctx, callers, n, st);
     return rc == STEREO_OK && pair ? finish_pairs(ctx, ps, n, st, true) : rc;
 }
 
@@ -789,7 +897,7 @@ static bool host_sample_is_8bit(const void* img, size_t step, int rows, int cols
 static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, int n_pairs, const HostPairIn* in,
                                      const HostDir* dirs, int n_dirs, int rows, int cols, int R, size_t disp_step, int elem) {
     if (ctx->force_path == STEREO_PATH_EXACT_F32 || ctx->force_path == STEREO_PATH_FAST_F32) return PIPE_NOT_APPLICABLE;
-    if (n_dirs == 2 && ctx->sgm_paths > 0) return PIPE_NOT_APPLICABLE;      // (SGM maps are computed whole, run_directions)
+    if (n_dirs == 2 && (ctx->sgm_paths > 0 || ctx->uniq > 0)) return PIPE_NOT_APPLICABLE;      // (SGM maps and the uniqueness pass are computed whole, run_directions)
     const auto t_call = std::chrono::steady_clock::now();       // (trace only)
     double t_pack = 0.0, t_ring = 0.0;
     auto since = [](std::chrono::steady_clock::time_point t0) { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(); };
@@ -1527,6 +1635,21 @@ int stereo_ctx_sgm_ncc_scale(const stereo_ctx* ctx) {
     return ctx->sgm_ncc_scale;
 }
 
+int stereo_ctx_set_uniqueness(stereo_ctx* ctx, int uniqueness_ratio) {
+    if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
+    if (uniqueness_ratio < 0 || uniqueness_ratio > 99) {
+        set_error("uniqueness ratio must be in [0, 99] (got %d)", uniqueness_ratio);
+        return STEREO_ERR_INVALID_ARG;
+    }
+    ctx->uniq = uniqueness_ratio;
+    return STEREO_OK;
+}
+
+int stereo_ctx_uniqueness(const stereo_ctx* ctx) {
+    if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
+    return ctx->uniq;
+}
+
 int stereo_filter_speckles_device(stereo_ctx* ctx, void* disp, size_t disp_step, int disp_elem_bytes, int rows, int cols, int new_val,
                                   int max_size, int max_diff, void* cuda_stream) {
     int rc = check_ctx(ctx);
@@ -1838,7 +1961,7 @@ static int pair_host(stereo_ctx* ctx, int cost, PixType type, const void* left, 
     const size_t row = size_t(cols) * (type == PixType::F32 ? 4 : 1), disp_row = size_t(cols) * elem;
     int rc = check_host_args(ctx, {left, right, disp_left, disp_right}, rows, cols, elem,
                              {{left_step, row}, {right_step, row}, {disp_step, disp_row}}, range);
-    if (rc == STEREO_OK) rc = check_pair_options(ctx, cost, elem, range, 0, rows, rows);      // (as run_directions would, but before staging)
+    if (rc == STEREO_OK) rc = check_pair_options(ctx, cost, type, elem, range, R, cols, 0, rows, rows);      // (as run_directions would, but before staging)
     if (rc != STEREO_OK) return rc;
     {
         const HostPairIn in{left, left_step, right, right_step};
@@ -1922,7 +2045,7 @@ static int pair_band_host(stereo_ctx* ctx, int cost, PixType type, const void* l
     int h0 = 0, h1 = 0;
     rc = stereo_band_halo_rows(rows, row_begin, row_end, R, &h0, &h1);      // (rejects a bad band or window radius)
     if (rc != STEREO_OK) return rc;
-    rc = check_pair_options(ctx, cost, elem, range, row_begin, row_end, rows);      // (as run_directions would, but before staging)
+    rc = check_pair_options(ctx, cost, type, elem, range, R, cols, row_begin, row_end, rows);      // (as run_directions would, but before staging)
     if (rc != STEREO_OK) return rc;
     const int nh = h1 - h0;
     HostRows in[2] = {{static_cast<const char*>(left) + size_t(h0) * left_step, left_step, size_t(cols)},
@@ -2006,7 +2129,7 @@ static int pair_batch_host(stereo_ctx* ctx, int cost, PixType type, int n_pairs,
     if (n_pairs <= 0) { set_error("n_pairs must be positive"); return STEREO_ERR_INVALID_ARG; }
     int rc = check_host_args(ctx, {left, right, disp_left, disp_right}, rows, cols, disp_elem_bytes,
                              {{img_step, size_t(cols) * px}, {disp_step, size_t(cols) * disp_elem_bytes}}, disparity_range);
-    if (rc == STEREO_OK) rc = check_pair_options(ctx, cost, disp_elem_bytes, disparity_range, 0, rows, rows);
+    if (rc == STEREO_OK) rc = check_pair_options(ctx, cost, type, disp_elem_bytes, disparity_range, window_rad, cols, 0, rows, rows);
     if (rc != STEREO_OK) return rc;
     {   // pipelined: item i+1 uploads while item i computes and item i-1 downloads (3 device slots)
         std::vector<HostPairIn> in(n_pairs);

@@ -171,6 +171,19 @@ class Context:
         """The NCC cost scale q of SGM (0: NCC pair calls refused while SGM is on)."""
         return int(_capi.lib().stereo_ctx_sgm_ncc_scale(self._h))
 
+    def set_uniqueness(self, ratio: Optional[int]) -> None:
+        """Pair calls: StereoSGBM's uniqueness ratio u (1 .. 99), before the left-right check and the speckle filter.  In
+        each map a pixel gets ``-(disparity_range + 1)`` when a present candidate more than one disparity away from the
+        winner has ``V(d) * (100 - u) < V* * 100``, V the SGM sum or, with SGM off, the SSD window cost (NCC needs SGM).
+        ``None`` or 0 switches it off (the default)."""
+        v = 0 if ratio is None else int(ratio)
+        _check(_capi.lib().stereo_ctx_set_uniqueness(self._h, v), "stereo_ctx_set_uniqueness")
+
+    @property
+    def uniqueness(self) -> int:
+        """The uniqueness ratio of pair calls (0: off)."""
+        return int(_capi.lib().stereo_ctx_uniqueness(self._h))
+
     def set_host_threads(self, threads: int) -> None:
         """Host threads that convert CV_32FC1 host images to u8 before the upload (0 = automatic, -1 = off)."""
         _check(_capi.lib().stereo_ctx_set_host_threads(self._h, int(threads)), "stereo_ctx_set_host_threads")
@@ -326,6 +339,11 @@ class MultiGpu:
         """:meth:`Context.set_sgm_ncc_scale` on every device's context: ``C = q - floor(float32(q * s))`` of the NCC
         score s, 0 refuses NCC pair calls while SGM is on."""
         _check(_capi.lib().stereo_mgpu_set_sgm_ncc_scale(self._h, int(q)), "stereo_mgpu_set_sgm_ncc_scale")
+
+    def set_uniqueness(self, ratio: Optional[int]) -> None:
+        """:meth:`Context.set_uniqueness` on every device's context (row-band sharded pairs refuse while it is on)."""
+        v = 0 if ratio is None else int(ratio)
+        _check(_capi.lib().stereo_mgpu_set_uniqueness(self._h, v), "stereo_mgpu_set_uniqueness")
 
     def disparity_pair_bands(self, cost: int, left: np.ndarray, right: np.ndarray, window_rad: int, disparity_range: int,
                              dtype=np.int8) -> Tuple[np.ndarray, np.ndarray]:
