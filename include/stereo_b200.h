@@ -315,6 +315,47 @@ int stereo_ctx_set_uniqueness(stereo_ctx* ctx, int uniqueness_ratio);
 /* The context's current u (0: off); STEREO_ERR_INVALID_ARG for a null context. */
 int stereo_ctx_uniqueness(const stereo_ctx* ctx);
 
+/* StereoBM's X-Sobel prefilter (preFilterCap, PREFILTER_XSOBEL) and texture threshold (textureThreshold) of pair calls.
+ * cap = 0 (the default) switches both off; texture_threshold must then be 0, and results are exactly those without them.
+ * 1 <= cap <= 63 (StereoBM's range) switches the prefilter on for the pair entry points of this context that compute whole
+ * maps - pair host and device, f32 and u8, the batches; texture_threshold >= 0 adds the threshold (0 never fires).  Anything
+ * else returns STEREO_ERR_INVALID_ARG and keeps the old setting.
+ *   P = pf(I, cap), per image (OpenCV's prefilterXSobel), 8-bit: columns 0 and cols - 1 get cap; when rows is odd, the whole
+ *   last row gets cap (OpenCV filters rows in pairs; rows == 1 too); every other pixel takes rows a = y - 1 and b = y + 1
+ *   reflected 101-style (-1 -> 1, rows -> rows - 2) and
+ *       v = (I[a][x+1] - I[a][x-1]) + 2 (I[y][x+1] - I[y][x-1]) + (I[b][x+1] - I[b][x-1]),   P = min(max(v, -cap), cap) + cap
+ *   exactly for u8 images.  f32 images (OpenCV takes 8U only): d = fl32(I[.][x+1] - I[.][x-1]) per row,
+ *   v = fl32(fl32(d_a + 2 d_y) + d_b), P = cap + clamp(rint(v), -cap, cap) rounding half to even, P = cap where v is NaN;
+ *   for 8-bit-valued float images this equals the u8 result.
+ *   Matching: pf(left) and pf(right) are computed once per pair; the L->R map matches ref pf(left) in tgt pf(right), R->L the
+ *   other way round, with every definition above (SSD, NCC, SGM with the NCC scale, the uniqueness ratio) applied to the
+ *   prefiltered images as to given ones.  Float pair calls then run as u8 calls (no classification, no host round trip).
+ *   Texture: with T = texture_threshold, a pixel of a map gets the sentinel -(disparity_range + 1) when the sum of |P(q) - cap|
+ *   over the (2R + 1)^2 window centred on it (coordinates clamped to the image, the matcher's replicate padding) is < T, P the
+ *   map's own reference image prefiltered.  OpenCV thresholds its left map only; here both maps, each against its own
+ *   reference, as for the uniqueness ratio.
+ *   Order: prefilter -> block matcher or SGM -> uniqueness ratio -> texture threshold -> left-right check -> speckle filter.
+ * Refused with STEREO_ERR_UNSUPPORTED before anything is enqueued, uploaded or written: row bands other than the whole image
+ * (stereo_disparity_pair_band_halo_u8_device, stereo_disparity_pair_band_{u8,f32}_host) and
+ * stereo_mgpu_disparity_pair_bands_* (the odd-height rule needs whole images: prefilter them with stereo_prefilter_*_device
+ * below and call the band entry points with it off), and a texture threshold whose sentinel does not fit the map (the
+ * left-right check's rule).  Single-direction and stereo_disparity_refgpu_* calls ignore the setting.  Host pair calls take
+ * the staged whole-image path (CV_32FC1 host images are uploaded as floats).  The prefiltered images live in a grow-only
+ * buffer of the context (2 x rows x align256(cols) bytes per pair of a launch sequence): after one call of a shape, device
+ * calls of that shape allocate nothing and stay capturable in CUDA graphs. */
+int stereo_ctx_set_prefilter(stereo_ctx* ctx, int cap, int texture_threshold);
+/* The context's current cap (0: off) and texture threshold; STEREO_ERR_INVALID_ARG for a null argument. */
+int stereo_ctx_prefilter(const stereo_ctx* ctx, int* cap, int* texture_threshold);
+
+/* pf(src, cap) as defined above, one rows x cols image of DEVICE memory into the 8-bit DEVICE image dst, asynchronously on
+ * cuda_stream (nullptr: the context's stream).  For callers that shard a pair by row bands: prefilter the whole images, then
+ * call the band entry points with the option off.  Bytes past cols in each dst row are never written.  STEREO_ERR_INVALID_ARG:
+ * a null pointer, a non-positive size, a step smaller than its row, a cap outside 1 .. 63, or a dst that overlaps src. */
+int stereo_prefilter_u8_device(stereo_ctx* ctx, const uint8_t* src, size_t src_step, int rows, int cols, int cap,
+                               uint8_t* dst, size_t dst_step, void* cuda_stream);
+int stereo_prefilter_f32_device(stereo_ctx* ctx, const float* src, size_t src_step, int rows, int cols, int cap,
+                                uint8_t* dst, size_t dst_step, void* cuda_stream);
+
 /* ---- single direction, HOST buffers (the drop-in form) ------------------------------------ */
 /*
  * One disparity map for reference image `ref` searched in `tgt` over [min_disp, max_disp].
@@ -551,6 +592,9 @@ int stereo_mgpu_set_sgm_ncc_scale(stereo_mgpu* mg, int q);
 /* stereo_ctx_set_uniqueness on every device's context.  Pair batches shard whole pairs and so give the single-GPU result;
  * row-band sharded pairs return STEREO_ERR_UNSUPPORTED while it is on. */
 int stereo_mgpu_set_uniqueness(stereo_mgpu* mg, int uniqueness_ratio);
+/* stereo_ctx_set_prefilter on every device's context.  Pair batches shard whole pairs and so give the single-GPU result;
+ * row-band sharded pairs return STEREO_ERR_UNSUPPORTED while it is on. */
+int stereo_mgpu_set_prefilter(stereo_mgpu* mg, int cap, int texture_threshold);
 /* Batches (BASELINE config 5): same arguments as stereo_disparity_pair_batch_{u8,f32}_host. */
 int stereo_mgpu_disparity_pair_batch_u8_host(stereo_mgpu* mg, int cost, int n_pairs,
                                              const uint8_t* left, const uint8_t* right, size_t img_step, size_t pair_stride,

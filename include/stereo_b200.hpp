@@ -204,6 +204,12 @@ inline void setUniqueness(int uniquenessRatio, stereo_ctx* ctx = nullptr) {
     check(stereo_ctx_set_uniqueness(ctx ? ctx : default_ctx(), uniquenessRatio), "stereo_ctx_set_uniqueness");
 }
 
+// StereoBM's X-Sobel prefilter (preFilterCap, 1 .. 63) and texture threshold (textureThreshold, >= 0) of the pair calls on
+// `ctx` (default: the default context); cap 0 (with threshold 0) switches both off (stereo_ctx_set_prefilter).
+inline void setPrefilter(int cap, int textureThreshold = 0, stereo_ctx* ctx = nullptr) {
+    check(stereo_ctx_set_prefilter(ctx ? ctx : default_ctx(), cap, textureThreshold), "stereo_ctx_set_prefilter");
+}
+
 // Kernel time of the last call on the default context, the quantity the reference logs as
 // "disparitySSDKernel execution took {} ms" (DisparitySSD.cu:203).
 inline float lastKernelMs() { return stereo_ctx_last_kernel_ms(default_ctx()); }
@@ -256,6 +262,9 @@ public:
     void setSgmNccScale(int q) { check(stereo_mgpu_set_sgm_ncc_scale(mg_, q), "stereo_mgpu_set_sgm_ncc_scale"); }
     void setUniqueness(int uniquenessRatio) {
         check(stereo_mgpu_set_uniqueness(mg_, uniquenessRatio), "stereo_mgpu_set_uniqueness");
+    }
+    void setPrefilter(int cap, int textureThreshold = 0) {
+        check(stereo_mgpu_set_prefilter(mg_, cap, textureThreshold), "stereo_mgpu_set_prefilter");
     }
 
     // disparitySSDPair / disparityNCorrPair (main.cpp:21-78) with the output rows sharded over the devices

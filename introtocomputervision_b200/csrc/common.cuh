@@ -111,6 +111,9 @@ struct stereo_ctx {
     int sgm_p1 = 0, sgm_p2 = 0;   // ... with these penalties
     int sgm_ncc_scale = 0;    // ... and, for NCC pair calls, this integer scale of the NCC cost (0: NCC refused)
     int uniq = 0;             // pair calls: StereoSGBM's uniquenessRatio, 1 .. 99 (0: off)
+    int pf_cap = 0;           // pair calls: StereoBM's X-Sobel prefilter with this preFilterCap, 1 .. 63 (0: off) ...
+    int pf_texture = 0;       // ... and this textureThreshold (0: off)
+    sb::Arena pf;             // the prefiltered images of a pair call, live while the arena is reset (grow-only)
     // device time of the hot kernels only (fast_*_kernel), per direction, for the roofline report
     static constexpr int HOT_EVENTS = 16;
     cudaEvent_t hot0[HOT_EVENTS] = {}, hot1[HOT_EVENTS] = {};

@@ -75,8 +75,8 @@ int pair_bands(stereo_mgpu* mg, int cost, const T* left, size_t left_step, const
                int window_rad, int disparity_range, void* disp_left, void* disp_right, size_t disp_step, int elem, bool f32) {
     if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
     if (rows <= 0) { sb::set_error("rows must be positive"); return STEREO_ERR_INVALID_ARG; }
-    // speckle regions and SGM paths cross band seams and the uniqueness pass works on whole images: no band is filtered,
-    // aggregated or checked on its own (and no whole-pair call stands in for the bands)
+    // speckle regions and SGM paths cross band seams and the uniqueness pass and the prefilter work on whole images: no band
+    // is filtered, aggregated, checked or prefiltered on its own (and no whole-pair call stands in for the bands)
     for (stereo_ctx* c : mg->ctx) {
         int max_size = 0, max_diff = 0, paths = 0, p1 = 0, p2 = 0;
         stereo_ctx_speckle_filter(c, &max_size, &max_diff);
@@ -88,6 +88,12 @@ int pair_bands(stereo_mgpu* mg, int cost, const T* left, size_t left_step, const
         if (paths > 0) { sb::set_error("SGM on: row-band sharded pairs are not aggregated (shard whole pairs)"); return STEREO_ERR_UNSUPPORTED; }
         if (stereo_ctx_uniqueness(c) > 0) {
             sb::set_error("uniqueness ratio on: row-band sharded pairs are not checked (shard whole pairs)");
+            return STEREO_ERR_UNSUPPORTED;
+        }
+        int cap = 0, texture = 0;
+        stereo_ctx_prefilter(c, &cap, &texture);
+        if (cap > 0) {
+            sb::set_error("prefilter on: row-band sharded pairs are not prefiltered (shard whole pairs, or prefilter the whole images)");
             return STEREO_ERR_UNSUPPORTED;
         }
     }
@@ -197,6 +203,15 @@ int stereo_mgpu_set_uniqueness(stereo_mgpu* mg, int uniqueness_ratio) {
     if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
     for (stereo_ctx* c : mg->ctx) {
         const int rc = stereo_ctx_set_uniqueness(c, uniqueness_ratio);
+        if (rc != STEREO_OK) return rc;
+    }
+    return STEREO_OK;
+}
+
+int stereo_mgpu_set_prefilter(stereo_mgpu* mg, int cap, int texture_threshold) {
+    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
+    for (stereo_ctx* c : mg->ctx) {
+        const int rc = stereo_ctx_set_prefilter(c, cap, texture_threshold);
         if (rc != STEREO_OK) return rc;
     }
     return STEREO_OK;

@@ -8,6 +8,7 @@
 #include "lrcheck.cuh"
 #include "speckle.cuh"
 #include "sgm.cuh"
+#include "prefilter.cuh"
 #include "host_pack.hpp"
 
 #include <atomic>
@@ -114,12 +115,12 @@ static void pair_problems(Problem* ps, int np, int k, int cost, PixType type, co
 
 // ---- pair options: uniqueness ratio, left-right check (lrcheck.cuh), speckle filter (speckle.cuh), SGM (sgm.cuh) -------
 
-// The uniqueness ratio, the check and the filter mark removed pixels with -(range + 1), which must fit the maps' element
-// type.  (An int8 map of more than 127 disparities already holds wrapped values.)
+// The uniqueness ratio, the texture threshold, the check and the filter mark removed pixels with -(range + 1), which must
+// fit the maps' element type.  (An int8 map of more than 127 disparities already holds wrapped values.)
 static int check_lr_sentinel(int elem, int range) {
     if (range <= (elem == 1 ? 127 : elem == 2 ? 32767 : 32768)) return STEREO_OK;
-    set_error("uniqueness ratio / left-right check / speckle filter: the sentinel -(%d + 1) does not fit a %d-byte disparity element",
-              range, elem);
+    set_error("uniqueness ratio / texture threshold / left-right check / speckle filter: the sentinel -(%d + 1) does not fit a "
+              "%d-byte disparity element", range, elem);
     return STEREO_ERR_UNSUPPORTED;
 }
 
@@ -133,17 +134,23 @@ static int check_uniq_bound(int R, double M) {
 }
 
 // What a pair call must satisfy for the context's options, checked once per call before anything is staged or enqueued:
-// the sentinel fits (uniqueness ratio, left-right check or speckle filter on), SGM aggregates the SSD cost or, with an NCC
-// scale set, the NCC cost, and SGM paths, speckle regions and the uniqueness pass get whole maps.  The uniqueness ratio on
-// block-matcher maps needs the SSD cost, at most 512 candidates after clipping and, for 8-bit images, check_uniq_bound with
-// M = 255^2 (float images: after their classification, check_uniq_classified).  run_sgm checks SGM's candidate count and
-// int32 bound.
+// the sentinel fits (uniqueness ratio, texture threshold, left-right check or speckle filter on), SGM aggregates the SSD
+// cost or, with an NCC scale set, the NCC cost, and the prefilter, SGM paths, speckle regions and the uniqueness pass get
+// whole maps.  The uniqueness ratio on block-matcher maps needs the SSD cost, at most 512 candidates after clipping and,
+// for 8-bit images, check_uniq_bound with M = 255^2 (float images: after their classification, check_uniq_classified;
+// with the prefilter on every call matches 8-bit images).  run_sgm checks SGM's candidate count and int32 bound.
 static int check_pair_options(const stereo_ctx* ctx, int cost, PixType type, int elem, int range, int R, int cols, int row_begin,
                               int row_end, int rows) {
     const bool sgm = ctx->sgm_paths > 0, spk = ctx->spk_max_size > 0, uniq = ctx->uniq > 0, whole = row_begin == 0 && row_end == rows;
-    if (ctx->lr_max_diff >= 0 || spk || uniq) {
+    if (ctx->pf_cap > 0) type = PixType::U8;
+    if (ctx->lr_max_diff >= 0 || spk || uniq || ctx->pf_texture > 0) {
         const int rc = check_lr_sentinel(elem, range);
         if (rc != STEREO_OK) return rc;
+    }
+    if (ctx->pf_cap > 0 && !whole) {
+        set_error("prefilter: rows [%d, %d) are not the whole map (its odd-height rule needs whole images: prefilter them with "
+                  "stereo_prefilter_*_device and call the band entry points with it off)", row_begin, row_end);
+        return STEREO_ERR_UNSUPPORTED;
     }
     if (uniq && !whole) {
         set_error("uniqueness ratio: rows [%d, %d) are not the whole map (the uniqueness pass works on whole images)", row_begin, row_end);
@@ -213,9 +220,22 @@ static size_t finish_scratch_bytes(const stereo_ctx* ctx, int n, int rows, int c
     return ctx->spk_max_size > 0 ? speckle_scratch_bytes(n, rows, cols) : 0;
 }
 
-// The context's left-right check and speckle filter on the maps of the n/2 pairs of ps (laid out as pair_problems builds
-// them), in that order (StereoSGBM's): the check on the rows of ps, then, once `maps_complete` says every row of the maps
-// is computed, the filter on the whole maps.
+// The texture threshold on the n whole maps of ps, each against its own reference image, which prefilter_pairs made.
+static int texture_maps(stereo_ctx* ctx, const Problem* ps, int n, int sentinel, cudaStream_t st) {
+    static_assert(FMAXJOBS <= TX_MAXMAPS, "one texture launch covers the maps of one launch sequence");
+    const Problem& p = ps[0];
+    TxParams P{};
+    for (int k = 0; k < n; ++k)
+        P.map[k] = TxMap{static_cast<const uint8_t*>(ps[k].ref.ptr), ps[k].ref.step, ps[k].disp.ptr, ps[k].disp.step};
+    P.rows = p.rows; P.cols = p.cols; P.R = p.R; P.cap = ctx->pf_cap; P.threshold = ctx->pf_texture; P.sentinel = sentinel;
+    ctx->last_launches += 1;
+    return texture_launch(P, n, p.disp.elem, st);
+}
+
+// The context's texture threshold, left-right check and speckle filter on the maps of the n/2 pairs of ps (laid out as
+// pair_problems builds them), in that order (StereoBM's / StereoSGBM's): the threshold (whole maps only: the prefilter is
+// refused for bands) and the check on the rows of ps, then, once `maps_complete` says every row of the maps is computed,
+// the filter on the whole maps.
 static int finish_pairs(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t st, bool maps_complete) {
     static_assert(FMAXJOBS / 2 <= LR_MAXPAIRS, "one check launch covers the pairs of one launch sequence");
     static_assert(FMAXJOBS <= SPK_MAXMAPS, "one filter launch covers the maps of one launch sequence");
@@ -224,7 +244,8 @@ static int finish_pairs(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t 
     OutView maps[FMAXJOBS];
     for (int k = 0; k < n; ++k) maps[k] = ps[k].disp;
     int rc = STEREO_OK;
-    if (ctx->lr_max_diff >= 0) rc = lr_check_pairs(ctx, maps, n / 2, p.row_end - p.row_begin, p.cols, ctx->lr_max_diff, sentinel, st);
+    if (ctx->pf_cap > 0 && ctx->pf_texture > 0) rc = texture_maps(ctx, ps, n, sentinel, st);
+    if (rc == STEREO_OK && ctx->lr_max_diff >= 0) rc = lr_check_pairs(ctx, maps, n / 2, p.row_end - p.row_begin, p.cols, ctx->lr_max_diff, sentinel, st);
     if (rc != STEREO_OK || !maps_complete || ctx->spk_max_size <= 0) return rc;
     for (int k = 0; k < n; ++k) maps[k].ptr = static_cast<char*>(maps[k].ptr) - size_t(ps[k].row_begin) * maps[k].step;
     return speckle_maps(ctx, maps, n, p.rows, p.cols, sentinel, ctx->spk_max_size, ctx->spk_max_diff, st);
@@ -666,9 +687,44 @@ static int run_sgm(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bool u8
     return rc;
 }
 
+// ---- prefilter (prefilter.cuh) ----------------------------------------------------------------------------------------
+// Both images of every pair of ps (pair_problems' layout, whole images) prefiltered once, in one launch, into ctx->pf:
+// u8 images of align256(cols) pitch that stay live while the arena is reset.  Every problem is then repointed at them
+// (L->R: ref pf(left), tgt pf(right); R->L swapped), so everything after matches 8-bit images.  The buffer grows (after
+// quiesce) only for a larger shape: after one call of a shape nothing is allocated.
+static int prefilter_pairs(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
+    static_assert(FMAXJOBS <= PF_MAXIMGS, "one prefilter launch covers the images of one launch sequence");
+    const int np = n / 2;
+    const Problem& p = ps[0];
+    const size_t pitch = align256(p.cols), img = size_t(p.rows) * pitch;
+    if (size_t(n) * align256(img) > ctx->pf.cap) {
+        int rc = quiesce(ctx, st);
+        if (rc == STEREO_OK) rc = ctx->pf.reserve(size_t(n) * align256(img));
+        if (rc != STEREO_OK) return rc;
+    }
+    ctx->pf.reset();
+    const bool f32 = p.ref.type == PixType::F32;
+    PfParams P{};
+    for (int k = 0; k < np; ++k) {
+        uint8_t* l8 = static_cast<uint8_t*>(ctx->pf.take(img));
+        uint8_t* r8 = static_cast<uint8_t*>(ctx->pf.take(img));
+        if (!l8 || !r8) { set_error("prefilter buffer too small (internal)"); return STEREO_ERR_ALLOC; }
+        P.img[2 * k] = PfImage{ps[k].ref.ptr, l8, ps[k].ref.step, pitch};
+        P.img[2 * k + 1] = PfImage{ps[k].tgt.ptr, r8, ps[k].tgt.step, pitch};
+        ps[k].ref = ImageView{l8, pitch, PixType::U8};
+        ps[k].tgt = ImageView{r8, pitch, PixType::U8};
+        ps[np + k].ref = ps[k].tgt;
+        ps[np + k].tgt = ps[k].ref;
+    }
+    P.rows = p.rows; P.cols = p.cols; P.cap = ctx->pf_cap;
+    ctx->last_launches += 1;
+    return prefilter_launch(P, n, f32, st);
+}
+
 // Validates every direction, runs them - pairs with the context's SGM on by SGM, everything else on the kernel family
 // run_families picks - then, for pairs of block-matcher maps, applies the context's uniqueness ratio (run_uniqueness;
-// SGM maps apply it in their last path) and finishes pairs with the left-right check and speckle filter (finish_pairs).
+// SGM maps apply it in their last path) and finishes pairs with the texture threshold, the left-right check and the
+// speckle filter (finish_pairs).  Pairs with the prefilter on match the prefiltered images (prefilter_pairs) from the start.
 static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
     bool fast = ctx->force_path != STEREO_PATH_EXACT_F32, u8 = true;
     for (int i = 0; i < n; ++i) {
@@ -685,6 +741,10 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
     if (pair) {
         const Problem& p = ps[0];
         int rc = check_pair_options(ctx, p.cost, p.ref.type, p.disp.elem, ps[n / 2].dmax, p.R, p.cols, p.row_begin, p.row_end, p.rows);
+        if (rc == STEREO_OK && ctx->pf_cap > 0) {
+            rc = prefilter_pairs(ctx, ps, n, st);
+            u8 = true;
+        }
         size_t need = finish_scratch_bytes(ctx, n, p.rows, p.cols);
         if (uniq_pass && uniq_scratch_bytes(p) > need) need = uniq_scratch_bytes(p);      // (both directions have one shape)
         if (rc == STEREO_OK) rc = reserve_arena(ctx, st, need);
@@ -897,7 +957,8 @@ static bool host_sample_is_8bit(const void* img, size_t step, int rows, int cols
 static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, int n_pairs, const HostPairIn* in,
                                      const HostDir* dirs, int n_dirs, int rows, int cols, int R, size_t disp_step, int elem) {
     if (ctx->force_path == STEREO_PATH_EXACT_F32 || ctx->force_path == STEREO_PATH_FAST_F32) return PIPE_NOT_APPLICABLE;
-    if (n_dirs == 2 && (ctx->sgm_paths > 0 || ctx->uniq > 0)) return PIPE_NOT_APPLICABLE;      // (SGM maps and the uniqueness pass are computed whole, run_directions)
+    // (SGM maps, the uniqueness pass and the prefilter are computed whole, run_directions)
+    if (n_dirs == 2 && (ctx->sgm_paths > 0 || ctx->uniq > 0 || ctx->pf_cap > 0)) return PIPE_NOT_APPLICABLE;
     const auto t_call = std::chrono::steady_clock::now();       // (trace only)
     double t_pack = 0.0, t_ring = 0.0;
     auto since = [](std::chrono::steady_clock::time_point t0) { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(); };
@@ -1359,6 +1420,7 @@ int stereo_ctx_create(int device, stereo_ctx** ctx_out) {
     }
     int rc = fast_ctx_init(c);
     if (rc == STEREO_OK) rc = lr_check_init();
+    if (rc == STEREO_OK) rc = texture_init();
     if (rc != STEREO_OK) { stereo_ctx_destroy(c); return rc; }
     *ctx_out = c;
     return STEREO_OK;
@@ -1370,6 +1432,7 @@ void stereo_ctx_destroy(stereo_ctx* ctx) {
     if (ctx->stream) { cudaStreamSynchronize(ctx->stream); }
     ctx->arena.release();
     ctx->io.release();
+    ctx->pf.release();
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
     delete ctx->pool;
     if (ctx->d_flag) cudaFree(ctx->d_flag);
@@ -1648,6 +1711,59 @@ int stereo_ctx_set_uniqueness(stereo_ctx* ctx, int uniqueness_ratio) {
 int stereo_ctx_uniqueness(const stereo_ctx* ctx) {
     if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
     return ctx->uniq;
+}
+
+int stereo_ctx_set_prefilter(stereo_ctx* ctx, int cap, int texture_threshold) {
+    if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
+    if (cap < 0 || cap > 63 || texture_threshold < 0 || (cap == 0 && texture_threshold != 0)) {
+        set_error("prefilter: cap must be in [1, 63] (0: off) and the texture threshold >= 0 (0 while off) (got %d, %d)", cap,
+                  texture_threshold);
+        return STEREO_ERR_INVALID_ARG;
+    }
+    ctx->pf_cap = cap;
+    ctx->pf_texture = texture_threshold;
+    return STEREO_OK;
+}
+
+int stereo_ctx_prefilter(const stereo_ctx* ctx, int* cap, int* texture_threshold) {
+    if (!ctx || !cap || !texture_threshold) { set_error("null argument"); return STEREO_ERR_INVALID_ARG; }
+    *cap = ctx->pf_cap;
+    *texture_threshold = ctx->pf_texture;
+    return STEREO_OK;
+}
+
+// pf(src) into dst, one image, on the caller's stream.
+static int prefilter_device(stereo_ctx* ctx, const void* src, size_t src_step, size_t px, int rows, int cols, int cap, uint8_t* dst,
+                            size_t dst_step, void* cuda_stream) {
+    int rc = check_ctx(ctx);
+    if (rc != STEREO_OK) return rc;
+    if (!src || !dst) { set_error("null pointer"); return STEREO_ERR_INVALID_ARG; }
+    if (rows <= 0 || cols <= 0) { set_error("rows/cols must be positive (got %d x %d)", rows, cols); return STEREO_ERR_INVALID_ARG; }
+    if (rows > 32768 || cols > 32768) { set_error("image larger than 32768 in a dimension"); return STEREO_ERR_UNSUPPORTED; }
+    if (src_step < size_t(cols) * px || dst_step < size_t(cols)) { set_error("a step is smaller than its row"); return STEREO_ERR_INVALID_ARG; }
+    if (cap < 1 || cap > 63) { set_error("prefilter cap must be in [1, 63] (got %d)", cap); return STEREO_ERR_INVALID_ARG; }
+    const uintptr_t s0 = reinterpret_cast<uintptr_t>(src), s1 = s0 + size_t(rows - 1) * src_step + size_t(cols) * px;
+    const uintptr_t d0 = reinterpret_cast<uintptr_t>(dst), d1 = d0 + size_t(rows - 1) * dst_step + size_t(cols);
+    if (s0 < d1 && d0 < s1) { set_error("prefilter: dst overlaps src"); return STEREO_ERR_INVALID_ARG; }
+    cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream;
+    begin_call(ctx, st);
+    PfParams P{};
+    P.img[0] = PfImage{src, dst, src_step, dst_step};
+    P.rows = rows; P.cols = cols; P.cap = cap;
+    ctx->last_launches += 1;
+    rc = prefilter_launch(P, 1, px == 4, st);
+    end_call(ctx, st);
+    return rc;
+}
+
+int stereo_prefilter_u8_device(stereo_ctx* ctx, const uint8_t* src, size_t src_step, int rows, int cols, int cap, uint8_t* dst,
+                               size_t dst_step, void* cuda_stream) {
+    return prefilter_device(ctx, src, src_step, 1, rows, cols, cap, dst, dst_step, cuda_stream);
+}
+
+int stereo_prefilter_f32_device(stereo_ctx* ctx, const float* src, size_t src_step, int rows, int cols, int cap, uint8_t* dst,
+                                size_t dst_step, void* cuda_stream) {
+    return prefilter_device(ctx, src, src_step, 4, rows, cols, cap, dst, dst_step, cuda_stream);
 }
 
 int stereo_filter_speckles_device(stereo_ctx* ctx, void* disp, size_t disp_step, int disp_elem_bytes, int rows, int cols, int new_val,

@@ -184,6 +184,22 @@ class Context:
         """The uniqueness ratio of pair calls (0: off)."""
         return int(_capi.lib().stereo_ctx_uniqueness(self._h))
 
+    def set_prefilter(self, cap: Optional[int], texture_threshold: int = 0) -> None:
+        """Pair calls: StereoBM's X-Sobel prefilter with ``preFilterCap`` = ``cap`` (1 .. 63): both maps of a pair match
+        the clipped horizontal Sobel responses of the images (8-bit, in [0, 2 cap]) instead of their intensities.
+        ``texture_threshold`` > 0 adds StereoBM's ``textureThreshold``: a pixel whose window holds a sum of
+        ``|P - cap|`` below it gets ``-(disparity_range + 1)``, before the left-right check and the speckle filter.
+        ``None`` or 0 switches both off (the default)."""
+        v = 0 if cap is None else int(cap)
+        _check(_capi.lib().stereo_ctx_set_prefilter(self._h, v, int(texture_threshold)), "stereo_ctx_set_prefilter")
+
+    @property
+    def prefilter(self) -> Optional[Tuple[int, int]]:
+        """``(cap, texture_threshold)`` of the prefilter, or None when it is off."""
+        cap, tex = C.c_int(), C.c_int()
+        _check(_capi.lib().stereo_ctx_prefilter(self._h, C.byref(cap), C.byref(tex)), "stereo_ctx_prefilter")
+        return None if cap.value <= 0 else (cap.value, tex.value)
+
     def set_host_threads(self, threads: int) -> None:
         """Host threads that convert CV_32FC1 host images to u8 before the upload (0 = automatic, -1 = off)."""
         _check(_capi.lib().stereo_ctx_set_host_threads(self._h, int(threads)), "stereo_ctx_set_host_threads")
@@ -344,6 +360,11 @@ class MultiGpu:
         """:meth:`Context.set_uniqueness` on every device's context (row-band sharded pairs refuse while it is on)."""
         v = 0 if ratio is None else int(ratio)
         _check(_capi.lib().stereo_mgpu_set_uniqueness(self._h, v), "stereo_mgpu_set_uniqueness")
+
+    def set_prefilter(self, cap: Optional[int], texture_threshold: int = 0) -> None:
+        """:meth:`Context.set_prefilter` on every device's context (row-band sharded pairs refuse while it is on)."""
+        v = 0 if cap is None else int(cap)
+        _check(_capi.lib().stereo_mgpu_set_prefilter(self._h, v, int(texture_threshold)), "stereo_mgpu_set_prefilter")
 
     def disparity_pair_bands(self, cost: int, left: np.ndarray, right: np.ndarray, window_rad: int, disparity_range: int,
                              dtype=np.int8) -> Tuple[np.ndarray, np.ndarray]:
