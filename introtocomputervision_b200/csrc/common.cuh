@@ -74,6 +74,28 @@ struct Arena {
     void release();
 };
 
+// The pair options of a context: what pair calls do beyond the block matcher.  Single-direction calls ignore them.
+struct PairOptions {
+    int lr_max_diff = -1;     // left-right consistency check with this disp12MaxDiff (< 0: off)
+    int spk_max_size = 0;     // speckle filter of components up to this many pixels (0: off) ...
+    int spk_max_diff = 0;     // ... whose neighbours differ by at most this much
+    int sgm_paths = 0;        // semi-global matching over 4 or 8 paths (0: off) ...
+    int sgm_p1 = 0, sgm_p2 = 0;   // ... with these penalties
+    int sgm_ncc_scale = 0;    // ... and, for NCC pair calls, this integer scale of the NCC cost (0: NCC refused)
+    int uniq = 0;             // StereoSGBM's uniquenessRatio, 1 .. 99 (0: off)
+    int pf_cap = 0;           // StereoBM's X-Sobel prefilter with this preFilterCap, 1 .. 63 (0: off) ...
+    int pf_texture = 0;       // ... and this textureThreshold (0: off)
+
+    // Removed pixels are marked with -(range + 1), which must fit the maps' element type.
+    bool writes_sentinel() const { return lr_max_diff >= 0 || spk_max_size > 0 || uniq > 0 || pf_texture > 0; }
+    // Row bands are refused: speckle regions and SGM paths cross band seams, the uniqueness pass and the prefilter's
+    // odd-height rule work on whole images.
+    bool needs_whole_maps() const { return pf_cap > 0 || uniq > 0 || sgm_paths > 0 || spk_max_size > 0; }
+    // The maps are computed from whole images in one go, so the host pipeline's row bands do not apply.  (The speckle
+    // filter is not here: the pipeline filters an item's maps after its last band.)
+    bool computed_whole() const { return sgm_paths > 0 || uniq > 0 || pf_cap > 0; }
+};
+
 } // namespace sb
 
 struct stereo_ctx {
@@ -104,15 +126,7 @@ struct stereo_ctx {
     int force_path = 0;
     int pipe_bands = 0;       // 0 = automatic
     int fuse_pairs = 1;       // both maps of a pair from one cost volume where the problem allows it
-    int lr_max_diff = -1;     // pair calls: left-right consistency check with this disp12MaxDiff (< 0: off)
-    int spk_max_size = 0;     // pair calls: speckle filter of components up to this many pixels (0: off) ...
-    int spk_max_diff = 0;     // ... whose neighbours differ by at most this much
-    int sgm_paths = 0;        // pair calls: semi-global matching over 4 or 8 paths (0: off) ...
-    int sgm_p1 = 0, sgm_p2 = 0;   // ... with these penalties
-    int sgm_ncc_scale = 0;    // ... and, for NCC pair calls, this integer scale of the NCC cost (0: NCC refused)
-    int uniq = 0;             // pair calls: StereoSGBM's uniquenessRatio, 1 .. 99 (0: off)
-    int pf_cap = 0;           // pair calls: StereoBM's X-Sobel prefilter with this preFilterCap, 1 .. 63 (0: off) ...
-    int pf_texture = 0;       // ... and this textureThreshold (0: off)
+    sb::PairOptions opt;      // what pair calls do beyond the block matcher (stereo_ctx_set_lr_check .. _set_prefilter)
     sb::Arena pf;             // the prefiltered images of a pair call, live while the arena is reset (grow-only)
     // device time of the hot kernels only (fast_*_kernel), per direction, for the roofline report
     static constexpr int HOT_EVENTS = 16;

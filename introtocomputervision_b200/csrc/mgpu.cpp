@@ -12,7 +12,10 @@
 #include <thread>
 #include <vector>
 
-namespace sb { void set_error(const char* fmt, ...); }
+namespace sb {
+void set_error(const char* fmt, ...);
+const char* band_sharding_refusal(const stereo_ctx* ctx);
+}
 
 struct stereo_mgpu {
     std::vector<stereo_ctx*> ctx;
@@ -47,6 +50,17 @@ int for_each_device(stereo_mgpu* mg, F fn) {
     return STEREO_OK;
 }
 
+// One pair-option setter on the context of every device; stops at the first refusal.
+template <class... A>
+int set_all(stereo_mgpu* mg, int (*set)(stereo_ctx*, A...), A... args) {
+    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
+    for (stereo_ctx* c : mg->ctx) {
+        const int rc = set(c, args...);
+        if (rc != STEREO_OK) return rc;
+    }
+    return STEREO_OK;
+}
+
 template <class T>
 int pair_batch(stereo_mgpu* mg, int cost, int n_pairs, const T* left, const T* right, size_t img_step, size_t pair_stride, int rows,
                int cols, int window_rad, int disparity_range, void* disp_left, void* disp_right, size_t disp_step,
@@ -75,28 +89,8 @@ int pair_bands(stereo_mgpu* mg, int cost, const T* left, size_t left_step, const
                int window_rad, int disparity_range, void* disp_left, void* disp_right, size_t disp_step, int elem, bool f32) {
     if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
     if (rows <= 0) { sb::set_error("rows must be positive"); return STEREO_ERR_INVALID_ARG; }
-    // speckle regions and SGM paths cross band seams and the uniqueness pass and the prefilter work on whole images: no band
-    // is filtered, aggregated, checked or prefiltered on its own (and no whole-pair call stands in for the bands)
-    for (stereo_ctx* c : mg->ctx) {
-        int max_size = 0, max_diff = 0, paths = 0, p1 = 0, p2 = 0;
-        stereo_ctx_speckle_filter(c, &max_size, &max_diff);
-        stereo_ctx_sgm(c, &paths, &p1, &p2);
-        if (max_size > 0) {
-            sb::set_error("speckle filter on: row-band sharded pairs are not filtered (filter the gathered map with stereo_filter_speckles_device)");
-            return STEREO_ERR_UNSUPPORTED;
-        }
-        if (paths > 0) { sb::set_error("SGM on: row-band sharded pairs are not aggregated (shard whole pairs)"); return STEREO_ERR_UNSUPPORTED; }
-        if (stereo_ctx_uniqueness(c) > 0) {
-            sb::set_error("uniqueness ratio on: row-band sharded pairs are not checked (shard whole pairs)");
-            return STEREO_ERR_UNSUPPORTED;
-        }
-        int cap = 0, texture = 0;
-        stereo_ctx_prefilter(c, &cap, &texture);
-        if (cap > 0) {
-            sb::set_error("prefilter on: row-band sharded pairs are not prefiltered (shard whole pairs, or prefilter the whole images)");
-            return STEREO_ERR_UNSUPPORTED;
-        }
-    }
+    for (stereo_ctx* c : mg->ctx)
+        if (const char* why = sb::band_sharding_refusal(c)) { sb::set_error("%s", why); return STEREO_ERR_UNSUPPORTED; }
     int parts = int(mg->ctx.size());
     const int band = (rows + parts - 1) / parts;            // equal bands of ceil(rows / parts) rows, the last one(s) shorter or empty
     int rc = for_each_device(mg, [&](int k) -> int {
@@ -163,58 +157,20 @@ stereo_ctx* stereo_mgpu_ctx(stereo_mgpu* mg, int index) {
     return mg->ctx[index];
 }
 
-int stereo_mgpu_set_lr_check(stereo_mgpu* mg, int max_diff) {
-    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
-    for (stereo_ctx* c : mg->ctx) {
-        const int rc = stereo_ctx_set_lr_check(c, max_diff);
-        if (rc != STEREO_OK) return rc;
-    }
-    return STEREO_OK;
-}
+int stereo_mgpu_set_lr_check(stereo_mgpu* mg, int max_diff) { return set_all(mg, stereo_ctx_set_lr_check, max_diff); }
 
 int stereo_mgpu_set_speckle_filter(stereo_mgpu* mg, int max_size, int max_diff) {
-    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
-    for (stereo_ctx* c : mg->ctx) {
-        const int rc = stereo_ctx_set_speckle_filter(c, max_size, max_diff);
-        if (rc != STEREO_OK) return rc;
-    }
-    return STEREO_OK;
+    return set_all(mg, stereo_ctx_set_speckle_filter, max_size, max_diff);
 }
 
-int stereo_mgpu_set_sgm(stereo_mgpu* mg, int paths, int p1, int p2) {
-    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
-    for (stereo_ctx* c : mg->ctx) {
-        const int rc = stereo_ctx_set_sgm(c, paths, p1, p2);
-        if (rc != STEREO_OK) return rc;
-    }
-    return STEREO_OK;
-}
+int stereo_mgpu_set_sgm(stereo_mgpu* mg, int paths, int p1, int p2) { return set_all(mg, stereo_ctx_set_sgm, paths, p1, p2); }
 
-int stereo_mgpu_set_sgm_ncc_scale(stereo_mgpu* mg, int q) {
-    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
-    for (stereo_ctx* c : mg->ctx) {
-        const int rc = stereo_ctx_set_sgm_ncc_scale(c, q);
-        if (rc != STEREO_OK) return rc;
-    }
-    return STEREO_OK;
-}
+int stereo_mgpu_set_sgm_ncc_scale(stereo_mgpu* mg, int q) { return set_all(mg, stereo_ctx_set_sgm_ncc_scale, q); }
 
-int stereo_mgpu_set_uniqueness(stereo_mgpu* mg, int uniqueness_ratio) {
-    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
-    for (stereo_ctx* c : mg->ctx) {
-        const int rc = stereo_ctx_set_uniqueness(c, uniqueness_ratio);
-        if (rc != STEREO_OK) return rc;
-    }
-    return STEREO_OK;
-}
+int stereo_mgpu_set_uniqueness(stereo_mgpu* mg, int uniqueness_ratio) { return set_all(mg, stereo_ctx_set_uniqueness, uniqueness_ratio); }
 
 int stereo_mgpu_set_prefilter(stereo_mgpu* mg, int cap, int texture_threshold) {
-    if (!mg || mg->ctx.empty()) { sb::set_error("null multi-GPU context"); return STEREO_ERR_INVALID_ARG; }
-    for (stereo_ctx* c : mg->ctx) {
-        const int rc = stereo_ctx_set_prefilter(c, cap, texture_threshold);
-        if (rc != STEREO_OK) return rc;
-    }
-    return STEREO_OK;
+    return set_all(mg, stereo_ctx_set_prefilter, cap, texture_threshold);
 }
 
 int stereo_mgpu_disparity_pair_batch_u8_host(stereo_mgpu* mg, int cost, int n_pairs, const uint8_t* left, const uint8_t* right,

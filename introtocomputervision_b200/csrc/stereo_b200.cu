@@ -133,30 +133,67 @@ static int check_uniq_bound(int R, double M) {
     return STEREO_ERR_UNSUPPORTED;
 }
 
+// The options of PairOptions::needs_whole_maps, each with its refusal of a row band [%d, %d) by check_pair_options and of
+// row-band sharding by band_sharding_refusal.  An option's entry is on while its field is positive.  check_pair_options
+// names the first option on in this order, band_sharding_refusal the last.
+struct WholeMapOption {
+    int PairOptions::*field;
+    const char* band;
+    const char* sharding;
+};
+static const WholeMapOption WHOLE_MAP_OPTIONS[] = {
+    {&PairOptions::pf_cap,
+     "prefilter: rows [%d, %d) are not the whole map (its odd-height rule needs whole images: prefilter them with "
+     "stereo_prefilter_*_device and call the band entry points with it off)",
+     "prefilter on: row-band sharded pairs are not prefiltered (shard whole pairs, or prefilter the whole images)"},
+    {&PairOptions::uniq,
+     "uniqueness ratio: rows [%d, %d) are not the whole map (the uniqueness pass works on whole images)",
+     "uniqueness ratio on: row-band sharded pairs are not checked (shard whole pairs)"},
+    {&PairOptions::sgm_paths,
+     "SGM: rows [%d, %d) are not the whole map (vertical and diagonal paths cross band seams)",
+     "SGM on: row-band sharded pairs are not aggregated (shard whole pairs)"},
+    {&PairOptions::spk_max_size,
+     "speckle filter: rows [%d, %d) are not the whole map (filter the gathered map with stereo_filter_speckles_device)",
+     "speckle filter on: row-band sharded pairs are not filtered (filter the gathered map with stereo_filter_speckles_device)"},
+};
+
+// Why the row-band sharded pair calls (stereo_mgpu_disparity_pair_bands_*) refuse a context's options, or nullptr when
+// they do not.  No band is filtered, aggregated, checked or prefiltered on its own, and no whole-pair call stands in for
+// the bands: this holds for one device too, whose band is the whole image.
+const char* band_sharding_refusal(const stereo_ctx* ctx) {
+    if (!ctx->opt.needs_whole_maps()) return nullptr;
+    const int n = int(sizeof(WHOLE_MAP_OPTIONS) / sizeof(WHOLE_MAP_OPTIONS[0]));
+    for (int k = n - 1; k >= 0; --k)
+        if (ctx->opt.*WHOLE_MAP_OPTIONS[k].field > 0) return WHOLE_MAP_OPTIONS[k].sharding;
+    return nullptr;
+}
+
 // What a pair call must satisfy for the context's options, checked once per call before anything is staged or enqueued:
-// the sentinel fits (uniqueness ratio, texture threshold, left-right check or speckle filter on), SGM aggregates the SSD
-// cost or, with an NCC scale set, the NCC cost, and the prefilter, SGM paths, speckle regions and the uniqueness pass get
-// whole maps.  The uniqueness ratio on block-matcher maps needs the SSD cost, at most 512 candidates after clipping and,
-// for 8-bit images, check_uniq_bound with M = 255^2 (float images: after their classification, check_uniq_classified;
-// with the prefilter on every call matches 8-bit images).  run_sgm checks SGM's candidate count and int32 bound.
+// the sentinel fits (PairOptions::writes_sentinel), SGM aggregates the SSD cost or, with an NCC scale set, the NCC cost,
+// and the options of PairOptions::needs_whole_maps get whole maps.  The uniqueness ratio on block-matcher maps needs the
+// SSD cost, at most 512 candidates after clipping and, for 8-bit images, check_uniq_bound with M = 255^2 (float images:
+// after their classification, check_uniq_classified; with the prefilter on every call matches 8-bit images).  run_sgm
+// checks SGM's candidate count and int32 bound.
 static int check_pair_options(const stereo_ctx* ctx, int cost, PixType type, int elem, int range, int R, int cols, int row_begin,
                               int row_end, int rows) {
-    const bool sgm = ctx->sgm_paths > 0, spk = ctx->spk_max_size > 0, uniq = ctx->uniq > 0, whole = row_begin == 0 && row_end == rows;
-    if (ctx->pf_cap > 0) type = PixType::U8;
-    if (ctx->lr_max_diff >= 0 || spk || uniq || ctx->pf_texture > 0) {
+    const PairOptions& o = ctx->opt;
+    const bool sgm = o.sgm_paths > 0;
+    if (o.pf_cap > 0) type = PixType::U8;
+    if (o.writes_sentinel()) {
         const int rc = check_lr_sentinel(elem, range);
         if (rc != STEREO_OK) return rc;
     }
-    if (ctx->pf_cap > 0 && !whole) {
-        set_error("prefilter: rows [%d, %d) are not the whole map (its odd-height rule needs whole images: prefilter them with "
-                  "stereo_prefilter_*_device and call the band entry points with it off)", row_begin, row_end);
+    if (sgm && cost != STEREO_COST_SSD && o.sgm_ncc_scale == 0) {
+        set_error("SGM aggregates the SSD cost only while no NCC scale is set (stereo_ctx_set_sgm_ncc_scale; or switch SGM off for NCC calls)");
         return STEREO_ERR_UNSUPPORTED;
     }
-    if (uniq && !whole) {
-        set_error("uniqueness ratio: rows [%d, %d) are not the whole map (the uniqueness pass works on whole images)", row_begin, row_end);
-        return STEREO_ERR_UNSUPPORTED;
-    }
-    if (uniq && !sgm) {
+    if ((row_begin != 0 || row_end != rows) && o.needs_whole_maps())
+        for (const WholeMapOption& w : WHOLE_MAP_OPTIONS)
+            if (o.*w.field > 0) {
+                set_error(w.band, row_begin, row_end);
+                return STEREO_ERR_UNSUPPORTED;
+            }
+    if (o.uniq > 0 && !sgm) {
         if (cost != STEREO_COST_SSD) {
             set_error("uniqueness ratio: NCC block-matcher maps rank float32 scores, for which it has no rule (switch SGM on with an NCC scale)");
             return STEREO_ERR_UNSUPPORTED;
@@ -170,19 +207,6 @@ static int check_pair_options(const stereo_ctx* ctx, int cost, PixType type, int
             const int rc = check_uniq_bound(R, 255.0 * 255.0);
             if (rc != STEREO_OK) return rc;
         }
-    }
-    if (sgm && cost != STEREO_COST_SSD && ctx->sgm_ncc_scale == 0) {
-        set_error("SGM aggregates the SSD cost only while no NCC scale is set (stereo_ctx_set_sgm_ncc_scale; or switch SGM off for NCC calls)");
-        return STEREO_ERR_UNSUPPORTED;
-    }
-    if (sgm && !whole) {
-        set_error("SGM: rows [%d, %d) are not the whole map (vertical and diagonal paths cross band seams)", row_begin, row_end);
-        return STEREO_ERR_UNSUPPORTED;
-    }
-    if (spk && !whole) {
-        set_error("speckle filter: rows [%d, %d) are not the whole map (filter the gathered map with stereo_filter_speckles_device)",
-                  row_begin, row_end);
-        return STEREO_ERR_UNSUPPORTED;
     }
     return STEREO_OK;
 }
@@ -217,7 +241,7 @@ static int speckle_maps(stereo_ctx* ctx, const OutView* maps, int n, int rows, i
 
 // The arena scratch finish_pairs needs for the n maps of a pair call.
 static size_t finish_scratch_bytes(const stereo_ctx* ctx, int n, int rows, int cols) {
-    return ctx->spk_max_size > 0 ? speckle_scratch_bytes(n, rows, cols) : 0;
+    return ctx->opt.spk_max_size > 0 ? speckle_scratch_bytes(n, rows, cols) : 0;
 }
 
 // The texture threshold on the n whole maps of ps, each against its own reference image, which prefilter_pairs made.
@@ -227,7 +251,7 @@ static int texture_maps(stereo_ctx* ctx, const Problem* ps, int n, int sentinel,
     TxParams P{};
     for (int k = 0; k < n; ++k)
         P.map[k] = TxMap{static_cast<const uint8_t*>(ps[k].ref.ptr), ps[k].ref.step, ps[k].disp.ptr, ps[k].disp.step};
-    P.rows = p.rows; P.cols = p.cols; P.R = p.R; P.cap = ctx->pf_cap; P.threshold = ctx->pf_texture; P.sentinel = sentinel;
+    P.rows = p.rows; P.cols = p.cols; P.R = p.R; P.cap = ctx->opt.pf_cap; P.threshold = ctx->opt.pf_texture; P.sentinel = sentinel;
     ctx->last_launches += 1;
     return texture_launch(P, n, p.disp.elem, st);
 }
@@ -244,11 +268,11 @@ static int finish_pairs(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t 
     OutView maps[FMAXJOBS];
     for (int k = 0; k < n; ++k) maps[k] = ps[k].disp;
     int rc = STEREO_OK;
-    if (ctx->pf_cap > 0 && ctx->pf_texture > 0) rc = texture_maps(ctx, ps, n, sentinel, st);
-    if (rc == STEREO_OK && ctx->lr_max_diff >= 0) rc = lr_check_pairs(ctx, maps, n / 2, p.row_end - p.row_begin, p.cols, ctx->lr_max_diff, sentinel, st);
-    if (rc != STEREO_OK || !maps_complete || ctx->spk_max_size <= 0) return rc;
+    if (ctx->opt.pf_cap > 0 && ctx->opt.pf_texture > 0) rc = texture_maps(ctx, ps, n, sentinel, st);
+    if (rc == STEREO_OK && ctx->opt.lr_max_diff >= 0) rc = lr_check_pairs(ctx, maps, n / 2, p.row_end - p.row_begin, p.cols, ctx->opt.lr_max_diff, sentinel, st);
+    if (rc != STEREO_OK || !maps_complete || ctx->opt.spk_max_size <= 0) return rc;
     for (int k = 0; k < n; ++k) maps[k].ptr = static_cast<char*>(maps[k].ptr) - size_t(ps[k].row_begin) * maps[k].step;
-    return speckle_maps(ctx, maps, n, p.rows, p.cols, sentinel, ctx->spk_max_size, ctx->spk_max_diff, st);
+    return speckle_maps(ctx, maps, n, p.rows, p.cols, sentinel, ctx->opt.spk_max_size, ctx->opt.spk_max_diff, st);
 }
 
 // ---- exact path ---------------------------------------------------------------------------------
@@ -454,7 +478,7 @@ static int run_f32_pair(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
     ImageView u8[2];
     int cls = CLS_EXACT;
     rc = classify_images(ctx, p, st, u8, &cls);
-    if (rc == STEREO_OK && n == 2 && ctx->uniq > 0) rc = check_uniq_classified(ctx, p.R);      // (before any map is written)
+    if (rc == STEREO_OK && n == 2 && ctx->opt.uniq > 0) rc = check_uniq_classified(ctx, p.R);      // (before any map is written)
     if (rc != STEREO_OK) return rc;
     if (cls == CLS_EXACT) {
         for (int d = 0; d < n && rc == STEREO_OK; ++d) rc = run_exact_direction(ctx, ps[d], st);
@@ -534,8 +558,8 @@ static size_t sgm_scratch_bytes(const Problem& p) {
 // Every L_r is at most C_max + P2: S stays in int32 when paths (C_max + P2) <= 2^31 - 1.  C_max is (2R + 1)^2 M for SSD,
 // M the largest per-element term, and 2q for NCC.
 static int check_sgm_bound(const stereo_ctx* ctx, double c_max, const char* what) {
-    if (double(ctx->sgm_paths) * (c_max + ctx->sgm_p2) <= 2147483647.0) return STEREO_OK;
-    set_error("SGM: %d paths x (C_max %.0f [%s] + P2 %d) exceeds 2^31 - 1", ctx->sgm_paths, c_max, what, ctx->sgm_p2);
+    if (double(ctx->opt.sgm_paths) * (c_max + ctx->opt.sgm_p2) <= 2147483647.0) return STEREO_OK;
+    set_error("SGM: %d paths x (C_max %.0f [%s] + P2 %d) exceeds 2^31 - 1", ctx->opt.sgm_paths, c_max, what, ctx->opt.sgm_p2);
     return STEREO_ERR_UNSUPPORTED;
 }
 static int check_ssd_sgm_bound(const stereo_ctx* ctx, int R, double M) {
@@ -584,7 +608,7 @@ static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st,
     int32_t* C = static_cast<int32_t*>(ctx->arena.take(cells * 4));
     int32_t* S = static_cast<int32_t*>(ctx->arena.take(cells * 4));
     if (!C || !S) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
-    SgmNcc ncc{nullptr, nullptr, ctx->sgm_ncc_scale};
+    SgmNcc ncc{nullptr, nullptr, ctx->opt.sgm_ncc_scale};
     const bool is_ncc = p.cost == STEREO_COST_NCORR;
     if (is_ncc) {
         double* nref = static_cast<double*>(ctx->arena.take(size_t(p.rows) * p.cols * sizeof(double)));
@@ -603,10 +627,10 @@ static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st,
     } else {
         launch_sgm_cost(ctx, p, g, Lp, Rp, ncc, C, st);
     }
-    for (int k = 0; k < ctx->sgm_paths; ++k) {
-        const bool last = k == ctx->sgm_paths - 1;
-        const SgmOut out{last ? p.disp.ptr : nullptr, p.disp.step, p.disp.elem, g.dlo, ctx->uniq, sentinel, 0};
-        const int rc2 = launch_sgm_path(ctx, p, g, C, S, DIRS[k][0], DIRS[k][1], ctx->sgm_p1, ctx->sgm_p2, k == 0, out, st);
+    for (int k = 0; k < ctx->opt.sgm_paths; ++k) {
+        const bool last = k == ctx->opt.sgm_paths - 1;
+        const SgmOut out{last ? p.disp.ptr : nullptr, p.disp.step, p.disp.elem, g.dlo, ctx->opt.uniq, sentinel, 0};
+        const int rc2 = launch_sgm_path(ctx, p, g, C, S, DIRS[k][0], DIRS[k][1], ctx->opt.sgm_p1, ctx->opt.sgm_p2, k == 0, out, st);
         if (rc2 != STEREO_OK) return rc2;
     }
     SB_CUDA(cudaGetLastError());
@@ -636,7 +660,7 @@ static int run_uniqueness(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_
         int32_t* C = static_cast<int32_t*>(ctx->arena.take(size_t(p.rows) * p.cols * g.Dp * 4));
         if (!C) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
         launch_sgm_cost(ctx, p, g, Lp, Rp, SgmNcc{nullptr, nullptr, 0}, C, st);
-        const SgmOut out{p.disp.ptr, p.disp.step, p.disp.elem, g.dlo, ctx->uniq, sentinel, 1};
+        const SgmOut out{p.disp.ptr, p.disp.step, p.disp.elem, g.dlo, ctx->opt.uniq, sentinel, 1};
         rc = launch_sgm_path(ctx, p, g, C, nullptr, 1, 0, 0, 0, true, out, st);
         if (rc != STEREO_OK) return rc;
     }
@@ -661,7 +685,7 @@ static int run_sgm(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bool u8
         const size_t b = sgm_scratch_bytes(ps[i]);
         if (b > need) need = b;
     }
-    int rc = ncc ? check_sgm_bound(ctx, 2.0 * ctx->sgm_ncc_scale, "2q")
+    int rc = ncc ? check_sgm_bound(ctx, 2.0 * ctx->opt.sgm_ncc_scale, "2q")
            : u8 ? check_ssd_sgm_bound(ctx, ps[0].R, 255.0 * 255.0) : STEREO_OK;
     if (rc == STEREO_OK) rc = reserve_arena(ctx, st, need);
     if (rc != STEREO_OK) return rc;
@@ -716,7 +740,7 @@ static int prefilter_pairs(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st)
         ps[np + k].ref = ps[k].tgt;
         ps[np + k].tgt = ps[k].ref;
     }
-    P.rows = p.rows; P.cols = p.cols; P.cap = ctx->pf_cap;
+    P.rows = p.rows; P.cols = p.cols; P.cap = ctx->opt.pf_cap;
     ctx->last_launches += 1;
     return prefilter_launch(P, n, f32, st);
 }
@@ -737,11 +761,11 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
         u8 = u8 && p.ref.type == PixType::U8;
     }
     const bool pair = n >= 2;      // (every pair of a call has the same shape, band, range and element type)
-    const bool uniq_pass = pair && ctx->uniq > 0 && ctx->sgm_paths == 0;
+    const bool uniq_pass = pair && ctx->opt.uniq > 0 && ctx->opt.sgm_paths == 0;
     if (pair) {
         const Problem& p = ps[0];
         int rc = check_pair_options(ctx, p.cost, p.ref.type, p.disp.elem, ps[n / 2].dmax, p.R, p.cols, p.row_begin, p.row_end, p.rows);
-        if (rc == STEREO_OK && ctx->pf_cap > 0) {
+        if (rc == STEREO_OK && ctx->opt.pf_cap > 0) {
             rc = prefilter_pairs(ctx, ps, n, st);
             u8 = true;
         }
@@ -758,7 +782,7 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
     }
     Problem callers[FMAXJOBS];      // (run_f32_pair points ps at u8 copies in the arena, which the uniqueness pass reuses)
     for (int i = 0; uniq_pass && i < n; ++i) callers[i] = ps[i];
-    int rc = pair && ctx->sgm_paths > 0 ? run_sgm(ctx, ps, n, st, u8) : run_families(ctx, ps, n, st, fast, u8);
+    int rc = pair && ctx->opt.sgm_paths > 0 ? run_sgm(ctx, ps, n, st, u8) : run_families(ctx, ps, n, st, fast, u8);
     if (rc == STEREO_OK && uniq_pass) rc = run_uniqueness(ctx, callers, n, st);
     return rc == STEREO_OK && pair ? finish_pairs(ctx, ps, n, st, true) : rc;
 }
@@ -957,8 +981,7 @@ static bool host_sample_is_8bit(const void* img, size_t step, int rows, int cols
 static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, int n_pairs, const HostPairIn* in,
                                      const HostDir* dirs, int n_dirs, int rows, int cols, int R, size_t disp_step, int elem) {
     if (ctx->force_path == STEREO_PATH_EXACT_F32 || ctx->force_path == STEREO_PATH_FAST_F32) return PIPE_NOT_APPLICABLE;
-    // (SGM maps, the uniqueness pass and the prefilter are computed whole, run_directions)
-    if (n_dirs == 2 && (ctx->sgm_paths > 0 || ctx->uniq > 0 || ctx->pf_cap > 0)) return PIPE_NOT_APPLICABLE;
+    if (n_dirs == 2 && ctx->opt.computed_whole()) return PIPE_NOT_APPLICABLE;      // (run_directions computes them whole)
     const auto t_call = std::chrono::steady_clock::now();       // (trace only)
     double t_pack = 0.0, t_ring = 0.0;
     auto since = [](std::chrono::steady_clock::time_point t0) { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(); };
@@ -1012,7 +1035,7 @@ static int pairs_host_pipelined_body(stereo_ctx* ctx, int cost, PixType type, in
         }
     }
     // pairs with the speckle filter: an item's maps are filtered whole after its last band, then downloaded
-    const bool spk = n_dirs == 2 && ctx->spk_max_size > 0;
+    const bool spk = n_dirs == 2 && ctx->opt.spk_max_size > 0;
     const size_t finish = n_dirs == 2 ? finish_scratch_bytes(ctx, 2 * cp, rows, cols) : 0;
     if (finish > scratch) scratch = finish;
     constexpr int NSTG = 4;                               // pinned staging ring of the host-packed uploads
@@ -1626,11 +1649,11 @@ int stereo_ctx_set_fuse_pairs(stereo_ctx* ctx, int on) {
 
 int stereo_ctx_set_lr_check(stereo_ctx* ctx, int max_diff) {
     if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
-    ctx->lr_max_diff = max_diff < 0 ? -1 : max_diff;
+    ctx->opt.lr_max_diff = max_diff < 0 ? -1 : max_diff;
     return STEREO_OK;
 }
 
-int stereo_ctx_lr_check(const stereo_ctx* ctx) { return ctx ? ctx->lr_max_diff : -1; }
+int stereo_ctx_lr_check(const stereo_ctx* ctx) { return ctx ? ctx->opt.lr_max_diff : -1; }
 
 int stereo_lr_check_device(stereo_ctx* ctx, void* disp_left, void* disp_right, size_t disp_step, int disp_elem_bytes, int rows,
                            int cols, int disparity_range, int max_diff, void* cuda_stream) {
@@ -1656,15 +1679,15 @@ int stereo_lr_check_device(stereo_ctx* ctx, void* disp_left, void* disp_right, s
 int stereo_ctx_set_speckle_filter(stereo_ctx* ctx, int max_size, int max_diff) {
     if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
     if (max_size > 0 && max_diff < 0) { set_error("max_diff must be >= 0"); return STEREO_ERR_INVALID_ARG; }
-    ctx->spk_max_size = max_size > 0 ? max_size : 0;
-    ctx->spk_max_diff = max_size > 0 ? max_diff : 0;
+    ctx->opt.spk_max_size = max_size > 0 ? max_size : 0;
+    ctx->opt.spk_max_diff = max_size > 0 ? max_diff : 0;
     return STEREO_OK;
 }
 
 int stereo_ctx_speckle_filter(const stereo_ctx* ctx, int* max_size, int* max_diff) {
     if (!ctx || !max_size || !max_diff) { set_error("null argument"); return STEREO_ERR_INVALID_ARG; }
-    *max_size = ctx->spk_max_size;
-    *max_diff = ctx->spk_max_diff;
+    *max_size = ctx->opt.spk_max_size;
+    *max_diff = ctx->opt.spk_max_diff;
     return STEREO_OK;
 }
 
@@ -1672,30 +1695,30 @@ int stereo_ctx_set_sgm(stereo_ctx* ctx, int paths, int p1, int p2) {
     if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
     if (paths != 0 && paths != 4 && paths != 8) { set_error("SGM paths must be 0, 4 or 8 (got %d)", paths); return STEREO_ERR_INVALID_ARG; }
     if (p1 < 0 || p1 > p2) { set_error("SGM penalties need 0 <= P1 <= P2 (got %d, %d)", p1, p2); return STEREO_ERR_INVALID_ARG; }
-    ctx->sgm_paths = paths;
-    ctx->sgm_p1 = paths ? p1 : 0;
-    ctx->sgm_p2 = paths ? p2 : 0;
+    ctx->opt.sgm_paths = paths;
+    ctx->opt.sgm_p1 = paths ? p1 : 0;
+    ctx->opt.sgm_p2 = paths ? p2 : 0;
     return STEREO_OK;
 }
 
 int stereo_ctx_sgm(const stereo_ctx* ctx, int* paths, int* p1, int* p2) {
     if (!ctx || !paths || !p1 || !p2) { set_error("null argument"); return STEREO_ERR_INVALID_ARG; }
-    *paths = ctx->sgm_paths;
-    *p1 = ctx->sgm_p1;
-    *p2 = ctx->sgm_p2;
+    *paths = ctx->opt.sgm_paths;
+    *p1 = ctx->opt.sgm_p1;
+    *p2 = ctx->opt.sgm_p2;
     return STEREO_OK;
 }
 
 int stereo_ctx_set_sgm_ncc_scale(stereo_ctx* ctx, int q) {
     if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
     if (q < 0 || q > (1 << 24)) { set_error("SGM NCC scale must be in [0, 2^24] (got %d)", q); return STEREO_ERR_INVALID_ARG; }
-    ctx->sgm_ncc_scale = q;
+    ctx->opt.sgm_ncc_scale = q;
     return STEREO_OK;
 }
 
 int stereo_ctx_sgm_ncc_scale(const stereo_ctx* ctx) {
     if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
-    return ctx->sgm_ncc_scale;
+    return ctx->opt.sgm_ncc_scale;
 }
 
 int stereo_ctx_set_uniqueness(stereo_ctx* ctx, int uniqueness_ratio) {
@@ -1704,13 +1727,13 @@ int stereo_ctx_set_uniqueness(stereo_ctx* ctx, int uniqueness_ratio) {
         set_error("uniqueness ratio must be in [0, 99] (got %d)", uniqueness_ratio);
         return STEREO_ERR_INVALID_ARG;
     }
-    ctx->uniq = uniqueness_ratio;
+    ctx->opt.uniq = uniqueness_ratio;
     return STEREO_OK;
 }
 
 int stereo_ctx_uniqueness(const stereo_ctx* ctx) {
     if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
-    return ctx->uniq;
+    return ctx->opt.uniq;
 }
 
 int stereo_ctx_set_prefilter(stereo_ctx* ctx, int cap, int texture_threshold) {
@@ -1720,15 +1743,15 @@ int stereo_ctx_set_prefilter(stereo_ctx* ctx, int cap, int texture_threshold) {
                   texture_threshold);
         return STEREO_ERR_INVALID_ARG;
     }
-    ctx->pf_cap = cap;
-    ctx->pf_texture = texture_threshold;
+    ctx->opt.pf_cap = cap;
+    ctx->opt.pf_texture = texture_threshold;
     return STEREO_OK;
 }
 
 int stereo_ctx_prefilter(const stereo_ctx* ctx, int* cap, int* texture_threshold) {
     if (!ctx || !cap || !texture_threshold) { set_error("null argument"); return STEREO_ERR_INVALID_ARG; }
-    *cap = ctx->pf_cap;
-    *texture_threshold = ctx->pf_texture;
+    *cap = ctx->opt.pf_cap;
+    *texture_threshold = ctx->opt.pf_texture;
     return STEREO_OK;
 }
 

@@ -1,11 +1,14 @@
 """Calls of every pair entry point on small synthetic pairs, for the tests of the pair options (the left-right check, the
-speckle filter, SGM): the same images and maps through each entry point's own interface.  Needs a B200."""
+speckle filter, SGM, the uniqueness ratio, the prefilter): the same images and maps through each entry point's own
+interface, calls on outputs that must stay untouched, and the contexts the tests share.  Needs a B200."""
 import ctypes as C
 
 import numpy as np
+import pytest
 
 import introtocomputervision_b200 as sb
 from introtocomputervision_b200 import _capi, synth
+from test_entry_points import EXPECTED, ROWS
 
 FAMILIES = {            # images, window radius, output type
     "u8": ("u8", 3, np.int8),
@@ -14,6 +17,26 @@ FAMILIES = {            # images, window radius, output type
     "exact": ("u8", 8, np.int32),
 }
 ROWS_T, COLS_T, RANGE_T = 40, 150, 20
+
+PAIR_ENTRY_POINTS = [n for n in EXPECTED if n.startswith("stereo_disparity_pair_")]
+MGPU_ENTRY_POINTS = {"stereo_mgpu_disparity_pair_batch_u8_host": "stereo_disparity_pair_batch_u8_host",      # (called as)
+                     "stereo_mgpu_disparity_pair_batch_f32_host": "stereo_disparity_pair_batch_f32_host",
+                     "stereo_mgpu_disparity_pair_bands_u8_host": "stereo_disparity_pair_u8_host",
+                     "stereo_mgpu_disparity_pair_bands_f32_host": "stereo_disparity_pair_f32_host"}
+
+
+@pytest.fixture(scope="module")
+def gctx():
+    c = sb.Context(0)
+    yield c
+    c.close()
+
+
+@pytest.fixture(scope="module")
+def mg():
+    m = sb.MultiGpu([0, 0])
+    yield m
+    m.close()
 
 
 def _torch():
@@ -122,3 +145,56 @@ def _device_batch(ctx, Ls, Rs, win, rng, elem):
                                                           rows * cols * elem, elem, C.c_void_p(torch.cuda.current_stream().cuda_stream)))
     torch.cuda.synchronize()
     return out.cpu().numpy()
+
+
+def _fill(dev, shape, value):
+    a = np.full(shape, value, np.uint8)
+    return _torch().from_numpy(a).cuda() if dev else a
+
+
+def _untouched(h, entry, Ls, Rs, R, rng, cost=sb.COST_SSD, dt=np.int16):
+    """Calls the entry point (pair_device, batch_device, pair_host, batch_host or mgpu_batch) on outputs filled with 0x3C;
+    returns (status, outputs untouched)."""
+    lib = _capi.lib()
+    n, rows, cols = Ls.shape
+    elem = np.dtype(dt).itemsize
+    f32 = Ls.dtype == np.float32
+    step = cols * Ls.itemsize
+    if entry in ("pair_device", "batch_device"):
+        torch = _torch()
+        tl, tr = torch.from_numpy(Ls).cuda(), torch.from_numpy(Rs).cuda()
+        out = torch.full((2, n, rows, cols * elem), 0x3C, dtype=torch.uint8, device="cuda")
+        st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+        if entry == "pair_device":
+            fn = lib.stereo_disparity_pair_f32_device if f32 else lib.stereo_disparity_pair_u8_device
+            rc = fn(h.handle, cost, tl.data_ptr(), step, tr.data_ptr(), step, rows, cols, R, rng, out[0].data_ptr(), out[1].data_ptr(),
+                    cols * elem, elem, st)
+        else:
+            rc = lib.stereo_disparity_pair_batch_u8_device(h.handle, cost, n, tl.data_ptr(), tr.data_ptr(), cols, rows * cols, rows, cols,
+                                                           R, rng, out[0].data_ptr(), out[1].data_ptr(), cols * elem, rows * cols * elem,
+                                                           elem, st)
+        torch.cuda.synchronize()
+        return rc, bool((out == 0x3C).all().item())
+    out = np.full((2, n, rows, cols * elem), 0x3C, np.uint8)
+    handle = h._h if isinstance(h, sb.MultiGpu) else h.handle
+    if entry == "pair_host":
+        fn = lib.stereo_disparity_pair_f32_host if f32 else lib.stereo_disparity_pair_u8_host
+        rc = fn(handle, cost, Ls.ctypes.data, step, Rs.ctypes.data, step, rows, cols, R, rng, out[0].ctypes.data, out[1].ctypes.data,
+                cols * elem, elem)
+    else:
+        prefix = "stereo_mgpu_" if entry == "mgpu_batch" else "stereo_"
+        fn = getattr(lib, prefix + ("disparity_pair_batch_f32_host" if f32 else "disparity_pair_batch_u8_host"))
+        rc = fn(handle, cost, n, Ls.ctypes.data, Rs.ctypes.data, step, rows * step, rows, cols, R, rng, out[0].ctypes.data,
+                out[1].ctypes.data, cols * elem, rows * cols * elem, elem)
+    return rc, bool((out == 0x3C).all())
+
+
+def _whole_band_args(name, args):
+    """test_entry_points._args of a band entry point, with the band [4, 12) widened to the whole image [0, ROWS)."""
+    a = list(args)
+    i = a.index(4)
+    assert a[i + 1] == 12
+    a[i], a[i + 1] = 0, ROWS
+    if name == "stereo_disparity_pair_band_halo_u8_device":
+        a[i + 2], a[i + 3] = 0, ROWS
+    return a

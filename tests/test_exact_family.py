@@ -18,20 +18,12 @@ from lr_oracle import lr_check
 from speckle_oracle import filter_speckles
 import introtocomputervision_b200 as sb
 from introtocomputervision_b200 import _capi, synth
+from pair_calls import _ok, _torch
 
 pytestmark = pytest.mark.gpu
 
 NCC_SCORE_RTOL = 1e-5
 UNSUP, RANGE = _capi.ERR_UNSUPPORTED, _capi.ERR_INVALID_RANGE
-
-
-def _torch():
-    import torch
-    return torch
-
-
-def _ok(rc, where=""):
-    assert rc == _capi.STEREO_OK, f"{where}: {rc} ({_capi.last_error()})"
 
 
 def _tdt(dt):

@@ -12,35 +12,11 @@ import oracle
 from lr_oracle import lr_check
 import introtocomputervision_b200 as sb
 from introtocomputervision_b200 import _capi, synth
-from pair_calls import COLS_T, FAMILIES, RANGE_T, _images, _run, _set_fuse
-from test_entry_points import EXPECTED, PITCH, ROWS, _args
+from pair_calls import COLS_T, FAMILIES, RANGE_T, _images, _ok, _run, _set_fuse, _torch, gctx, mg
 
 pytestmark = pytest.mark.gpu
 
 ARG, RANGE, UNSUP = _capi.ERR_INVALID_ARG, _capi.ERR_INVALID_RANGE, _capi.ERR_UNSUPPORTED
-
-
-def _torch():
-    import torch
-    return torch
-
-
-def _ok(rc, where=""):
-    assert rc == _capi.STEREO_OK, f"{where}: {rc} ({_capi.last_error()})"
-
-
-@pytest.fixture(scope="module")
-def lctx():
-    c = sb.Context(0)
-    yield c
-    c.close()
-
-
-@pytest.fixture(scope="module")
-def mg():
-    m = sb.MultiGpu([0, 0])
-    yield m
-    m.close()
 
 
 # ---- 1. the kernel alone ---------------------------------------------------------------------------------------------
@@ -71,7 +47,7 @@ KERNEL_CASES = [(e, c) for e in (1, 2, 4) for c in (1, 7, 640, 3840)] + [(1, 204
 
 
 @pytest.mark.parametrize("elem,cols", KERNEL_CASES)
-def test_kernel_alone_equals_the_oracle(lctx, elem, cols):
+def test_kernel_alone_equals_the_oracle(gctx, elem, cols):
     torch = _torch()
     dt = {1: np.int8, 2: np.int16, 4: np.int32}[elem]
     rng = {1: 127, 2: 32767 if cols == 32768 else 700, 4: 32768 if cols == 32768 else 5000}[elem]
@@ -83,10 +59,10 @@ def test_kernel_alone_equals_the_oracle(lctx, elem, cols):
         hl, hr = _padded(dl, pad), _padded(dr, pad)
         tl, tr = torch.from_numpy(hl).cuda(), torch.from_numpy(hr).cuda()
         side.wait_stream(torch.cuda.current_stream())
-        rc = _capi.lib().stereo_lr_check_device(lctx.handle, tl.data_ptr(), tr.data_ptr(), hl.shape[1], elem, rows, cols, rng,
+        rc = _capi.lib().stereo_lr_check_device(gctx.handle, tl.data_ptr(), tr.data_ptr(), hl.shape[1], elem, rows, cols, rng,
                                                 max_diff, C.c_void_p(side.cuda_stream))
         _ok(rc, "stereo_lr_check_device")
-        assert lctx.last_launches == 1
+        assert gctx.last_launches == 1
         torch.cuda.synchronize()
         ol, orr = tl.cpu().numpy(), tr.cpu().numpy()
         wl, wr = lr_check(dl, dr, rng, max_diff)
@@ -99,14 +75,14 @@ def test_kernel_alone_equals_the_oracle(lctx, elem, cols):
             assert 0.05 < kept < 0.95, kept
 
 
-def test_kernel_alone_argument_checks(lctx):
+def test_kernel_alone_argument_checks(gctx):
     torch = _torch()
     buf = torch.zeros((2, 4, 256), dtype=torch.uint8, device="cuda")
     a, b = buf[0].data_ptr(), buf[1].data_ptr()
     lib = _capi.lib()
 
     def call(l=a, r=b, step=256, elem=2, rows=4, cols=64, rng=10, max_diff=1):
-        return lib.stereo_lr_check_device(lctx.handle, l, r, step, elem, rows, cols, rng, max_diff, None)
+        return lib.stereo_lr_check_device(gctx.handle, l, r, step, elem, rows, cols, rng, max_diff, None)
 
     assert call() == _capi.STEREO_OK
     assert call(l=None) == ARG and call(r=None) == ARG
@@ -117,7 +93,7 @@ def test_kernel_alone_argument_checks(lctx):
     assert call(elem=1, rng=128) == UNSUP and call(elem=2, rng=32768) == UNSUP
     assert call(elem=1, rng=127) == _capi.STEREO_OK and call(elem=4, rng=32768) == _capi.STEREO_OK
     assert lib.stereo_lr_check_device(None, a, b, 256, 2, 4, 64, 10, 1, None) == ARG
-    lctx.synchronize()
+    gctx.synchronize()
 
 
 # ---- 2. every pair entry point ---------------------------------------------------------------------------------------
@@ -145,13 +121,13 @@ def _on_equals_oracle_of_off(h, entry, cost, Ls, Rs, win, rng, dt, max_diff):
 @pytest.mark.parametrize("fuse", [True, False])
 @pytest.mark.parametrize("cost", [sb.COST_SSD, sb.COST_NCORR])
 @pytest.mark.parametrize("entry", ENTRIES)
-def test_every_pair_entry_point_equals_the_oracle_check(lctx, mg, entry, cost, fuse, family):
+def test_every_pair_entry_point_equals_the_oracle_check(gctx, mg, entry, cost, fuse, family):
     kind, win, dt = FAMILIES[family]
     if kind != "u8" and entry in ("batch_device", "band_halo_device"):
         pytest.skip("8-bit device entry point")
     if kind == "noisy" and entry == "band_host":
         pytest.skip("the host row-band entry points take 8-bit-valued images only")
-    h = mg if entry.startswith("mgpu_") else lctx
+    h = mg if entry.startswith("mgpu_") else gctx
     n = 5 if "batch" in entry else 1
     Ls, Rs = _images(kind, n, 300 + 7 * ENTRIES.index(entry))
     _set_fuse(h, fuse)
@@ -163,95 +139,42 @@ def test_every_pair_entry_point_equals_the_oracle_check(lctx, mg, entry, cost, f
 
 @pytest.mark.parametrize("bands", [0, 3])
 @pytest.mark.parametrize("kind", ["u8", "f32"])
-def test_host_pipeline_items_and_bands(lctx, bands, kind):
+def test_host_pipeline_items_and_bands(gctx, bands, kind):
     Ls, Rs = _images(kind, 7, 900)
-    lctx.set_pipe_bands(bands)
+    gctx.set_pipe_bands(bands)
     try:
         for cost in (sb.COST_SSD, sb.COST_NCORR):
-            _on_equals_oracle_of_off(lctx, "batch_host", cost, Ls, Rs, 3, RANGE_T, np.int16, 0)
+            _on_equals_oracle_of_off(gctx, "batch_host", cost, Ls, Rs, 3, RANGE_T, np.int16, 0)
     finally:
-        lctx.set_pipe_bands(0)
+        gctx.set_pipe_bands(0)
 
 
 # ---- 3. against the reference at the ps2 shape ---------------------------------------------------------------------
 
-def test_ps2_shape_ssd_pair_equals_the_reference_checked(lctx):
+def test_ps2_shape_ssd_pair_equals_the_reference_checked(gctx):
     L, Rt, _ = synth.make_pair(511, 640, 96, 4242)
     Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
     want_l, want_r = lr_check(oracle.ssd_fast(Lf, Rf, 7, -96, 0), oracle.ssd_fast(Rf, Lf, 7, 0, 96), 96, 1)
-    lctx.set_lr_check(1)
+    gctx.set_lr_check(1)
     try:
-        dl, dr = sb.disparitySSDPair(Lf, Rf, sb.DisparityConfig(7, 96), ctx=lctx)
+        dl, dr = sb.disparitySSDPair(Lf, Rf, sb.DisparityConfig(7, 96), ctx=gctx)
     finally:
-        lctx.set_lr_check(None)
+        gctx.set_lr_check(None)
     assert np.array_equal(dl, oracle.narrow_i8(want_l)) and np.array_equal(dr, oracle.narrow_i8(want_r))
     assert 0.01 < float(np.mean(want_l == -97)) < 0.5
 
 
-# ---- 4. default and off ---------------------------------------------------------------------------------------------
+# ---- 4. twice the range ---------------------------------------------------------------------------------------------
 
-def test_off_again_is_byte_identical_to_a_fresh_context(lctx):
-    Ls, Rs = _images("u8", 3, 77)
-    fresh = sb.Context(0)
-    try:
-        assert fresh.lr_check is None
-        for entry in ("pair_host", "pair_device", "batch_device"):
-            for cost in (sb.COST_SSD, sb.COST_NCORR):
-                want = _run(fresh, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                lctx.set_lr_check(2)
-                assert lctx.lr_check == 2
-                _run(lctx, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                lctx.set_lr_check(-5)
-                assert lctx.lr_check is None
-                got = _run(lctx, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1]), (entry, cost)
-    finally:
-        fresh.close()
-        lctx.set_lr_check(None)
-
-
-def test_single_direction_and_refgpu_calls_ignore_the_check(lctx):
-    torch = _torch()
-    L, Rt, _ = synth.make_pair(48, 160, 24, 515)
-    Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
-    lib = _capi.lib()
-
-    def singles(c):
-        out = [c.disparity(sb.COST_SSD, Lf, Rf, 3, -20, 0, dtype=np.int16), c.disparity(sb.COST_NCORR, L, Rt, 3, 0, 20),
-               c.disparity_refgpu(sb.COST_SSD, Lf, Rf, 3, -20, 0)]
-        st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-        tl, tr = torch.from_numpy(L).cuda(), torch.from_numpy(Rt).cuda()
-        o = torch.zeros((3, 48, 160), dtype=torch.int16, device="cuda")
-        _ok(lib.stereo_disparity_u8_device(c.handle, 0, tl.data_ptr(), 160, tr.data_ptr(), 160, 48, 160, 3, -20, 0, o[0].data_ptr(),
-                                           320, 2, None, 0, st))
-        _ok(lib.stereo_disparity_band_u8_device(c.handle, 0, tl.data_ptr(), 160, tr.data_ptr(), 160, 48, 160, 10, 30, 3, 0, 20,
-                                                o[1][10].data_ptr(), 320, 2, st))
-        _ok(lib.stereo_disparity_band_halo_u8_device(c.handle, 0, tl[6].data_ptr(), 160, tr[6].data_ptr(), 160, 48, 160, 10, 30, 6,
-                                                     34, 3, -20, 0, o[2][10].data_ptr(), 320, 2, st))
-        torch.cuda.synchronize()
-        return out + [o.cpu().numpy()]
-
-    fresh = sb.Context(0)
-    try:
-        want = singles(fresh)
-        lctx.set_lr_check(0)
-        got = singles(lctx)
-    finally:
-        fresh.close()
-        lctx.set_lr_check(None)
-    for a, b in zip(got, want):
-        assert np.array_equal(a, b)
-
-
-def test_twice_the_range_only_drops_partners_outside_the_image(lctx):
+def test_twice_the_range_only_drops_partners_outside_the_image(gctx):
     Ls, Rs = _images("u8", 1, 31)
     rng, cols = RANGE_T, COLS_T
-    off_l, off_r = _on_equals_oracle_of_off(lctx, "pair_host", sb.COST_SSD, Ls, Rs, 3, rng, np.int16, 2 * rng)
-    lctx.set_lr_check(2 * rng)
+    off_l, off_r = _on_equals_oracle_of_off(gctx, "pair_host", sb.COST_SSD, Ls, Rs, 3, rng, np.int16, 2 * rng)
+    gctx.set_lr_check(2 * rng)
     try:
-        on_l, on_r = _run(lctx, "pair_host", sb.COST_SSD, Ls, Rs, 3, rng, np.int16)
+        on_l, on_r = _run(gctx, "pair_host", sb.COST_SSD, Ls, Rs, 3, rng, np.int16)
     finally:
-        lctx.set_lr_check(None)
+        gctx.set_lr_check(None)
     x = np.arange(cols)
     n_outside = 0
     for off, on in ((off_l[0], on_l[0]), (off_r[0], on_r[0])):
@@ -262,50 +185,9 @@ def test_twice_the_range_only_drops_partners_outside_the_image(lctx):
     assert n_outside > 0
 
 
-# ---- 5. the sentinel rule -------------------------------------------------------------------------------------------
+# ---- 5. graph capture -------------------------------------------------------------------------------------------------
 
-PAIR_ENTRY_POINTS = [n for n in EXPECTED if n.startswith("stereo_disparity_pair_")]
-MGPU_ENTRY_POINTS = {"stereo_mgpu_disparity_pair_batch_u8_host": "stereo_disparity_pair_batch_u8_host",
-                     "stereo_mgpu_disparity_pair_batch_f32_host": "stereo_disparity_pair_batch_f32_host",
-                     "stereo_mgpu_disparity_pair_bands_u8_host": "stereo_disparity_pair_u8_host",
-                     "stereo_mgpu_disparity_pair_bands_f32_host": "stereo_disparity_pair_f32_host"}
-
-
-@pytest.mark.parametrize("elem,rng", [(1, 128), (2, 32768)])
-@pytest.mark.parametrize("name", PAIR_ENTRY_POINTS + list(MGPU_ENTRY_POINTS))
-def test_sentinel_that_does_not_fit_is_rejected_before_anything_runs(lctx, mg, name, elem, rng):
-    torch = _torch()
-    h = mg if name.startswith("stereo_mgpu_") else lctx
-    as_name = MGPU_ENTRY_POINTS.get(name, name)
-    dev = as_name.endswith("_device")
-    imgs = [np.zeros((2, ROWS, PITCH), np.uint8) for _ in range(2)]
-    outs = [np.full((2, ROWS, PITCH), 0x3C, np.uint8) for _ in range(2)]
-    if dev:
-        imgs = [torch.from_numpy(a).cuda() for a in imgs]
-        outs = [torch.from_numpy(a).cuda() for a in outs]
-        ptrs = [t.data_ptr() for t in imgs + outs]
-    else:
-        ptrs = [a.ctypes.data for a in imgs + outs]
-    handle = h._h if isinstance(h, sb.MultiGpu) else h.handle
-    fn = getattr(_capi.lib(), name)
-    args = _args(as_name, handle, ptrs, rng=rng, elem=elem)
-    h.set_lr_check(1)
-    try:
-        rc = fn(*args)
-        torch.cuda.synchronize()
-        assert rc == UNSUP, f"{name}: {rc} ({_capi.last_error()})"
-        for o in outs:
-            a = o.cpu().numpy() if dev else o
-            assert (a == 0x3C).all(), f"{name} wrote its outputs"
-    finally:
-        h.set_lr_check(None)
-    _ok(fn(*args), name)
-    torch.cuda.synchronize()
-
-
-# ---- 6. graph capture -------------------------------------------------------------------------------------------------
-
-def test_band_halo_pair_call_with_the_check_replays_in_a_cuda_graph(lctx):
+def test_band_halo_pair_call_with_the_check_replays_in_a_cuda_graph(gctx):
     torch = _torch()
     rows, cols, win, rng, r0, r1 = 64, 200, 4, 30, 16, 48
     L, Rt, _ = synth.make_pair(rows, cols, rng + 4, 2024)
@@ -318,13 +200,13 @@ def test_band_halo_pair_call_with_the_check_replays_in_a_cuda_graph(lctx):
 
     def call(o):
         _ok(_capi.lib().stereo_disparity_pair_band_halo_u8_device(
-            lctx.handle, sb.COST_SSD, tl[h0.value].data_ptr(), cols, tr[h0.value].data_ptr(), cols, rows, cols, r0, r1, h0.value,
+            gctx.handle, sb.COST_SSD, tl[h0.value].data_ptr(), cols, tr[h0.value].data_ptr(), cols, rows, cols, r0, r1, h0.value,
             h1.value, win, rng, o[0].data_ptr(), o[1].data_ptr(), cols * 2, 2, C.c_void_p(s.cuda_stream)))
 
     try:
         with torch.cuda.stream(s):
             call(outs["off"])
-            lctx.set_lr_check(1)
+            gctx.set_lr_check(1)
             call(outs["eager"])
         s.synchronize()
         g = torch.cuda.CUDAGraph()
@@ -334,7 +216,7 @@ def test_band_halo_pair_call_with_the_check_replays_in_a_cuda_graph(lctx):
         g.replay()
         torch.cuda.synchronize()
     finally:
-        lctx.set_lr_check(None)
+        gctx.set_lr_check(None)
     off, eager, graph = (outs[k].cpu().numpy() for k in ("off", "eager", "graph"))
     assert np.array_equal(graph, eager)
     wl, wr = lr_check(off[0], off[1], rng, 1)

@@ -13,7 +13,7 @@ import oracle
 from introtocomputervision_b200 import _capi, synth
 from lr_oracle import lr_check
 from ncc_check import check_ncc_map
-from pair_calls import FAMILIES, RANGE_T, _device_batch, _images, _run, _set_fuse
+from pair_calls import FAMILIES, RANGE_T, _device_batch, _images, _ok, _run, _set_fuse, _torch, gctx, mg
 from prefilter_oracle import pf, texture_keep, texture_sum
 from sgm_ncc_oracle import sgm_pair as sgm_ncc_pair
 from sgm_oracle import cost_volume, sgm_pair
@@ -25,29 +25,6 @@ pytestmark = pytest.mark.gpu
 ARG, UNSUP = _capi.ERR_INVALID_ARG, _capi.ERR_UNSUPPORTED
 ENTRIES = ["pair_host", "pair_device", "batch_device", "batch_host", "band_host", "band_halo_device", "mgpu_batch"]
 NCC_AGREE = 0.99        # clipped responses form plateaus: more near-ties than raw images (each one is checked against tau)
-
-
-def _torch():
-    import torch
-    return torch
-
-
-def _ok(rc, where=""):
-    assert rc == _capi.STEREO_OK, f"{where}: {rc} ({_capi.last_error()})"
-
-
-@pytest.fixture(scope="module")
-def gctx():
-    c = sb.Context(0)
-    yield c
-    c.close()
-
-
-@pytest.fixture(scope="module")
-def mg():
-    m = sb.MultiGpu([0, 0])
-    yield m
-    m.close()
 
 
 def _threshold(img, cap, R, q=0.2):
@@ -273,60 +250,7 @@ def test_prefiltered_bands_equal_the_whole_pair_call(gctx, rows):
         assert np.array_equal(ol.cpu().numpy(), want[0]) and np.array_equal(orr.cpu().numpy(), want[1]), (rows, cost)
 
 
-# ---- 6. refusals and the setting ----------------------------------------------------------------------------------------
-
-def test_partial_bands_and_mgpu_bands_are_refused(gctx, mg):
-    torch = _torch()
-    lib = _capi.lib()
-    rows, cols, win, rng = 48, 96, 3, 16
-    L, Rt, _ = synth.make_pair(rows, cols, rng + 4, 88)
-    Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
-    gctx.set_prefilter(31, 0)
-    mg.set_prefilter(31, 0)
-    try:
-        for r0, r1 in ((0, 24), (24, 48), (10, 20)):
-            for fn, a, b in ((lib.stereo_disparity_pair_band_u8_host, L, Rt), (lib.stereo_disparity_pair_band_f32_host, Lf, Rf)):
-                ol, orr = np.full((rows, cols * 2), 0x3C, np.uint8), np.full((rows, cols * 2), 0x3C, np.uint8)
-                rc = fn(gctx.handle, sb.COST_SSD, a.ctypes.data, a.strides[0], b.ctypes.data, b.strides[0], rows, cols, r0, r1, win, rng,
-                        ol[r0:].ctypes.data, orr[r0:].ctypes.data, cols * 2, 2)
-                assert rc == UNSUP and (ol == 0x3C).all() and (orr == 0x3C).all(), (fn.__name__, r0, r1, rc)
-            h0, h1 = C.c_int(), C.c_int()
-            _ok(lib.stereo_band_halo_rows(rows, r0, r1, win, C.byref(h0), C.byref(h1)))
-            tl, tr = torch.from_numpy(L).cuda(), torch.from_numpy(Rt).cuda()
-            ol = torch.full((rows, cols * 2), 0x3C, dtype=torch.uint8, device="cuda")
-            orr = torch.full_like(ol, 0x3C)
-            rc = lib.stereo_disparity_pair_band_halo_u8_device(gctx.handle, sb.COST_SSD, tl[h0.value].data_ptr(), cols, tr[h0.value].data_ptr(),
-                                                               cols, rows, cols, r0, r1, h0.value, h1.value, win, rng, ol[r0].data_ptr(),
-                                                               orr[r0].data_ptr(), cols * 2, 2, None)
-            torch.cuda.synchronize()
-            assert rc == UNSUP and (ol == 0x3C).all().item() and (orr == 0x3C).all().item(), ("band_halo", r0, r1, rc)
-        for fn, a, b in ((lib.stereo_mgpu_disparity_pair_bands_u8_host, L, Rt), (lib.stereo_mgpu_disparity_pair_bands_f32_host, Lf, Rf)):
-            ol, orr = np.full((rows, cols * 2), 0x3C, np.uint8), np.full((rows, cols * 2), 0x3C, np.uint8)
-            rc = fn(mg._h, sb.COST_SSD, a.ctypes.data, a.strides[0], b.ctypes.data, b.strides[0], rows, cols, win, rng,
-                    ol.ctypes.data, orr.ctypes.data, cols * 2, 2)
-            assert rc == UNSUP and (ol == 0x3C).all() and (orr == 0x3C).all(), (fn.__name__, rc)
-    finally:
-        gctx.set_prefilter(None)
-        mg.set_prefilter(None)
-    dl, dr = mg.disparity_pair_bands(sb.COST_SSD, L, Rt, win, rng, dtype=np.int16)      # off again: served
-    assert dl.shape == (rows, cols)
-
-
-@pytest.mark.parametrize("entry", ["pair_device", "batch_device", "pair_host", "batch_host", "mgpu_batch"])
-def test_a_texture_sentinel_that_does_not_fit_is_refused(gctx, mg, entry):
-    from test_uniqueness import _untouched
-    h = mg if entry.startswith("mgpu_") else gctx
-    Ls, Rs = _images("u8", 2, 31)
-    try:
-        h.set_prefilter(31, 10)
-        rc, untouched = _untouched(h, entry, Ls, Rs, 3, 128, dt=np.int8)            # -(128 + 1) does not fit int8
-        assert rc == UNSUP and untouched, (entry, rc)
-        h.set_prefilter(31, 0)                                                       # the prefilter alone writes no sentinel
-        rc, _ = _untouched(h, entry, Ls, Rs, 3, 128, dt=np.int8)
-        _ok(rc, entry)
-    finally:
-        h.set_prefilter(None)
-
+# ---- 6. refusals of the standalone calls --------------------------------------------------------------------------------
 
 def test_standalone_refusals(gctx):
     torch = _torch()
@@ -355,69 +279,6 @@ def test_standalone_refusals(gctx):
         assert fn(*args) == ARG, (fn.__name__, args)
     torch.cuda.synchronize()
     assert (dst == 0x3C).all().item() and (src == 0).all().item() and (srcf == 0).all().item()
-
-
-def test_setter_getter_and_mgpu_setter(mg):
-    lib = _capi.lib()
-    fresh = sb.Context(0)
-    try:
-        assert fresh.prefilter is None
-        a, b = C.c_int(), C.c_int()
-        assert lib.stereo_ctx_set_prefilter(None, 31, 0) == ARG
-        assert lib.stereo_ctx_prefilter(None, C.byref(a), C.byref(b)) == ARG
-        assert lib.stereo_ctx_prefilter(fresh.handle, None, C.byref(b)) == ARG
-        assert lib.stereo_mgpu_set_prefilter(None, 31, 0) == ARG
-        fresh.set_prefilter(31, 10)
-        for cap, t in ((64, 0), (-1, 0), (0, 5), (31, -1), (100, 10), (0, -1)):
-            assert lib.stereo_ctx_set_prefilter(fresh.handle, cap, t) == ARG, (cap, t)
-            assert fresh.prefilter == (31, 10), (cap, t)          # the old setting stays
-        for cap, t in ((1, 0), (63, 1 << 30), (5, 0), (20, 7)):
-            fresh.set_prefilter(cap, t)
-            assert fresh.prefilter == (cap, t)
-        fresh.set_prefilter(0)
-        assert fresh.prefilter is None
-        fresh.set_prefilter(9)
-        fresh.set_prefilter(None)
-        assert fresh.prefilter is None
-        with pytest.raises(sb.StereoError):
-            mg.set_prefilter(64)
-        mg.set_prefilter(7, 3)
-        for i in range(mg.device_count):
-            _ok(lib.stereo_ctx_prefilter(lib.stereo_mgpu_ctx(mg._h, i), C.byref(a), C.byref(b)))
-            assert (a.value, b.value) == (7, 3)
-    finally:
-        fresh.close()
-        mg.set_prefilter(None)
-
-
-def test_off_again_is_byte_identical_and_singles_ignore_it(gctx):
-    Ls, Rs = _images("u8", 2, 2700)
-    fresh = sb.Context(0)
-    try:
-        for entry in ("pair_host", "pair_device", "batch_device", "batch_host"):
-            for cost in (sb.COST_SSD, sb.COST_NCORR):
-                want = _run(fresh, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                gctx.set_prefilter(31, 40)
-                on = _run(gctx, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                assert (on[0] != want[0]).any()
-                gctx.set_prefilter(None)
-                got = _run(gctx, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1]), (entry, cost)
-        L, Rt = Ls[0], Rs[0]
-        Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
-
-        def singles(c):
-            return [c.disparity(sb.COST_SSD, Lf, Rf, 3, -20, 0, dtype=np.int16), c.disparity(sb.COST_SSD, L, Rt, 3, -20, 0),
-                    c.disparity(sb.COST_NCORR, L, Rt, 3, 0, 20), c.disparity_refgpu(sb.COST_SSD, Lf, Rf, 3, -20, 0)]
-
-        want = singles(fresh)
-        gctx.set_prefilter(31, 40)
-        got = singles(gctx)
-        for a, b in zip(got, want):
-            assert np.array_equal(a, b)
-    finally:
-        fresh.close()
-        gctx.set_prefilter(None)
 
 
 # ---- 7. graph capture ----------------------------------------------------------------------------------------------------

@@ -14,7 +14,7 @@ import oracle
 from introtocomputervision_b200 import _capi, synth
 from lr_oracle import lr_check
 from ncc_check import score_at
-from pair_calls import FAMILIES, RANGE_T, _images, _run
+from pair_calls import FAMILIES, RANGE_T, _images, _ok, _run, _torch, _untouched, gctx, mg
 from sgm_ncc_oracle import quantise, sgm_pair
 from speckle_oracle import filter_speckles
 
@@ -23,29 +23,6 @@ pytestmark = pytest.mark.gpu
 ARG, UNSUP = _capi.ERR_INVALID_ARG, _capi.ERR_UNSUPPORTED
 ENTRIES = ["pair_host", "pair_device", "batch_device", "batch_host", "band_host", "band_halo_device", "mgpu_batch"]
 NCC = sb.COST_NCORR
-
-
-def _torch():
-    import torch
-    return torch
-
-
-def _ok(rc, where=""):
-    assert rc == _capi.STEREO_OK, f"{where}: {rc} ({_capi.last_error()})"
-
-
-@pytest.fixture(scope="module")
-def gctx():
-    c = sb.Context(0)
-    yield c
-    c.close()
-
-
-@pytest.fixture(scope="module")
-def mg():
-    m = sb.MultiGpu([0, 0])
-    yield m
-    m.close()
 
 
 def _kind_images(kind, n, seed):
@@ -228,42 +205,6 @@ def test_reference_contrast_problem_at_full_size(gctx):
 
 # ---- 3. rejections -----------------------------------------------------------------------------------------------------
 
-def _untouched_call(h, entry, Ls, Rs, R, rng, cost=NCC, dt=np.int16):
-    """Calls the entry point on outputs filled with 0x3C; returns (status, outputs untouched)."""
-    torch = _torch()
-    lib = _capi.lib()
-    n, rows, cols = Ls.shape
-    elem = np.dtype(dt).itemsize
-    f32 = Ls.dtype == np.float32
-    step = cols * Ls.itemsize
-    if entry in ("pair_device", "batch_device"):
-        tl, tr = torch.from_numpy(Ls).cuda(), torch.from_numpy(Rs).cuda()
-        out = torch.full((2, n, rows, cols * elem), 0x3C, dtype=torch.uint8, device="cuda")
-        st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-        if entry == "pair_device":
-            fn = lib.stereo_disparity_pair_f32_device if f32 else lib.stereo_disparity_pair_u8_device
-            rc = fn(h.handle, cost, tl.data_ptr(), step, tr.data_ptr(), step, rows, cols, R, rng, out[0].data_ptr(), out[1].data_ptr(),
-                    cols * elem, elem, st)
-        else:
-            rc = lib.stereo_disparity_pair_batch_u8_device(h.handle, cost, n, tl.data_ptr(), tr.data_ptr(), cols, rows * cols, rows, cols,
-                                                           R, rng, out[0].data_ptr(), out[1].data_ptr(), cols * elem, rows * cols * elem,
-                                                           elem, st)
-        torch.cuda.synchronize()
-        return rc, bool((out == 0x3C).all().item())
-    out = np.full((2, n, rows, cols * elem), 0x3C, np.uint8)
-    handle = h._h if isinstance(h, sb.MultiGpu) else h.handle
-    if entry == "pair_host":
-        fn = lib.stereo_disparity_pair_f32_host if f32 else lib.stereo_disparity_pair_u8_host
-        rc = fn(handle, cost, Ls.ctypes.data, step, Rs.ctypes.data, step, rows, cols, R, rng, out[0].ctypes.data, out[1].ctypes.data,
-                cols * elem, elem)
-    else:
-        prefix = "stereo_mgpu_" if entry == "mgpu_batch" else "stereo_"
-        fn = getattr(lib, prefix + ("disparity_pair_batch_f32_host" if f32 else "disparity_pair_batch_u8_host"))
-        rc = fn(handle, cost, n, Ls.ctypes.data, Rs.ctypes.data, step, rows * step, rows, cols, R, rng, out[0].ctypes.data,
-                out[1].ctypes.data, cols * elem, rows * cols * elem, elem)
-    return rc, bool((out == 0x3C).all())
-
-
 HOST_ENTRIES = ["pair_host", "batch_host", "mgpu_batch"]
 
 
@@ -273,11 +214,11 @@ def test_scale_zero_still_refuses_ncc(gctx, mg, entry):
     Ls, Rs = _images("u8", 2, 5)
     _set(h, 0, 4, 1, 10)
     try:
-        rc, untouched = _untouched_call(h, entry, Ls, Rs, 3, RANGE_T)
+        rc, untouched = _untouched(h, entry, Ls, Rs, 3, RANGE_T, cost=NCC)
         assert rc == UNSUP and untouched, (entry, rc)
         assert "SSD" in _capi.last_error()
         h.set_sgm_ncc_scale(100)                                    # the same call with a scale is served
-        rc, untouched = _untouched_call(h, entry, Ls, Rs, 3, RANGE_T)
+        rc, untouched = _untouched(h, entry, Ls, Rs, 3, RANGE_T, cost=NCC)
         _ok(rc, entry)
         assert not untouched
     finally:
@@ -294,10 +235,10 @@ def test_the_int32_bound_is_exact(gctx, paths, q):
         for R in (0, 7):
             _set(gctx, q, paths, 0, p2)
             try:
-                rc, _ = _untouched_call(gctx, entry, a, b, R, 10)
+                rc, _ = _untouched(gctx, entry, a, b, R, 10, cost=NCC)
                 _ok(rc, f"{entry} at the bound")
                 gctx.set_sgm(paths, 0, p2 + 1)
-                rc, untouched = _untouched_call(gctx, entry, a, b, R, 10)
+                rc, untouched = _untouched(gctx, entry, a, b, R, 10, cost=NCC)
                 assert rc == UNSUP and untouched, (entry, R, rc)
             finally:
                 _reset(gctx)
@@ -312,9 +253,9 @@ def test_non_finite_images_are_rejected(gctx, mg, entry):
         for bad in (np.nan, np.inf, -np.inf):
             L2 = Ls.copy()
             L2[:, 7, 11] = bad
-            rc, untouched = _untouched_call(h, entry, L2, Rs, 1, RANGE_T)
+            rc, untouched = _untouched(h, entry, L2, Rs, 1, RANGE_T, cost=NCC)
             assert rc == UNSUP and untouched, (entry, bad, rc)
-        rc, untouched = _untouched_call(h, entry, Ls, Rs, 1, RANGE_T)
+        rc, untouched = _untouched(h, entry, Ls, Rs, 1, RANGE_T, cost=NCC)
         _ok(rc, entry)
     finally:
         _reset(h)
@@ -326,82 +267,15 @@ def test_too_many_candidates_are_rejected(gctx):
     Rs = g.integers(0, 256, (1, 8, 1000)).astype(np.uint8)
     _set(gctx, 1000, 4, 10, 100)
     try:
-        rc, untouched = _untouched_call(gctx, "pair_device", Ls, Rs, 1, 600)
+        rc, untouched = _untouched(gctx, "pair_device", Ls, Rs, 1, 600, cost=NCC)
         assert rc == UNSUP and untouched and "candidates" in _capi.last_error()
-        rc, _ = _untouched_call(gctx, "pair_device", Ls, Rs, 1, 511)               # 512 candidates: served
+        rc, _ = _untouched(gctx, "pair_device", Ls, Rs, 1, 511, cost=NCC)               # 512 candidates: served
         _ok(rc)
     finally:
         _reset(gctx)
 
 
-def _fill(dev, shape, value):
-    a = np.full(shape, value, np.uint8)
-    return _torch().from_numpy(a).cuda() if dev else a
-
-
-def test_partial_bands_and_mgpu_bands_are_rejected(gctx, mg):
-    torch = _torch()
-    lib = _capi.lib()
-    rows, cols, win, rng = 48, 96, 3, 16
-    L, Rt, _ = synth.make_pair(rows, cols, rng + 4, 88)
-    Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
-    _set(gctx, 1000, 4, 20, 200)
-    _set(mg, 1000, 4, 20, 200)
-    try:
-        for r0, r1 in ((0, 24), (24, 48), (10, 20)):
-            for fn, a, b in ((lib.stereo_disparity_pair_band_u8_host, L, Rt), (lib.stereo_disparity_pair_band_f32_host, Lf, Rf)):
-                ol, orr = _fill(False, (rows, cols * 2), 0x3C), _fill(False, (rows, cols * 2), 0x3C)
-                rc = fn(gctx.handle, NCC, a.ctypes.data, a.strides[0], b.ctypes.data, b.strides[0], rows, cols, r0, r1, win, rng,
-                        ol[r0:].ctypes.data, orr[r0:].ctypes.data, cols * 2, 2)
-                assert rc == UNSUP and (ol == 0x3C).all() and (orr == 0x3C).all(), (fn.__name__, r0, r1, rc)
-            h0, h1 = C.c_int(), C.c_int()
-            _ok(lib.stereo_band_halo_rows(rows, r0, r1, win, C.byref(h0), C.byref(h1)))
-            tl, tr = torch.from_numpy(L).cuda(), torch.from_numpy(Rt).cuda()
-            ol, orr = _fill(True, (rows, cols * 2), 0x3C), _fill(True, (rows, cols * 2), 0x3C)
-            rc = lib.stereo_disparity_pair_band_halo_u8_device(gctx.handle, NCC, tl[h0.value].data_ptr(), cols, tr[h0.value].data_ptr(),
-                                                               cols, rows, cols, r0, r1, h0.value, h1.value, win, rng, ol[r0].data_ptr(),
-                                                               orr[r0].data_ptr(), cols * 2, 2, None)
-            torch.cuda.synchronize()
-            assert rc == UNSUP and (ol == 0x3C).all().item() and (orr == 0x3C).all().item(), ("band_halo", r0, r1, rc)
-        for fn, a, b in ((lib.stereo_mgpu_disparity_pair_bands_u8_host, L, Rt), (lib.stereo_mgpu_disparity_pair_bands_f32_host, Lf, Rf)):
-            ol, orr = _fill(False, (rows, cols * 2), 0x3C), _fill(False, (rows, cols * 2), 0x3C)
-            rc = fn(mg._h, NCC, a.ctypes.data, a.strides[0], b.ctypes.data, b.strides[0], rows, cols, win, rng,
-                    ol.ctypes.data, orr.ctypes.data, cols * 2, 2)
-            assert rc == UNSUP and (ol == 0x3C).all() and (orr == 0x3C).all(), (fn.__name__, rc)
-    finally:
-        _reset(gctx)
-        _reset(mg)
-
-
-# ---- 4. the setting ----------------------------------------------------------------------------------------------------
-
-def test_setter_checks_and_default_state(mg):
-    lib = _capi.lib()
-    fresh = sb.Context(0)
-    try:
-        assert fresh.sgm_ncc_scale == 0
-        assert lib.stereo_ctx_set_sgm_ncc_scale(None, 5) == ARG
-        assert lib.stereo_ctx_sgm_ncc_scale(None) == ARG
-        assert lib.stereo_mgpu_set_sgm_ncc_scale(None, 5) == ARG
-        fresh.set_sgm_ncc_scale(1000)
-        for bad in (-1, -(1 << 24), (1 << 24) + 1, 1 << 30, 2 ** 31 - 1):
-            assert lib.stereo_ctx_set_sgm_ncc_scale(fresh.handle, bad) == ARG, bad
-            assert fresh.sgm_ncc_scale == 1000, bad                    # the old setting stays
-        for q in (1, 1 << 24, 0, 77):
-            fresh.set_sgm_ncc_scale(q)
-            assert fresh.sgm_ncc_scale == q
-        fresh.set_sgm(8, 1, 2)                                         # SGM on and off again: q stays
-        fresh.set_sgm(None)
-        assert fresh.sgm_ncc_scale == 77 and fresh.sgm is None
-        with pytest.raises(sb.StereoError):
-            mg.set_sgm_ncc_scale(-3)
-        mg.set_sgm_ncc_scale(4096)
-        for i in range(mg.device_count):
-            assert lib.stereo_ctx_sgm_ncc_scale(lib.stereo_mgpu_ctx(mg._h, i)) == 4096
-    finally:
-        fresh.close()
-        mg.set_sgm_ncc_scale(0)
-
+# ---- 4. settings that change nothing -----------------------------------------------------------------------------------
 
 def test_settings_that_change_nothing(gctx):
     Ls, Rs = _images("u8", 2, 79)
@@ -423,6 +297,10 @@ def test_settings_that_change_nothing(gctx):
             without = _run(gctx, entry, sb.COST_SSD, a, b, 3, RANGE_T, np.int16)
             assert np.array_equal(with_q[0], without[0]) and np.array_equal(with_q[1], without[1]), entry
             gctx.set_sgm(None)
+        fresh.set_sgm_ncc_scale(77)                                    # SGM on and off again: q stays
+        fresh.set_sgm(8, 1, 2)
+        fresh.set_sgm(None)
+        assert fresh.sgm_ncc_scale == 77 and fresh.sgm is None
     finally:
         fresh.close()
         _reset(gctx)

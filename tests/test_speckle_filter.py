@@ -13,37 +13,13 @@ import introtocomputervision_b200 as sb
 from introtocomputervision_b200 import _capi, synth
 from lr_oracle import lr_check
 from speckle_oracle import filter_speckles
-from pair_calls import FAMILIES, RANGE_T, _device_batch, _images, _run, _set_fuse
-from test_entry_points import EXPECTED, PITCH, ROWS, _args
+from pair_calls import FAMILIES, RANGE_T, _device_batch, _images, _ok, _run, _set_fuse, _torch, gctx, mg
 
 pytestmark = pytest.mark.gpu
 
 ARG, UNSUP = _capi.ERR_INVALID_ARG, _capi.ERR_UNSUPPORTED
 DT = {1: np.int8, 2: np.int16, 4: np.int32}
 MAX_SIZE, MAX_DIFF = 30, 0
-
-
-def _torch():
-    import torch
-    return torch
-
-
-def _ok(rc, where=""):
-    assert rc == _capi.STEREO_OK, f"{where}: {rc} ({_capi.last_error()})"
-
-
-@pytest.fixture(scope="module")
-def sctx():
-    c = sb.Context(0)
-    yield c
-    c.close()
-
-
-@pytest.fixture(scope="module")
-def mg():
-    m = sb.MultiGpu([0, 0])
-    yield m
-    m.close()
 
 
 # ---- 1. the kernel alone ---------------------------------------------------------------------------------------------
@@ -113,7 +89,7 @@ def _check_kernel(ctx, d, new_val, settings, min_changed=0.0):
 
 @pytest.mark.parametrize("elem", [1, 2, 4])
 @pytest.mark.parametrize("kind", ["serpentine", "comb", "checker", "whole", "blobs"])
-def test_kernel_alone_adversarial_maps(sctx, elem, kind):
+def test_kernel_alone_adversarial_maps(gctx, elem, kind):
     rows, cols, nv = 150, 333, -100
     g = np.random.default_rng(elem * 10 + len(kind))
     d = {"serpentine": _serpentine(rows, cols), "comb": _comb(rows, cols), "checker": _checker(rows, cols, 2),
@@ -126,10 +102,10 @@ def test_kernel_alone_adversarial_maps(sctx, elem, kind):
                 "checker": [(1, 2), (1, 3), (2, 3)],                      # max_diff 2: all singletons; 3: one component
                 "whole": [(big, 0), (big - 1, 0)],
                 "blobs": [(20, 0), (100, 1), (400, 2), (0, 1)]}[kind]
-    _check_kernel(sctx, d, nv, settings)
+    _check_kernel(gctx, d, nv, settings)
 
 
-def test_kernel_alone_int32_near_the_limits(sctx):
+def test_kernel_alone_int32_near_the_limits(gctx):
     lo, hi = np.iinfo(np.int32).min, np.iinfo(np.int32).max
     g = np.random.default_rng(5)
     rows, cols = 70, 90
@@ -137,7 +113,7 @@ def test_kernel_alone_int32_near_the_limits(sctx):
     d = d.astype(np.int32)
     d[g.random((rows, cols)) < 0.1] = 0
     # lo and hi differ by 2^32 - 1, more than any max_diff: a 32-bit difference would wrap to 1 and link them
-    _check_kernel(sctx, d, 0, [(30, 1), (30, 2), (rows * cols, 2 ** 31 - 1), (5, 2 ** 31 - 1)])
+    _check_kernel(gctx, d, 0, [(30, 1), (30, 2), (rows * cols, 2 ** 31 - 1), (5, 2 ** 31 - 1)])
 
 
 SHAPES = [(1, 1), (1, 640), (640, 1), (7, 640), (2160, 3840), (2, 32768), (32768, 2)]
@@ -145,32 +121,32 @@ SHAPES = [(1, 1), (1, 640), (640, 1), (7, 640), (2160, 3840), (2, 32768), (32768
 
 @pytest.mark.parametrize("elem", [1, 2, 4])
 @pytest.mark.parametrize("shape", SHAPES)
-def test_kernel_alone_shapes(sctx, elem, shape):
+def test_kernel_alone_shapes(gctx, elem, shape):
     rows, cols = shape
     nv = -100
     g = np.random.default_rng(rows * 7 + cols + elem)
     d = _blobs(g, rows, cols).astype(DT[elem])
     d[g.random((rows, cols)) < 0.05] = nv
     settings = [(20, 1), (1, 0)] if rows * cols < 10 ** 6 else [(100, 1)]
-    _check_kernel(sctx, d, nv, settings, min_changed=0.001 if rows * cols > 100 else 0.0)
+    _check_kernel(gctx, d, nv, settings, min_changed=0.001 if rows * cols > 100 else 0.0)
 
 
-def test_kernel_alone_4k_serpentine(sctx):
+def test_kernel_alone_4k_serpentine(gctx):
     d = _serpentine(2160, 3840).astype(np.int16)
-    _check_kernel(sctx, d, -300, [(2160 * 3840 // 2 + 600, 0)], min_changed=0.4)
+    _check_kernel(gctx, d, -300, [(2160 * 3840 // 2 + 600, 0)], min_changed=0.4)
 
 
-def test_kernel_alone_argument_checks(sctx):
+def test_kernel_alone_argument_checks(gctx):
     torch = _torch()
     buf = torch.zeros((4, 256), dtype=torch.uint8, device="cuda")
     a = buf.data_ptr()
     lib = _capi.lib()
 
-    def call(p=a, step=256, elem=2, rows=4, cols=64, nv=-11, max_size=5, max_diff=1, ctx=sctx.handle):
+    def call(p=a, step=256, elem=2, rows=4, cols=64, nv=-11, max_size=5, max_diff=1, ctx=gctx.handle):
         return lib.stereo_filter_speckles_device(ctx, p, step, elem, rows, cols, nv, max_size, max_diff, None)
 
     assert call() == _capi.STEREO_OK and call(max_size=0) == _capi.STEREO_OK
-    assert sctx.last_launches == 0
+    assert gctx.last_launches == 0
     assert call(p=None) == ARG and call(ctx=None) == ARG
     assert call(rows=0) == ARG and call(cols=0) == ARG and call(rows=-1) == ARG
     assert call(rows=32769) == UNSUP and call(cols=32769, step=32769 * 2) == UNSUP
@@ -179,7 +155,7 @@ def test_kernel_alone_argument_checks(sctx):
     assert call(elem=1, nv=-129) == ARG and call(elem=1, nv=128) == ARG and call(elem=2, nv=32768) == ARG
     assert call(elem=1, nv=-128) == _capi.STEREO_OK and call(elem=2, nv=-32768) == _capi.STEREO_OK
     assert call(elem=4, nv=-2 ** 31) == _capi.STEREO_OK
-    sctx.synchronize()
+    gctx.synchronize()
 
 
 # ---- 2. every pair entry point ---------------------------------------------------------------------------------------
@@ -218,13 +194,13 @@ def _filtered_equals_oracle_of_off(h, entry, cost, Ls, Rs, win, rng, dt, lr, max
 @pytest.mark.parametrize("fuse", [True, False])
 @pytest.mark.parametrize("cost", [sb.COST_SSD, sb.COST_NCORR])
 @pytest.mark.parametrize("entry", ENTRIES)
-def test_every_pair_entry_point_equals_the_oracle_filter(sctx, mg, entry, cost, fuse, family, lr):
+def test_every_pair_entry_point_equals_the_oracle_filter(gctx, mg, entry, cost, fuse, family, lr):
     kind, win, dt = FAMILIES[family]
     if kind != "u8" and entry in ("batch_device", "band_halo_device"):
         pytest.skip("8-bit device entry point")
     if kind == "noisy" and entry == "band_host":
         pytest.skip("the host row-band entry points take 8-bit-valued images only")
-    h = mg if entry.startswith("mgpu_") else sctx
+    h = mg if entry.startswith("mgpu_") else gctx
     n = 5 if "batch" in entry else 1
     Ls, Rs = _images(kind, n, 500 + 7 * ENTRIES.index(entry))
     _set_fuse(h, fuse)
@@ -237,47 +213,47 @@ def test_every_pair_entry_point_equals_the_oracle_filter(sctx, mg, entry, cost, 
 
 @pytest.mark.parametrize("bands", [0, 3])
 @pytest.mark.parametrize("kind", ["u8", "f32"])
-def test_host_pipeline_items_and_bands(sctx, bands, kind):
+def test_host_pipeline_items_and_bands(gctx, bands, kind):
     Ls, Rs = _images(kind, 7, 901)
-    sctx.set_pipe_bands(bands)
+    gctx.set_pipe_bands(bands)
     try:
         for cost in (sb.COST_SSD, sb.COST_NCORR):
             for lr in (False, True):
-                _filtered_equals_oracle_of_off(sctx, "batch_host", cost, Ls, Rs, 3, RANGE_T, np.int16, lr, 30, 0)
+                _filtered_equals_oracle_of_off(gctx, "batch_host", cost, Ls, Rs, 3, RANGE_T, np.int16, lr, 30, 0)
     finally:
-        sctx.set_pipe_bands(0)
+        gctx.set_pipe_bands(0)
 
 
-def test_launches_of_a_filtered_pair_call(sctx):
+def test_launches_of_a_filtered_pair_call(gctx):
     Ls, Rs = _images("u8", 1, 41)
-    sctx.set_speckle_filter(None)
-    _run(sctx, "pair_device", sb.COST_SSD, Ls, Rs, 3, RANGE_T, np.int16)
-    off = sctx.last_launches
-    sctx.set_speckle_filter(MAX_SIZE, MAX_DIFF)
+    gctx.set_speckle_filter(None)
+    _run(gctx, "pair_device", sb.COST_SSD, Ls, Rs, 3, RANGE_T, np.int16)
+    off = gctx.last_launches
+    gctx.set_speckle_filter(MAX_SIZE, MAX_DIFF)
     try:
-        _run(sctx, "pair_device", sb.COST_SSD, Ls, Rs, 3, RANGE_T, np.int16)
-        assert sctx.last_launches == off + 4
+        _run(gctx, "pair_device", sb.COST_SSD, Ls, Rs, 3, RANGE_T, np.int16)
+        assert gctx.last_launches == off + 4
     finally:
-        sctx.set_speckle_filter(None)
+        gctx.set_speckle_filter(None)
 
 
 # ---- 3. / 4. full-size batches ---------------------------------------------------------------------------------------
 
 @pytest.mark.parametrize("shape,nd,win,n,elem", [((720, 1280), 64, 4, 16, 1), ((2160, 3840), 256, 5, 1, 2)])
-def test_full_size_batch_equals_the_oracle(sctx, shape, nd, win, n, elem):
+def test_full_size_batch_equals_the_oracle(gctx, shape, nd, win, n, elem):
     rows, cols = shape
     rng = nd - 1
     pairs = [synth.make_pair(rows, cols, nd, 60 + i)[:2] for i in range(min(n, 4))]
     Ls = np.stack([pairs[i % len(pairs)][0] for i in range(n)])
     Rs = np.stack([pairs[i % len(pairs)][1] for i in range(n)])
-    sctx.set_speckle_filter(None)
-    off = _device_batch(sctx, Ls, Rs, win, rng, elem)
-    sctx.set_speckle_filter(100, 1)
+    gctx.set_speckle_filter(None)
+    off = _device_batch(gctx, Ls, Rs, win, rng, elem)
+    gctx.set_speckle_filter(100, 1)
     try:
-        on = _device_batch(sctx, Ls, Rs, win, rng, elem)
-        launches = sctx.last_launches
+        on = _device_batch(gctx, Ls, Rs, win, rng, elem)
+        launches = gctx.last_launches
     finally:
-        sctx.set_speckle_filter(None)
+        gctx.set_speckle_filter(None)
     cache = {}
     for side in (0, 1):
         for i in range(n):
@@ -287,187 +263,13 @@ def test_full_size_batch_equals_the_oracle(sctx, shape, nd, win, n, elem):
             assert np.array_equal(on[side, i], cache[key]), (side, i)
     assert np.mean(on != off) > 0.002
     if n == 16:
-        _device_batch(sctx, Ls, Rs, win, rng, elem)
-        assert launches == sctx.last_launches + 4    # every map of the 16 pairs in one set of filter launches
+        _device_batch(gctx, Ls, Rs, win, rng, elem)
+        assert launches == gctx.last_launches + 4    # every map of the 16 pairs in one set of filter launches
 
 
-# ---- 5. rejections, default and off ----------------------------------------------------------------------------------
+# ---- 5. graph capture -------------------------------------------------------------------------------------------------
 
-def _fill(dev, shape, value):
-    torch = _torch()
-    a = np.full(shape, value, np.uint8)
-    return torch.from_numpy(a).cuda() if dev else a
-
-
-def test_partial_bands_are_rejected_and_write_nothing(sctx, mg):
-    torch = _torch()
-    lib = _capi.lib()
-    rows, cols, win, rng = 48, 96, 3, 16
-    L, Rt, _ = synth.make_pair(rows, cols, rng + 4, 88)
-    Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
-    sctx.set_speckle_filter(MAX_SIZE, MAX_DIFF)
-    mg.set_speckle_filter(MAX_SIZE, MAX_DIFF)
-    try:
-        for r0, r1 in ((0, 24), (24, 48), (10, 20)):
-            for fn, a, b in ((lib.stereo_disparity_pair_band_u8_host, L, Rt), (lib.stereo_disparity_pair_band_f32_host, Lf, Rf)):
-                ol, orr = _fill(False, (rows, cols * 2), 0x3C), _fill(False, (rows, cols * 2), 0x3C)
-                rc = fn(sctx.handle, sb.COST_SSD, a.ctypes.data, a.strides[0], b.ctypes.data, b.strides[0], rows, cols, r0, r1, win, rng,
-                        ol[r0:].ctypes.data, orr[r0:].ctypes.data, cols * 2, 2)
-                assert rc == UNSUP, (fn.__name__, r0, r1, rc)
-                assert (ol == 0x3C).all() and (orr == 0x3C).all()
-            h0, h1 = C.c_int(), C.c_int()
-            _ok(lib.stereo_band_halo_rows(rows, r0, r1, win, C.byref(h0), C.byref(h1)))
-            tl, tr = torch.from_numpy(L).cuda(), torch.from_numpy(Rt).cuda()
-            ol, orr = _fill(True, (rows, cols * 2), 0x3C), _fill(True, (rows, cols * 2), 0x3C)
-            rc = lib.stereo_disparity_pair_band_halo_u8_device(sctx.handle, sb.COST_SSD, tl[h0.value].data_ptr(), cols, tr[h0.value].data_ptr(),
-                                                               cols, rows, cols, r0, r1, h0.value, h1.value, win, rng, ol[r0].data_ptr(),
-                                                               orr[r0].data_ptr(), cols * 2, 2, None)
-            torch.cuda.synchronize()
-            assert rc == UNSUP, ("band_halo", r0, r1, rc)
-            assert (ol == 0x3C).all().item() and (orr == 0x3C).all().item()
-        for fn, a, b in ((lib.stereo_mgpu_disparity_pair_bands_u8_host, L, Rt), (lib.stereo_mgpu_disparity_pair_bands_f32_host, Lf, Rf),
-                         # float images that are not 8-bit: no whole-pair call stands in for the refused bands either
-                         (lib.stereo_mgpu_disparity_pair_bands_f32_host, synth.noisy_variant(L, 1), synth.noisy_variant(Rt, 2))):
-            ol, orr = _fill(False, (rows, cols * 2), 0x3C), _fill(False, (rows, cols * 2), 0x3C)
-            rc = fn(mg._h, sb.COST_SSD, a.ctypes.data, a.strides[0], b.ctypes.data, b.strides[0], rows, cols, win, rng,
-                    ol.ctypes.data, orr.ctypes.data, cols * 2, 2)
-            assert rc == UNSUP, (fn.__name__, rc)
-            assert (ol == 0x3C).all() and (orr == 0x3C).all()
-    finally:
-        sctx.set_speckle_filter(None)
-        mg.set_speckle_filter(None)
-    # off again: the same partial band is computed
-    ol = np.zeros((rows, cols), np.int16)
-    orr = np.zeros((rows, cols), np.int16)
-    _ok(lib.stereo_disparity_pair_band_u8_host(sctx.handle, sb.COST_SSD, L.ctypes.data, cols, Rt.ctypes.data, cols, rows, cols, 10, 20,
-                                               win, rng, ol[10:].ctypes.data, orr[10:].ctypes.data, cols * 2, 2))
-    dl, dr = mg.disparity_pair_bands(sb.COST_SSD, L, Rt, win, rng, dtype=np.int16)
-    assert dl.shape == (rows, cols)
-
-
-PAIR_ENTRY_POINTS = [n for n in EXPECTED if n.startswith("stereo_disparity_pair_")]
-MGPU_ENTRY_POINTS = {"stereo_mgpu_disparity_pair_batch_u8_host": "stereo_disparity_pair_batch_u8_host",
-                     "stereo_mgpu_disparity_pair_batch_f32_host": "stereo_disparity_pair_batch_f32_host"}
-
-
-@pytest.mark.parametrize("elem,rng", [(1, 128), (2, 32768)])
-@pytest.mark.parametrize("name", PAIR_ENTRY_POINTS + list(MGPU_ENTRY_POINTS))
-def test_sentinel_that_does_not_fit_is_rejected_with_the_filter_alone(sctx, mg, name, elem, rng):
-    torch = _torch()
-    h = mg if name.startswith("stereo_mgpu_") else sctx
-    as_name = MGPU_ENTRY_POINTS.get(name, name)
-    dev = as_name.endswith("_device")
-    imgs = [_fill(dev, (2, ROWS, PITCH), 0) for _ in range(2)]
-    outs = [_fill(dev, (2, ROWS, PITCH), 0x3C) for _ in range(2)]
-    ptrs = [t.data_ptr() for t in imgs + outs] if dev else [a.ctypes.data for a in imgs + outs]
-    handle = h._h if isinstance(h, sb.MultiGpu) else h.handle
-    fn = getattr(_capi.lib(), name)
-    # (the band entry points are called with a band of the whole image here: the sentinel alone rejects them)
-    args = _args(as_name, handle, ptrs, rng=rng, elem=elem)
-    if "band" in as_name:
-        args = _whole_band_args(as_name, args)
-    h.set_speckle_filter(MAX_SIZE, MAX_DIFF)
-    try:
-        rc = fn(*args)
-        torch.cuda.synchronize()
-        assert rc == UNSUP, f"{name}: {rc} ({_capi.last_error()})"
-        assert "sentinel" in _capi.last_error()
-        for o in outs:
-            a = o.cpu().numpy() if dev else o
-            assert (a == 0x3C).all(), f"{name} wrote its outputs"
-    finally:
-        h.set_speckle_filter(None)
-    _ok(fn(*args), name)
-    torch.cuda.synchronize()
-
-
-def _whole_band_args(name, args):
-    """test_entry_points._args of a band entry point, with the band [4, 12) widened to the whole image [0, ROWS)."""
-    a = list(args)
-    i = a.index(4)
-    assert a[i + 1] == 12
-    a[i], a[i + 1] = 0, ROWS
-    if name == "stereo_disparity_pair_band_halo_u8_device":
-        a[i + 2], a[i + 3] = 0, ROWS
-    return a
-
-
-def test_setter_checks_and_default_state(sctx, mg):
-    lib = _capi.lib()
-    fresh = sb.Context(0)
-    try:
-        assert fresh.speckle_filter is None
-        assert lib.stereo_ctx_set_speckle_filter(None, 5, 1) == ARG
-        assert lib.stereo_mgpu_set_speckle_filter(None, 5, 1) == ARG
-        assert lib.stereo_ctx_set_speckle_filter(fresh.handle, 5, -1) == ARG
-        assert fresh.speckle_filter is None
-        _ok(lib.stereo_ctx_set_speckle_filter(fresh.handle, 0, -1))          # off: max_diff does not matter
-        _ok(lib.stereo_ctx_set_speckle_filter(fresh.handle, -3, 7))
-        assert fresh.speckle_filter is None
-        fresh.set_speckle_filter(40, 2)
-        assert fresh.speckle_filter == (40, 2)
-        fresh.set_speckle_filter(7)
-        assert fresh.speckle_filter == (7, 1)
-        fresh.set_speckle_filter(None)
-        assert fresh.speckle_filter is None
-        with pytest.raises(sb.StereoError):
-            fresh.set_speckle_filter(10, -1)
-        with pytest.raises(sb.StereoError):
-            mg.set_speckle_filter(10, -1)
-        size, diff = C.c_int(), C.c_int()
-        assert lib.stereo_ctx_speckle_filter(None, C.byref(size), C.byref(diff)) == ARG
-        mg.set_speckle_filter(9, 0)
-        for i in range(mg.device_count):
-            _ok(lib.stereo_ctx_speckle_filter(lib.stereo_mgpu_ctx(mg._h, i), C.byref(size), C.byref(diff)))
-            assert (size.value, diff.value) == (9, 0)
-        mg.set_speckle_filter(None)
-    finally:
-        fresh.close()
-        mg.set_speckle_filter(None)
-
-
-def test_off_again_is_byte_identical_to_a_fresh_context(sctx):
-    Ls, Rs = _images("u8", 3, 78)
-    fresh = sb.Context(0)
-    try:
-        for entry in ("pair_host", "pair_device", "batch_device", "batch_host"):
-            for cost in (sb.COST_SSD, sb.COST_NCORR):
-                want = _run(fresh, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                sctx.set_speckle_filter(MAX_SIZE, MAX_DIFF)
-                on = _run(sctx, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                sctx.set_speckle_filter(0)
-                assert sctx.speckle_filter is None
-                got = _run(sctx, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1]), (entry, cost)
-                assert (on[0] != want[0]).any()
-    finally:
-        fresh.close()
-        sctx.set_speckle_filter(None)
-
-
-def test_single_direction_and_refgpu_calls_ignore_the_filter(sctx):
-    L, Rt, _ = synth.make_pair(48, 160, 24, 516)
-    Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
-
-    def singles(c):
-        return [c.disparity(sb.COST_SSD, Lf, Rf, 3, -20, 0, dtype=np.int16), c.disparity(sb.COST_NCORR, L, Rt, 3, 0, 20),
-                c.disparity_refgpu(sb.COST_SSD, Lf, Rf, 3, -20, 0)]
-
-    fresh = sb.Context(0)
-    try:
-        want = singles(fresh)
-        sctx.set_speckle_filter(1000, 3)
-        got = singles(sctx)
-    finally:
-        fresh.close()
-        sctx.set_speckle_filter(None)
-    for a, b in zip(got, want):
-        assert np.array_equal(a, b)
-
-
-# ---- 6. graph capture -------------------------------------------------------------------------------------------------
-
-def test_device_pair_call_with_the_filter_replays_in_a_cuda_graph(sctx):
+def test_device_pair_call_with_the_filter_replays_in_a_cuda_graph(gctx):
     torch = _torch()
     rows, cols, win, rng = 120, 256, 3, 30
     inputs = [synth.make_pair(rows, cols, rng + 4, 3030 + k)[:2] for k in range(3)]
@@ -483,15 +285,15 @@ def test_device_pair_call_with_the_filter_replays_in_a_cuda_graph(sctx):
 
     offc = sb.Context(0)
     try:
-        sctx.set_speckle_filter(MAX_SIZE, MAX_DIFF)
+        gctx.set_speckle_filter(MAX_SIZE, MAX_DIFF)
         with torch.cuda.stream(s):
-            call(sctx)                                  # warm-up: sizes the scratch arena
+            call(gctx)                                  # warm-up: sizes the scratch arena
         s.synchronize()
         g = torch.cuda.CUDAGraph()
         out.fill_(99)
         torch.cuda.synchronize()
         with torch.cuda.graph(g, stream=s, capture_error_mode="thread_local"):
-            call(sctx)
+            call(gctx)
         assert (out == 99).all().item()                 # captured, not run
         for L, Rt in inputs[1:]:
             tl.copy_(torch.from_numpy(L))
@@ -507,4 +309,4 @@ def test_device_pair_call_with_the_filter_replays_in_a_cuda_graph(sctx):
             assert (want_l != off_l).any()
     finally:
         offc.close()
-        sctx.set_speckle_filter(None)
+        gctx.set_speckle_filter(None)

@@ -10,7 +10,7 @@ import pytest
 import introtocomputervision_b200 as sb
 from introtocomputervision_b200 import _capi, synth
 from lr_oracle import lr_check
-from pair_calls import RANGE_T, _device_batch, _images, _run, _set_fuse
+from pair_calls import RANGE_T, _device_batch, _images, _ok, _run, _set_fuse, _torch, _untouched, gctx, mg
 from sgm_ncc_oracle import clip_range
 from sgm_ncc_oracle import cost_volume as ncc_cost_volume
 from sgm_oracle import aggregate, cost_volume, winner
@@ -21,29 +21,6 @@ pytestmark = pytest.mark.gpu
 
 ARG, UNSUP = _capi.ERR_INVALID_ARG, _capi.ERR_UNSUPPORTED
 ENTRIES = ["pair_host", "pair_device", "batch_device", "batch_host", "band_host", "band_halo_device", "mgpu_batch"]
-
-
-def _torch():
-    import torch
-    return torch
-
-
-def _ok(rc, where=""):
-    assert rc == _capi.STEREO_OK, f"{where}: {rc} ({_capi.last_error()})"
-
-
-@pytest.fixture(scope="module")
-def gctx():
-    c = sb.Context(0)
-    yield c
-    c.close()
-
-
-@pytest.fixture(scope="module")
-def mg():
-    m = sb.MultiGpu([0, 0])
-    yield m
-    m.close()
 
 
 def _directions(L, Rt, rng):
@@ -255,42 +232,6 @@ def test_full_size_4k_pair_on_spread_rows(gctx):
 
 # ---- 5. refusals ----------------------------------------------------------------------------------------------------------
 
-def _untouched(h, entry, Ls, Rs, R, rng, cost=sb.COST_SSD, dt=np.int16):
-    """Calls the entry point on outputs filled with 0x3C; returns (status, outputs untouched)."""
-    lib = _capi.lib()
-    n, rows, cols = Ls.shape
-    elem = np.dtype(dt).itemsize
-    f32 = Ls.dtype == np.float32
-    step = cols * Ls.itemsize
-    if entry in ("pair_device", "batch_device"):
-        torch = _torch()
-        tl, tr = torch.from_numpy(Ls).cuda(), torch.from_numpy(Rs).cuda()
-        out = torch.full((2, n, rows, cols * elem), 0x3C, dtype=torch.uint8, device="cuda")
-        st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-        if entry == "pair_device":
-            fn = lib.stereo_disparity_pair_f32_device if f32 else lib.stereo_disparity_pair_u8_device
-            rc = fn(h.handle, cost, tl.data_ptr(), step, tr.data_ptr(), step, rows, cols, R, rng, out[0].data_ptr(), out[1].data_ptr(),
-                    cols * elem, elem, st)
-        else:
-            rc = lib.stereo_disparity_pair_batch_u8_device(h.handle, cost, n, tl.data_ptr(), tr.data_ptr(), cols, rows * cols, rows, cols,
-                                                           R, rng, out[0].data_ptr(), out[1].data_ptr(), cols * elem, rows * cols * elem,
-                                                           elem, st)
-        torch.cuda.synchronize()
-        return rc, bool((out == 0x3C).all().item())
-    out = np.full((2, n, rows, cols * elem), 0x3C, np.uint8)
-    handle = h._h if isinstance(h, sb.MultiGpu) else h.handle
-    if entry == "pair_host":
-        fn = lib.stereo_disparity_pair_f32_host if f32 else lib.stereo_disparity_pair_u8_host
-        rc = fn(handle, cost, Ls.ctypes.data, step, Rs.ctypes.data, step, rows, cols, R, rng, out[0].ctypes.data, out[1].ctypes.data,
-                cols * elem, elem)
-    else:
-        prefix = "stereo_mgpu_" if entry == "mgpu_batch" else "stereo_"
-        fn = getattr(lib, prefix + ("disparity_pair_batch_f32_host" if f32 else "disparity_pair_batch_u8_host"))
-        rc = fn(handle, cost, n, Ls.ctypes.data, Rs.ctypes.data, step, rows * step, rows, cols, R, rng, out[0].ctypes.data,
-                out[1].ctypes.data, cols * elem, rows * cols * elem, elem)
-    return rc, bool((out == 0x3C).all())
-
-
 REFUSE_ENTRIES = ["pair_device", "batch_device", "pair_host", "batch_host", "mgpu_batch"]
 
 
@@ -342,112 +283,7 @@ def test_float_bound_and_non_finite_images_are_refused(gctx, mg, entry):
         h.set_uniqueness(0)
 
 
-def test_partial_bands_and_mgpu_bands_are_refused(gctx, mg):
-    torch = _torch()
-    lib = _capi.lib()
-    rows, cols, win, rng = 48, 96, 3, 16
-    L, Rt, _ = synth.make_pair(rows, cols, rng + 4, 88)
-    Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
-    gctx.set_uniqueness(10)
-    mg.set_uniqueness(10)
-    try:
-        for r0, r1 in ((0, 24), (24, 48), (10, 20)):
-            for fn, a, b in ((lib.stereo_disparity_pair_band_u8_host, L, Rt), (lib.stereo_disparity_pair_band_f32_host, Lf, Rf)):
-                ol, orr = np.full((rows, cols * 2), 0x3C, np.uint8), np.full((rows, cols * 2), 0x3C, np.uint8)
-                rc = fn(gctx.handle, sb.COST_SSD, a.ctypes.data, a.strides[0], b.ctypes.data, b.strides[0], rows, cols, r0, r1, win, rng,
-                        ol[r0:].ctypes.data, orr[r0:].ctypes.data, cols * 2, 2)
-                assert rc == UNSUP and (ol == 0x3C).all() and (orr == 0x3C).all(), (fn.__name__, r0, r1, rc)
-            h0, h1 = C.c_int(), C.c_int()
-            _ok(lib.stereo_band_halo_rows(rows, r0, r1, win, C.byref(h0), C.byref(h1)))
-            tl, tr = torch.from_numpy(L).cuda(), torch.from_numpy(Rt).cuda()
-            ol = torch.full((rows, cols * 2), 0x3C, dtype=torch.uint8, device="cuda")
-            orr = torch.full_like(ol, 0x3C)
-            rc = lib.stereo_disparity_pair_band_halo_u8_device(gctx.handle, sb.COST_SSD, tl[h0.value].data_ptr(), cols, tr[h0.value].data_ptr(),
-                                                               cols, rows, cols, r0, r1, h0.value, h1.value, win, rng, ol[r0].data_ptr(),
-                                                               orr[r0].data_ptr(), cols * 2, 2, None)
-            torch.cuda.synchronize()
-            assert rc == UNSUP and (ol == 0x3C).all().item() and (orr == 0x3C).all().item(), ("band_halo", r0, r1, rc)
-        for fn, a, b in ((lib.stereo_mgpu_disparity_pair_bands_u8_host, L, Rt), (lib.stereo_mgpu_disparity_pair_bands_f32_host, Lf, Rf)):
-            ol, orr = np.full((rows, cols * 2), 0x3C, np.uint8), np.full((rows, cols * 2), 0x3C, np.uint8)
-            rc = fn(mg._h, sb.COST_SSD, a.ctypes.data, a.strides[0], b.ctypes.data, b.strides[0], rows, cols, win, rng,
-                    ol.ctypes.data, orr.ctypes.data, cols * 2, 2)
-            assert rc == UNSUP and (ol == 0x3C).all() and (orr == 0x3C).all(), (fn.__name__, rc)
-    finally:
-        gctx.set_uniqueness(0)
-        mg.set_uniqueness(0)
-    dl, dr = mg.disparity_pair_bands(sb.COST_SSD, L, Rt, win, rng, dtype=np.int16)      # off again: served
-    assert dl.shape == (rows, cols)
-
-
-# ---- 6. the setting -------------------------------------------------------------------------------------------------------
-
-def test_setter_getter_and_mgpu_setter(mg):
-    lib = _capi.lib()
-    fresh = sb.Context(0)
-    try:
-        assert fresh.uniqueness == 0
-        assert lib.stereo_ctx_set_uniqueness(None, 10) == ARG
-        assert lib.stereo_ctx_uniqueness(None) == ARG
-        assert lib.stereo_mgpu_set_uniqueness(None, 10) == ARG
-        fresh.set_uniqueness(15)
-        for bad in (-1, 100, 101, -100, 1 << 20):
-            assert lib.stereo_ctx_set_uniqueness(fresh.handle, bad) == ARG, bad
-            assert fresh.uniqueness == 15, bad                      # the old setting stays
-        for v in (1, 99, 0, 42):
-            fresh.set_uniqueness(v)
-            assert fresh.uniqueness == v
-        fresh.set_uniqueness(None)
-        assert fresh.uniqueness == 0
-        with pytest.raises(sb.StereoError):
-            mg.set_uniqueness(100)
-        mg.set_uniqueness(7)
-        for i in range(mg.device_count):
-            assert lib.stereo_ctx_uniqueness(lib.stereo_mgpu_ctx(mg._h, i)) == 7
-    finally:
-        fresh.close()
-        mg.set_uniqueness(0)
-
-
-def test_off_again_is_byte_identical_to_a_fresh_context(gctx):
-    Ls, Rs = _images("u8", 3, 79)
-    fresh = sb.Context(0)
-    try:
-        for entry in ("pair_host", "pair_device", "batch_device", "batch_host"):
-            for cost in (sb.COST_SSD, sb.COST_NCORR):
-                want = _run(fresh, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                if cost == sb.COST_SSD:
-                    gctx.set_uniqueness(30)
-                    on = _run(gctx, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                    assert (on[0] != want[0]).any()
-                gctx.set_uniqueness(0)
-                got = _run(gctx, entry, cost, Ls, Rs, 3, RANGE_T, np.int16)
-                assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1]), (entry, cost)
-    finally:
-        fresh.close()
-        gctx.set_uniqueness(0)
-
-
-def test_single_direction_and_refgpu_calls_ignore_the_setting(gctx):
-    L, Rt, _ = synth.make_pair(48, 160, 24, 517)
-    Lf, Rf = L.astype(np.float32), Rt.astype(np.float32)
-
-    def singles(c):
-        return [c.disparity(sb.COST_SSD, Lf, Rf, 3, -20, 0, dtype=np.int16), c.disparity(sb.COST_SSD, L, Rt, 3, -20, 0),
-                c.disparity(sb.COST_NCORR, L, Rt, 3, 0, 20), c.disparity_refgpu(sb.COST_SSD, Lf, Rf, 3, -20, 0)]
-
-    fresh = sb.Context(0)
-    try:
-        want = singles(fresh)
-        gctx.set_uniqueness(50)
-        got = singles(gctx)
-    finally:
-        fresh.close()
-        gctx.set_uniqueness(0)
-    for a, b in zip(got, want):
-        assert np.array_equal(a, b)
-
-
-# ---- 7. graph capture ----------------------------------------------------------------------------------------------------
+# ---- 6. graph capture ----------------------------------------------------------------------------------------------------
 
 def test_device_pair_call_replays_in_a_cuda_graph(gctx):
     torch = _torch()
