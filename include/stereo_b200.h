@@ -315,6 +315,44 @@ int stereo_ctx_set_uniqueness(stereo_ctx* ctx, int uniqueness_ratio);
 /* The context's current u (0: off); STEREO_ERR_INVALID_ARG for a null context. */
 int stereo_ctx_uniqueness(const stereo_ctx* ctx);
 
+/* Sub-pixel disparity of pair calls: StereoSGBM's 1/16-pixel fixed point (DISP_SHIFT = 4), the parabola through the cost of
+ * the winner and the costs of its two neighbours.
+ * on = 0 (the default) switches it off, and results are then exactly those without it.  on = 1 switches it on for the pair
+ * entry points of this context that compute whole maps - pair host and device, f32 and u8, the batches; any other value
+ * returns STEREO_ERR_INVALID_ARG and keeps the old setting.
+ * For each map of each pair, V is the value the map minimises over the present candidates, as for the uniqueness ratio:
+ * S(p, d) for SGM maps (SSD cost, or NCC cost with scale q), the single-direction SSD window sum C(p, d) for block-matcher
+ * maps.  Present is as defined for SGM above (SSD: xp + d in [0, Wp - 1]; NCC: x + d in [0, cols - 1]), each inside the
+ * direction's candidate range.  With d the map's integer value at the pixel after every other step (uniqueness ratio,
+ * texture threshold, left-right check, speckle filter), the pixel is written as
+ *     16 sentinel                                                  where d is the sentinel -(disparity_range + 1),
+ *     16 d + ((V(d-1) - V(d+1)) 16 + den) / (2 den),
+ *            den = max(V(d-1) + V(d+1) - 2 V(d), 1)               where d - 1 and d + 1 are both present,
+ *     16 d                                                         otherwise (a range edge or an absent neighbour),
+ * in 64-bit, with C division (truncation toward zero): StereoSGBM's formula ("do subpixel quadratic interpolation",
+ * stereosgbm.cpp) over ascending signed d, so L->R maps stay negative.  V(d) is the first minimum, so the offset lies in
+ * [-7, 8] and (out + 7) >> 4 is the integer map without the option at every pixel, the sentinel included.  A block-matcher
+ * pixel that accepted no candidate holds 0, a range edge in both directions, and stays 0.  Two differences from OpenCV:
+ * the left-right check, the speckle filter and the texture threshold run on the integer maps, before the refinement
+ * (OpenCV's validateDisparity and filterSpeckles see the 16S values); and both maps of a pair are refined, each against its
+ * own V (OpenCV refines its left map only), as for the uniqueness ratio.
+ *   Order: prefilter -> block matcher or SGM -> uniqueness ratio -> texture threshold -> left-right check -> speckle filter
+ *   -> sub-pixel.
+ * Refused with STEREO_ERR_UNSUPPORTED before anything is enqueued, uploaded or written: 1-byte maps; 2-byte maps with
+ * disparity_range > 2047 (16 (disparity_range + 1) must fit); NCC pair calls with SGM off (the NCC block matcher ranks
+ * float32 scores, which have no integer V; NCC SGM maps are served); row bands other than the whole image
+ * (stereo_disparity_pair_band_halo_u8_device, stereo_disparity_pair_band_{u8,f32}_host) and
+ * stereo_mgpu_disparity_pair_bands_*.  Single-direction and stereo_disparity_refgpu_* calls ignore the setting.  Host pair
+ * calls take the staged whole-image path.
+ * SGM maps: the last path kernel stores each pixel's offset in a grow-only buffer of the context (1 byte per pixel and map of
+ * a launch sequence), applied by one launch at the end.  Block-matcher maps come from the same kernels as without it (same
+ * last path, same fused pairs); a pass at the end pads each image once (4 bytes per padded pixel, from the context's arena)
+ * and recomputes V(d - 1), V(d), V(d + 1) of each pixel.  After one call of a shape, device calls of that shape allocate
+ * nothing and stay capturable in CUDA graphs. */
+int stereo_ctx_set_subpixel(stereo_ctx* ctx, int on);
+/* The context's current setting (0: off, 1: on); STEREO_ERR_INVALID_ARG for a null context. */
+int stereo_ctx_subpixel(const stereo_ctx* ctx);
+
 /* StereoBM's X-Sobel prefilter (preFilterCap, PREFILTER_XSOBEL) and texture threshold (textureThreshold) of pair calls.
  * cap = 0 (the default) switches both off; texture_threshold must then be 0, and results are exactly those without them.
  * 1 <= cap <= 63 (StereoBM's range) switches the prefilter on for the pair entry points of this context that compute whole
@@ -595,6 +633,9 @@ int stereo_mgpu_set_uniqueness(stereo_mgpu* mg, int uniqueness_ratio);
 /* stereo_ctx_set_prefilter on every device's context.  Pair batches shard whole pairs and so give the single-GPU result;
  * row-band sharded pairs return STEREO_ERR_UNSUPPORTED while it is on. */
 int stereo_mgpu_set_prefilter(stereo_mgpu* mg, int cap, int texture_threshold);
+/* stereo_ctx_set_subpixel on every device's context.  Pair batches shard whole pairs and so give the single-GPU result;
+ * row-band sharded pairs return STEREO_ERR_UNSUPPORTED while it is on. */
+int stereo_mgpu_set_subpixel(stereo_mgpu* mg, int on);
 /* Batches (BASELINE config 5): same arguments as stereo_disparity_pair_batch_{u8,f32}_host. */
 int stereo_mgpu_disparity_pair_batch_u8_host(stereo_mgpu* mg, int cost, int n_pairs,
                                              const uint8_t* left, const uint8_t* right, size_t img_step, size_t pair_stride,

@@ -204,6 +204,12 @@ inline void setUniqueness(int uniquenessRatio, stereo_ctx* ctx = nullptr) {
     check(stereo_ctx_set_uniqueness(ctx ? ctx : default_ctx(), uniquenessRatio), "stereo_ctx_set_uniqueness");
 }
 
+// Sub-pixel disparity (StereoSGBM's 1/16-pixel fixed point) of the pair calls on `ctx` (default: the default context): true
+// writes 16 d + offset, false switches it off (stereo_ctx_set_subpixel).
+inline void setSubpixel(bool on, stereo_ctx* ctx = nullptr) {
+    check(stereo_ctx_set_subpixel(ctx ? ctx : default_ctx(), on ? 1 : 0), "stereo_ctx_set_subpixel");
+}
+
 // StereoBM's X-Sobel prefilter (preFilterCap, 1 .. 63) and texture threshold (textureThreshold, >= 0) of the pair calls on
 // `ctx` (default: the default context); cap 0 (with threshold 0) switches both off (stereo_ctx_set_prefilter).
 inline void setPrefilter(int cap, int textureThreshold = 0, stereo_ctx* ctx = nullptr) {
@@ -266,6 +272,7 @@ public:
     void setPrefilter(int cap, int textureThreshold = 0) {
         check(stereo_mgpu_set_prefilter(mg_, cap, textureThreshold), "stereo_mgpu_set_prefilter");
     }
+    void setSubpixel(bool on) { check(stereo_mgpu_set_subpixel(mg_, on ? 1 : 0), "stereo_mgpu_set_subpixel"); }
 
     // disparitySSDPair / disparityNCorrPair (main.cpp:21-78) with the output rows sharded over the devices
     void disparityPairBands(int cost, const MatT& left, const MatT& right, size_t windowRad, int disparityRange, MatT& disparityLeft,

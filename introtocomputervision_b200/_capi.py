@@ -67,6 +67,9 @@ SIGNATURES = {
     "stereo_ctx_set_prefilter": (_i, [_vp, _i, _i]),
     "stereo_ctx_prefilter": (_i, [_vp, C.POINTER(_i), C.POINTER(_i)]),
     "stereo_mgpu_set_prefilter": (_i, [_vp, _i, _i]),
+    "stereo_ctx_set_subpixel": (_i, [_vp, _i]),
+    "stereo_ctx_subpixel": (_i, [_vp]),
+    "stereo_mgpu_set_subpixel": (_i, [_vp, _i]),
     "stereo_prefilter_u8_device": (_i, [_vp, _vp, _sz, _i, _i, _i, _vp, _sz, _vp]),
     "stereo_prefilter_f32_device": (_i, [_vp, _vp, _sz, _i, _i, _i, _vp, _sz, _vp]),
     "stereo_ctx_synchronize": (_i, [_vp, _vp]),

@@ -85,15 +85,16 @@ struct PairOptions {
     int uniq = 0;             // StereoSGBM's uniquenessRatio, 1 .. 99 (0: off)
     int pf_cap = 0;           // StereoBM's X-Sobel prefilter with this preFilterCap, 1 .. 63 (0: off) ...
     int pf_texture = 0;       // ... and this textureThreshold (0: off)
+    int subpix = 0;           // StereoSGBM's sub-pixel disparity, 1/16-pixel fixed point, after every other step (0: off)
 
     // Removed pixels are marked with -(range + 1), which must fit the maps' element type.
     bool writes_sentinel() const { return lr_max_diff >= 0 || spk_max_size > 0 || uniq > 0 || pf_texture > 0; }
-    // Row bands are refused: speckle regions and SGM paths cross band seams, the uniqueness pass and the prefilter's
-    // odd-height rule work on whole images.
-    bool needs_whole_maps() const { return pf_cap > 0 || uniq > 0 || sgm_paths > 0 || spk_max_size > 0; }
+    // Row bands are refused: speckle regions and SGM paths cross band seams, the uniqueness pass, the sub-pixel pass and
+    // the prefilter's odd-height rule work on whole images.
+    bool needs_whole_maps() const { return pf_cap > 0 || uniq > 0 || sgm_paths > 0 || spk_max_size > 0 || subpix > 0; }
     // The maps are computed from whole images in one go, so the host pipeline's row bands do not apply.  (The speckle
     // filter is not here: the pipeline filters an item's maps after its last band.)
-    bool computed_whole() const { return sgm_paths > 0 || uniq > 0 || pf_cap > 0; }
+    bool computed_whole() const { return sgm_paths > 0 || uniq > 0 || pf_cap > 0 || subpix > 0; }
 };
 
 } // namespace sb
@@ -128,6 +129,7 @@ struct stereo_ctx {
     int fuse_pairs = 1;       // both maps of a pair from one cost volume where the problem allows it
     sb::PairOptions opt;      // what pair calls do beyond the block matcher (stereo_ctx_set_lr_check .. _set_prefilter)
     sb::Arena pf;             // the prefiltered images of a pair call, live while the arena is reset (grow-only)
+    sb::Arena sp;             // the SGM maps' sub-pixel offsets of a pair call, live while the arena is reset (grow-only)
     // device time of the hot kernels only (fast_*_kernel), per direction, for the roofline report
     static constexpr int HOT_EVENTS = 16;
     cudaEvent_t hot0[HOT_EVENTS] = {}, hot1[HOT_EVENTS] = {};

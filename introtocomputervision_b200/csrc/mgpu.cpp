@@ -169,6 +169,8 @@ int stereo_mgpu_set_sgm_ncc_scale(stereo_mgpu* mg, int q) { return set_all(mg, s
 
 int stereo_mgpu_set_uniqueness(stereo_mgpu* mg, int uniqueness_ratio) { return set_all(mg, stereo_ctx_set_uniqueness, uniqueness_ratio); }
 
+int stereo_mgpu_set_subpixel(stereo_mgpu* mg, int on) { return set_all(mg, stereo_ctx_set_subpixel, on); }
+
 int stereo_mgpu_set_prefilter(stereo_mgpu* mg, int cap, int texture_threshold) {
     return set_all(mg, stereo_ctx_set_prefilter, cap, texture_threshold);
 }

@@ -18,6 +18,7 @@
 #pragma once
 #include "common.cuh"
 #include "exact.cuh"
+#include "subpixel.cuh"
 
 namespace sb {
 
@@ -163,8 +164,10 @@ __host__ __device__ inline int sgm_lines(int rows, int cols, int dy, int dx) {
 
 // The map the last path writes (ptr == nullptr: none).  uniq: the uniqueness ratio (0: off), whose rejected pixels get
 // `sentinel`.  only_invalid: the block matcher's map is already there; store only the sentinel, also at pixels whose every
-// present V is >= 99999999 (the reference's initial best cost, so its map holds the default 0 there).
-struct SgmOut { void* ptr; size_t step; int elem; int dlo; int uniq; int sentinel; int only_invalid; };
+// present V is >= 99999999 (the reference's initial best cost, so its map holds the default 0 there).  subpix (nullptr:
+// off): rows x cols bytes that receive each pixel's sub-pixel offset of the winner (subpixel.cuh's subpix_offset of S(j* - 1),
+// S(j*), S(j* + 1); 0 where a neighbour is absent).
+struct SgmOut { void* ptr; size_t step; int elem; int dlo; int uniq; int sentinel; int only_invalid; int8_t* subpix; };
 
 constexpr unsigned SGM_BM_NO_WINNER = 99999999u;
 
@@ -274,6 +277,19 @@ sgm_path_kernel(const int32_t* __restrict__ C, int32_t* __restrict__ S, int rows
             bool unique;
             const int jw = sgm_winner<K>(sn, lane, out.uniq, &vbest, &unique);
             const bool invalid = !unique || (out.only_invalid && vbest >= SGM_BM_NO_WINNER);
+            int off = 0;
+            if (out.subpix) {
+                // S(j* - 1) and S(j* + 1) from the lanes that hold them, by selects over constant register indices
+                unsigned vm = 0xFFFFFFFFu, vp = 0xFFFFFFFFu;
+#pragma unroll
+                for (int i = 0; i < K; ++i) {
+                    if (lane * K + i == jw - 1) vm = sn[i];
+                    if (lane * K + i == jw + 1) vp = sn[i];
+                }
+                vm = __reduce_min_sync(0xffffffffu, vm);
+                vp = __reduce_min_sync(0xffffffffu, vp);
+                if (vm != 0xFFFFFFFFu && vp != 0xFFFFFFFFu) off = subpix_offset(vm, vbest, vp);
+            }
             if (lane == 0 && (invalid || !out.only_invalid)) {
                 const long long pix = base / Dp;
                 const int py = int(pix / cols), px = int(pix - (long long)py * cols);
@@ -282,6 +298,7 @@ sgm_path_kernel(const int32_t* __restrict__ C, int32_t* __restrict__ S, int rows
                 if (out.elem == 1) reinterpret_cast<int8_t*>(row)[px] = int8_t(uint8_t(uint32_t(dv) & 0xFFu));
                 else if (out.elem == 2) reinterpret_cast<int16_t*>(row)[px] = int16_t(dv);
                 else reinterpret_cast<int32_t*>(row)[px] = dv;
+                if (out.subpix) out.subpix[size_t(py) * cols + px] = int8_t(off);
             }
         }
         base += stride;

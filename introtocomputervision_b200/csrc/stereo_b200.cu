@@ -9,6 +9,7 @@
 #include "speckle.cuh"
 #include "sgm.cuh"
 #include "prefilter.cuh"
+#include "subpixel.cuh"
 #include "host_pack.hpp"
 
 #include <atomic>
@@ -133,6 +134,14 @@ static int check_uniq_bound(int R, double M) {
     return STEREO_ERR_UNSUPPORTED;
 }
 
+// Sub-pixel maps hold 16 d + offset, d in [-(range + 1), range] and the offset in [-7, 8], so 16 (range + 1) must fit:
+// never a 1-byte map, a 2-byte map up to range 2047.  (The option marks no pixel itself: this is not check_lr_sentinel.)
+static int check_subpixel_fit(int elem, int range) {
+    if (elem == 4 || (elem == 2 && range <= 2047)) return STEREO_OK;
+    set_error("sub-pixel disparity: 16 x (%d + 1) does not fit a %d-byte disparity element", range, elem);
+    return STEREO_ERR_UNSUPPORTED;
+}
+
 // The options of PairOptions::needs_whole_maps, each with its refusal of a row band [%d, %d) by check_pair_options and of
 // row-band sharding by band_sharding_refusal.  An option's entry is on while its field is positive.  check_pair_options
 // names the first option on in this order, band_sharding_refusal the last.
@@ -155,6 +164,9 @@ static const WholeMapOption WHOLE_MAP_OPTIONS[] = {
     {&PairOptions::spk_max_size,
      "speckle filter: rows [%d, %d) are not the whole map (filter the gathered map with stereo_filter_speckles_device)",
      "speckle filter on: row-band sharded pairs are not filtered (filter the gathered map with stereo_filter_speckles_device)"},
+    {&PairOptions::subpix,
+     "sub-pixel disparity: rows [%d, %d) are not the whole map (the sub-pixel pass works on whole images)",
+     "sub-pixel disparity on: row-band sharded pairs are not refined (shard whole pairs)"},
 };
 
 // Why the row-band sharded pair calls (stereo_mgpu_disparity_pair_bands_*) refuse a context's options, or nullptr when
@@ -170,7 +182,8 @@ const char* band_sharding_refusal(const stereo_ctx* ctx) {
 
 // What a pair call must satisfy for the context's options, checked once per call before anything is staged or enqueued:
 // the sentinel fits (PairOptions::writes_sentinel), SGM aggregates the SSD cost or, with an NCC scale set, the NCC cost,
-// and the options of PairOptions::needs_whole_maps get whole maps.  The uniqueness ratio on block-matcher maps needs the
+// and the options of PairOptions::needs_whole_maps get whole maps.  Sub-pixel maps fit (check_subpixel_fit) and, with SGM
+// off, need the SSD cost.  The uniqueness ratio on block-matcher maps needs the
 // SSD cost, at most 512 candidates after clipping and, for 8-bit images, check_uniq_bound with M = 255^2 (float images:
 // after their classification, check_uniq_classified; with the prefilter on every call matches 8-bit images).  run_sgm
 // checks SGM's candidate count and int32 bound.
@@ -182,6 +195,14 @@ static int check_pair_options(const stereo_ctx* ctx, int cost, PixType type, int
     if (o.writes_sentinel()) {
         const int rc = check_lr_sentinel(elem, range);
         if (rc != STEREO_OK) return rc;
+    }
+    if (o.subpix > 0) {
+        const int rc = check_subpixel_fit(elem, range);
+        if (rc != STEREO_OK) return rc;
+        if (!sgm && cost != STEREO_COST_SSD) {
+            set_error("sub-pixel disparity: NCC block-matcher maps rank float32 scores, which have no integer cost (switch SGM on with an NCC scale)");
+            return STEREO_ERR_UNSUPPORTED;
+        }
     }
     if (sgm && cost != STEREO_COST_SSD && o.sgm_ncc_scale == 0) {
         set_error("SGM aggregates the SSD cost only while no NCC scale is set (stereo_ctx_set_sgm_ncc_scale; or switch SGM off for NCC calls)");
@@ -598,7 +619,8 @@ static int launch_sgm_path(stereo_ctx* ctx, const Problem& p, const SgmShape& g,
 // One direction by SGM into p.disp, on scratch the caller reserved.  ref / tgt: the caller's images (u8 or float).
 // `per_cell`: NCC on float images that are not 8-bit-valued, whose numerators are summed cell by cell (sgm_ncc_cell_kernel).
 // `sentinel`: the value of pixels the uniqueness ratio rejects.
-static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st, bool per_cell, int sentinel) {
+// `subpix`: rows x cols bytes for the sub-pixel offsets of the map (nullptr: off).
+static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st, bool per_cell, int sentinel, int8_t* subpix) {
     static constexpr int DIRS[8][2] = {{0, 1}, {0, -1}, {1, 0}, {-1, 0}, {1, 1}, {1, -1}, {-1, 1}, {-1, -1}};
     const SgmShape g = sgm_shape(p);
     const size_t cells = size_t(p.rows) * p.cols * g.Dp;
@@ -629,7 +651,7 @@ static int run_sgm_direction(stereo_ctx* ctx, const Problem& p, cudaStream_t st,
     }
     for (int k = 0; k < ctx->opt.sgm_paths; ++k) {
         const bool last = k == ctx->opt.sgm_paths - 1;
-        const SgmOut out{last ? p.disp.ptr : nullptr, p.disp.step, p.disp.elem, g.dlo, ctx->opt.uniq, sentinel, 0};
+        const SgmOut out{last ? p.disp.ptr : nullptr, p.disp.step, p.disp.elem, g.dlo, ctx->opt.uniq, sentinel, 0, last ? subpix : nullptr};
         const int rc2 = launch_sgm_path(ctx, p, g, C, S, DIRS[k][0], DIRS[k][1], ctx->opt.sgm_p1, ctx->opt.sgm_p2, k == 0, out, st);
         if (rc2 != STEREO_OK) return rc2;
     }
@@ -660,7 +682,7 @@ static int run_uniqueness(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_
         int32_t* C = static_cast<int32_t*>(ctx->arena.take(size_t(p.rows) * p.cols * g.Dp * 4));
         if (!C) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
         launch_sgm_cost(ctx, p, g, Lp, Rp, SgmNcc{nullptr, nullptr, 0}, C, st);
-        const SgmOut out{p.disp.ptr, p.disp.step, p.disp.elem, g.dlo, ctx->opt.uniq, sentinel, 1};
+        const SgmOut out{p.disp.ptr, p.disp.step, p.disp.elem, g.dlo, ctx->opt.uniq, sentinel, 1, nullptr};
         rc = launch_sgm_path(ctx, p, g, C, nullptr, 1, 0, 0, 0, true, out, st);
         if (rc != STEREO_OK) return rc;
     }
@@ -706,7 +728,8 @@ static int run_sgm(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st, bool u8
     ctx->last_path = STEREO_PATH_SGM;
     for (int i = 0; i < n && rc == STEREO_OK; ++i) {
         ctx->arena.reset();
-        rc = run_sgm_direction(ctx, ps[i], st, per_cell, -(ps[n / 2].dmax + 1));
+        int8_t* off = ctx->opt.subpix > 0 ? reinterpret_cast<int8_t*>(ctx->sp.base) + size_t(i) * ps[i].rows * ps[i].cols : nullptr;
+        rc = run_sgm_direction(ctx, ps[i], st, per_cell, -(ps[n / 2].dmax + 1), off);
     }
     return rc;
 }
@@ -745,10 +768,59 @@ static int prefilter_pairs(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st)
     return prefilter_launch(P, n, f32, st);
 }
 
+// ---- sub-pixel disparity (subpixel.cuh) -------------------------------------------------------------------------------
+
+// The SGM maps' offsets of the n directions of a launch sequence in ctx->sp, n x rows x cols bytes that stay live while the
+// arena is reset.  The buffer grows (after quiesce) only for a larger shape: after one call of a shape nothing is allocated.
+static int reserve_subpix_offsets(stereo_ctx* ctx, cudaStream_t st, size_t bytes) {
+    if (bytes <= ctx->sp.cap) return STEREO_OK;
+    const int rc = quiesce(ctx, st);
+    return rc != STEREO_OK ? rc : ctx->sp.reserve(bytes);
+}
+
+// The block-matcher pass's scratch: each image of the n/2 pairs padded once (both directions of a pair read the same two).
+static size_t subpix_scratch_bytes(const Problem& p, int n) {
+    return size_t(n) * align256(padded_elems(p) * sizeof(float)) + 4096;
+}
+
+// The last step of a pair call: every map of the n directions of ps (pair_problems' layout, whole maps, the caller's or the
+// prefiltered images) rewritten in place in 1/16 pixels.  SGM maps apply the offsets their last path stored in ctx->sp;
+// block-matcher SSD maps pad the images once into the arena, which the caller sized for subpix_scratch_bytes, and
+// recompute V(d - 1), V(d), V(d + 1) of each final d.
+static int subpixel_maps(stereo_ctx* ctx, const Problem* ps, int n, cudaStream_t st, bool sgm) {
+    static_assert(FMAXJOBS <= SP_MAXMAPS, "one sub-pixel launch covers the maps of one launch sequence");
+    const Problem& p = ps[0];
+    const int np = n / 2;
+    SpParams P{};
+    P.rows = p.rows; P.cols = p.cols; P.R = p.R; P.sentinel = -(ps[np].dmax + 1);
+    for (int k = 0; k < n; ++k) P.map[k] = SpMap{ps[k].disp.ptr, ps[k].disp.step, nullptr, nullptr, nullptr, ps[k].dmin, ps[k].dmax};
+    if (sgm) {
+        for (int k = 0; k < n; ++k) P.map[k].off = reinterpret_cast<const int8_t*>(ctx->sp.base) + size_t(k) * p.rows * p.cols;
+        ctx->last_launches += 1;
+        return subpix_apply_launch(P, n, p.disp.elem, st);
+    }
+    ctx->arena.reset();
+    const size_t guard = size_t(p.R) + 64;
+    SpPadParams Q{};
+    Q.rows = p.rows; Q.cols = p.cols; Q.R = p.R;
+    for (int k = 0; k < np; ++k) {
+        float* l = static_cast<float*>(ctx->arena.take(padded_elems(p) * sizeof(float)));
+        float* r = static_cast<float*>(ctx->arena.take(padded_elems(p) * sizeof(float)));
+        if (!l || !r) { set_error("scratch arena too small (internal)"); return STEREO_ERR_ALLOC; }
+        Q.img[2 * k] = SpImage{ps[k].ref.ptr, ps[k].ref.step, l + guard};
+        Q.img[2 * k + 1] = SpImage{ps[k].tgt.ptr, ps[k].tgt.step, r + guard};
+        P.map[k].Lp = P.map[np + k].Rp = l + guard;
+        P.map[k].Rp = P.map[np + k].Lp = r + guard;
+    }
+    ctx->last_launches += 2;
+    return subpix_bm_launch(Q, n, P, n, p.disp.elem, p.ref.type == PixType::U8, st);
+}
+
 // Validates every direction, runs them - pairs with the context's SGM on by SGM, everything else on the kernel family
 // run_families picks - then, for pairs of block-matcher maps, applies the context's uniqueness ratio (run_uniqueness;
 // SGM maps apply it in their last path) and finishes pairs with the texture threshold, the left-right check and the
-// speckle filter (finish_pairs).  Pairs with the prefilter on match the prefiltered images (prefilter_pairs) from the start.
+// speckle filter (finish_pairs), and last refines them to 1/16 pixel (subpixel_maps).  Pairs with the prefilter on match
+// the prefiltered images (prefilter_pairs) from the start.
 static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) {
     bool fast = ctx->force_path != STEREO_PATH_EXACT_F32, u8 = true;
     for (int i = 0; i < n; ++i) {
@@ -762,6 +834,7 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
     }
     const bool pair = n >= 2;      // (every pair of a call has the same shape, band, range and element type)
     const bool uniq_pass = pair && ctx->opt.uniq > 0 && ctx->opt.sgm_paths == 0;
+    const bool subpix = pair && ctx->opt.subpix > 0, sgm = pair && ctx->opt.sgm_paths > 0;
     if (pair) {
         const Problem& p = ps[0];
         int rc = check_pair_options(ctx, p.cost, p.ref.type, p.disp.elem, ps[n / 2].dmax, p.R, p.cols, p.row_begin, p.row_end, p.rows);
@@ -771,7 +844,9 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
         }
         size_t need = finish_scratch_bytes(ctx, n, p.rows, p.cols);
         if (uniq_pass && uniq_scratch_bytes(p) > need) need = uniq_scratch_bytes(p);      // (both directions have one shape)
+        if (subpix && !sgm && subpix_scratch_bytes(p, n) > need) need = subpix_scratch_bytes(p, n);
         if (rc == STEREO_OK) rc = reserve_arena(ctx, st, need);
+        if (rc == STEREO_OK && subpix && sgm) rc = reserve_subpix_offsets(ctx, st, size_t(n) * p.rows * p.cols);
         if (rc == STEREO_OK && uniq_pass && !u8 && !(fast && n <= 2)) {
             // float images the exact kernels take without a classification: classify them for the bound
             ImageView copies[2];
@@ -780,11 +855,12 @@ static int run_directions(stereo_ctx* ctx, Problem* ps, int n, cudaStream_t st) 
         }
         if (rc != STEREO_OK) return rc;
     }
-    Problem callers[FMAXJOBS];      // (run_f32_pair points ps at u8 copies in the arena, which the uniqueness pass reuses)
-    for (int i = 0; uniq_pass && i < n; ++i) callers[i] = ps[i];
-    int rc = pair && ctx->opt.sgm_paths > 0 ? run_sgm(ctx, ps, n, st, u8) : run_families(ctx, ps, n, st, fast, u8);
+    Problem callers[FMAXJOBS];      // (run_f32_pair points ps at u8 copies in the arena, which the later passes reuse)
+    for (int i = 0; (uniq_pass || subpix) && i < n; ++i) callers[i] = ps[i];
+    int rc = sgm ? run_sgm(ctx, ps, n, st, u8) : run_families(ctx, ps, n, st, fast, u8);
     if (rc == STEREO_OK && uniq_pass) rc = run_uniqueness(ctx, callers, n, st);
-    return rc == STEREO_OK && pair ? finish_pairs(ctx, ps, n, st, true) : rc;
+    if (rc == STEREO_OK && pair) rc = finish_pairs(ctx, ps, n, st, true);
+    return rc == STEREO_OK && subpix ? subpixel_maps(ctx, callers, n, st, sgm) : rc;
 }
 
 // Every call of a context shares one scratch arena (and the classification flag), so calls are ordered: a call
@@ -1456,6 +1532,7 @@ void stereo_ctx_destroy(stereo_ctx* ctx) {
     ctx->arena.release();
     ctx->io.release();
     ctx->pf.release();
+    ctx->sp.release();
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
     delete ctx->pool;
     if (ctx->d_flag) cudaFree(ctx->d_flag);
@@ -1734,6 +1811,18 @@ int stereo_ctx_set_uniqueness(stereo_ctx* ctx, int uniqueness_ratio) {
 int stereo_ctx_uniqueness(const stereo_ctx* ctx) {
     if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
     return ctx->opt.uniq;
+}
+
+int stereo_ctx_set_subpixel(stereo_ctx* ctx, int on) {
+    if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
+    if (on != 0 && on != 1) { set_error("sub-pixel disparity: on must be 0 or 1 (got %d)", on); return STEREO_ERR_INVALID_ARG; }
+    ctx->opt.subpix = on;
+    return STEREO_OK;
+}
+
+int stereo_ctx_subpixel(const stereo_ctx* ctx) {
+    if (!ctx) { set_error("null context"); return STEREO_ERR_INVALID_ARG; }
+    return ctx->opt.subpix;
 }
 
 int stereo_ctx_set_prefilter(stereo_ctx* ctx, int cap, int texture_threshold) {

@@ -200,6 +200,19 @@ class Context:
         _check(_capi.lib().stereo_ctx_prefilter(self._h, C.byref(cap), C.byref(tex)), "stereo_ctx_prefilter")
         return None if cap.value <= 0 else (cap.value, tex.value)
 
+    def set_subpixel(self, on: Optional[bool]) -> None:
+        """Pair calls: StereoSGBM's sub-pixel disparity, the last step after the speckle filter.  Every map then holds
+        ``16 d + offset`` (1/16 pixel, the sentinel becomes ``16 * sentinel``), the offset from the parabola through the
+        costs of d - 1, d and d + 1 (SGM sums or, with SGM off, SSD window costs; NCC needs SGM).  Needs 2-byte maps
+        (range <= 2047) or 4-byte maps.  ``True`` switches it on, ``False`` or ``None`` off (the default)."""
+        v = 0 if on is None else int(on)
+        _check(_capi.lib().stereo_ctx_set_subpixel(self._h, v), "stereo_ctx_set_subpixel")
+
+    @property
+    def subpixel(self) -> bool:
+        """Whether pair calls write sub-pixel maps."""
+        return bool(_capi.lib().stereo_ctx_subpixel(self._h))
+
     def set_host_threads(self, threads: int) -> None:
         """Host threads that convert CV_32FC1 host images to u8 before the upload (0 = automatic, -1 = off)."""
         _check(_capi.lib().stereo_ctx_set_host_threads(self._h, int(threads)), "stereo_ctx_set_host_threads")
@@ -365,6 +378,11 @@ class MultiGpu:
         """:meth:`Context.set_prefilter` on every device's context (row-band sharded pairs refuse while it is on)."""
         v = 0 if cap is None else int(cap)
         _check(_capi.lib().stereo_mgpu_set_prefilter(self._h, v, int(texture_threshold)), "stereo_mgpu_set_prefilter")
+
+    def set_subpixel(self, on: Optional[bool]) -> None:
+        """:meth:`Context.set_subpixel` on every device's context (row-band sharded pairs refuse while it is on)."""
+        v = 0 if on is None else int(on)
+        _check(_capi.lib().stereo_mgpu_set_subpixel(self._h, v), "stereo_mgpu_set_subpixel")
 
     def disparity_pair_bands(self, cost: int, left: np.ndarray, right: np.ndarray, window_rad: int, disparity_range: int,
                              dtype=np.int8) -> Tuple[np.ndarray, np.ndarray]:
